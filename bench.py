@@ -23,6 +23,8 @@ A step is one pass of the hot path over the whole corpus.
 `--impl reference` times the CPU reference arm: the oracle port of the reference's deflate (the reference
 itself is TypeScript and there is no JavaScript engine in this image; baseline/node_bench.mjs is run instead
 when `node` is on PATH), one independent stream per host thread, on the same workload.
+`--dump-outputs DIR` writes what the last timed step computed to DIR/<name>.npy (see dump_outputs), so that two
+builds can be compared output for output on the same seeded corpus.
 """
 from __future__ import annotations
 
@@ -40,6 +42,7 @@ import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: the benchmark writes nothing into it
 
 METRIC = "deflate_input_GBps"
 UNIT = "GB/s"
@@ -191,6 +194,26 @@ def lz_issue(prof_key, n_bytes, lz_avg_ms, clocks, torch, dev, level):
     return None
 
 
+def sample_windows(n, budget=8 << 20, win=16384):
+    """Start offsets and width of the windows dumped of an n-byte output: all of it up to `budget` bytes, else
+    budget // win windows of `win` bytes at fixed, seeded positions, in order."""
+    import numpy as np
+    if n <= budget:
+        return [0], n
+    return (np.sort(np.random.default_rng(0).choice(n // win, budget // win, replace=False)) * win).tolist(), win
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as path/<name>.npy (float32 byte values, float64 offsets, lengths and checksums:
+    both exact), at most 64 MB in all."""
+    import numpy as np
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def lz_traffic(n_bytes, level):
     tpath = os.path.join(ROOT, "profiles", "roofline_traffic.json")
     try:
@@ -337,6 +360,16 @@ def run_single(args, torch, dev, local_rank):
     clocks = sampler.stop()
     ms_step = ms_total / args.steps
     value = n / (ms_step / 1e3) / 1e9
+    if args.dump_outputs:
+        # what deflate_batch_dev hands its caller after the last timed step: every chunk's byte offset and bit
+        # length, the totals, and the concatenated raw streams (a seeded sample of them beyond 8 MiB)
+        last = bufs.read_result()
+        starts, win = sample_windows(int(last.total_out_bytes))
+        dump_outputs(args.dump_outputs, {
+            "chunk_byte_offsets": bufs.out_off.cpu().numpy().astype(np.float64),
+            "chunk_bits": bufs.out_bits.cpu().numpy().astype(np.float64),
+            "totals": np.array([last.total_out_bytes, last.total_out_bits, last.check, last.n_blocks], dtype=np.float64),
+            "compressed_bytes": torch.cat([bufs.out[p: p + win] for p in starts]).cpu().numpy().astype(np.float32)})
 
     # ---- e2e: host buffers through zs_deflate_batch ----
     lib = capi.load()
@@ -892,6 +925,14 @@ def run_sharded(args, torch, dist, dev, rank, local_rank, world):
             pos += len(piece)
         verified = bool(ok and d.eof and pos == total and adler == plan.check and d.unused_data == b"")
         ratio = len(stream) / total
+        if args.dump_outputs:
+            # the last timed step's parts stitched into the one zlib stream, with the exchange step's plan
+            s = np.frombuffer(stream, dtype=np.uint8)
+            starts, win = sample_windows(s.size)
+            dump_outputs(args.dump_outputs, {
+                "part_bit_offsets": np.array(plan.bit_offset, dtype=np.float64),
+                "totals": np.array([len(stream), plan.total_bits, plan.check, plan.total_len], dtype=np.float64),
+                "compressed_bytes": np.concatenate([s[p: p + win] for p in starts]).astype(np.float32)})
     flag = torch.tensor([1 if (verified or rank != 0) else 0], device=dev)
     dist.broadcast(flag, 0)
 
@@ -1013,7 +1054,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--force-sharded", action="store_true", help="run the N > 1 code path with however many ranks there are "
                     "(one rank: a check of that path on a single GPU, not a bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy: the "
+                    "compressed bytes (a fixed, seeded 8 MiB sample of them when longer), offsets and totals")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has no such outputs")
     if args.impl == "reference":
         return run_reference(args)
 

@@ -1,13 +1,15 @@
 """CPU: what can be checked of bench.py without a GPU -- the reference arm (`--impl reference`: the oracle port of the
 reference's deflate on the host cores, a bounded sample per step) prints ONE JSON line with the contract's keys for
 the N = 1 and the N > 1 workload, a non-zero rank of a torchrun launch prints nothing, and the product arm refuses to
-run without a CUDA device (there is no CPU fallback)."""
+run without a CUDA device (there is no CPU fallback).  On a GPU: what --dump-outputs writes is the timed path's output."""
 import json
 import os
 import subprocess
 import sys
 
-from conftest import ROOT
+import pytest
+
+from conftest import ROOT, pkg
 
 BENCH = os.path.join(ROOT, "bench.py")
 
@@ -44,3 +46,50 @@ def test_product_arm_needs_a_gpu():
         return
     p = _run(["--steps", "1", "--warmup", "1", "--size-mib", "16"])
     assert p.returncode != 0 and "no CUDA device" in (p.stderr + p.stdout)
+
+
+def test_arguments_refused(tmp_path):
+    """No timed step at all, and a dump of the reference arm (which computes nothing on the GPU), are usage errors."""
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        p = _run([*args, "--size-mib", "16"])
+        assert p.returncode == 2 and "error" in p.stderr
+    assert not any(tmp_path.iterdir())
+
+
+def test_sample_windows():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench", BENCH)
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    assert bench.sample_windows(1000) == ([0], 1000)
+    starts, win = bench.sample_windows(300 << 20)
+    assert win == 16384 and len(starts) * win == 8 << 20 and starts == sorted(set(starts))
+    assert all(p % win == 0 and p + win <= 300 << 20 for p in starts) and bench.sample_windows(300 << 20) == (starts, win)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_timed_path_outputs(gpu_ctx, tmp_path):
+    """--dump-outputs of the N = 1 path: every chunk's raw stream, primed with the 32 KiB before it, decodes to the
+    seeded corpus, and the offsets, bit lengths and totals agree with each other and with the JSON line."""
+    import zlib
+
+    import numpy as np
+    import torch
+    p = _run(["--steps", "2", "--warmup", "1", "--size-mib", "8", "--no-extra", "--no-cpu", "--dump-outputs", str(tmp_path)])
+    assert p.returncode == 0, p.stderr[-2000:]
+    line = json.loads([l for l in p.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 2
+    d = {f.stem: np.load(f) for f in tmp_path.iterdir()}
+    assert sorted(d) == ["chunk_bits", "chunk_byte_offsets", "compressed_bytes", "totals"]
+    assert d["compressed_bytes"].dtype == np.float32 and all(d[k].dtype == np.float64 for k in ("chunk_bits", "chunk_byte_offsets", "totals"))
+    off = d["chunk_byte_offsets"].astype(np.int64)
+    total = int(d["totals"][0])
+    assert off.size == 129 and off[0] == 0 and off[-1] == total == d["compressed_bytes"].size   # 8 MiB compress to less than the 8 MiB dumped whole
+    assert total == round(line["compressed_ratio"] * (8 << 20))
+    assert np.all((d["chunk_bits"] + 7) // 8 == np.diff(off))
+    corpus = pkg("corpus").text_torch(8 << 20, torch.device("cuda", 0), seed=0xC0FFEE).cpu().numpy().tobytes()
+    z = d["compressed_bytes"].astype(np.uint8).tobytes()
+    for i in range(off.size - 1):
+        lo = i * 65536
+        dec = zlib.decompressobj(-15, zdict=corpus[max(0, lo - 32768): lo]) if lo else zlib.decompressobj(-15)
+        assert dec.decompress(z[off[i]: off[i + 1]]) == corpus[lo: lo + 65536] and dec.eof, i
