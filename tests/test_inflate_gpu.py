@@ -279,6 +279,77 @@ def test_fuzzed_streams_same_verdict_and_message(gpu_ctx, oracle, monkeypatch, k
     assert n_err > 100
 
 
+def _gzip_header(flg, method=8, hcrc_ok=True):
+    h = bytes([0x1F, 0x8B, method, flg]) + (123456789).to_bytes(4, "little") + b"\x00\x03"
+    if flg & 4:
+        h += (5).to_bytes(2, "little") + b"ab\x00cd"
+    if flg & 8:
+        h += b"name.txt\x00"
+    if flg & 16:
+        h += b"a comment\x00"
+    if flg & 2:
+        h += ((zlib.crc32(h) & 0xFFFF) ^ (0 if hcrc_ok else 1)).to_bytes(2, "little")
+    return h
+
+
+def _zlib_header(cinfo=7, method=8, fdict=False, fcheck_ok=True):
+    cmf, flg = cinfo << 4 | method, 0x80 | (0x20 if fdict else 0)
+    flg += (31 - (cmf * 256 + flg) % 31) % 31
+    return bytes([cmf, flg + (0 if fcheck_ok else 1)]) + (b"\x01\x02\x03\x04" if fdict else b"")
+
+
+@pytest.mark.parametrize("kernel", ["warp", "thread"])
+def test_wrapper_header_and_trailer_verdicts(gpu_ctx, oracle, monkeypatch, kernel):
+    """zlib and gzip wrappers built by hand -- every combination of the gzip header fields, a right and a wrong
+    header crc, truncation at every header byte and inside the trailer, reserved flags, other methods, a bad
+    FCHECK, a window above 32 KiB, FDICT -- decoded as windowBits 15, 31 and 47 by both kernels: status,
+    message, output and consumed input must be the reference's."""
+    monkeypatch.setenv("ZS_INFLATE_TPS" if kernel == "thread" else "ZS_INFLATE_WARP", "1")
+    data = make_text(3000, 17)
+    co = zlib.compressobj(6, 8, -15)
+    body = co.compress(data) + co.flush()
+    gz_trailer = zlib.crc32(data).to_bytes(4, "little") + len(data).to_bytes(4, "little")
+    z_trailer = zlib.adler32(data).to_bytes(4, "big")
+    streams = []
+    for flg in range(32):   # FTEXT 1, FHCRC 2, FEXTRA 4, FNAME 8, FCOMMENT 16
+        streams.append(_gzip_header(flg) + body + gz_trailer)
+        if flg & 2:
+            streams.append(_gzip_header(flg, hcrc_ok=False) + body + gz_trailer)
+    full = _gzip_header(31)
+    streams += [full[:k] for k in range(len(full))]
+    streams += [_gzip_header(8 | bit) + body + gz_trailer for bit in (0x20, 0x40, 0x80)]
+    streams.append(_gzip_header(0, method=7) + body + gz_trailer)
+    gz = _gzip_header(0) + body + gz_trailer
+    streams += [gz[:-k] for k in range(1, 9)]
+    for cinfo, method, ok in ((7, 8, True), (0, 8, True), (7, 7, True), (7, 8, False), (8, 8, True), (15, 8, True)):
+        streams.append(_zlib_header(cinfo, method, fcheck_ok=ok) + body + z_trailer)
+    zd = _zlib_header(fdict=True)
+    streams += [zd[:k] for k in range(len(zd) + 1)] + [zd + body + z_trailer]
+    zs = _zlib_header() + body + z_trailer
+    streams += [zs[:-k] for k in range(1, 5)]
+    streams += [streams[0]] * (32 - len(streams))   # ZS_INFLATE_TPS applies to batches of 32 streams or more
+    cap = len(data) + 64
+    seen = set()
+    for wb in (15, 31, 47):
+        r = _run(streams, wb, [cap] * len(streams))
+        for i, s in enumerate(streams):
+            st = oracle.InflateStream(wb)
+            ret, out, used = st.step(s, cap, oracle.Z_FINISH)
+            what = (kernel, wb, i, int(r.status[i]), ret, r.message(i), st.msg)
+            assert int(r.status[i]) == ret, what
+            assert r.output(i) == out, what
+            if ret == oracle.Z_DATA_ERROR:
+                # (after a data error the reference's count includes the bytes already in its bit buffer)
+                assert r.message(i) == st.msg, what
+            else:
+                assert int(r.in_used[i]) == used, (what, int(r.in_used[i]), used)
+            seen.add((ret, st.msg))
+            st.close()
+    assert {oracle.Z_STREAM_END, oracle.Z_NEED_DICT, oracle.Z_BUF_ERROR} <= {ret for ret, _ in seen}
+    assert {"header crc mismatch", "unknown header flags set", "unknown compression method", "incorrect header check",
+            "invalid window size"} <= {msg for _, msg in seen}
+
+
 def test_randomised_soak_inflate_and_api(gpu_ctx):
     """tools/soak_inflate.py for a few seconds: random batches (valid, truncated, corrupted, too-small
     outputs; zlib / gzip / raw / auto / deflate64) on both kernels against the oracle, and random piece /

@@ -26,12 +26,6 @@ using namespace zsinf;
 
 constexpr int kWarps = 4;
 
-__device__ __forceinline__ uint32_t crc_bitwise(uint32_t crc, unsigned byte) {
-    crc ^= byte;
-    for (int k = 0; k < 8; k++) crc = (crc & 1u) ? (0xedb88320u ^ (crc >> 1)) : (crc >> 1);
-    return crc;
-}
-
 __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a) {
     __shared__ WarpArena s_arena[kWarps];
     __shared__ FixedTables s_fixed;
@@ -49,22 +43,12 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
 
     for (uint64_t sidx = (uint64_t)blockIdx.x * kWarps + wid; sidx < a.n; sidx += (uint64_t)gridDim.x * kWarps) {
         BitReader br;
-        br.base = a.d_in;
-        br.pos = a.d_in_off[sidx];
-        br.end = a.d_in_off[sidx + 1];
-        br.safe_end = safe_end;
-        br.hold = 0;
-        br.bits = 0;
+        uint64_t cap, dict_len;
+        const uint8_t* dict;
+        open_stream(a, sidx, safe_end, br, cap, dict, dict_len);
         const uint64_t in_start = br.pos;
         uint8_t* out = a.d_out + a.d_out_off[sidx];
-        const uint64_t cap = a.d_out_off[sidx + 1] - a.d_out_off[sidx];
         uint64_t op = 0;
-        const uint8_t* dict = nullptr;
-        uint64_t dict_len = 0;
-        if (a.d_dict && a.d_dict_rng) {
-            dict = a.d_dict + a.d_dict_rng[2 * sidx];
-            dict_len = a.d_dict_rng[2 * sidx + 1] - a.d_dict_rng[2 * sidx];
-        }
         int status = ZS_OK;  // ZS_OK while running
         int detail = D_NONE;
         unsigned tflags = 0;  // 1 zlib trailer, 2 gzip trailer
@@ -90,72 +74,7 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
                 else br.drop((unsigned)(sb & 7u));
             }
         }
-        // ---- wrapper header: HEAD..HCRC / DICTID of inflate() (inflate.ts:377-593) ----
-        if (a.wrap && !skip_header) {
-            if (!br.need(16)) {
-                status = ZS_BUF_ERROR;
-            } else {
-                unsigned h = br.peek(16);
-                if ((a.wrap & 2) && h == 0x8b1fu) {
-                    uint32_t hcrc = crc_bitwise(crc_bitwise(0xffffffffu, 0x1f), 0x8b);
-                    br.drop(16);
-                    // FLAGS
-                    if (!br.need(16)) status = ZS_BUF_ERROR;
-                    unsigned flg = 0;
-                    if (status == ZS_OK) {
-                        unsigned w = br.take(16);
-                        flg = w >> 8;
-                        if ((w & 0xff) != 8) { status = ZS_DATA_ERROR; detail = D_METHOD; }
-                        else if (w & 0xe000) { status = ZS_DATA_ERROR; detail = D_HDR_FLAGS; }
-                        hcrc = crc_bitwise(crc_bitwise(hcrc, w & 0xff), w >> 8);
-                    }
-                    // TIME(4) XFL OS
-                    for (int k = 0; k < 6 && status == ZS_OK; k++) {
-                        if (!br.need(8)) status = ZS_BUF_ERROR;
-                        else hcrc = crc_bitwise(hcrc, br.take(8));
-                    }
-                    if (status == ZS_OK && (flg & 4)) {  // FEXTRA
-                        unsigned xlen = 0;
-                        if (!br.need(16)) status = ZS_BUF_ERROR;
-                        else {
-                            xlen = br.take(16);
-                            hcrc = crc_bitwise(crc_bitwise(hcrc, xlen & 0xff), xlen >> 8);
-                        }
-                        while (status == ZS_OK && xlen--) {
-                            if (!br.need(8)) status = ZS_BUF_ERROR;
-                            else hcrc = crc_bitwise(hcrc, br.take(8));
-                        }
-                    }
-                    for (int which = 0; which < 2 && status == ZS_OK; which++) {  // FNAME, FCOMMENT
-                        if (!(flg & (which ? 16 : 8))) continue;
-                        for (;;) {
-                            if (!br.need(8)) { status = ZS_BUF_ERROR; break; }
-                            unsigned c = br.take(8);
-                            hcrc = crc_bitwise(hcrc, c);
-                            if (c == 0) break;
-                        }
-                    }
-                    if (status == ZS_OK && (flg & 2)) {  // FHCRC
-                        if (!br.need(16)) status = ZS_BUF_ERROR;
-                        else if (br.take(16) != ((~hcrc) & 0xffffu)) { status = ZS_DATA_ERROR; detail = D_HDR_CRC; }
-                    }
-                    tflags = 2;
-                } else if (!(a.wrap & 1) || (((h & 0xff) << 8) + (h >> 8)) % 31) {
-                    status = ZS_DATA_ERROR; detail = D_HEADER_CHECK;
-                } else if ((h & 0xf) != 8) {
-                    status = ZS_DATA_ERROR; detail = D_METHOD;
-                } else if (((h >> 4) & 0xf) + 8 > 15) {
-                    status = ZS_DATA_ERROR; detail = D_WINDOW;
-                } else {
-                    br.drop(16);
-                    tflags = 1;
-                    if (h & 0x2000) {  // FDICT: DICTID follows; preset dictionaries for zlib streams
-                        if (!br.need(32)) status = ZS_BUF_ERROR;  // are host-side framing (INTEGRATION.md)
-                        else { br.drop(32); status = ZS_NEED_DICT; }
-                    }
-                }
-            }
-        }
+        if (a.wrap && !skip_header) read_wrapper_header(br, a.wrap, status, detail, tflags);
 
         if (a.d_hdr_state) {
             // header only: where the blocks start, for the segment-parallel decoder
@@ -255,13 +174,8 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
                     // a symbol pulls at most 8 bytes: two refills of 32 bits
                     while (in_rem >= 8u && out_rem) {
                         if (br.bits <= 32) ZS_FAST_REFILL();
-                        uint32_t here = lcode[(unsigned)br.hold & lmask];
-                        unsigned used = E_BITS(here);
-                        if (E_OP(here) && (E_OP(here) & 0xf0u) == 0) {  // second-level table
-                            const uint32_t first = here;
-                            here = lcode[E_VAL(first) + (((unsigned)br.hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
-                            used = E_BITS(first) + E_BITS(here);
-                        }
+                        unsigned used;
+                        uint32_t here = table_lookup<true>(lcode, lmask, br.hold, used);
                         const unsigned lop = E_OP(here);
                         if (lop == 0) {  // literal
                             br.drop(used);
@@ -279,13 +193,7 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
                         const unsigned len = E_VAL(here) + (((unsigned)(br.hold >> used)) & ((1u << xb) - 1u));
                         br.drop(used + xb);
                         if (br.bits <= 32) ZS_FAST_REFILL();
-                        here = dcode[(unsigned)br.hold & dmask];
-                        used = E_BITS(here);
-                        if ((E_OP(here) & 0xf0u) == 0) {
-                            const uint32_t first = here;
-                            here = dcode[E_VAL(first) + (((unsigned)br.hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
-                            used = E_BITS(first) + E_BITS(here);
-                        }
+                        here = table_lookup<false>(dcode, dmask, br.hold, used);
                         xb = E_OP(here) & 15u;
                         const unsigned dist = E_VAL(here) + (((unsigned)(br.hold >> used)) & ((1u << xb) - 1u));
                         if ((E_OP(here) & 64u) || dist > back0 + made || len > out_rem) {
@@ -333,13 +241,8 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
                 }
                 // ---- careful path: one symbol with every test of inflate() (also reached for the tail of a buffer)
                 br.refill();
-                uint32_t here = lcode[(unsigned)br.hold & lmask];
-                unsigned used = E_BITS(here);
-                if (E_OP(here) && (E_OP(here) & 0xf0u) == 0) {  // second-level table
-                    uint32_t first = here;
-                    here = lcode[E_VAL(first) + (((unsigned)br.hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
-                    used = E_BITS(first) + E_BITS(here);
-                }
+                unsigned used;
+                uint32_t here = table_lookup<true>(lcode, lmask, br.hold, used);
                 if (used > br.bits) { status = ZS_BUF_ERROR; break; }
                 unsigned lop = E_OP(here);
                 if (lop == 0) {  // literal
@@ -358,13 +261,7 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
                 unsigned len = E_VAL(here) + br.take(xb);
                 // distance
                 br.refill();
-                here = dcode[(unsigned)br.hold & dmask];
-                used = E_BITS(here);
-                if ((E_OP(here) & 0xf0u) == 0) {
-                    uint32_t first = here;
-                    here = dcode[E_VAL(first) + (((unsigned)br.hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
-                    used = E_BITS(first) + E_BITS(here);
-                }
+                here = table_lookup<false>(dcode, dmask, br.hold, used);
                 if (used > br.bits) { status = ZS_BUF_ERROR; break; }
                 if (E_OP(here) & 64) { status = ZS_DATA_ERROR; detail = D_DIST_CODE; break; }
                 xb = E_OP(here) & 15u;
@@ -388,35 +285,9 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
             }
         }
 
-        // ---- trailer: CHECK / LENGTH (inflate.ts:1006-1037) ----
-        if (status == ZS_OK) {
-            br.align_byte();
-            if (tflags) {
-                if (!br.need(32)) status = ZS_BUF_ERROR;
-                else {
-                    uint32_t w = (uint32_t)br.hold;
-                    br.drop(32);
-                    t_check = tflags == 1 ? __byte_perm(w, 0, 0x0123) : w;
-                }
-                if (status == ZS_OK && tflags == 2) {
-                    if (!br.need(32)) status = ZS_BUF_ERROR;
-                    else { t_isize = (uint32_t)br.hold; br.drop(32); }
-                }
-            }
-            if (status == ZS_OK) status = ZS_STREAM_END;
-        }
+        read_trailer(br, tflags, status, t_check, t_isize);
         if (lane == 0) {
-            a.d_out_len[sidx] = op;
-            // a Z_BUF_ERROR with output space left means the input ran dry: the reference has
-            // pulled every available byte by then (PULLBYTE, inflate.ts:1147-1158)
-            uint64_t used_in = (status == ZS_BUF_ERROR && op < cap) ? br.end - in_start
-                                                                    : br.pos - (br.bits >> 3) - in_start;
-            if (a.d_in_used) a.d_in_used[sidx] = used_in;
-            a.d_status[sidx] = status;
-            a.d_detail[sidx] = detail;
-            a.d_trailer[2 * sidx] = t_check;
-            a.d_trailer[2 * sidx + 1] = t_isize;
-            a.d_flags[sidx] = (status == ZS_STREAM_END) ? tflags : 0u;
+            store_result(a, sidx, br, in_start, op, cap, status, detail, tflags, t_check, t_isize);
             if (a.d_block_mark) { a.d_block_mark[2 * sidx] = mark_bit; a.d_block_mark[2 * sidx + 1] = mark_out; }
         }
         __syncwarp();

@@ -1,6 +1,8 @@
-// zs_inflate_common.cuh -- pieces shared by the warp-per-stream inflate kernel (zs_inflate.cu) and the
-// segment-parallel decoder of one stream (zs_inflate_par.cu): decode-table entries, the warp-parallel table
-// construction, the bit reader and the dynamic block header.
+// zs_inflate_common.cuh -- pieces shared by the warp-per-stream inflate kernel (zs_inflate.cu), the
+// thread-per-stream kernel (zs_inflate_tps.cu) and the segment-parallel decoder of one stream
+// (zs_inflate_par.cu): decode-table entries and their lookup, the warp-parallel table construction, the bit
+// reader, the dynamic block header, and the stream setup, wrapper header, trailer and result record of a
+// batch stream.
 //
 // The decode tables have the layout of the reference's inflate_table (src/mod/inflate/inftrees.ts:62-307):
 // a root table of `root` bits whose entries are symbols (replicated for shorter codes) or pointers to
@@ -254,6 +256,155 @@ struct BitReader {
         bits = __shfl_sync(ZS_FULL_MASK, bits, 0);
     }
 };
+
+// One symbol's entry of a decode table: the root entry for the low bits of `hold` or, where that points to a
+// sub-table, the entry there; `used` receives the bits of the code.  A literal/length root entry is a pointer
+// when its op is non-zero with no bit of 0xf0 set; a distance root entry is never op 0, so the test is one
+// compare shorter.
+template <bool kLitLen>
+__device__ __forceinline__ uint32_t table_lookup(const uint32_t* table, unsigned mask, uint64_t hold, unsigned& used) {
+    uint32_t here = table[(unsigned)hold & mask];
+    used = E_BITS(here);
+    if ((!kLitLen || E_OP(here)) && (E_OP(here) & 0xf0u) == 0) {
+        const uint32_t first = here;
+        here = table[E_VAL(first) + (((unsigned)hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
+        used = E_BITS(first) + E_BITS(here);
+    }
+    return here;
+}
+
+// ---- one stream of a batch (inflate_kernel, inflate_tps_kernel) --------------------------------------
+
+// The reader over stream sidx's input, its output capacity and its preset dictionary (none: dict_len = 0).
+// (The output pointer, a.d_out + a.d_out_off[sidx], is formed by the kernel: formed here, it changed how
+// inflate_kernel's fast loop computes the addresses of its match copies.)
+__device__ __forceinline__ void open_stream(const zs_inflate_args& a, uint64_t sidx, uint64_t safe_end, BitReader& br,
+                                            uint64_t& cap, const uint8_t*& dict, uint64_t& dict_len) {
+    br.base = a.d_in;
+    br.pos = a.d_in_off[sidx];
+    br.end = a.d_in_off[sidx + 1];
+    br.safe_end = safe_end;
+    br.hold = 0;
+    br.bits = 0;
+    cap = a.d_out_off[sidx + 1] - a.d_out_off[sidx];
+    dict = nullptr;
+    dict_len = 0;
+    if (a.d_dict && a.d_dict_rng) {
+        dict = a.d_dict + a.d_dict_rng[2 * sidx];
+        dict_len = a.d_dict_rng[2 * sidx + 1] - a.d_dict_rng[2 * sidx];
+    }
+}
+
+__device__ __forceinline__ uint32_t crc_bitwise(uint32_t crc, unsigned byte) {
+    crc ^= byte;
+    for (int k = 0; k < 8; k++) crc = (crc & 1u) ? (0xedb88320u ^ (crc >> 1)) : (crc >> 1);
+    return crc;
+}
+
+// Wrapper header: HEAD..HCRC / DICTID of inflate() (inflate.ts:377-593).  wrap: bit 0 zlib, bit 1 gzip.
+// A bad or truncated header sets status (and detail); FDICT sets ZS_NEED_DICT.  tflags: 1 zlib trailer,
+// 2 gzip trailer.
+__device__ __forceinline__ void read_wrapper_header(BitReader& br, int wrap, int& status, int& detail, unsigned& tflags) {
+    if (!br.need(16)) {
+        status = ZS_BUF_ERROR;
+    } else {
+        unsigned h = br.peek(16);
+        if ((wrap & 2) && h == 0x8b1fu) {
+            uint32_t hcrc = crc_bitwise(crc_bitwise(0xffffffffu, 0x1f), 0x8b);
+            br.drop(16);
+            // FLAGS
+            if (!br.need(16)) status = ZS_BUF_ERROR;
+            unsigned flg = 0;
+            if (status == ZS_OK) {
+                unsigned w = br.take(16);
+                flg = w >> 8;
+                if ((w & 0xff) != 8) { status = ZS_DATA_ERROR; detail = D_METHOD; }
+                else if (w & 0xe000) { status = ZS_DATA_ERROR; detail = D_HDR_FLAGS; }
+                hcrc = crc_bitwise(crc_bitwise(hcrc, w & 0xff), w >> 8);
+            }
+            // TIME(4) XFL OS
+            for (int k = 0; k < 6 && status == ZS_OK; k++) {
+                if (!br.need(8)) status = ZS_BUF_ERROR;
+                else hcrc = crc_bitwise(hcrc, br.take(8));
+            }
+            if (status == ZS_OK && (flg & 4)) {  // FEXTRA
+                unsigned xlen = 0;
+                if (!br.need(16)) status = ZS_BUF_ERROR;
+                else {
+                    xlen = br.take(16);
+                    hcrc = crc_bitwise(crc_bitwise(hcrc, xlen & 0xff), xlen >> 8);
+                }
+                while (status == ZS_OK && xlen--) {
+                    if (!br.need(8)) status = ZS_BUF_ERROR;
+                    else hcrc = crc_bitwise(hcrc, br.take(8));
+                }
+            }
+            for (int which = 0; which < 2 && status == ZS_OK; which++) {  // FNAME, FCOMMENT
+                if (!(flg & (which ? 16 : 8))) continue;
+                for (;;) {
+                    if (!br.need(8)) { status = ZS_BUF_ERROR; break; }
+                    unsigned c = br.take(8);
+                    hcrc = crc_bitwise(hcrc, c);
+                    if (c == 0) break;
+                }
+            }
+            if (status == ZS_OK && (flg & 2)) {  // FHCRC
+                if (!br.need(16)) status = ZS_BUF_ERROR;
+                else if (br.take(16) != ((~hcrc) & 0xffffu)) { status = ZS_DATA_ERROR; detail = D_HDR_CRC; }
+            }
+            tflags = 2;
+        } else if (!(wrap & 1) || (((h & 0xff) << 8) + (h >> 8)) % 31) {
+            status = ZS_DATA_ERROR; detail = D_HEADER_CHECK;
+        } else if ((h & 0xf) != 8) {
+            status = ZS_DATA_ERROR; detail = D_METHOD;
+        } else if (((h >> 4) & 0xf) + 8 > 15) {
+            status = ZS_DATA_ERROR; detail = D_WINDOW;
+        } else {
+            br.drop(16);
+            tflags = 1;
+            if (h & 0x2000) {  // FDICT: DICTID follows; preset dictionaries for zlib streams
+                if (!br.need(32)) status = ZS_BUF_ERROR;  // are host-side framing (INTEGRATION.md)
+                else { br.drop(32); status = ZS_NEED_DICT; }
+            }
+        }
+    }
+}
+
+// Trailer: CHECK / LENGTH (inflate.ts:1006-1037), read when the blocks ended well (status ZS_OK, which
+// becomes ZS_STREAM_END).  check / isize receive the stored values; inflate_verify_kernel compares them.
+__device__ __forceinline__ void read_trailer(BitReader& br, unsigned tflags, int& status, uint32_t& check, uint32_t& isize) {
+    if (status == ZS_OK) {
+        br.align_byte();
+        if (tflags) {
+            if (!br.need(32)) status = ZS_BUF_ERROR;
+            else {
+                uint32_t w = (uint32_t)br.hold;
+                br.drop(32);
+                check = tflags == 1 ? __byte_perm(w, 0, 0x0123) : w;
+            }
+            if (status == ZS_OK && tflags == 2) {
+                if (!br.need(32)) status = ZS_BUF_ERROR;
+                else { isize = (uint32_t)br.hold; br.drop(32); }
+            }
+        }
+        if (status == ZS_OK) status = ZS_STREAM_END;
+    }
+}
+
+// The per-stream result record.  A Z_BUF_ERROR with output space left means the input ran dry: the reference
+// has pulled every available byte by then (PULLBYTE, inflate.ts:1147-1158).
+__device__ __forceinline__ void store_result(const zs_inflate_args& a, uint64_t sidx, const BitReader& br, uint64_t in_start,
+                                             uint64_t op, uint64_t cap, int status, int detail, unsigned tflags,
+                                             uint32_t check, uint32_t isize) {
+    a.d_out_len[sidx] = op;
+    const uint64_t used_in = (status == ZS_BUF_ERROR && op < cap) ? br.end - in_start : br.pos - (br.bits >> 3) - in_start;
+    if (a.d_in_used) a.d_in_used[sidx] = used_in;
+    a.d_status[sidx] = status;
+    a.d_detail[sidx] = detail;
+    a.d_trailer[2 * sidx] = check;
+    a.d_trailer[2 * sidx + 1] = isize;
+    a.d_flags[sidx] = (status == ZS_STREAM_END) ? tflags : 0u;
+}
 
 static __constant__ uint8_t c_bl_order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
 

@@ -381,13 +381,8 @@ __device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, c
         bool block_ok = false;
         for (;;) {
             br.refill();
-            uint32_t here = lcode[(unsigned)br.hold & lmask];
-            unsigned used = E_BITS(here);
-            if (E_OP(here) && (E_OP(here) & 0xf0u) == 0) {
-                const uint32_t first = here;
-                here = lcode[E_VAL(first) + (((unsigned)br.hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
-                used = E_BITS(first) + E_BITS(here);
-            }
+            unsigned used;
+            uint32_t here = table_lookup<true>(lcode, lmask, br.hold, used);
             if (used > br.bits) break;
             const unsigned lop = E_OP(here);
             if (lop == 0) {
@@ -403,13 +398,7 @@ __device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, c
             br.drop(used);
             const unsigned len = E_VAL(here) + br.take(xb);
             br.refill();
-            here = dcode[(unsigned)br.hold & dmask];
-            used = E_BITS(here);
-            if ((E_OP(here) & 0xf0u) == 0) {
-                const uint32_t first = here;
-                here = dcode[E_VAL(first) + (((unsigned)br.hold >> E_BITS(first)) & ((1u << E_OP(first)) - 1u))];
-                used = E_BITS(first) + E_BITS(here);
-            }
+            here = table_lookup<false>(dcode, dmask, br.hold, used);
             if (used > br.bits) break;
             if (E_OP(here) & 64) break;
             xb = E_OP(here) & 15u;
@@ -663,10 +652,7 @@ __global__ void par_finish_kernel(ParArgs a) {
 // scratch slots of zs_api.cu reserved for this path
 enum { SCR_P_CAND = 25, SCR_P_SEG = 26, SCR_P_PLAN = 27, SCR_P_SYM = 28, SCR_P_WIN = 29, SCR_P_STATE = 30, SCR_P_GMAP = 33 };
 
-int zs_launch_inflate_header(zs_ctx* ctx, const zs_inflate_args& a, uint64_t* d_state);   // zs_inflate.cu
-
 // One stream, wrapper header already located: a.d_resume receives where inflate_kernel continues.
-// d_state: [5] = bit position of the first block (or ~0), [6] = trailer flags, filled by zs_launch_inflate_header.
 int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
                                const uint8_t* d_hist, uint64_t hist_len, uint64_t* d_state, uint64_t* d_resume) {
     ParArgs p;

@@ -18,15 +18,11 @@
 // code.  The dispatcher (zs_launch_inflate) picks this kernel for >= 32768 streams.
 #include <cstdio>
 
-#include "zs_common.cuh"
+#include "zs_inflate_common.cuh"
 
 namespace {
 
-enum {
-    D_NONE = 0, D_HEADER_CHECK, D_METHOD, D_WINDOW, D_HDR_FLAGS, D_HDR_CRC, D_BLOCK_TYPE, D_STORED_LEN,
-    D_TOO_MANY, D_TOO_MANY_9, D_CODE_LENGTHS, D_BIT_REPEAT, D_NO_EOB, D_LITLEN_SET, D_DIST_SET, D_LITLEN_CODE,
-    D_DIST_CODE, D_TOO_FAR, D_DATA_CHECK, D_LENGTH_CHECK
-};
+using namespace zsinf;
 
 // Per-thread table layout.  Shared memory per stream decides how many warps an SM holds (the kernel is
 // latency-bound: 7 warps per SM with 928 bytes per stream, 11 with 640), so the sorted symbols are
@@ -58,36 +54,6 @@ struct Tab {
         const unsigned sh = (i & 3u) * 4u;
         x = (uint16_t)((x & ~(15u << sh)) | (v << sh));
     }
-};
-
-__constant__ uint8_t c_order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-
-// per-thread bit reader (same semantics as BitReader in zs_inflate.cu)
-struct Bits {
-    const uint8_t* base;
-    uint64_t pos, end, safe_end;
-    uint64_t hold;
-    unsigned bits;
-    __device__ __forceinline__ void refill() {
-        if (bits <= 32) {
-            if (end - pos >= 4) {
-                hold |= (uint64_t)zs_ld32(base, pos, safe_end) << bits;
-                bits += 32;
-                pos += 4;
-            } else {
-                while (pos < end && bits <= 56) {
-                    hold |= (uint64_t)__ldg(base + pos) << bits;
-                    bits += 8;
-                    pos++;
-                }
-            }
-        }
-    }
-    __device__ __forceinline__ bool need(unsigned n) { if (bits < n) refill(); return bits >= n; }
-    __device__ __forceinline__ unsigned peek(unsigned n) const { return (unsigned)hold & ((1u << n) - 1u); }
-    __device__ __forceinline__ void drop(unsigned n) { hold >>= n; bits -= n; }
-    __device__ __forceinline__ unsigned take(unsigned n) { unsigned v = peek(n); drop(n); return v; }
-    __device__ __forceinline__ void unload() { pos -= bits >> 3; hold = 0; bits = 0; }
 };
 
 // Canonical tables from code lengths lens[first .. first+n): the verdicts of inflate_table
@@ -185,6 +151,8 @@ __device__ __forceinline__ int decode_sym_fast(const Tab& T, const LimSet& L, ui
     return (int)sym;
 }
 
+// len_sym / dist_sym (zs_inflate_common.cuh) in the form this kernel needs: extra bits and an invalid flag
+// instead of a table op, which made the kernel 16 SASS instructions longer when decoded from the op.
 __device__ __forceinline__ void len_base(unsigned idx, bool d64, unsigned& base, unsigned& xb, bool& invalid) {
     invalid = false;
     if (idx < 28) {
@@ -210,12 +178,6 @@ __device__ __forceinline__ void dist_base(unsigned idx, bool d64, unsigned& base
     }
 }
 
-__device__ __forceinline__ uint32_t crc_bitwise(uint32_t crc, unsigned byte) {
-    crc ^= byte;
-    for (int k = 0; k < 8; k++) crc = (crc & 1u) ? (0xedb88320u ^ (crc >> 1)) : (crc >> 1);
-    return crc;
-}
-
 __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_inflate_args a) {
     __shared__ __align__(16) uint8_t s_tab[kWarpsPerCta][kArenaBytes];
     const unsigned lane = zs_lane();
@@ -227,88 +189,18 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
     const uint64_t safe_end = (in_total + 7) & ~7ull;
 
     for (uint64_t sidx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; sidx < a.n; sidx += (uint64_t)gridDim.x * blockDim.x) {
-        Bits br;
-        br.base = a.d_in;
-        br.pos = a.d_in_off[sidx];
-        br.end = a.d_in_off[sidx + 1];
-        br.safe_end = safe_end;
-        br.hold = 0;
-        br.bits = 0;
+        BitReader br;
+        uint64_t cap, dict_len;
+        const uint8_t* dict;
+        open_stream(a, sidx, safe_end, br, cap, dict, dict_len);
         const uint64_t in_start = br.pos;
         uint8_t* out = a.d_out + a.d_out_off[sidx];
-        const uint64_t cap = a.d_out_off[sidx + 1] - a.d_out_off[sidx];
         uint64_t op = 0;
-        const uint8_t* dict = nullptr;
-        uint64_t dict_len = 0;
-        if (a.d_dict && a.d_dict_rng) {
-            dict = a.d_dict + a.d_dict_rng[2 * sidx];
-            dict_len = a.d_dict_rng[2 * sidx + 1] - a.d_dict_rng[2 * sidx];
-        }
         int status = ZS_OK, detail = D_NONE;
         unsigned tflags = 0;
         uint32_t t_check = 0, t_isize = 0;
 
-        // ---- wrapper header (inflate.ts:377-593) ----
-        if (a.wrap) {
-            if (!br.need(16)) {
-                status = ZS_BUF_ERROR;
-            } else {
-                const unsigned h = br.peek(16);
-                if ((a.wrap & 2) && h == 0x8b1fu) {
-                    uint32_t hcrc = crc_bitwise(crc_bitwise(0xffffffffu, 0x1f), 0x8b);
-                    br.drop(16);
-                    unsigned flg = 0;
-                    if (!br.need(16)) status = ZS_BUF_ERROR;
-                    if (status == ZS_OK) {
-                        const unsigned w = br.take(16);
-                        flg = w >> 8;
-                        if ((w & 0xff) != 8) { status = ZS_DATA_ERROR; detail = D_METHOD; }
-                        else if (w & 0xe000) { status = ZS_DATA_ERROR; detail = D_HDR_FLAGS; }
-                        hcrc = crc_bitwise(crc_bitwise(hcrc, w & 0xff), w >> 8);
-                    }
-                    for (int k = 0; k < 6 && status == ZS_OK; k++) {
-                        if (!br.need(8)) status = ZS_BUF_ERROR;
-                        else hcrc = crc_bitwise(hcrc, br.take(8));
-                    }
-                    if (status == ZS_OK && (flg & 4)) {
-                        unsigned xlen = 0;
-                        if (!br.need(16)) status = ZS_BUF_ERROR;
-                        else { xlen = br.take(16); hcrc = crc_bitwise(crc_bitwise(hcrc, xlen & 0xff), xlen >> 8); }
-                        while (status == ZS_OK && xlen--) {
-                            if (!br.need(8)) status = ZS_BUF_ERROR;
-                            else hcrc = crc_bitwise(hcrc, br.take(8));
-                        }
-                    }
-                    for (int which = 0; which < 2 && status == ZS_OK; which++) {
-                        if (!(flg & (which ? 16 : 8))) continue;
-                        for (;;) {
-                            if (!br.need(8)) { status = ZS_BUF_ERROR; break; }
-                            const unsigned c = br.take(8);
-                            hcrc = crc_bitwise(hcrc, c);
-                            if (c == 0) break;
-                        }
-                    }
-                    if (status == ZS_OK && (flg & 2)) {
-                        if (!br.need(16)) status = ZS_BUF_ERROR;
-                        else if (br.take(16) != ((~hcrc) & 0xffffu)) { status = ZS_DATA_ERROR; detail = D_HDR_CRC; }
-                    }
-                    tflags = 2;
-                } else if (!(a.wrap & 1) || (((h & 0xff) << 8) + (h >> 8)) % 31) {
-                    status = ZS_DATA_ERROR; detail = D_HEADER_CHECK;
-                } else if ((h & 0xf) != 8) {
-                    status = ZS_DATA_ERROR; detail = D_METHOD;
-                } else if (((h >> 4) & 0xf) + 8 > 15) {
-                    status = ZS_DATA_ERROR; detail = D_WINDOW;
-                } else {
-                    br.drop(16);
-                    tflags = 1;
-                    if (h & 0x2000) {
-                        if (!br.need(32)) status = ZS_BUF_ERROR;
-                        else { br.drop(32); status = ZS_NEED_DICT; }
-                    }
-                }
-            }
-        }
+        if (a.wrap) read_wrapper_header(br, a.wrap, status, detail, tflags);
 
         // ---- blocks ----
         bool last = false;
@@ -318,7 +210,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
             const unsigned type = br.take(2);
             unsigned lmin = 1, dmin = 1;
             if (type == 0) {
-                br.drop(br.bits & 7u);
+                br.align_byte();
                 if (!br.need(32)) { status = ZS_BUF_ERROR; break; }
                 const unsigned w = (unsigned)br.hold;
                 if ((w & 0xffffu) != ((w >> 16) ^ 0xffffu)) { status = ZS_DATA_ERROR; detail = D_STORED_LEN; break; }
@@ -346,7 +238,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
                 bool trunc = false;
                 for (unsigned i = 0; i < ncode; i++) {
                     if (!br.need(3)) { trunc = true; break; }
-                    T.len_set(c_order[i], br.take(3));
+                    T.len_set(c_bl_order[i], br.take(3));
                 }
                 if (trunc) { status = ZS_BUF_ERROR; break; }
                 unsigned cmin = 1;
@@ -484,31 +376,8 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
             }
         }
 
-        // ---- trailer (inflate.ts:1006-1037) ----
-        if (status == ZS_OK) {
-            br.drop(br.bits & 7u);
-            if (tflags) {
-                if (!br.need(32)) status = ZS_BUF_ERROR;
-                else {
-                    const uint32_t w = (uint32_t)br.hold;
-                    br.drop(32);
-                    t_check = tflags == 1 ? __byte_perm(w, 0, 0x0123) : w;
-                }
-                if (status == ZS_OK && tflags == 2) {
-                    if (!br.need(32)) status = ZS_BUF_ERROR;
-                    else { t_isize = (uint32_t)br.hold; br.drop(32); }
-                }
-            }
-            if (status == ZS_OK) status = ZS_STREAM_END;
-        }
-        a.d_out_len[sidx] = op;
-        const uint64_t used_in = (status == ZS_BUF_ERROR && op < cap) ? br.end - in_start : br.pos - (br.bits >> 3) - in_start;
-        if (a.d_in_used) a.d_in_used[sidx] = used_in;
-        a.d_status[sidx] = status;
-        a.d_detail[sidx] = detail;
-        a.d_trailer[2 * sidx] = t_check;
-        a.d_trailer[2 * sidx + 1] = t_isize;
-        a.d_flags[sidx] = (status == ZS_STREAM_END) ? tflags : 0u;
+        read_trailer(br, tflags, status, t_check, t_isize);
+        store_result(a, sidx, br, in_start, op, cap, status, detail, tflags, t_check, t_isize);
     }
 }
 
