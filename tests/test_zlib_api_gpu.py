@@ -306,7 +306,7 @@ def test_inflate_without_finish_reaches_stream_end(gpu_ctx):
     for wbits in (15, 31, -15):
         co = zlib.compressobj(6, zlib.DEFLATED, wbits)
         stream = co.compress(data) + co.flush()
-        assert len(stream) > (512 << 10)          # beyond the every-call threshold of the shim
+        assert len(stream) > (512 << 10)          # far beyond the shim's every-call threshold (64 KiB, kEveryCallBelow)
         s = Z.createInflateStream()
         assert Z.inflateInit2_(s, wbits) == Z.Z_OK
         out = bytearray()

@@ -261,6 +261,7 @@ struct InflateState {
     size_t out_pushed = 0;          // bytes of `out` already copied to `ready`
     size_t next_attempt = 0;
     bool fresh_input = false;       // input has arrived since the last attempt
+    uint32_t in_tail = 1;           // the last 4 input bytes received, across calls (big endian; 1 = none yet)
     double attempt_end = 0.0;       // monotonic clock at the end of the last attempt ...
     double attempt_cost = 0.0;      // ... and how long it took (seconds): the pacing of a long stream's attempts
     size_t out_cap_hint = 1 << 20;
@@ -981,6 +982,8 @@ int zs_stream_inflate(zs_stream* strm, int flush) {
         if (strm->avail_in) {
             const double t_ins0 = now_s();
             if (!st->in.append(strm->next_in, (size_t)strm->avail_in, 0)) { strm->msg = "insufficient memory"; return ZS_MEM_ERROR; }
+            for (size_t i = strm->avail_in > 4 ? (size_t)strm->avail_in - 4 : 0; i < strm->avail_in; i++)
+                st->in_tail = st->in_tail << 8 | strm->next_in[i];
             st->t_insert += now_s() - t_ins0;
             strm->next_in += strm->avail_in;
             strm->total_in += strm->avail_in;
@@ -1005,8 +1008,16 @@ int zs_stream_inflate(zs_stream* strm, int flush) {
         //    producing output, which the zlib contract allows.
         //    (Round 2 first doubled the batches of a long stream -- an attempt when as much input as had been seen had
         //    arrived again: 0.22-0.26 GB/s for a 64 MiB stream fed in 32 KiB slices, nine attempts of ~20 ms.)
+        //  * whatever the pace, on a call that brings input which ends with a sync / full flush marker (00 00 ff ff,
+        //    possibly split across calls): a request/response peer hands over one flushed message per call and waits
+        //    for its reply, so the message must be decoded now.  A memory-fed caller's slice almost never ends on a
+        //    marker, so bulk input keeps its pacing;
+        //  * and on a call that brings input while the last block is decoded and only the trailer is missing: finishing
+        //    the stream is host work plus one checksum, and Z_STREAM_END with the hand-back of what follows the
+        //    trailer through avail_in belongs to the call that brings its last byte.
         if (in0) st->fresh_input = true;
-        bool due = flush != ZS_NO_FLUSH || st->in.size() >= st->next_attempt || (in0 == 0 && st->fresh_input);
+        bool due = flush != ZS_NO_FLUSH || st->in.size() >= st->next_attempt || (in0 == 0 && st->fresh_input) ||
+                   (in0 && (st->in_tail == 0x0000ffffu || st->await_trailer));
         if (!due && st->fresh_input && now_s() - st->attempt_end >= kPaceFactor * st->attempt_cost) due = true;
         if (due && !st->in.empty()) {
             const double t_begin = now_s();
@@ -1094,6 +1105,7 @@ int zs_stream_inflate_reset(zs_stream* strm) {
     st->ready_pos = st->out_pushed = 0;
     st->next_attempt = 0;
     st->fresh_input = false;
+    st->in_tail = 1;
     st->attempt_end = st->attempt_cost = 0.0;
     st->body = st->await_trailer = false;
     st->start_bit = 0;
