@@ -34,7 +34,8 @@
 //                         candidates, compares in the shared-memory ring, 16-bit ring indices);
 //                         every position is searched speculatively, which is what makes the
 //                         chain walk 960-wide.  Greedy levels: compares stop at nice_length inside
-//                         the loop, the winners are extended together behind it.  Lazy levels: the
+//                         the loop, the winners are extended together behind it; each greedy level
+//                         has its own kernel, and level 1's walk is four straight-line rounds.  Lazy levels: the
 //                         batch walks in lock step with a straggler stop, and a candidate is first
 //                         tested on the four bytes that end at index best_len;
 //        resolve (wide) : greedy / lazy rule per position, 5 rounds of pointer doubling per batch
@@ -88,10 +89,12 @@ constexpr unsigned kMaxSegChunks = 256;  // chunks per segment (boundary table i
 
 struct LevelCfg { int lazy_fn, good, lazy, nice, chain; };
 // CONFIGURATION_TABLE, deflate.ts:86-103
-__constant__ LevelCfg c_levels[10] = {
+constexpr LevelCfg kLevels[10] = {
     {0, 0, 0, 0, 0},      {0, 4, 4, 8, 4},      {0, 4, 5, 16, 8},      {0, 4, 6, 32, 32},
     {1, 4, 4, 16, 16},    {1, 8, 16, 32, 32},   {1, 8, 16, 128, 128},  {1, 8, 32, 128, 256},
     {1, 32, 128, 258, 1024}, {1, 32, 258, 258, 4096}};
+// A row of the table as a compile-time constant in device code (kernels specialised for one level)
+__host__ __device__ constexpr LevelCfg level_cfg(int level) { return kLevels[level]; }
 
 // prep word: hash | nearest lower peer lane << 16 | has peer << 21 | last of its group << 22 | valid << 23
 constexpr uint32_t PREP_HAS_PRED = 1u << 21, PREP_LAST = 1u << 22, PREP_VALID = 1u << 23;
@@ -120,14 +123,13 @@ struct LzArgs {
     const uint64_t* in_off;    // [n_chunks+1] relative to org
     uint32_t n_chunks, seg_chunks, n_seg, max_bpc;
     uint32_t n_big, seg_small;   // segments [0, n_big) hold seg_chunks chunks, the later ones seg_small (see zs_launch_lz77)
-    int level;
+    LevelCfg cfg;              // kLevels[level] (kernels specialised for one level use their own compile-time copy)
     int strategy;              // ZS_STRATEGY_* (FILTERED and RLE act here)
     int cross;                 // 1: matches may reach before the chunk start (PRIME / STITCHED)
     uint32_t* sym;
     uint32_t* chunk_nblk;
     uint32_t* blk_desc;
     uint32_t* seg_counter;
-    int debug;                 // ZS_LZ_PROF builds: chain override in bits 8..
     unsigned stop_after, stop_active;   // lazy levels: straggler stop of the chain walk (search_lazy_endwin)
 };
 
@@ -395,19 +397,21 @@ __device__ __forceinline__ unsigned match_length(const Smem& S, unsigned ci, uns
 
 // [cs, ce) is the chunk that holds q.
 // kMode: 0 greedy levels (1-3), 2 Z_RLE.  (The lazy levels 4-9 use search_lazy_endwin below.)
+// kLevel: 0 = cfg is read at run time, 1-3 = cfg is the compile-time row kLevels[kLevel].
 // Work bounds of the lazy levels on periodic data: a chain is "dense" when the hop to the candidate is at most
 // kDenseHop positions -- runs and short periods, not ordinary text or DNA-like data, whose ties and good
 // matches must not cut the search short (measured: +5.8 % size on a 4-letter alphabet at level 6 when they did).
 constexpr unsigned kDenseHop = 8;       // hops this short mark a run / a short period
 constexpr int kInteriorChain = 16;      // candidates left once a good match turns out to lie inside a longer one
-template <int kMode>
+template <int kMode, int kLevel>
 __device__ __forceinline__ uint32_t search_position(const Smem& S, const LevelCfg& cfg, const RangeCtx& c, uint32_t q,
                                                     uint32_t cs, uint32_t ce) {
     static_assert(kMode == 0 || kMode == 2, "levels 4-9 go through search_lazy_endwin");
     const uint32_t room = ce - q;
     const unsigned max_len = room < 258u ? room : 258u;
     const unsigned pi = (c.cb + q) & (kRing - 1u);
-    const uint32_t pw0 = ring32(S, pi), pw1 = ring32(S, pi + 4);
+    const uint2 pw = ring64(S, pi);
+    const uint32_t pw0 = pw.x, pw1 = pw.y;
     const uint32_t lit = (pw0 & 0xffu) << 24;
     if (max_len < 3) return lit;
     if (kMode == 2) {
@@ -430,6 +434,40 @@ __device__ __forceinline__ uint32_t search_position(const Smem& S, const LevelCf
     const unsigned max_back = back < kMaxDist ? back : kMaxDist;
     unsigned best_len = 2, best_dist = 0, best_ci = pi;
     unsigned ci = pi, dist = 0;
+    if constexpr (kLevel != 0 && level_cfg(kLevel).nice <= 8) {
+        // Level 1 (chain 4, nice 8): the whole walk fits in the first eight bytes, so it runs as max_chain
+        // straight-line rounds, each one hop and one 8-byte compare per lane that is still walking, with no
+        // branch for the compiler to stop at: the hop of round r+1 is issued together with the window loads of
+        // round r.  There is no collision test: a candidate that differs in its first three bytes has a length
+        // below 3 and cannot beat best_len = 2.  A lane stops at the chain's end or once it holds a match of nice.
+        // (At level 1 the loop below costs about 10 warp instructions per input byte at 17 of 32 lanes active:
+        // profiles/lz77_r2b_l1_summary.md.)
+        bool alive = true;
+        unsigned delta = S.prev[ci & 32767u];
+#pragma unroll
+        for (int round = 0; round < level_cfg(kLevel).chain; ++round) {
+            dist += delta;
+            alive = alive && dist <= max_back;
+            ci = (ci - delta) & (kRing - 1u);
+            // a lane that is done reads at its own position (consecutive across the batch: no extra bank
+            // conflicts) instead of branching around the loads
+            const unsigned li = alive ? ci : pi;
+            const uint2 cw = ring64(S, li);
+            if (round + 1 < level_cfg(kLevel).chain) delta = S.prev[li & 32767u];
+            const uint32_t x0 = cw.x ^ pw0, x1 = cw.y ^ pw1;
+            // bytes equal from the start: trailing zero bits of the 64-bit xor / 8, without a branch
+            // ((x - 1) & ~x has the trailing zeros of x as ones: 32 of them for x = 0, so 8 bytes for equal words)
+            const uint32_t xw = x0 ? x0 : x1;
+            unsigned len = ((x0 ? 0u : 32u) + __popc((xw - 1u) & ~xw)) >> 3;
+            if (len > max_len) len = max_len;
+            if (alive && len > best_len) {
+                best_len = len;
+                best_dist = dist;
+                best_ci = ci;
+            }
+            alive = alive && len < nice;
+        }
+    } else
     for (int chain = cfg.chain; chain > 0; --chain) {
         unsigned delta;
         if (!chain_hop(S, ci, dist, max_back, delta)) break;
@@ -782,17 +820,20 @@ __device__ __forceinline__ uint32_t resolved_frontier(uint32_t searched, uint32_
 }
 
 // kMode 1: levels 4-9 (deflate_slow's rules); 0: levels 1-3, greedy; 2: Z_RLE, greedy with distance 1 only.
-template <int kMode>
+// kLevel (greedy levels): 0 = the level's parameters come from a.cfg, 1-3 = that level's row at compile time.
+template <int kMode, int kLevel>
 __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
+    static_assert(kLevel == 0 || (kMode == 0 && kLevel <= 3), "only the greedy levels are specialised");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& S = *reinterpret_cast<Smem*>(smem_raw);
     const unsigned wid = threadIdx.x >> 5, lane = zs_lane();
-    LevelCfg cfg = c_levels[a.level];
+    LevelCfg cfg = a.cfg;
+    if constexpr (kLevel != 0) {
+        constexpr LevelCfg row = level_cfg(kLevel);
+        cfg = row;
+    }
     const StopCfg stop = {a.stop_after, a.stop_active};
     (void)stop;
-#ifdef ZS_LZ_PROF
-    if (a.debug >> 8) cfg.chain = a.debug >> 8;
-#endif
 
 #ifdef ZS_LZ_BULK
     if (threadIdx.x == 0) mbar_init(&S.stage_bar, 1);   // published by the first __syncthreads of the segment loop
@@ -1018,7 +1059,7 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
                             }
                             // (the end-window filter of the lazy levels costs the greedy levels 7 % on text: chains of 4
                             // have nothing to filter)
-                            r = search_position<kMode == 1 ? 0 : kMode>(S, cfg, rc, q, cs, ce);
+                            r = search_position<kMode == 1 ? 0 : kMode, kLevel>(S, cfg, rc, q, cs, ce);
                         }
                         if (q < n) S.res[res_slot(q)] = r;
                     }
@@ -1118,10 +1159,14 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     // the opt-in to > 48 KB of dynamic shared memory is a per-device function attribute
     static bool attr_set[64] = {false};
     const int dev_slot = ctx->device >= 0 && ctx->device < 64 ? ctx->device : 0;
+    // lz77_kernel<0, 0> is the greedy levels with their parameters read at run time, <0, L> level L specialised
+    using LzKernel = void (*)(LzArgs);
+    static const LzKernel kGreedy[4] = {lz77_kernel<0, 0>, lz77_kernel<0, 1>, lz77_kernel<0, 2>, lz77_kernel<0, 3>};
     if (!attr_set[dev_slot] || ctx->device >= 64) {
-        ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
-        ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
-        ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+        for (LzKernel k : kGreedy)
+            ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+        ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+        ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
         attr_set[dev_slot] = true;
     }
     LzArgs a;
@@ -1134,7 +1179,7 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     a.in_off = p.d_in_off;
     a.n_chunks = p.n_chunks;
     a.max_bpc = p.max_bpc;
-    a.level = p.level;
+    a.cfg = kLevels[p.level];
     a.strategy = p.strategy;
     a.cross = (p.mode == ZS_MODE_STITCHED || (p.flags & ZS_FLAG_PRIME)) ? 1 : 0;
     // Segments: runs of consecutive chunks that go through the pipeline as one range, sharing one set
@@ -1175,14 +1220,21 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     a.chunk_nblk = p.d_chunk_nblk;
     a.blk_desc = p.d_blk_desc;
     a.seg_counter = p.d_seg_counter;
-    a.debug = 0;
     // straggler stop of the lazy levels (policy constants; the environment overrides exist for the A/B tools)
     a.stop_after = 8;
     a.stop_active = 8;
     if (const char* e = getenv("ZS_LZ_STOP_AFTER")) a.stop_after = (unsigned)atoi(e);
     if (const char* e = getenv("ZS_LZ_STOP_ACTIVE")) a.stop_active = (unsigned)atoi(e);
+    // ZS_LZ_GREEDY_GENERIC=1: the greedy levels through lz77_kernel<0, 0>, the reference the level-specialised
+    // kernels are compared with (same output, byte for byte)
+    bool greedy_generic = false;
+    if (const char* e = getenv("ZS_LZ_GREEDY_GENERIC")) greedy_generic = atoi(e) != 0;
 #ifdef ZS_LZ_PROF
-    if (getenv("ZS_LZ_DEBUG")) a.debug = atoi(getenv("ZS_LZ_DEBUG"));
+    // chain override in bits 8.. (the specialised kernels have theirs compiled in)
+    if (const char* e = getenv("ZS_LZ_DEBUG"); e && (atoi(e) >> 8)) {
+        a.cfg.chain = atoi(e) >> 8;
+        greedy_generic = true;
+    }
 #endif
     if (p.level == 0 || p.strategy == ZS_STRATEGY_HUFFMAN_ONLY) {
         const bool stored = p.level == 0;
@@ -1204,11 +1256,12 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     cudaMemcpyToSymbol(g_prof, zero, sizeof(zero));
 #endif
     if (a.strategy == ZS_STRATEGY_RLE) {
-        ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<2><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
-    } else if (a.level >= 4) {
-        ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<1><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
+        ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<2, 0><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
+    } else if (p.level >= 4) {
+        ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<1, 0><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
     } else {
-        ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<0><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
+        const LzKernel k = kGreedy[greedy_generic ? 0 : p.level];
+        ZS_KERNEL(ctx, "lz77_kernel", k<<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
     }
 #ifdef ZS_LZ_PROF
     {
