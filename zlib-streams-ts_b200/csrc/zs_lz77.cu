@@ -43,8 +43,8 @@
 //                         then two adjacent batches are composed into one 64-position hop (lazy
 //                         levels: resolve and emit pairs are claimed from a counter by the warps
 //                         that are done searching);
-//        parse   (thin) : chains the 64-position hops with register shuffles (entry of the next
-//                         hop = exit of this one), counts symbols, cuts blocks every <= 16383
+//        parse   (thin) : chains the 64-position hops, one shared-memory load each (entry of the
+//                         next hop = exit of this one), counts symbols, cuts blocks every <= 16383
 //                         symbols (lit_bufsize - 1, deflate.ts:323,336);
 //        emit    (wide) : writes the packed symbols of every batch at the index the parse gave it.
 //     The link stage runs at most 2 steps ahead of a searcher, so restricting matches to
@@ -135,7 +135,7 @@ struct LzArgs {
 
 #ifdef ZS_LZ_PROF
 // cycle counters: [0] thin insert, [1] thin parse, [2] wide warps (summed), [3] whole step incl.
-// barrier (warp 0), [4] steps
+// barrier (warp 0), [4] steps, [5] slowest wide warp of each step (summed)
 __device__ unsigned long long g_prof[16];
 #define PROF_T(i) if (lane == 0) atomicAdd(&g_prof[i], (unsigned long long)(clock64() - t_begin))
 #else
@@ -285,12 +285,14 @@ __device__ __forceinline__ uint32_t prep_batch(const Smem& S, const RangeCtx& c,
 // Only the head[] accesses are ordered (read the old head, then publish the batch's last position of
 // every hash); that is all the thin warp does.  Turning the old head into the prev[] link is
 // independent per position and is done by the wide warps one step later.
-__device__ __forceinline__ void head_exchange(Smem& S, uint32_t p16, uint32_t w, uint16_t* oldh) {
-    const unsigned h = w & 0x7fffu;
-    unsigned old = 0;
-    if ((w & PREP_VALID) && !(w & PREP_HAS_PRED)) old = S.head[h];
-    if (w & PREP_LAST) S.head[h] = (uint16_t)(p16 + zs_lane());
-    oldh[zs_lane()] = (uint16_t)old;
+// The link reads the old head only for a valid position without an in-batch peer, so every lane loads it
+// unconditionally (an invalid prep word reads head[0]): per batch that leaves one load of the prep word, the
+// head[] load and store, the oldh[] store and the value p + lane.
+__device__ __forceinline__ void head_exchange(Smem& S, uint32_t p, uint32_t w, uint16_t* oldh) {
+    const unsigned h = w & ((1u << kHashBits) - 1u);
+    const uint16_t old = S.head[h];
+    if (w & PREP_LAST) S.head[h] = (uint16_t)p;
+    oldh[zs_lane()] = old;
     __syncwarp();  // orders this batch's head[] stores before the next batch's loads
 }
 __device__ __forceinline__ void link_batch(Smem& S, const RangeCtx& c, uint32_t q0, uint32_t w, unsigned old) {
@@ -711,69 +713,82 @@ __device__ __forceinline__ unsigned below(unsigned b) { return b >= 32u ? 0xffff
 // to emit) and the index of its first symbol go to the pb ring; the wide warps write the symbols one
 // step later (emit_batch).  Matches never cross a chunk boundary, so the chain lands on every
 // boundary; a boundary strictly inside a pair splits the hop (rare: once per chunk).
-// kBoundary = false is the chain without any boundary test, for groups no boundary can touch (every
-// instruction on this chain costs 15-25 cycles).
+// The chain is the thin warp's whole cost: it shares its SM sub-partition with seven issue-bound wide
+// warps, so every instruction of a hop costs 6-7 cycles.  A hop entering pair q0 at offset s needs one
+// word, mj[q0 + s].y (the pair fields for s < 32, the batch fields of the second batch for s >= 32),
+// loaded on the chain as a broadcast.
+// kRare = false: groups that no chunk boundary can touch and that cannot fill the open block (a pair adds
+// at most 64 symbols), i.e. nearly all of them: unrolled, without a branch.  kRare = true: every other
+// group, a plain loop with the boundary and block-cut tests per hop.
 constexpr int kParseGroup = 16;
-template <bool kBoundary>
+template <bool kRare>
 __device__ __forceinline__ void parse_group(Smem& S, const LzArgs& a, const RangeCtx& rc, ParseState& ps, uint32_t c0,
                                             uint32_t qb, int np) {
     const unsigned lane = zs_lane();
     const uint32_t n = rc.n;
-    unsigned ya[kParseGroup], yb[kParseGroup];   // mj[].y of this lane in the first / second batch of each pair
-#pragma unroll
+    unsigned pb_entry = 64u, pb_sym = 0;   // lane u: entry offset and first symbol of pair u
+    uint32_t pos = qb + ps.skip;           // kRare = false: the position the chain stands on
+    constexpr int kUnroll = kRare ? 1 : kParseGroup;
+#pragma unroll kUnroll
     for (int u = 0; u < kParseGroup; ++u) {
-        const uint32_t q = qb + 64u * u + lane;
-        ya[u] = (u < np && q < n) ? S.mj[mj_slot(q)].y : (32u | (32u << 16));
-        yb[u] = (u < np && q + 32 < n) ? S.mj[mj_slot(q + 32)].y : 32u;
-    }
-#pragma unroll
-    for (int u = 0; u < kParseGroup; ++u) {
-        if (u < np) {
-            const uint32_t q0 = qb + 64u * u;
-            unsigned entry = 64u;
-            const uint32_t first_sym = ps.nsym;
-            if (ps.skip >= 64) {
-                ps.skip -= 64;
-            } else {
-                unsigned s = ps.skip;
-                entry = s;
-                while (kBoundary && ps.nb < q0 + 64u) {
-                    // sub-hop [s, b): the symbols of the visited positions before the boundary
-                    const unsigned b = ps.nb - q0;
-                    unsigned c;
-                    if (b <= s) {
-                        c = 0;   // an empty chunk; position q0 + s may be the end of the range, whose mj[] slot is stale
-                    } else if (s < 32u) {
-                        const uint2 m = S.mj[mj_slot(q0 + s)];
-                        c = __popc(m.x & below(b));
-                        if (b > 32u) {
-                            // the chain enters the second batch at xa <= b - 32; at xa == b - 32 it stands on the
-                            // boundary already (and that slot of mj[] is stale when b is the end of the range)
-                            const unsigned xa = mj_exit(m.y) - 32u;
-                            if (xa < b - 32u) c += __popc(S.mj[mj_slot(q0 + 32u + xa)].x & below(b - 32u));
-                        }
-                    } else {
-                        c = __popc(S.mj[mj_slot(q0 + s)].x & below(b - 32u));
+        if (u >= np) break;
+        const uint32_t q0 = qb + 64u * u;
+        const uint32_t first_sym = ps.nsym;
+        unsigned entry = 64u;
+        if constexpr (!kRare) {
+            // The group ends more than 258 positions before the next boundary, so pos < n and every exit lies
+            // in a later pair.  A pair the previous match covers (pos >= q0 + 64) reads a word it does not use.
+            const bool hop = pos < q0 + 64u, first = pos < q0 + 32u;
+            const unsigned y = S.mj[mj_slot(pos)].y;
+            const unsigned cnt = first ? mj_pair_count(y) : mj_count(y);
+            const unsigned e = (y >> (first ? 16u : 0u)) & 0x1ffu;   // exit relative to the pair, - 32
+            ps.nsym += hop ? cnt : 0u;
+            entry = hop ? pos - q0 : 64u;
+            if (hop) pos = q0 + 32u + e;
+        } else if (ps.skip >= 64) {
+            ps.skip -= 64;
+        } else {
+            unsigned s = ps.skip;
+            entry = s;
+            while (ps.nb < q0 + 64u) {
+                // sub-hop [s, b): the symbols of the visited positions before the boundary
+                const unsigned b = ps.nb - q0;
+                unsigned c;
+                if (b <= s) {
+                    c = 0;   // an empty chunk; position q0 + s may be the end of the range, whose mj[] slot is stale
+                } else if (s < 32u) {
+                    const uint2 m = S.mj[mj_slot(q0 + s)];
+                    c = __popc(m.x & below(b));
+                    if (b > 32u) {
+                        // the chain enters the second batch at xa <= b - 32; at xa == b - 32 it stands on the
+                        // boundary already (and that slot of mj[] is stale when b is the end of the range)
+                        const unsigned xa = mj_exit(m.y) - 32u;
+                        if (xa < b - 32u) c += __popc(S.mj[mj_slot(q0 + 32u + xa)].x & below(b - 32u));
                     }
-                    if (ps.nsym - ps.blk_sym0 + c > kSymLimit) close_block(a, rc, ps, c0, q0 + s);
-                    ps.nsym += c;
-                    close_chunk(S, a, rc, ps, c0);
-                    s = b;
+                } else {
+                    c = __popc(S.mj[mj_slot(q0 + s)].x & below(b - 32u));
                 }
-                // the serial chain: register shuffles only
-                const unsigned wa = __shfl_sync(ZS_FULL_MASK, ya[u], s & 31u);
-                const unsigned wb = __shfl_sync(ZS_FULL_MASK, yb[u], s & 31u);
-                unsigned cnt, exit_rel;
-                if (s < 32) { cnt = mj_pair_count(wa); exit_rel = mj_pair_exit(wa); }
-                else { cnt = mj_count(wb); exit_rel = 32u + mj_exit(wb); }
-                if (ps.nsym - ps.blk_sym0 + cnt > kSymLimit) close_block(a, rc, ps, c0, q0 + s);  // rare
-                ps.nsym += cnt;
-                ps.skip = exit_rel >= 64u ? exit_rel - 64u : 0u;   // < 64 only where the range ends
-                while (kBoundary && ps.nb <= q0 + exit_rel) close_chunk(S, a, rc, ps, c0);   // landed on a boundary
+                if (ps.nsym - ps.blk_sym0 + c > kSymLimit) close_block(a, rc, ps, c0, q0 + s);
+                ps.nsym += c;
+                close_chunk(S, a, rc, ps, c0);
+                s = b;
             }
-            if (lane == 0) S.pb[(q0 >> 6) & (kPbRing - 1u)] = make_uint2(entry, first_sym);
+            // past the end of the range (it ends inside this pair) nothing is visited: the mj[] slots are stale
+            unsigned cnt = 0, exit_rel = 64u;
+            if (q0 + s < n) {
+                const unsigned y = S.mj[mj_slot(q0 + s)].y;
+                if (s < 32) { cnt = mj_pair_count(y); exit_rel = mj_pair_exit(y); }
+                else { cnt = mj_count(y); exit_rel = 32u + mj_exit(y); }
+            }
+            if (ps.nsym - ps.blk_sym0 + cnt > kSymLimit) close_block(a, rc, ps, c0, q0 + s);
+            ps.nsym += cnt;
+            ps.skip = exit_rel >= 64u ? exit_rel - 64u : 0u;   // < 64 only where the range ends
+            while (ps.nb <= q0 + exit_rel) close_chunk(S, a, rc, ps, c0);   // landed on a boundary
         }
+        if (lane == (unsigned)u) { pb_entry = entry; pb_sym = first_sym; }
     }
+    if constexpr (!kRare) ps.skip = pos - (qb + 64u * np);
+    if (lane < (unsigned)np) S.pb[((qb >> 6) + lane) & (kPbRing - 1u)] = make_uint2(pb_entry, pb_sym);
 }
 
 // Wide emit: the symbols of one batch.  The pair's entry offset and first symbol index come from
@@ -837,6 +852,12 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
 
 #ifdef ZS_LZ_BULK
     if (threadIdx.x == 0) mbar_init(&S.stage_bar, 1);   // published by the first __syncthreads of the segment loop
+#endif
+#ifdef ZS_LZ_PROF
+    // slowest wide warp of step k: prof_wmax[k & 1], reset by thread 0 behind the barrier of step k (no
+    // warp reaches step k + 2 before that)
+    __shared__ unsigned long long prof_wmax[2];
+    if (threadIdx.x < 2) prof_wmax[threadIdx.x] = 0;
 #endif
     for (;;) {
         if (threadIdx.x == 0) S.seg = atomicAdd(a.seg_counter, 1u);
@@ -970,11 +991,11 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
                 }
 #endif
                 if (k >= 1 && k - 1 < nsteps) {
-                    const uint32_t p16 = rc.cb + q_prep - kStep;
-                    const uint32_t* pw = S.prep + s_ins * kStep;
+                    const uint32_t p = rc.cb + q_prep - kStep + lane;
+                    const uint32_t* pw = S.prep + s_ins * kStep + lane;
                     uint16_t* oh = S.oldh + ((k - 1) & 1u) * kStep;
-#pragma unroll 8
-                    for (int u = 0; u < kSearchWarps; ++u) head_exchange(S, p16 + 32u * u, pw[32 * u + lane], oh + 32 * u);
+#pragma unroll
+                    for (int u = 0; u < kSearchWarps; ++u) head_exchange(S, p + 32u * u, pw[32 * u], oh + 32 * u);
                 }
 #ifdef ZS_LZ_BULK
                 // past the end of the input the window reads as zeros (the last steps of the last segment only)
@@ -1018,9 +1039,11 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
                 while (ps.ppos < r1) {
                     int np = (int)((r1 - ps.ppos + 63) / 64);
                     if (np > kParseGroup) np = kParseGroup;
-                    // a hop leaves its pair by at most 257 positions
-                    if (ps.nb > ps.ppos + 64u * (unsigned)np + 258u) parse_group<false>(S, a, rc, ps, c0, ps.ppos, np);
-                    else parse_group<true>(S, a, rc, ps, c0, ps.ppos, np);
+                    // a hop leaves its pair by at most 257 positions and adds at most 64 symbols
+                    if (ps.nb > ps.ppos + 64u * (unsigned)np + 258u && ps.nsym - ps.blk_sym0 + 64u * (unsigned)np <= kSymLimit)
+                        parse_group<false>(S, a, rc, ps, c0, ps.ppos, np);
+                    else
+                        parse_group<true>(S, a, rc, ps, c0, ps.ppos, np);
                     ps.ppos += 64u * np;
                 }
             } else {
@@ -1110,6 +1133,7 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
                 if (lane == 0) {
                     const int role = wid == kWarpInsert ? 0 : wid == kWarpParse ? 1 : 2;
                     atomicAdd(&g_prof[role], (unsigned long long)t_work);
+                    if (role == 2) atomicMax(&prof_wmax[k & 1u], (unsigned long long)t_work);
                     if (wid == 0) atomicAdd(&g_prof[4], 1ull);
                 }
             }
@@ -1120,7 +1144,11 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
             s_prep = s_prep == 2 ? 0u : s_prep + 1u;
             __syncthreads();
 #ifdef ZS_LZ_PROF
-            if (threadIdx.x == 0) atomicAdd(&g_prof[3], (unsigned long long)(clock64() - t_begin));
+            if (threadIdx.x == 0) {
+                atomicAdd(&g_prof[3], (unsigned long long)(clock64() - t_begin));
+                atomicAdd(&g_prof[5], prof_wmax[k & 1u]);
+                prof_wmax[k & 1u] = 0;
+            }
 #endif
         }
         if (wid == kWarpParse)
@@ -1269,8 +1297,8 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
         cudaStreamSynchronize(ctx->stream);
         cudaMemcpyFromSymbol(pr, g_prof, sizeof(pr));
         double st = pr[4] ? (double)pr[4] : 1.0;
-        fprintf(stderr, "[lz77 prof] level %d steps %llu  cycles/step: insert %.0f parse %.0f wide(avg warp) %.0f step %.0f | insert: ldg-issued %.0f prep-loaded %.0f inserted %.0f | parse chain done %.0f\n",
-                p.level, pr[4], pr[0] / st, pr[1] / st, pr[2] / st / kSearchWarps, pr[3] / st, pr[8] / st, pr[9] / st, pr[10] / st, pr[11] / st);
+        fprintf(stderr, "[lz77 prof] level %d steps %llu  cycles/step: insert %.0f parse %.0f wide(avg warp) %.0f wide(max warp) %.0f step %.0f | insert: ldg-issued %.0f prep-loaded %.0f inserted %.0f | parse chain done %.0f\n",
+                p.level, pr[4], pr[0] / st, pr[1] / st, pr[2] / st / kSearchWarps, pr[5] / st, pr[3] / st, pr[8] / st, pr[9] / st, pr[10] / st, pr[11] / st);
         fprintf(stderr, "[lz77 prof] chain-loop iterations: total %llu max %llu positions>100: %llu (last: best_len %llu at chunk offset %llu)\n",
                 pr[12], pr[13], pr[14], pr[15] >> 32, pr[15] & 0xffffffffull);
     }
