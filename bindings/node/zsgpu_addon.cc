@@ -39,10 +39,29 @@ napi_value Init(napi_env env, napi_callback_info info) {
     return rc == ZS_OK ? nullptr : throw_code(env, rc, "zs_ctx_create");   // no CPU fallback: it throws
 }
 
-// deflateBatch(input: Uint8Array, chunkSize, level, wrap, mode, flags, out: Uint8Array, outOff: BigUint64Array)
-//   -> {bytes, bits, check, blocks}                                   zs_deflate_batch
+// createDeflateDictionary(dict: Uint8Array) -> {handle, id}            zs_deflate_dict_create
+// (the handle is destroyed when it is garbage collected)
+void FreeDict(napi_env, void* data, void*) { zs_deflate_dict_destroy((zs_deflate_dict*)data); }
+napi_value CreateDeflateDictionary(napi_env env, napi_callback_info info) {
+    size_t argc = 1; napi_value a[1];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    uint8_t* p; size_t n;
+    if (argc < 1 || !u8(env, a[0], &p, &n)) return throw_code(env, ZS_STREAM_ERROR, "createDeflateDictionary");
+    zs_deflate_dict* d = nullptr;
+    int rc = zs_deflate_dict_create(g_ctx, p, n, &d);
+    if (rc != ZS_OK) return throw_code(env, rc, "zs_deflate_dict_create");
+    napi_value h, o;
+    napi_create_external(env, d, FreeDict, nullptr, &h);
+    napi_create_object(env, &o);
+    napi_set_named_property(env, o, "handle", h);
+    napi_set_named_property(env, o, "id", num(env, (double)zs_deflate_dict_id(d)));
+    return o;
+}
+
+// deflateBatch(input: Uint8Array, chunkSize, level, wrap, mode, flags, out: Uint8Array, outOff: BigUint64Array
+//              [, dictionary handle]) -> {bytes, bits, check, blocks}   zs_deflate_batch / zs_deflate_batch_dict
 napi_value DeflateBatch(napi_env env, napi_callback_info info) {
-    size_t argc = 8; napi_value a[8];
+    size_t argc = 9; napi_value a[9];
     napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
     uint8_t *in, *out; size_t n, cap;
     if (!u8(env, a[0], &in, &n) || !u8(env, a[6], &out, &cap)) return throw_code(env, ZS_STREAM_ERROR, "deflateBatch");
@@ -51,8 +70,13 @@ napi_value DeflateBatch(napi_env env, napi_callback_info info) {
     uint64_t* off = nullptr; size_t off_n = 0; napi_typedarray_type t; napi_value ab; size_t bo;
     napi_get_typedarray_info(env, a[7], &t, &off_n, (void**)&off, &ab, &bo);
     zs_deflate_result r;
-    int rc = zs_deflate_batch(g_ctx, in, n, nullptr, n_chunks, chunk, i32(env, a[2]), i32(env, a[3]), i32(env, a[4]),
-                              (uint32_t)i32(env, a[5]), out, cap, off_n >= n_chunks + 1 ? off : nullptr, nullptr, nullptr, &r);
+    void* dict = nullptr;
+    if (argc >= 9 && napi_get_value_external(env, a[8], &dict) != napi_ok) dict = nullptr;
+    int rc = dict ? zs_deflate_batch_dict(g_ctx, (const zs_deflate_dict*)dict, in, n, nullptr, n_chunks, chunk, i32(env, a[2]),
+                                          i32(env, a[3]), (uint32_t)i32(env, a[5]), out, cap,
+                                          off_n >= n_chunks + 1 ? off : nullptr, nullptr, nullptr, &r)
+                  : zs_deflate_batch(g_ctx, in, n, nullptr, n_chunks, chunk, i32(env, a[2]), i32(env, a[3]), i32(env, a[4]),
+                                     (uint32_t)i32(env, a[5]), out, cap, off_n >= n_chunks + 1 ? off : nullptr, nullptr, nullptr, &r);
     if (rc != ZS_OK) return throw_code(env, rc, "zs_deflate_batch");
     napi_value o; napi_create_object(env, &o);
     napi_set_named_property(env, o, "bytes", num(env, (double)r.total_out_bytes));
@@ -63,9 +87,10 @@ napi_value DeflateBatch(napi_env env, napi_callback_info info) {
 }
 
 // inflateBatch(input, inOff: BigUint64Array, windowBits, out, outOff: BigUint64Array, outLen: BigUint64Array,
-//              checks: Uint32Array, status: Int32Array) -> void        zs_inflate_batch
+//              checks: Uint32Array, status: Int32Array[, dicts: Uint8Array, dictRng: BigUint64Array (2 per stream)])
+//   -> void                                                            zs_inflate_batch
 napi_value InflateBatch(napi_env env, napi_callback_info info) {
-    size_t argc = 8; napi_value a[8];
+    size_t argc = 10; napi_value a[10];
     napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
     uint8_t *in, *out; size_t n_in, n_out;
     if (!u8(env, a[0], &in, &n_in) || !u8(env, a[3], &out, &n_out)) return throw_code(env, ZS_STREAM_ERROR, "inflateBatch");
@@ -76,9 +101,14 @@ napi_value InflateBatch(napi_env env, napi_callback_info info) {
     napi_get_typedarray_info(env, a[5], &t, &n3, &out_len, &ab, &bo);
     napi_get_typedarray_info(env, a[6], &t, &n4, &checks, &ab, &bo);
     napi_get_typedarray_info(env, a[7], &t, &n5, &status, &ab, &bo);
+    uint8_t* dict = nullptr; size_t n_dict = 0; void* dict_rng = nullptr; size_t n6 = 0;
+    if (argc >= 10 && u8(env, a[8], &dict, &n_dict)) {
+        napi_get_typedarray_info(env, a[9], &t, &n6, &dict_rng, &ab, &bo);
+        if (n6 < 2 * (n1 - 1)) return throw_code(env, ZS_STREAM_ERROR, "inflateBatch: dictRng needs 2 entries per stream");
+    }
     int rc = zs_inflate_batch(g_ctx, in, (const uint64_t*)in_off, (uint32_t)(n1 - 1), i32(env, a[2]), out,
                               (const uint64_t*)out_off, (uint64_t*)out_len, nullptr, (uint32_t*)checks, (int32_t*)status,
-                              nullptr, nullptr, 0);
+                              dict_rng ? dict : nullptr, (const uint64_t*)dict_rng, dict_rng ? n_dict : 0);
     return rc == ZS_OK ? nullptr : throw_code(env, rc, "zs_inflate_batch");
 }
 
@@ -229,6 +259,7 @@ napi_value InflateHeaderState(napi_env env, napi_callback_info info) {
 napi_value Register(napi_env env, napi_value exports) {
     const struct { const char* name; napi_callback fn; } fns[] = {
         {"init", Init}, {"deflateBatch", DeflateBatch}, {"inflateBatch", InflateBatch}, {"checksum", Checksum},
+        {"createDeflateDictionary", CreateDeflateDictionary},
         {"streamNew", StreamNew}, {"deflateInit2", DeflateInit2}, {"inflateInit2", InflateInit2}, {"process", Process},
         {"end", End}, {"setDictionary", SetDictionary}, {"inflateReset", InflateReset}, {"control", Control},
         {"deflatePending", DeflatePending}, {"deflateSetHeader", DeflateSetHeader},

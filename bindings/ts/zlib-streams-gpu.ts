@@ -147,15 +147,29 @@ export function crc32(crc = 0, buf?: Uint8Array, len?: number): number {        
 }
 
 // ---- new batch entry points (no reference analogue) ----
-export function deflateBatch(input: Uint8Array, opts: { chunkSize: number; level?: number; wrap?: 0 | 1 | 2; stitched?: boolean; prime?: boolean }) {
+// A preset dictionary prepared once for many deflateBatch calls (deflateSetDictionary for every chunk); `id` is
+// the DICTID zlib streams made with it carry (adler32 of the whole dictionary).
+export interface DeflateDictionary { handle: unknown; id: number }
+export function createDeflateDictionary(dict: Uint8Array): DeflateDictionary {
+  return addon.createDeflateDictionary(dict);
+}
+// With `dictionary` every chunk is an independent stream that starts from it (raw or zlib, not stitched or primed).
+export function deflateBatch(input: Uint8Array, opts: { chunkSize: number; level?: number; wrap?: 0 | 1 | 2; stitched?: boolean; prime?: boolean;
+                                                       strategy?: number; dictionary?: DeflateDictionary }) {
   const nChunks = Math.max(1, Math.ceil(input.length / opts.chunkSize));
-  const out = new Uint8Array(input.length + 6 * nChunks * (Math.floor(opts.chunkSize / 16351) + 2) + 26 * nChunks + 64);
+  const out = new Uint8Array(input.length + 6 * nChunks * (Math.floor(opts.chunkSize / 16351) + 2) + 26 * nChunks + 64 +
+    (opts.dictionary ? 4 * nChunks : 0));
   const off = new BigUint64Array(nChunks + 1);
-  const r = addon.deflateBatch(input, opts.chunkSize, opts.level ?? 6, opts.wrap ?? 0, opts.stitched ? 1 : 0,
-    opts.prime ? 1 : 0, out, off);
+  if (opts.dictionary && (opts.stitched || opts.prime))
+    throw new Error("deflateBatch: a dictionary call compresses every chunk as its own stream (not stitched, not primed)");
+  const flags = (opts.prime ? 1 : 0) | ((opts.strategy ?? 0) << 8);
+  const r = opts.dictionary
+    ? addon.deflateBatch(input, opts.chunkSize, opts.level ?? 6, opts.wrap ?? 0, 0, flags, out, off, opts.dictionary.handle)
+    : addon.deflateBatch(input, opts.chunkSize, opts.level ?? 6, opts.wrap ?? 0, opts.stitched ? 1 : 0, flags, out, off);
   return { data: out.subarray(0, r.bytes), offsets: off, check: r.check, bits: r.bits };
 }
-export function inflateBatch(streams: Uint8Array[], windowBits: number, outCaps: number[]) {
+// dictionaries[i]: preset dictionary of stream i (raw streams, and zlib streams whose DICTID names it)
+export function inflateBatch(streams: Uint8Array[], windowBits: number, outCaps: number[], dictionaries?: (Uint8Array | undefined)[]) {
   const n = streams.length;
   const inOff = new BigUint64Array(n + 1), outOff = new BigUint64Array(n + 1);
   streams.forEach((s, i) => { inOff[i + 1] = inOff[i] + BigInt(s.length); outOff[i + 1] = outOff[i] + BigInt(outCaps[i]); });
@@ -163,6 +177,15 @@ export function inflateBatch(streams: Uint8Array[], windowBits: number, outCaps:
   streams.forEach((s, i) => input.set(s, Number(inOff[i])));
   const out = new Uint8Array(Number(outOff[n]) + 16), outLen = new BigUint64Array(n);
   const checks = new Uint32Array(n), status = new Int32Array(n);
-  addon.inflateBatch(input, inOff, windowBits, out, outOff, outLen, checks, status);
+  if (dictionaries) {
+    const rng = new BigUint64Array(2 * n);
+    let total = 0;
+    for (let i = 0; i < n; i++) { rng[2 * i] = BigInt(total); total += dictionaries[i]?.length ?? 0; rng[2 * i + 1] = BigInt(total); }
+    const blob = new Uint8Array(total + 1);
+    for (let i = 0; i < n; i++) if (dictionaries[i]) blob.set(dictionaries[i]!, Number(rng[2 * i]));
+    addon.inflateBatch(input, inOff, windowBits, out, outOff, outLen, checks, status, blob, rng);
+  } else {
+    addon.inflateBatch(input, inOff, windowBits, out, outOff, outLen, checks, status);
+  }
   return { out, outOff, outLen, checks, status };
 }

@@ -166,6 +166,43 @@ ZS_API int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint
                     int level, int wrap, uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_bits,
                     zs_deflate_result* result);
 
+/* ---- preset dictionary for batch deflate (deflateSetDictionary, deflate.ts:367-424, once for many
+ *      records).  Many small records compress far better against a shared dictionary; the batch calls
+ *      below compress every chunk as one whole stream that starts from it. ---- */
+typedef struct zs_deflate_dict zs_deflate_dict;
+
+/* Copies the dictionary to the context's device and builds the match finder's tables from it once (about
+ * 128 KiB of device memory).  Like deflateSetDictionary, only the last 32 KiB of a longer dictionary are
+ * used; an empty one is allowed.  Synchronises.  The handle may be used by any context on the same device. */
+ZS_API int zs_deflate_dict_create(zs_ctx* ctx, const uint8_t* dict, uint64_t dict_len, zs_deflate_dict** out);
+/* DICTID: adler32 of the WHOLE dictionary (what a zlib stream made with it names, and what an inflater
+ * compares with the dictionary it is given). */
+ZS_API uint32_t zs_deflate_dict_id(const zs_deflate_dict* d);
+/* Frees the dictionary (waits for the device).  Destroy it before the context it was created with. */
+ZS_API void zs_deflate_dict_destroy(zs_deflate_dict* d);
+
+/* Batch deflate against a prepared dictionary: the arguments of zs_deflate_batch_dev without history and
+ * mode.  Every chunk becomes an independent stream compressed as deflateSetDictionary + deflate(Z_FINISH)
+ * would: matches reach back into the dictionary's last 32 KiB (in this engine at most 32768 - 1920 bytes
+ * before the matching position, as everywhere: DESIGN.md 3.1), and the output of a chunk is byte-identical to
+ * zs_deflate_batch_dev with ZS_FLAG_PRIME on a buffer holding the dictionary's last <= 32 KiB followed by the
+ * chunk alone.  wrap: ZS_WRAP_RAW, or ZS_WRAP_ZLIB with FDICT set and the 4-byte DICTID after the 2-byte
+ * header when the dictionary is not empty (6 + body + 4 bytes per stream; the adler32 trailer covers the
+ * chunk alone).  ZS_WRAP_GZIP returns ZS_STREAM_ERROR (deflate.ts:372), as does any flag other than the
+ * strategy (PRIME, SYNC, part flags).  Level 0, Z_HUFFMAN_ONLY and Z_RLE produce the same blocks as without
+ * the dictionary (only the framing changes).  out_cap: zs_deflate_batch_bound(in_len, n_chunks, max_chunk,
+ * wrap, ZS_MODE_INDEPENDENT) + 4 * n_chunks is always enough. */
+ZS_API int zs_deflate_batch_dict_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* d_in, uint64_t in_len,
+                                     const uint64_t* d_in_off, uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk,
+                                     int level, int wrap, uint32_t flags, uint8_t* d_out, uint64_t out_cap,
+                                     uint64_t* d_out_off, uint64_t* d_out_bits, uint32_t* d_checks,
+                                     zs_deflate_result* d_result);
+/* Host-buffer variant, sliced and pipelined like zs_deflate_batch (slicing cannot change the output). */
+ZS_API int zs_deflate_batch_dict(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len,
+                                 const uint64_t* in_off, uint32_t n_chunks, uint32_t chunk_size, int level, int wrap,
+                                 uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits,
+                                 uint32_t* checks, zs_deflate_result* result);
+
 /* Bit-granular stitch (no reference analogue; deflatePrime, deflate.ts:528, is the reference's
  * "insert bits at a bit offset" primitive): OR `n_bits` bits of d_src into d_dst starting at bit
  * `dst_bit_off`.  The destination bits must be zero beforehand. */
@@ -188,8 +225,11 @@ ZS_API int zs_huffman_blocks(zs_ctx* ctx, const uint32_t* freq, const uint32_t* 
  * Stream i is d_in[d_in_off[i] .. d_in_off[i+1]); its output goes to d_out[d_out_off[i] ..
  * d_out_off[i+1]) (capacity).  window_bits as inflateInit2_ (inflate.ts:174): 15 zlib, -15 raw,
  * 31 gzip, 47 auto-detect zlib/gzip, -16 raw deflate64.  Optional per-stream preset dictionary
- * (raw streams, inflateSetDictionary inflate.ts:1220): stream i uses d_dict[d_dict_rng[2i] ..
- * d_dict_rng[2i+1]).  Per stream: d_out_len = bytes produced, d_in_used = bytes consumed
+ * (inflateSetDictionary inflate.ts:1220-1249): stream i uses d_dict[d_dict_rng[2i] .. d_dict_rng[2i+1]).
+ * A raw stream decodes against it directly.  A zlib stream whose header has FDICT decodes against it when
+ * the adler32 of the whole range equals the stream's DICTID (inflate -> Z_NEED_DICT -> inflateSetDictionary
+ * -> inflate(Z_FINISH)); without a dictionary, or with another one, its status is Z_NEED_DICT.  An empty range
+ * is no dictionary (a deflater sets FDICT only for a non-empty one).  Per stream: d_out_len = bytes produced, d_in_used = bytes consumed
  * (total_in), d_checks = adler32/crc32 of the output, d_status = what inflate(strm, Z_FINISH)
  * returns (Z_STREAM_END, Z_DATA_ERROR, Z_BUF_ERROR, Z_NEED_DICT).  d_in_used / d_checks may be NULL.
  */
@@ -214,7 +254,8 @@ ZS_API int zs_inflate_batch(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_o
  * a symbolic 32 KiB window and resolved in order (csrc/zs_inflate_par.cu).  A stream without flush points is
  * cut at dynamic block headers located by search (trusted only when the segment before lands on them bit
  * exact); raw deflate64 (-16) is decoded by one warp.  The host-buffer call zs_inflate_batch with n = 1 and the
- * streaming shim take the same path.  d_dict: optional preset dictionary / earlier output (raw streams). */
+ * streaming shim take the same path.  d_dict: optional preset dictionary / earlier output (raw streams, and
+ * zlib streams with FDICT as in zs_inflate_batch_dev). */
 ZS_API int zs_inflate_stream_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int window_bits, uint8_t* d_out,
                           uint64_t out_cap, uint64_t* d_out_len, uint64_t* d_in_used, uint32_t* d_check,
                           int32_t* d_status, const uint8_t* d_dict, uint64_t dict_len);

@@ -70,13 +70,50 @@ class DeflateBatchDev:
         return DeflateResult.from_buffer_copy(raw)
 
 
+class DeflateDictionary:
+    """A preset dictionary prepared once for batch deflate (zs_deflate_dict_create): the device copy of its last
+    32 KiB and the match finder's tables built from them.  `dict_id` is the DICTID a zlib stream made with it
+    carries: adler32 of the whole dictionary.  Close it (or let it be collected) before its context goes."""
+
+    def __init__(self, data, ctx: Context | None = None):
+        self.ctx = ctx or default_context()
+        src = _as_u8(data)
+        h = C.c_void_p()
+        self._lib = capi.load()
+        rc = self._lib.zs_deflate_dict_create(self.ctx.handle, src.ctypes.data if src.size else None, src.size, C.byref(h))
+        self.ctx.check(rc, "zs_deflate_dict_create")
+        self._h = h
+        self.dict_id = int(self._lib.zs_deflate_dict_id(h))
+        self.size = int(src.size)
+
+    @property
+    def handle(self):
+        if not self._h:
+            raise ValueError("DeflateDictionary is closed")
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.zs_deflate_dict_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def deflate_batch_dev(d_in: torch.Tensor, chunk_size: int, level: int = 6, wrap: int = WRAP_RAW,
                       mode: int = MODE_INDEPENDENT, flags: int = 0, history: int = 0, in_off: torch.Tensor | None = None,
                       max_chunk: int | None = None, out: torch.Tensor | None = None, want_checks: bool = False,
-                      ctx: Context | None = None, reuse: DeflateBatchDev | None = None) -> DeflateBatchDev:
+                      ctx: Context | None = None, reuse: DeflateBatchDev | None = None,
+                      dictionary: DeflateDictionary | None = None) -> DeflateBatchDev:
     """Enqueue one batch deflate on device-resident input (no synchronisation).
 
     `d_in` may be a view whose first `history` preceding bytes (same storage) are valid history.
+    With `dictionary` every chunk is an independent stream that starts from it (zs_deflate_batch_dict_dev):
+    mode must be INDEPENDENT, history 0, and flags the strategy alone; a zlib stream then carries FDICT + DICTID.
     """
     assert d_in.is_cuda and d_in.dtype == torch.uint8 and d_in.is_contiguous()
     ctx = ctx or default_context(d_in.device.index)
@@ -93,11 +130,21 @@ def deflate_batch_dev(d_in: torch.Tensor, chunk_size: int, level: int = 6, wrap:
     else:
         if out is None:
             cap = int(capi.load().zs_deflate_batch_bound(n, n_chunks, mc, wrap, mode))
+            if dictionary is not None:
+                cap += 4 * n_chunks   # DICTID
             out = torch.empty(cap, dtype=torch.uint8, device=dev)
         out_off = torch.empty(n_chunks + 1, dtype=torch.int64, device=dev)
         out_bits = torch.empty(n_chunks, dtype=torch.int64, device=dev)
         checks = torch.empty(n_chunks, dtype=torch.int32, device=dev) if (want_checks or wrap != WRAP_RAW) else None
         result = torch.zeros(24, dtype=torch.uint8, device=dev)
+    if dictionary is not None:
+        if mode != MODE_INDEPENDENT or history:
+            raise ValueError("a dictionary call is INDEPENDENT and takes no history")
+        rc = capi.load().zs_deflate_batch_dict_dev(ctx.handle, dictionary.handle, _ptr(d_in), n, _ptr(in_off), n_chunks,
+                                                   chunk_size, mc, level, wrap, flags, _ptr(out), out.numel(),
+                                                   _ptr(out_off), _ptr(out_bits), _ptr(checks), _ptr(result))
+        ctx.check(rc, "zs_deflate_batch_dict_dev")
+        return DeflateBatchDev(out, out_off, out_bits, checks, result)
     rc = capi.load().zs_deflate_batch_dev(ctx.handle, _ptr(d_in), n, _ptr(in_off), n_chunks, chunk_size, mc, history,
                                           level, wrap, mode, flags, _ptr(out), out.numel(), _ptr(out_off),
                                           _ptr(out_bits), _ptr(checks), _ptr(result))
@@ -122,8 +169,11 @@ class DeflateBatchHost:
 
 
 def deflate_batch(data, chunk_size: int = 65536, level: int = 6, wrap: int = WRAP_RAW, mode: int = MODE_INDEPENDENT,
-                  flags: int = 0, in_off=None, ctx: Context | None = None) -> DeflateBatchHost:
-    """Host-buffer deflateBatch through zs_deflate_batch (H2D + kernels + D2H inside the call)."""
+                  flags: int = 0, in_off=None, ctx: Context | None = None,
+                  dictionary: DeflateDictionary | None = None) -> DeflateBatchHost:
+    """Host-buffer deflateBatch through zs_deflate_batch (H2D + kernels + D2H inside the call).
+
+    With `dictionary`: zs_deflate_batch_dict, every chunk an independent stream that starts from it."""
     ctx = ctx or default_context()
     src = _as_u8(data)
     n = src.size
@@ -137,16 +187,27 @@ def deflate_batch(data, chunk_size: int = 65536, level: int = 6, wrap: int = WRA
         mc = int((off_arr[1:] - off_arr[:-1]).max()) if n_chunks else 1
     lib = capi.load()
     cap = int(lib.zs_deflate_batch_bound(n, n_chunks, max(mc, 1), wrap, mode))
+    if dictionary is not None:
+        cap += 4 * n_chunks   # DICTID
     out = np.empty(cap, dtype=np.uint8)
     out_off = np.zeros(n_chunks + 1, dtype=np.uint64)
     out_bits = np.zeros(n_chunks, dtype=np.uint64)
     checks = np.zeros(n_chunks, dtype=np.uint32)
     res = DeflateResult()
-    rc = lib.zs_deflate_batch(ctx.handle, src.ctypes.data if n else None, n,
-                              off_arr.ctypes.data if off_arr is not None else None, n_chunks, chunk_size, level, wrap,
-                              mode, flags, out.ctypes.data, cap, out_off.ctypes.data, out_bits.ctypes.data,
-                              checks.ctypes.data, C.byref(res))
-    ctx.check(rc, "zs_deflate_batch")
+    if dictionary is not None:
+        if mode != MODE_INDEPENDENT:
+            raise ValueError("a dictionary call is INDEPENDENT")
+        rc = lib.zs_deflate_batch_dict(ctx.handle, dictionary.handle, src.ctypes.data if n else None, n,
+                                       off_arr.ctypes.data if off_arr is not None else None, n_chunks, chunk_size, level,
+                                       wrap, flags, out.ctypes.data, cap, out_off.ctypes.data, out_bits.ctypes.data,
+                                       checks.ctypes.data, C.byref(res))
+        ctx.check(rc, "zs_deflate_batch_dict")
+    else:
+        rc = lib.zs_deflate_batch(ctx.handle, src.ctypes.data if n else None, n,
+                                  off_arr.ctypes.data if off_arr is not None else None, n_chunks, chunk_size, level, wrap,
+                                  mode, flags, out.ctypes.data, cap, out_off.ctypes.data, out_bits.ctypes.data,
+                                  checks.ctypes.data, C.byref(res))
+        ctx.check(rc, "zs_deflate_batch")
     return DeflateBatchHost(out[: res.total_out_bytes].tobytes(), out_off, out_bits, checks, res.total_out_bytes,
                             res.total_out_bits, res.check, res.n_blocks)
 
@@ -210,7 +271,9 @@ def inflate_batch(streams, window_bits: int = 15, out_caps=None, dictionaries=No
     """Host-buffer inflateBatch: `streams` is a list of bytes-like objects (independent streams).
 
     `out_caps[i]` is the output capacity given to stream i (avail_out of a one-shot
-    inflate(strm, Z_FINISH)); `dictionaries[i]` an optional preset dictionary (raw streams).
+    inflate(strm, Z_FINISH)); `dictionaries[i]` an optional preset dictionary: a raw stream decodes against it,
+    a zlib stream with FDICT when its DICTID is the dictionary's adler32 (Z_NEED_DICT otherwise).  None or an
+    empty dictionary is no dictionary.
     """
     ctx = ctx or default_context()
     n = len(streams)

@@ -66,6 +66,15 @@ _PROTOTYPES = {
                                    C.c_void_p, C.POINTER(DeflateResult)]),
     "zs_deflate_part": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.c_uint32,
                                   C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(DeflateResult)]),
+    "zs_deflate_dict_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]),
+    "zs_deflate_dict_id": (C.c_uint32, [C.c_void_p]),
+    "zs_deflate_dict_destroy": (None, [C.c_void_p]),
+    "zs_deflate_batch_dict_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32,
+                                            C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64,
+                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "zs_deflate_batch_dict": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32,
+                                        C.c_int, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.POINTER(DeflateResult)]),
     "zs_bit_concat_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64]),
     "zs_huffman_blocks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_inflate_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_void_p,

@@ -143,3 +143,41 @@ def mixed_torch_range(lo: int, hi: int, device, seed: int = 0xB200, tile: int = 
         out[pos - lo: pos - lo + take] = uniq[o: o + take]
         pos += take
     return out
+
+
+_JSON_KEYS = ["id", "user", "name", "email", "created_at", "updated_at", "status", "type", "score", "tags", "region",
+              "device", "session", "latency_ms", "bytes", "path", "method", "code", "message", "level", "version",
+              "count", "enabled", "ratio", "parent", "owner", "priority", "source"]
+_JSON_WORDS = ["active", "pending", "closed", "error", "warning", "info", "debug", "GET", "POST", "PUT", "eu-west-1",
+               "us-east-2", "ap-south-1", "mobile", "desktop", "tablet", "admin", "guest", "premium", "trial", "/api/v1/items",
+               "/api/v1/users", "/login", "/search", "timeout", "ok", "not found", "alpha", "beta", "gamma"]
+
+
+def json_pool(n: int, seed: int = 0x4A53) -> bytes:
+    """About n bytes of JSON-like rows (one object per line: a fixed key vocabulary, words, numbers, dates), the
+    kind of small records a preset dictionary is for.  Deterministic in `seed`."""
+    rng = np.random.default_rng(seed)
+    rows = []
+    size = 0
+    while size < n:
+        nk = int(rng.integers(4, 12))
+        keys = rng.choice(len(_JSON_KEYS), size=nk, replace=False)
+        parts = []
+        for k in sorted(keys):
+            key = _JSON_KEYS[k]
+            kind = int(rng.integers(0, 5))
+            if kind == 0:
+                v = str(int(rng.integers(0, 10 ** int(rng.integers(1, 9)))))
+            elif kind == 1:
+                v = '"%s"' % _JSON_WORDS[int(rng.integers(0, len(_JSON_WORDS)))]
+            elif kind == 2:
+                v = "%.3f" % float(rng.random() * 1000)
+            elif kind == 3:
+                v = '"2026-%02d-%02dT%02d:%02d:%02dZ"' % tuple(int(x) for x in rng.integers([1, 1, 0, 0, 0], [13, 29, 24, 60, 60]))
+            else:
+                v = "true" if rng.random() < 0.5 else "false"
+            parts.append('"%s": %s' % (key, v))
+        row = ("{" + ", ".join(parts) + "}\n").encode()
+        rows.append(row)
+        size += len(row)
+    return b"".join(rows)[:n]

@@ -86,6 +86,12 @@ int zs_set_cuda_error(zs_ctx* ctx, cudaError_t e, const char* where) {
 
 namespace {
 
+// dictionary ranges [begin, end) -> (begin, length) for the checksum kernels
+__global__ void dict_ranges_kernel(const uint64_t* rng, uint64_t* off, uint64_t* len, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) { off[i] = rng[2 * i]; len[i] = rng[2 * i + 1] - rng[2 * i]; }
+}
+
 __global__ void make_chunk_offsets_kernel(uint64_t* off, uint64_t len, uint64_t chunk, uint32_t n) {
     uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i <= n) {
@@ -248,13 +254,15 @@ int zs_checksum(zs_ctx* ctx, int kind, const uint8_t* buf, uint64_t len, uint32_
     return zs_checksum_dev(ctx, kind, d_in, len, init, result);
 }
 
+}  // extern "C"
+
 // ---- deflate ------------------------------------------------------------------------------------------
-int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, const uint64_t* d_in_off,
-                         uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk, uint32_t history, int level,
-                         int wrap, int mode, uint32_t flags, uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off,
-                         uint64_t* d_out_bits, uint32_t* d_checks, zs_deflate_result* d_result) {
-    if (ctx) bind_device(ctx);
-    if (!ctx) return ZS_STREAM_ERROR;
+// zs_deflate_batch_dev, and zs_deflate_batch_dict_dev with `dict` (INDEPENDENT, no history, checked by the caller)
+static int deflate_batch_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* d_in, uint64_t in_len,
+                             const uint64_t* d_in_off, uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk,
+                             uint32_t history, int level, int wrap, int mode, uint32_t flags, uint8_t* d_out,
+                             uint64_t out_cap, uint64_t* d_out_off, uint64_t* d_out_bits, uint32_t* d_checks,
+                             zs_deflate_result* d_result) {
     if (level == -1) level = 6;
     // argument rules of deflateInit2_ (deflate.ts:263-297) that apply to the batch form
     if (level < 0 || level > 9) return bad_arg(ctx, "deflate: level must be 0..9");
@@ -286,6 +294,7 @@ int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, cons
     p.max_bpc = max_chunk / 16351u + 2u;
     p.level = level; p.wrap = wrap; p.mode = mode; p.flags = flags; p.strategy = strategy;
     p.seg_hint = ctx->seg_hint;
+    p.dict = dict;
     const size_t slots = (size_t)n_chunks * p.max_bpc;
 
     uint64_t* off = (uint64_t*)zs_scratch_get(ctx, SCR_D_OFF, (size_t)(n_chunks + 1) * 8);
@@ -350,6 +359,95 @@ int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, cons
     return zs_launch_huffman(ctx, p);
 }
 
+extern "C" {
+
+int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, const uint64_t* d_in_off,
+                         uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk, uint32_t history, int level,
+                         int wrap, int mode, uint32_t flags, uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off,
+                         uint64_t* d_out_bits, uint32_t* d_checks, zs_deflate_result* d_result) {
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    return deflate_batch_dev(ctx, nullptr, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, history, level, wrap,
+                             mode, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result);
+}
+
+// ---- preset dictionaries ------------------------------------------------------------------------------
+int zs_deflate_dict_create(zs_ctx* ctx, const uint8_t* dict, uint64_t dict_len, zs_deflate_dict** out) {
+    if (ctx) bind_device(ctx);
+    if (!ctx || !out || (dict_len && !dict)) return bad_arg(ctx, "deflate_dict_create: bad arguments");
+    *out = nullptr;
+    // deflateSetDictionary (deflate.ts:367-424): only the last w_size bytes are used; DICTID covers them all
+    const uint64_t used = dict_len < 32768 ? dict_len : 32768;
+    zs_deflate_dict* d = new zs_deflate_dict();
+    d->device = ctx->device;
+    d->len = (uint32_t)used;
+    // the whole dictionary (for DICTID) and its used tail (16-byte aligned, for the build) are needed only here
+    uint8_t *d_whole = nullptr, *d_tail = nullptr;
+    auto fail = [&](int rc) {
+        cudaFree(d_whole); cudaFree(d_tail); cudaFree(d->d_img);
+        delete d;
+        return rc;
+    };
+    cudaError_t e = cudaMalloc(&d_tail, 32768 + 64);
+    if (e == cudaSuccess) e = cudaMalloc(&d->d_img, zs_lz77_dict_image_bytes());
+    if (e == cudaSuccess && dict_len) e = cudaMalloc(&d_whole, dict_len);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_tail, 0, 32768 + 64, ctx->stream);
+    if (e == cudaSuccess && dict_len) e = cudaMemcpyAsync(d_whole, dict, dict_len, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && used)
+        e = cudaMemcpyAsync(d_tail, d_whole + (dict_len - used), used, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e != cudaSuccess) return fail(zs_set_cuda_error(ctx, e, "deflate_dict_create"));
+    // DICTID on the device with the checksum kernels
+    uint32_t* d_id = (uint32_t*)zs_scratch_get(ctx, SCR_SMALL, 256);
+    if (!d_id) return fail(ZS_MEM_ERROR);
+    int rc = zs_launch_checksum_whole(ctx, 0, d_whole, dict_len, 1u, d_id);
+    if (rc != ZS_OK) return fail(rc);
+    e = cudaMemcpyAsync(&d->id, d_id, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(zs_set_cuda_error(ctx, e, "deflate_dict_create"));
+    rc = zs_lz77_dict_build(ctx, d_tail, d->len, d->d_img);   // synchronises
+    if (rc != ZS_OK) return fail(rc);
+    cudaFree(d_whole);
+    cudaFree(d_tail);
+    *out = d;
+    return ZS_OK;
+}
+
+uint32_t zs_deflate_dict_id(const zs_deflate_dict* d) { return d ? d->id : 1u; }
+
+void zs_deflate_dict_destroy(zs_deflate_dict* d) {
+    if (!d) return;
+    // called from garbage collectors at any time: the caller's current device is left as it was
+    int prev = -1;
+    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
+    cudaSetDevice(d->device);
+    cudaDeviceSynchronize();   // a call that uses the tables may still be queued on any stream of the device
+    cudaFree(d->d_img);
+    if (prev >= 0 && prev != d->device) cudaSetDevice(prev);
+    delete d;
+}
+
+// the arguments zlib refuses with a dictionary (deflateSetDictionary, deflate.ts:372) and those the batch form
+// has no meaning for: every chunk is one whole independent stream
+static int check_dict_call(zs_ctx* ctx, const zs_deflate_dict* dict, int wrap, uint32_t flags) {
+    if (!dict) return bad_arg(ctx, "deflate_batch_dict: no dictionary");
+    if (dict->device != ctx->device) return bad_arg(ctx, "deflate_batch_dict: dictionary prepared for another device");
+    if (wrap != ZS_WRAP_RAW && wrap != ZS_WRAP_ZLIB) return bad_arg(ctx, "deflate_batch_dict: gzip streams take no dictionary (deflate.ts:372)");
+    if (flags & ~(7u << 8)) return bad_arg(ctx, "deflate_batch_dict: flags carry the strategy only");
+    return ZS_OK;
+}
+
+int zs_deflate_batch_dict_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* d_in, uint64_t in_len,
+                              const uint64_t* d_in_off, uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk, int level,
+                              int wrap, uint32_t flags, uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off,
+                              uint64_t* d_out_bits, uint32_t* d_checks, zs_deflate_result* d_result) {
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    const int rc = check_dict_call(ctx, dict, wrap, flags);
+    if (rc != ZS_OK) return rc;
+    return deflate_batch_dev(ctx, dict, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, 0, level, wrap,
+                             ZS_MODE_INDEPENDENT, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result);
+}
+
 // Host-buffer deflate of a large batch, software-pipelined: the batch is cut into slices of whole waves of
 // LZ77 segments, and the H2D copy of slice s+1, the kernels of slice s and the D2H copy of slice s-1 run
 // concurrently on three streams.
@@ -359,10 +457,10 @@ int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, cons
 //  so slices concatenate byte-wise (5 bytes per slice more than the single-shot stream).  `history` bytes
 //  before `in` are readable and primed against; the trailer of a whole stream (deflate.ts:964-988) is
 //  written here from the combined checksums.
-static int deflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t history, uint32_t n_chunks,
-                                   uint32_t chunk_size, int level, int wrap, int mode, uint32_t flags, uint8_t* out,
-                                   uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits, uint32_t* checks,
-                                   zs_deflate_result* result) {
+static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len,
+                                   uint32_t history, uint32_t n_chunks, uint32_t chunk_size, int level, int wrap, int mode,
+                                   uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits,
+                                   uint32_t* checks, zs_deflate_result* result) {
     constexpr int kMaxSlices = 16;
     const bool stitched = mode == ZS_MODE_STITCHED;
     // Same LZ77 segmentation as the single-shot call over the whole batch; a slice is a whole number
@@ -411,7 +509,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, uint64_t in_l
     }
     zs_deflate_result* h_res = (zs_deflate_result*)ctx->h_pin;
     const uint64_t slice_bytes = (uint64_t)slice_chunks * chunk_size;
-    const uint64_t region = zs_deflate_batch_bound(slice_bytes, slice_chunks, chunk_size, wrap, mode);
+    const uint64_t region = zs_deflate_batch_bound(slice_bytes, slice_chunks, chunk_size, wrap, mode) + (dict ? 4ull * slice_chunks : 0);
     const uint64_t region_al = (region + 255) & ~255ull;
     if (!stitched) history = 0;
     if (history > 32768) history = 32768;
@@ -453,9 +551,9 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, uint64_t in_l
         } else if (flags & ZS_FLAG_PRIME) {
             hist = (uint32_t)(b0 < 32768 ? b0 : 32768);
         }
-        int rc = zs_deflate_batch_dev(ctx, d_in + b0, len, nullptr, nc, chunk_size, chunk_size, hist, level, wrap,
-                                      mode, sflags, d_out + region_al * s, region, d_ooff + c0 + s,
-                                      d_obits + c0, want_checks ? d_cks + c0 : nullptr, d_res + s);
+        int rc = deflate_batch_dev(ctx, dict, d_in + b0, len, nullptr, nc, chunk_size, chunk_size, hist, level, wrap,
+                                   mode, sflags, d_out + region_al * s, region, d_ooff + c0 + s,
+                                   d_obits + c0, want_checks ? d_cks + c0 : nullptr, d_res + s);
         if (rc != ZS_OK) return rc;
         ZS_CUDA_TRY(ctx, cudaEventRecord(ev_k[s], ctx->stream));
         // The 24-byte results come back on their own stream: the bulk D2H copies below are issued as
@@ -532,10 +630,10 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, uint64_t in_l
 }
 
 // Shared body of zs_deflate_batch / zs_deflate_part: `history` readable bytes lie before `in`.
-static int deflate_batch_host(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t history, const uint64_t* in_off,
-                              uint32_t n_chunks, uint32_t chunk_size, int level, int wrap, int mode, uint32_t flags,
-                              uint8_t* out, uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits, uint32_t* checks,
-                              zs_deflate_result* result) {
+static int deflate_batch_host(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len,
+                              uint32_t history, const uint64_t* in_off, uint32_t n_chunks, uint32_t chunk_size, int level,
+                              int wrap, int mode, uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off,
+                              uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result) {
     if (!out || !result || (in_len && !in) || n_chunks == 0) return bad_arg(ctx, "deflate: null buffer or zero chunks");
     if (history && !in) return bad_arg(ctx, "deflate: history without an input pointer");
     if (history > 32768) history = 32768;
@@ -552,8 +650,8 @@ static int deflate_batch_host(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, u
     }
     // Large batches with fixed chunking are software-pipelined (see deflate_batch_pipelined).
     if (!in_off && n_chunks >= 512 && chunk_size >= 4096 && !(mode == ZS_MODE_STITCHED && (flags & ZS_FLAG_PRIME)))
-        return deflate_batch_pipelined(ctx, in, in_len, history, n_chunks, chunk_size, level, wrap, mode, flags, out, out_cap,
-                                       out_off, out_bits, checks, result);
+        return deflate_batch_pipelined(ctx, dict, in, in_len, history, n_chunks, chunk_size, level, wrap, mode, flags, out,
+                                       out_cap, out_off, out_bits, checks, result);
     if (mode != ZS_MODE_STITCHED) history = 0;
     uint8_t* d_in_base = (uint8_t*)zs_scratch_get(ctx, SCR_H_IN, 32768 + in_len + 64);
     uint8_t* d_out = (uint8_t*)zs_scratch_get(ctx, SCR_H_OUT, out_cap + 64);
@@ -568,8 +666,8 @@ static int deflate_batch_host(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, u
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in - history, in - history, in_len + history, cudaMemcpyHostToDevice, ctx->stream));
     if (in_off)
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_off, in_off, (size_t)(n_chunks + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = zs_deflate_batch_dev(ctx, d_in, in_len, in_off ? d_off : nullptr, n_chunks, chunk_size, max_chunk, history, level,
-                                  wrap, mode, flags, d_out, out_cap, d_ooff, d_ooff + n_chunks + 1, d_checks, d_result);
+    int rc = deflate_batch_dev(ctx, dict, d_in, in_len, in_off ? d_off : nullptr, n_chunks, chunk_size, max_chunk, history,
+                               level, wrap, mode, flags, d_out, out_cap, d_ooff, d_ooff + n_chunks + 1, d_checks, d_result);
     if (rc != ZS_OK) return rc;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(result, d_result, sizeof(zs_deflate_result), cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -594,8 +692,20 @@ int zs_deflate_batch(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, const uint
                      uint64_t* out_off, uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result) {
     if (ctx) bind_device(ctx);
     if (!ctx) return ZS_STREAM_ERROR;
-    return deflate_batch_host(ctx, in, in_len, 0, in_off, n_chunks, chunk_size, level, wrap, mode, flags, out, out_cap,
+    return deflate_batch_host(ctx, nullptr, in, in_len, 0, in_off, n_chunks, chunk_size, level, wrap, mode, flags, out, out_cap,
                               out_off, out_bits, checks, result);
+}
+
+int zs_deflate_batch_dict(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len, const uint64_t* in_off,
+                          uint32_t n_chunks, uint32_t chunk_size, int level, int wrap, uint32_t flags, uint8_t* out,
+                          uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result) {
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    const int rc = check_dict_call(ctx, dict, wrap, flags);
+    if (rc != ZS_OK) return rc;
+    // every chunk is its own segment in a dictionary call, so slicing a large batch cannot change the output
+    return deflate_batch_host(ctx, dict, in, in_len, 0, in_off, n_chunks, chunk_size, level, wrap, ZS_MODE_INDEPENDENT, flags,
+                              out, out_cap, out_off, out_bits, checks, result);
 }
 
 int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t history, uint32_t chunk_size, int level,
@@ -606,8 +716,8 @@ int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t hi
     if (flags & ZS_FLAG_PRIME) return bad_arg(ctx, "deflate: ZS_FLAG_PRIME does not apply to a part of a stream");
     const uint64_t nc = in_len ? (in_len + chunk_size - 1) / chunk_size : 1;
     if (nc > 0xffffffffull) return bad_arg(ctx, "deflate: too many chunks");
-    return deflate_batch_host(ctx, in, in_len, history, nullptr, (uint32_t)nc, chunk_size, level, wrap, ZS_MODE_STITCHED, flags,
-                              out, out_cap, nullptr, out_bits, nullptr, result);
+    return deflate_batch_host(ctx, nullptr, in, in_len, history, nullptr, (uint32_t)nc, chunk_size, level, wrap, ZS_MODE_STITCHED,
+                              flags, out, out_cap, nullptr, out_bits, nullptr, result);
 }
 
 int zs_bit_concat_dev(zs_ctx* ctx, uint8_t* d_dst, uint64_t dst_bit_off, const uint8_t* d_src, uint64_t n_bits) {
@@ -638,8 +748,8 @@ int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_
     }
     if (window_bits && (window_bits < 8 || window_bits > (d64 ? 16 : 15))) return bad_arg(ctx, "inflate: windowBits out of range");
 
-    // misc scratch: detail[n] trailer[2n] flags[n] adler[n] crc[n]
-    uint32_t* misc = (uint32_t*)zs_scratch_get(ctx, SCR_I_MISC, (size_t)n * 6 * 4);
+    // misc scratch: detail[n] trailer[2n] flags[n] adler[n] crc[n] dict_adler[n] | dict off[n] len[n] (u64)
+    uint32_t* misc = (uint32_t*)zs_scratch_get(ctx, SCR_I_MISC, (size_t)n * 7 * 4 + 16 + (size_t)n * 16);
     if (!misc) return ZS_MEM_ERROR;
     zs_inflate_args a;
     a.d_in = d_in; a.d_in_off = d_in_off; a.n = n; a.wrap = wrap; a.deflate64 = d64;
@@ -649,6 +759,16 @@ int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_
     a.d_trailer = misc + n;
     a.d_flags = misc + 3 * (size_t)n;
     a.d_dict = d_dict; a.d_dict_rng = d_dict_rng;
+    a.d_dict_adler = nullptr;
+    if ((wrap & 1) && d_dict && d_dict_rng) {
+        // zlib streams with FDICT are decoded when their DICTID is the adler32 of the dictionary they were given
+        uint32_t* d_da = misc + 6 * (size_t)n;
+        uint64_t* d_doff = (uint64_t*)(((uintptr_t)(misc + 7 * (size_t)n) + 15) & ~(uintptr_t)15);
+        ZS_KERNEL(ctx, "dict_ranges_kernel", dict_ranges_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(d_dict_rng, d_doff, d_doff + n, n));
+        const int rc0 = zs_launch_checksum_segments(ctx, 0, d_dict, d_doff, d_doff + n, n, d_da);
+        if (rc0 != ZS_OK) return rc0;
+        a.d_dict_adler = d_da;
+    }
     a.d_start_bit = nullptr; a.d_block_mark = nullptr;
     if (ctx->inflate_resume && n == 1) {
         // one stream of the streaming shim: [0] start bit (in), [1..2] block mark (out)

@@ -139,6 +139,15 @@ __device__ __forceinline__ unsigned zs_dist_base(unsigned code) {  // base of (d
 
 #endif  // __CUDACC__
 
+// A prepared preset dictionary (zs_deflate_dict_create): the match finder's tables built from the last
+// <= 32 KiB of the caller's dictionary, with those bytes in their ring (layout private to zs_lz77.cu).
+struct zs_deflate_dict {
+    int device;
+    uint32_t len;        // bytes used: the last min(dict_len, 32768)
+    uint32_t id;         // adler32 of the whole dictionary (DICTID)
+    uint8_t* d_img;      // saved tables
+};
+
 // ---- kernel entry points (host wrappers, one per .cu) ---------------------------------------------
 // checksum
 int zs_launch_checksum_segments(zs_ctx* ctx, int kind, const uint8_t* d_buf, const uint64_t* d_off,
@@ -169,6 +178,7 @@ struct zs_inflate_args {
     uint32_t* d_flags;    // [n]: 1 = has zlib trailer (adler), 2 = has gzip trailer (crc)
     const uint8_t* d_dict;
     const uint64_t* d_dict_rng;
+    const uint32_t* d_dict_adler;   // [n]: adler32 of each stream's dictionary range (zlib streams with FDICT), or nullptr
     int force_tps;        // tests: 1 = thread-per-stream kernel for any batch of >= 32 streams, -1 = never
     // streaming shim (warp kernel only): decode raw blocks from this bit of each stream instead of
     // from its start, and report where the last block that was begun starts: [2n] = (bit offset in the
@@ -222,7 +232,12 @@ struct zs_deflate_plan {
     uint32_t* d_check_total;  // 1
     zs_deflate_result* d_result;
     int32_t* d_error;         // device flag: ZS_BUF_ERROR if out_cap too small
+    const zs_deflate_dict* dict;   // zs_deflate_batch_dict*: every chunk starts from this dictionary, or nullptr
 };
 int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p);
+// Runs d_dict[0, len) (len <= 32768, 16-byte aligned, readable to len rounded up to 16) through the match
+// finder's insert stages alone and writes the saved tables to d_img (zs_lz77_dict_image_bytes()).
+int zs_lz77_dict_build(zs_ctx* ctx, const uint8_t* d_dict, uint32_t len, uint8_t* d_img);
+size_t zs_lz77_dict_image_bytes();
 int zs_launch_huffman(zs_ctx* ctx, const zs_deflate_plan& p);
 int zs_launch_bit_concat(zs_ctx* ctx, uint8_t* d_dst, uint64_t dst_bit_off, const uint8_t* d_src, uint64_t n_bits);

@@ -675,7 +675,13 @@ struct LayoutArgs {
     zs_deflate_result* result;
     int32_t* error;
     const uint32_t* check_total;
+    int fdict;            // zlib wrapper with a preset dictionary: FDICT + DICTID, a 6-byte header
 };
+
+// bytes of the wrapper header in front of every stream (INDEPENDENT) or of the stream (STITCHED)
+__device__ __forceinline__ uint64_t wrap_header_bytes(int wrap, int fdict) {
+    return wrap == ZS_WRAP_ZLIB ? (fdict ? 6 : 2) : wrap == ZS_WRAP_GZIP ? 10 : 0;
+}
 
 __device__ __forceinline__ unsigned stored_pad(uint64_t bitpos_after_hdr) { return (unsigned)((8u - (bitpos_after_hdr & 7u)) & 7u); }
 
@@ -730,7 +736,7 @@ __global__ void __launch_bounds__(kScanThreads) layout_scan_kernel(LayoutArgs a)
     __shared__ uint64_t s_len[32];
     __shared__ uint64_t s_tile_len;
     const unsigned lane = zs_lane(), wid = threadIdx.x >> 5;
-    const uint64_t H = a.wrap == ZS_WRAP_ZLIB ? 2 : a.wrap == ZS_WRAP_GZIP ? 10 : 0;
+    const uint64_t H = wrap_header_bytes(a.wrap, a.fdict);
     const uint64_t T = a.wrap == ZS_WRAP_ZLIB ? 4 : a.wrap == ZS_WRAP_GZIP ? 8 : 0;
     const bool stitched = a.mode == ZS_MODE_STITCHED;
     uint64_t pos = 0;  // INDEPENDENT: bytes; STITCHED: bits
@@ -818,7 +824,7 @@ __global__ void layout_blocks_kernel(LayoutArgs a) {
     if (c >= a.n_chunks) return;
     const uint32_t nb = a.chunk_nblk[c];
     const bool stitched = a.mode == ZS_MODE_STITCHED;
-    const uint64_t H = a.wrap == ZS_WRAP_ZLIB ? 2 : a.wrap == ZS_WRAP_GZIP ? 10 : 0;
+    const uint64_t H = wrap_header_bytes(a.wrap, a.fdict);
     uint64_t pos = stitched ? a.out_off[c] : 8 * (a.out_off[c] + H);
     const bool chunk_final = stitched ? (c + 1 == a.n_chunks && !(a.flags & ZS_FLAG_NOT_LAST)) : true;
     for (uint32_t j = 0; j < nb; j++) {
@@ -853,6 +859,8 @@ struct EncodeArgs {
     const zs_deflate_result* result;
     const int32_t* error;
     int level;
+    int fdict;            // see LayoutArgs
+    uint32_t dict_id;     // DICTID: adler32 of the whole preset dictionary
 };
 
 __device__ __forceinline__ void or_bits_global(uint32_t* out32, uint64_t bitpos, uint64_t v, unsigned n) {
@@ -1039,8 +1047,13 @@ __global__ void frame_kernel(EncodeArgs a) {
             const int strategy = (int)((a.flags >> 8) & 7u);
             unsigned lf = (strategy >= ZS_STRATEGY_HUFFMAN_ONLY || a.level < 2) ? 0u : a.level < 6 ? 1u : a.level == 6 ? 2u : 3u;
             header |= lf << 6;
+            if (a.fdict) header |= 0x20u;   // PRESET_DICT: deflate() sets it when a dictionary was given (strstart != 0)
             header += 31u - header % 31u;
             hp[0] = (uint8_t)(header >> 8); hp[1] = (uint8_t)header;
+            if (a.fdict) {   // DICTID, big-endian (putShortMSB twice)
+                hp[2] = (uint8_t)(a.dict_id >> 24); hp[3] = (uint8_t)(a.dict_id >> 16);
+                hp[4] = (uint8_t)(a.dict_id >> 8); hp[5] = (uint8_t)a.dict_id;
+            }
         } else if (a.wrap == ZS_WRAP_GZIP) {
             hp[0] = 0x1f; hp[1] = 0x8b; hp[2] = 8;
             for (int k = 3; k < 8; k++) hp[k] = 0;
@@ -1059,7 +1072,7 @@ __global__ void frame_kernel(EncodeArgs a) {
             ck = *a.check_total;
             isize = a.in_off[a.n_chunks];
         } else {
-            const uint64_t H = a.wrap == ZS_WRAP_ZLIB ? 2 : 10;
+            const uint64_t H = wrap_header_bytes(a.wrap, a.fdict);
             tp = a.out + a.out_off[c] + H + ((a.out_bits[c] + 7) >> 3);
             ck = a.checks[c];
             isize = a.in_off[c + 1] - a.in_off[c];
@@ -1150,6 +1163,7 @@ int zs_launch_huffman(zs_ctx* ctx, const zs_deflate_plan& p) {
     l.in_off = p.d_in_off; l.chunk_nblk = p.d_chunk_nblk; l.blk_hdr = p.d_blk_hdr; l.blk_bits = p.d_blk_bits;
     l.chunk_pr = p.d_chunk_pr; l.out_off = p.d_out_off; l.out_bits = p.d_out_bits; l.out_cap = p.out_cap;
     l.result = p.d_result; l.error = p.d_error; l.check_total = p.d_check_total;
+    l.fdict = p.dict != nullptr && p.dict->len > 0;
     const unsigned cgrid = (p.n_chunks + 127) / 128;
     ZS_KERNEL(ctx, "layout_chunks_kernel", layout_chunks_kernel<<<cgrid, 128, 0, ctx->stream>>>(l));
     ZS_KERNEL(ctx, "layout_scan_kernel", layout_scan_kernel<<<1, kScanThreads, 0, ctx->stream>>>(l));
@@ -1163,6 +1177,7 @@ int zs_launch_huffman(zs_ctx* ctx, const zs_deflate_plan& p) {
     e.blk_code = p.d_blk_code; e.blk_hdr = p.d_blk_hdr; e.blk_abs = p.d_blk_bits; e.out_off = p.d_out_off;
     e.out_bits = p.d_out_bits; e.checks = p.d_checks; e.check_total = p.d_check_total; e.out = p.d_out;
     e.result = p.d_result; e.error = p.d_error; e.level = p.level;
+    e.fdict = l.fdict; e.dict_id = p.dict ? p.dict->id : 0u;
     ZS_KERNEL(ctx, "encode_kernel", encode_kernel<<<(unsigned)nblk_slots, kEncThreads, 0, ctx->stream>>>(e));
     ZS_KERNEL(ctx, "frame_kernel", frame_kernel<<<cgrid, 128, 0, ctx->stream>>>(e));
     ZS_KERNEL(ctx, "count_blocks_kernel", count_blocks_kernel<<<1, 256, 0, ctx->stream>>>(p.d_chunk_nblk, p.n_chunks, p.d_result, p.d_check_total));

@@ -74,7 +74,8 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(zs_inflate_args a)
                 else br.drop((unsigned)(sb & 7u));
             }
         }
-        if (a.wrap && !skip_header) read_wrapper_header(br, a.wrap, status, detail, tflags);
+        if (a.wrap && !skip_header)
+            read_wrapper_header(br, a.wrap, status, detail, tflags, a.d_dict_adler && dict_len ? a.d_dict_adler + sidx : nullptr);
 
         if (a.d_hdr_state) {
             // header only: where the blocks start, for the segment-parallel decoder

@@ -302,9 +302,11 @@ __device__ __forceinline__ uint32_t crc_bitwise(uint32_t crc, unsigned byte) {
 }
 
 // Wrapper header: HEAD..HCRC / DICTID of inflate() (inflate.ts:377-593).  wrap: bit 0 zlib, bit 1 gzip.
-// A bad or truncated header sets status (and detail); FDICT sets ZS_NEED_DICT.  tflags: 1 zlib trailer,
-// 2 gzip trailer.
-__device__ __forceinline__ void read_wrapper_header(BitReader& br, int wrap, int& status, int& detail, unsigned& tflags) {
+// A bad or truncated header sets status (and detail).  FDICT: decoding goes on when the stream's dictionary
+// was given (a non-empty range: no deflater sets FDICT for an empty one) and its adler32 (*dict_adler) equals DICTID -- inflateSetDictionary after Z_NEED_DICT,
+// inflate.ts:1220-1249 -- and stops with ZS_NEED_DICT otherwise.  tflags: 1 zlib trailer, 2 gzip trailer.
+__device__ __forceinline__ void read_wrapper_header(BitReader& br, int wrap, int& status, int& detail, unsigned& tflags,
+                                                    const uint32_t* dict_adler) {
     if (!br.need(16)) {
         status = ZS_BUF_ERROR;
     } else {
@@ -362,9 +364,13 @@ __device__ __forceinline__ void read_wrapper_header(BitReader& br, int wrap, int
         } else {
             br.drop(16);
             tflags = 1;
-            if (h & 0x2000) {  // FDICT: DICTID follows; preset dictionaries for zlib streams
-                if (!br.need(32)) status = ZS_BUF_ERROR;  // are host-side framing (INTEGRATION.md)
-                else { br.drop(32); status = ZS_NEED_DICT; }
+            if (h & 0x2000) {  // FDICT: DICTID follows (big-endian)
+                if (!br.need(32)) status = ZS_BUF_ERROR;
+                else {
+                    const uint32_t id = __byte_perm((uint32_t)br.hold, 0, 0x0123);
+                    br.drop(32);
+                    if (!dict_adler || *dict_adler != id) status = ZS_NEED_DICT;
+                }
             }
         }
     }

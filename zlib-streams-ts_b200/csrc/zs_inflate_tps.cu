@@ -200,7 +200,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
         unsigned tflags = 0;
         uint32_t t_check = 0, t_isize = 0;
 
-        if (a.wrap) read_wrapper_header(br, a.wrap, status, detail, tflags);
+        if (a.wrap) read_wrapper_header(br, a.wrap, status, detail, tflags, a.d_dict_adler && dict_len ? a.d_dict_adler + sidx : nullptr);
 
         // ---- blocks ----
         bool last = false;

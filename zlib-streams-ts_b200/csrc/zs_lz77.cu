@@ -52,6 +52,7 @@
 //     does not depend on scheduling (tables are reset per segment).
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 
 #include "zs_common.cuh"
 
@@ -131,7 +132,23 @@ struct LzArgs {
     uint32_t* blk_desc;
     uint32_t* seg_counter;
     unsigned stop_after, stop_active;   // lazy levels: straggler stop of the chain walk (search_lazy_endwin)
+    // lz77_dict_kernel only (every segment is one chunk, see DictImage): the prepared dictionary's saved
+    // tables (nullptr: build them -- the call's one chunk is the dictionary), where a build writes them,
+    // and the dictionary's length (<= 32 KiB)
+    const uint8_t* dict_img;
+    uint8_t* dict_save;
+    uint32_t dict_len;
 };
+
+// The tables of a prepared dictionary (zs_deflate_dict), as lz77_dict_kernel leaves them after running the
+// dictionary alone through prep / insert / link with range offset q = ring index (the dictionary's first
+// byte at q = 0): head[] and prev[] as they lie in shared memory, then ring[0, 32 KiB) and its guard mirror.
+// Every position whose three hash bytes lie inside the dictionary is inserted; the last two are not (their
+// hash needs the chunk's first two bytes: deflateSetDictionary leaves s->insert = 2, deflate.ts:367-424).
+constexpr unsigned kImgTables = (1u << kHashBits) * 2u + 32768u * 2u;   // head[] + prev[]
+constexpr unsigned kImgRing = kImgTables;                               // ring[0, 32768)
+constexpr unsigned kImgGuard = kImgRing + 32768u;                       // ring[kRing, kRing + kRingGuard)
+constexpr unsigned kImgBytes = kImgGuard + kRingGuard;
 
 #ifdef ZS_LZ_PROF
 // cycle counters: [0] thin insert, [1] thin parse, [2] wide warps (summed), [3] whole step incl.
@@ -169,6 +186,24 @@ __device__ __forceinline__ void stage_window(Smem& S, const LzArgs& a, uint64_t 
         *reinterpret_cast<uint4*>(S.ring + idx) = v;
         if (idx < kRingGuard) *reinterpret_cast<uint4*>(S.ring + kRing + idx) = v;
     }
+}
+
+// Dictionary kernel: the 16 bytes of range offsets [ql, ql + 16) that come from the input, byte q at absolute
+// index g0 + q (g0 = the chunk's first absolute index - its range offset, negative for a chunk near the start
+// of the buffer).  The chunk starts at any byte, so the ring line is assembled from five aligned words;
+// words before index 0 or at / past safe16 (the input's end rounded up to 16) read as zeros.
+__device__ __forceinline__ uint4 dict_src_line(const LzArgs& a, int64_t g0, int64_t safe16, uint32_t ql) {
+    const int64_t g = g0 + (int64_t)ql;
+    const int64_t al = g - (g & 3);
+    const unsigned sh = (unsigned)(g & 3) * 8u;
+    uint32_t w[5];
+#pragma unroll
+    for (int k = 0; k < 5; ++k) {
+        const int64_t at = al + 4 * k;
+        w[k] = (at >= 0 && at < safe16) ? __ldg(reinterpret_cast<const uint32_t*>(a.buf + at)) : 0u;
+    }
+    return make_uint4(__funnelshift_r(w[0], w[1], sh), __funnelshift_r(w[1], w[2], sh), __funnelshift_r(w[2], w[3], sh),
+                      __funnelshift_r(w[3], w[4], sh));
 }
 
 // ---- bulk-async staging (Blackwell: the copy engine moves the window, no thread does) ------------
@@ -247,15 +282,18 @@ struct RangeCtx {
     uint32_t nc;     // chunks in the segment
     int cross;       // matches may reach before the chunk start
     unsigned min_len;  // shortest match worth emitting: 3, or 6 with Z_FILTERED at the lazy levels (deflate.ts:1381-1387)
+    uint32_t ins_lo;   // dictionary kernel: first position prep inserts
 };
 
 // ---- stage 1: prep (wide) -----------------------------------------------------------------------
 // 32 consecutive positions starting at offset q0; positions >= limit (end of the step being inserted)
 // or without three readable bytes are not inserted.
+template <bool kDict = false>
 __device__ __forceinline__ uint32_t prep_batch(const Smem& S, const RangeCtx& c, uint32_t q0, uint32_t limit) {
     const unsigned lane = zs_lane();
     const uint32_t q = q0 + lane;
-    const bool valid = q < limit && q + 2 < c.tail;
+    // (dictionary kernel: the positions below ins_lo are in the restored tables already)
+    const bool valid = q < limit && q + 2 < c.tail && (!kDict || q >= c.ins_lo);
     unsigned h = 0;
     if (valid) h = hash3(win32(S, c.cb + q));
     // lanes with the same hash: kHashBits independent ballots (measured faster than one MATCH.ANY,
@@ -836,8 +874,17 @@ __device__ __forceinline__ uint32_t resolved_frontier(uint32_t searched, uint32_
 
 // kMode 1: levels 4-9 (deflate_slow's rules); 0: levels 1-3, greedy; 2: Z_RLE, greedy with distance 1 only.
 // kLevel (greedy levels): 0 = the level's parameters come from a.cfg, 1-3 = that level's row at compile time.
-template <int kMode, int kLevel>
-__global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
+// kDict: lz77_dict_kernel -- every segment is one chunk whose range starts with the prepared dictionary.
+// The range offset q is the ring index itself (cb = 0): the dictionary's last <= 32 KiB at q = [0, L), the
+// chunk at q = [L, L + len).  At segment start the CTA restores the saved tables and the dictionary's ring
+// bytes (DictImage) instead of zeroing head[] / prev[], inserts from L - 2 on (the two positions the build
+// deferred) and searches from L on, with the 32-position batches on the grid of the PRIME path for a range that
+// starts at the dictionary.  The chunk is staged from global memory with plain loads (it starts at any byte,
+// so the ring and the input are not congruent modulo 16 as the bulk copies need).  The output equals that of
+// the PRIME path on a buffer holding the dictionary followed by the chunk.  With dict_img == nullptr the call
+// builds the image instead: its one chunk is the dictionary, inserted and nothing searched.
+template <int kMode, int kLevel, bool kDict>
+__device__ __forceinline__ void lz77_run(const LzArgs& a) {
     static_assert(kLevel == 0 || (kMode == 0 && kLevel <= 3), "only the greedy levels are specialised");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& S = *reinterpret_cast<Smem*>(smem_raw);
@@ -851,7 +898,7 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
     (void)stop;
 
 #ifdef ZS_LZ_BULK
-    if (threadIdx.x == 0) mbar_init(&S.stage_bar, 1);   // published by the first __syncthreads of the segment loop
+    if (!kDict && threadIdx.x == 0) mbar_init(&S.stage_bar, 1);   // published by the first __syncthreads of the segment loop
 #endif
 #ifdef ZS_LZ_PROF
     // slowest wide warp of step k: prof_wmax[k & 1], reset by thread 0 behind the barrier of step k (no
@@ -873,7 +920,16 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
 
         // fresh tables per segment: the output never depends on which CTA ran which segment
         if (threadIdx.x == 0) S.claim[0] = 0;
-        {
+        if (kDict && a.dict_img) {
+            // the dictionary's tables and ring bytes, from L2 (one image for every chunk of the call)
+            const uint4* src = reinterpret_cast<const uint4*>(a.dict_img);
+            uint4* ht = reinterpret_cast<uint4*>(S.head);   // prev[] follows head[], as in the image
+            for (unsigned i = threadIdx.x; i < kImgTables / 16u; i += kThreads) ht[i] = __ldg(src + i);
+            const unsigned nring = (a.dict_len + 15u) / 16u;
+            for (unsigned i = threadIdx.x; i < nring; i += kThreads) reinterpret_cast<uint4*>(S.ring)[i] = __ldg(src + kImgRing / 16u + i);
+            for (unsigned i = threadIdx.x; i < kRingGuard / 16u; i += kThreads)
+                reinterpret_cast<uint4*>(S.ring + kRing)[i] = __ldg(src + kImgGuard / 16u + i);
+        } else {
             uint4* z = reinterpret_cast<uint4*>(S.head);
             const unsigned nz = (sizeof(S.head) + sizeof(S.prev)) / sizeof(uint4);
 #ifdef ZS_LZ_PREV_DELTA
@@ -892,7 +948,9 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
         const uint64_t seg_start = a.org + off0;
         const uint64_t seg_end = a.org + a.in_off[c1];
         uint64_t prime0 = seg_start;
-        if (a.cross) {
+        if (kDict) {
+            prime0 = 0;   // unused: the range offset is the ring index
+        } else if (a.cross) {
             prime0 = seg_start > a.valid_lo + 32768 ? seg_start - 32768 : a.valid_lo;
             prime0 = (prime0 + 31) & ~31ull;
             if (prime0 > seg_start) prime0 = seg_start;
@@ -904,13 +962,25 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
         rc.nc = nc;
         rc.cross = a.cross;
         rc.min_len = (kMode == 1 && a.strategy == ZS_STRATEGY_FILTERED) ? 6u : 3u;
-        {
+        uint32_t q_src = 0, q_start = 0;   // dictionary kernel: range offset of the chunk's first byte, first step
+        if constexpr (kDict) {
+            // build: the chunk is the dictionary (q = [0, L), nothing compressed); use: it follows the dictionary
+            const uint32_t L = a.dict_len;
+            q_src = a.dict_img ? L : 0u;
+            rc.q_data = L;
+            rc.n = q_src + (uint32_t)(seg_end - seg_start);
+            rc.pre = 0;
+            rc.tail = rc.n;   // as on the PRIME path with the chunk alone in the call: its last two positions are not inserted
+            rc.ins_lo = a.dict_img ? (L >= 2u ? L - 2u : 0u) : 0u;
+            q_start = rc.ins_lo & ~63u;   // a whole aligned pair of batches: the PRIME path's grid
+            if (threadIdx.x < 2) S.bnd[threadIdx.x] = threadIdx.x ? rc.n : rc.q_data;
+        } else {
             const uint64_t pre = a.cross ? prime0 - a.valid_lo : 0;
             rc.pre = pre < kMaxDist ? (uint32_t)pre : kMaxDist;
             const uint64_t tail = a.data_end - prime0;
             rc.tail = tail < 0xffffffffull ? (uint32_t)tail : 0xffffffffu;
+            for (unsigned j = threadIdx.x; j <= nc; j += kThreads) S.bnd[j] = (uint32_t)(a.in_off[c0 + j] - off0) + rc.q_data;
         }
-        for (unsigned j = threadIdx.x; j <= nc; j += kThreads) S.bnd[j] = (uint32_t)(a.in_off[c0 + j] - off0) + rc.q_data;
         // Staging addresses positions relative to base16 (the 16-byte line that holds the range's first byte):
         // after iteration k the ring holds everything below stage_rel(k + 1) = q_prep + 3 steps + guard, rounded up.
         const uint64_t base16 = prime0 & ~15ull;
@@ -920,11 +990,31 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
             return d < 0xfffffff0ull ? (uint32_t)d : 0xfffffff0u;
         }();
         // look-ahead for the first two steps of the range
-        stage_window(S, a, base16, base16 + ((p0lo + 2u * kStep + kRingGuard + 15u) & ~15u), threadIdx.x, kThreads);
+        const int64_t g0 = (int64_t)seg_start - (int64_t)q_src;   // dictionary kernel: absolute index of range offset 0
+        const int64_t dsafe16 = (int64_t)((a.data_end + 15) & ~15ull);
+        if constexpr (kDict) {
+            __syncthreads();   // the restored ring line that holds q_src is merged below
+            const uint32_t to = (q_start + 2u * kStep + kRingGuard + 15u) & ~15u;
+            for (uint32_t ql = (q_src & ~15u) + 16u * threadIdx.x; ql < to; ql += 16u * kThreads) {
+                uint4 v = dict_src_line(a, g0, dsafe16, ql);
+                const unsigned idx = ql & (kRing - 1u);
+                if (ql < q_src) {   // the dictionary's last bytes share this line with the chunk's first ones
+                    const uint4 d = *reinterpret_cast<const uint4*>(S.ring + idx);
+                    const unsigned keep = q_src - ql;   // 1..15 bytes from the dictionary
+                    auto m = [&](unsigned w) { return keep >= 4u * w + 4u ? 0xffffffffu : keep <= 4u * w ? 0u : (1u << (8u * (keep - 4u * w))) - 1u; };
+                    v.x = (d.x & m(0)) | (v.x & ~m(0)); v.y = (d.y & m(1)) | (v.y & ~m(1));
+                    v.z = (d.z & m(2)) | (v.z & ~m(2)); v.w = (d.w & m(3)) | (v.w & ~m(3));
+                }
+                *reinterpret_cast<uint4*>(S.ring + idx) = v;
+                if (idx < kRingGuard) *reinterpret_cast<uint4*>(S.ring + kRing + idx) = v;
+            }
+        } else {
+            stage_window(S, a, base16, base16 + ((p0lo + 2u * kStep + kRingGuard + 15u) & ~15u), threadIdx.x, kThreads);
+        }
         __syncthreads();
 
         const uint32_t n = rc.n;
-        const uint32_t nsteps = (n + kStep - 1) / kStep;
+        const uint32_t nsteps = (n - q_start + kStep - 1) / kStep;
         const uint32_t n_iter = nsteps + 6;
         // The staging barrier completes one phase per step; a segment uses an even number of them (one empty phase
         // more after an odd number of steps), so the parity to wait for is k & 1 in every segment.  (Re-initialising
@@ -941,9 +1031,9 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
         unsigned js = 0;
         uint32_t cs_w = rc.q_data, ce_w = S.bnd[1];
         // per-iteration uniform state, kept incrementally (no multiplies / 64-bit math in the loop)
-        uint32_t q_prep = 0;                 // first position of the step being prepped (k * kStep)
+        uint32_t q_prep = q_start;           // first position of the step being prepped (q_start + k * kStep)
         unsigned s_prep = 0;                 // prep[] buffer of step k (k % 3)
-        uint32_t searched = 0;               // positions searched before this iteration
+        uint32_t searched = q_start;         // positions searched before this iteration
         uint32_t r0 = qd64, r1 = qd64, r2 = qd64, r3 = qd64;   // resolved frontier after iteration k, k-1, k-2, k-3
 
         for (uint32_t k = 0; k < n_iter; ++k) {
@@ -955,7 +1045,34 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
             if (r0 < qd64) r0 = qd64;
             const unsigned s_ins = s_prep == 0 ? 2u : s_prep - 1u;     // (k - 1) % 3
             const unsigned s_link = s_ins == 0 ? 2u : s_ins - 1u;      // (k - 2) % 3
-            if (wid == kWarpInsert) {
+            if (kDict && wid == kWarpInsert) {
+                // the same look-ahead as below, from the chunk through registers (range offset = ring index)
+                const uint32_t stage_from = (q_prep + 2u * kStep + kRingGuard + 15u) & ~15u;
+                const uint32_t stage_to = k < nsteps ? (q_prep + 3u * kStep + kRingGuard + 15u) & ~15u : stage_from;
+                constexpr int kStageVec = (kStep + 16 + 511) / 512;   // 16-byte vectors per lane and step (covers a step)
+                uint4 sv[kStageVec];
+#pragma unroll
+                for (int v = 0; v < kStageVec; ++v) {
+                    const uint32_t pos = stage_from + 16u * (lane + 32 * v);
+                    sv[v] = pos < stage_to ? dict_src_line(a, g0, dsafe16, pos) : make_uint4(0, 0, 0, 0);
+                }
+                if (k >= 1 && k - 1 < nsteps) {
+                    const uint32_t p = q_prep - kStep + lane;
+                    const uint32_t* pw = S.prep + s_ins * kStep + lane;
+                    uint16_t* oh = S.oldh + ((k - 1) & 1u) * kStep;
+#pragma unroll
+                    for (int u = 0; u < kSearchWarps; ++u) head_exchange(S, p + 32u * u, pw[32 * u], oh + 32 * u);
+                }
+#pragma unroll
+                for (int v = 0; v < kStageVec; ++v) {
+                    const uint32_t pos = stage_from + 16u * (lane + 32 * v);
+                    if (pos < stage_to) {
+                        const unsigned idx = pos & (kRing - 1u);
+                        *reinterpret_cast<uint4*>(S.ring + idx) = sv[v];
+                        if (idx < kRingGuard) *reinterpret_cast<uint4*>(S.ring + kRing + idx) = sv[v];
+                    }
+                }
+            } else if (wid == kWarpInsert) {
                 // Bytes the next iteration reads (prep of step k+1, look-ahead of the search of step
                 // k-2) replace positions 64 KiB older, which nobody reads any more.
                 const uint32_t stage_from = (p0lo + q_prep + 2u * kStep + kRingGuard + 15u) & ~15u;
@@ -1051,7 +1168,7 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
                 // prep of step k
                 if (k < nsteps) {
                     const uint32_t se = q_prep + kStep < n ? q_prep + kStep : n;
-                    S.prep[s_prep * kStep + i] = prep_batch(S, rc, q_prep + 32u * wid, se);
+                    S.prep[s_prep * kStep + i] = prep_batch<kDict>(S, rc, q_prep + 32u * wid, se);
                 }
                 // link of step k-2 (its head exchange ran in the previous iteration)
                 if (k >= 2 && k - 2 < nsteps)
@@ -1154,8 +1271,21 @@ __global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) {
         if (wid == kWarpParse)
             while (ps.jc < nc) close_chunk(S, a, rc, ps, c0);   // chunks that end with the range (and empty ones after it)
         __syncthreads();
+        if (kDict && a.dict_save) {   // build: the tables as the chunks of later calls start from them (DictImage)
+            uint4* dst = reinterpret_cast<uint4*>(a.dict_save);
+            const uint4* ht = reinterpret_cast<const uint4*>(S.head);
+            for (unsigned i = threadIdx.x; i < kImgTables / 16u; i += kThreads) dst[i] = ht[i];
+            for (unsigned i = threadIdx.x; i < 32768u / 16u; i += kThreads) dst[kImgRing / 16u + i] = reinterpret_cast<const uint4*>(S.ring)[i];
+            for (unsigned i = threadIdx.x; i < kRingGuard / 16u; i += kThreads)
+                dst[kImgGuard / 16u + i] = reinterpret_cast<const uint4*>(S.ring + kRing)[i];
+        }
     }
 }
+
+template <int kMode, int kLevel>
+__global__ void __launch_bounds__(kThreads, 1) lz77_kernel(LzArgs a) { lz77_run<kMode, kLevel, false>(a); }
+template <int kMode, int kLevel>
+__global__ void __launch_bounds__(kThreads, 1) lz77_dict_kernel(LzArgs a) { lz77_run<kMode, kLevel, true>(a); }
 
 // Level 0 (deflate_stored, deflate.ts:1140-1279) and Z_HUFFMAN_ONLY (deflate_huff, :1525-1560) need no
 // match finder: the blocks of a chunk are cut at fixed input lengths -- 65535 bytes per stored block,
@@ -1190,10 +1320,15 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     // lz77_kernel<0, 0> is the greedy levels with their parameters read at run time, <0, L> level L specialised
     using LzKernel = void (*)(LzArgs);
     static const LzKernel kGreedy[4] = {lz77_kernel<0, 0>, lz77_kernel<0, 1>, lz77_kernel<0, 2>, lz77_kernel<0, 3>};
+    static const LzKernel kGreedyDict[4] = {lz77_dict_kernel<0, 0>, lz77_dict_kernel<0, 1>, lz77_dict_kernel<0, 2>,
+                                            lz77_dict_kernel<0, 3>};
     if (!attr_set[dev_slot] || ctx->device >= 64) {
         for (LzKernel k : kGreedy)
             ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+        for (LzKernel k : kGreedyDict)
+            ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
         ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+        ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_dict_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
         ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
         attr_set[dev_slot] = true;
     }
@@ -1210,6 +1345,17 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     a.cfg = kLevels[p.level];
     a.strategy = p.strategy;
     a.cross = (p.mode == ZS_MODE_STITCHED || (p.flags & ZS_FLAG_PRIME)) ? 1 : 0;
+    a.dict_img = nullptr;
+    a.dict_save = nullptr;
+    a.dict_len = 0;
+    // A dictionary call: every chunk is its own segment (it must see the dictionary, not the chunk before it).
+    // Z_RLE looks one byte back only and keeps its kernel: there the dictionary changes the framing alone.
+    const bool with_dict = p.dict != nullptr && p.strategy != ZS_STRATEGY_RLE;
+    if (with_dict) {
+        a.cross = 1;
+        a.dict_img = p.dict->d_img;
+        a.dict_len = p.dict->len;
+    }
     // Segments: runs of consecutive chunks that go through the pipeline as one range, sharing one set
     // of hash tables.  A segment pays the pipeline fill/drain (6 steps) and, with cross-chunk
     // matching, one 32 KiB insert-only priming pass.
@@ -1232,6 +1378,7 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
         seg_chunks = (uint32_t)sc;
     }
     if (a.cross && p.seg_hint) seg_chunks = p.seg_hint < kMaxSegChunks ? p.seg_hint : kMaxSegChunks;
+    if (with_dict) seg_chunks = 1;
     // The CTAs claim segments in index order from an atomic counter, so what the kernel waits for at the end
     // is at most one segment: the last quarter of the chunks is cut into segments a quarter of the size
     // (measured on 8192 x 256 KiB chunks, level 6: 630 equal segments = 4.26 waves over 148 SMs, 14.5 GB/s;
@@ -1283,7 +1430,10 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
     unsigned long long zero[16] = {0};
     cudaMemcpyToSymbol(g_prof, zero, sizeof(zero));
 #endif
-    if (a.strategy == ZS_STRATEGY_RLE) {
+    if (with_dict) {
+        const LzKernel k = p.level >= 4 ? lz77_dict_kernel<1, 0> : kGreedyDict[greedy_generic ? 0 : p.level];
+        ZS_KERNEL(ctx, "lz77_dict_kernel", k<<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
+    } else if (a.strategy == ZS_STRATEGY_RLE) {
         ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<2, 0><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
     } else if (p.level >= 4) {
         ZS_KERNEL(ctx, "lz77_kernel", lz77_kernel<1, 0><<<grid, kThreads, sizeof(Smem), ctx->stream>>>(a));
@@ -1303,5 +1453,49 @@ int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p) {
                 pr[12], pr[13], pr[14], pr[15] >> 32, pr[15] & 0xffffffffull);
     }
 #endif
+    return ZS_OK;
+}
+
+size_t zs_lz77_dict_image_bytes() { return kImgBytes; }
+
+int zs_lz77_dict_build(zs_ctx* ctx, const uint8_t* d_dict, uint32_t len, uint8_t* d_img) {
+    if (len > 32768u || (reinterpret_cast<uintptr_t>(d_dict) & 15u)) return ZS_STREAM_ERROR;
+    // (the use launch sets the shared-memory opt-in of every dictionary kernel; the build runs <1, 0>)
+    ZS_CUDA_TRY(ctx, cudaFuncSetAttribute(lz77_dict_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+    // one chunk, the dictionary; nothing is searched, so the symbol and block outputs are a few words of scratch
+    uint64_t* work = nullptr;
+    ZS_CUDA_TRY(ctx, cudaMalloc(&work, 64 * sizeof(uint64_t)));
+    const uint64_t off[2] = {0, len};
+    cudaError_t e = cudaMemcpyAsync(work, off, sizeof(off), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(work + 2, 0, 62 * sizeof(uint64_t), ctx->stream);
+    if (e != cudaSuccess) { cudaFree(work); return zs_set_cuda_error(ctx, e, "dictionary build"); }
+    LzArgs a;
+    memset(&a, 0, sizeof(a));
+    a.buf = d_dict;
+    a.org = 0;
+    a.valid_lo = 0;
+    a.data_end = len;
+    a.in_off = work;
+    a.n_chunks = 1; a.seg_chunks = 1; a.n_seg = 1; a.max_bpc = 1;
+    a.n_big = 1; a.seg_small = 1;
+    a.cfg = kLevels[6];
+    a.strategy = ZS_STRATEGY_DEFAULT;
+    a.cross = 1;
+    a.seg_counter = reinterpret_cast<uint32_t*>(work + 2);
+    a.chunk_nblk = reinterpret_cast<uint32_t*>(work + 3);
+    a.blk_desc = reinterpret_cast<uint32_t*>(work + 4);
+    a.sym = reinterpret_cast<uint32_t*>(work + 8);
+    a.stop_after = 8; a.stop_active = 8;
+    a.dict_img = nullptr;
+    a.dict_save = d_img;
+    a.dict_len = len;
+    zs_prof_begin(ctx, "lz77_dict_build");
+    lz77_dict_kernel<1, 0><<<1, kThreads, sizeof(Smem), ctx->stream>>>(a);
+    zs_prof_end(ctx);
+    ctx->launches++;
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    cudaFree(work);
+    if (e != cudaSuccess) return zs_set_cuda_error(ctx, e, "lz77_dict_build");
     return ZS_OK;
 }
