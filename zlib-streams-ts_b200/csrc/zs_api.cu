@@ -7,23 +7,12 @@
 
 #include "zs_common.cuh"
 
-// ---- scratch slots ---------------------------------------------------------------------------------
-enum {
-    SCR_CK_OFF = 0, SCR_CK_PART = 1, SCR_SMALL = 2,
-    SCR_D_SYM = 3, SCR_D_NBLK = 4, SCR_D_DESC = 5, SCR_D_FREQ = 6, SCR_D_CODE = 7, SCR_D_HDR = 8, SCR_D_BITS = 9,
-    SCR_D_PR = 10, SCR_D_OFF = 11, SCR_D_CHECKS = 12,
-    SCR_I_MISC = 13,
-    // (SCR_H_IN, SCR_H_OUT and SCR_H_RES are named by number in zs_stream.cu: run_part)
-    SCR_H_IN = 14, SCR_H_OUT = 15, SCR_H_OFF = 16, SCR_H_OFF2 = 17, SCR_H_RES = 18, SCR_H_DICT = 19, SCR_H_RNG = 20,
-    SCR_D_OUTOFF = 21, SCR_D_OUTBITS = 22, SCR_H_CHECKS = 23, SCR_I_RESUME = 24,
-    // 25..29: zs_inflate_par.cu
-    SCR_P_STATE = 30, SCR_I_STREAM = 31, SCR_H_DETAIL = 32,
-};
 constexpr uint64_t kParMinInput = 128u << 10;   // shorter streams are decoded by one warp
 
-void* zs_scratch_get(zs_ctx* ctx, int slot, size_t bytes) {
+// ---- scratch (slots: zs_common.cuh) -----------------------------------------------------------------
+void* zs_scratch_get(zs_ctx* ctx, zs_scratch_slot slot, size_t bytes) {
     zs_scratch& s = ctx->scr[slot];
-    if (slot == SCR_H_OUT) ctx->h_out_gen++;
+    s.gen++;
     if (bytes == 0) bytes = 16;
     if (s.cap >= bytes) return s.p;
     if (s.p) {
@@ -108,6 +97,27 @@ int bad_arg(zs_ctx* ctx, const char* msg) {
     return ZS_STREAM_ERROR;
 }
 
+// The copy streams and events of the pipelined host-buffer paths, created by the first such call.
+int ensure_copy_streams(zs_ctx* ctx) {
+    if (ctx->s_in) return ZS_OK;
+    ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_in, cudaStreamNonBlocking));
+    ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_out, cudaStreamNonBlocking));
+    ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_res, cudaStreamNonBlocking));
+    for (int s = 0; s < kMaxPipeSlices; s++)
+        for (cudaEvent_t* e : {&ctx->ev_in[s], &ctx->ev_kern[s], &ctx->ev_res[s]})
+            ZS_CUDA_TRY(ctx, cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    ZS_CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->ev_fence, cudaEventDisableTiming));
+    return ZS_OK;
+}
+
+// Everything issued so far on the context stream (the caller's producers, this call's uploads) comes before
+// whatever the copy streams do next.
+int fence_copy_streams(zs_ctx* ctx) {
+    ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_fence, ctx->stream));
+    for (cudaStream_t s : {ctx->s_in, ctx->s_out, ctx->s_res}) ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(s, ctx->ev_fence, 0));
+    return ZS_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -151,8 +161,10 @@ void zs_ctx_destroy(zs_ctx* ctx) {
     if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
     if (ctx->s_out) cudaStreamDestroy(ctx->s_out);
     if (ctx->s_res) cudaStreamDestroy(ctx->s_res);
-    for (auto e : ctx->ev)
-        if (e) cudaEventDestroy(e);
+    for (int s = 0; s < kMaxPipeSlices; s++)
+        for (cudaEvent_t e : {ctx->ev_in[s], ctx->ev_kern[s], ctx->ev_res[s]})
+            if (e) cudaEventDestroy(e);
+    if (ctx->ev_fence) cudaEventDestroy(ctx->ev_fence);
     if (ctx->prof) {
         zs_profile* pr = (zs_profile*)ctx->prof;
         for (auto& r : pr->recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -257,12 +269,13 @@ int zs_checksum(zs_ctx* ctx, int kind, const uint8_t* buf, uint64_t len, uint32_
 }  // extern "C"
 
 // ---- deflate ------------------------------------------------------------------------------------------
-// zs_deflate_batch_dev, and zs_deflate_batch_dict_dev with `dict` (INDEPENDENT, no history, checked by the caller)
+// zs_deflate_batch_dev, and zs_deflate_batch_dict_dev with `dict` (INDEPENDENT, no history, checked by the caller).
+// seg_hint: 0, or the LZ77 segment size (chunks) of the whole batch when this call compresses a slice of it.
 static int deflate_batch_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* d_in, uint64_t in_len,
                              const uint64_t* d_in_off, uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk,
                              uint32_t history, int level, int wrap, int mode, uint32_t flags, uint8_t* d_out,
                              uint64_t out_cap, uint64_t* d_out_off, uint64_t* d_out_bits, uint32_t* d_checks,
-                             zs_deflate_result* d_result) {
+                             zs_deflate_result* d_result, uint32_t seg_hint) {
     if (level == -1) level = 6;
     // argument rules of deflateInit2_ (deflate.ts:263-297) that apply to the batch form
     if (level < 0 || level > 9) return bad_arg(ctx, "deflate: level must be 0..9");
@@ -293,7 +306,7 @@ static int deflate_batch_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uin
     p.d_in = d_in; p.in_len = in_len; p.history = history; p.n_chunks = n_chunks; p.max_chunk = max_chunk;
     p.max_bpc = max_chunk / 16351u + 2u;
     p.level = level; p.wrap = wrap; p.mode = mode; p.flags = flags; p.strategy = strategy;
-    p.seg_hint = ctx->seg_hint;
+    p.seg_hint = seg_hint;
     p.dict = dict;
     const size_t slots = (size_t)n_chunks * p.max_bpc;
 
@@ -368,7 +381,7 @@ int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, cons
     if (ctx) bind_device(ctx);
     if (!ctx) return ZS_STREAM_ERROR;
     return deflate_batch_dev(ctx, nullptr, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, history, level, wrap,
-                             mode, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result);
+                             mode, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0);
 }
 
 // ---- preset dictionaries ------------------------------------------------------------------------------
@@ -445,7 +458,7 @@ int zs_deflate_batch_dict_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
     const int rc = check_dict_call(ctx, dict, wrap, flags);
     if (rc != ZS_OK) return rc;
     return deflate_batch_dev(ctx, dict, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, 0, level, wrap,
-                             ZS_MODE_INDEPENDENT, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result);
+                             ZS_MODE_INDEPENDENT, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0);
 }
 
 // Host-buffer deflate of a large batch, software-pipelined: the batch is cut into slices of whole waves of
@@ -462,6 +475,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
                                    uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits,
                                    uint32_t* checks, zs_deflate_result* result) {
     constexpr int kMaxSlices = 16;
+    static_assert(kMaxSlices <= kMaxPipeSlices, "one event per slice");
     const bool stitched = mode == ZS_MODE_STITCHED;
     // Same LZ77 segmentation as the single-shot call over the whole batch; a slice is a whole number
     // of waves of segments (one segment per SM and wave), so that no SM idles inside a slice.
@@ -497,12 +511,8 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
     }
     uint32_t slice_chunks = 0;   // the largest slice: sizes the per-slice output regions
     for (int i = 0; i < n_slices; i++) slice_chunks = cb[i + 1] - cb[i] > slice_chunks ? cb[i + 1] - cb[i] : slice_chunks;
-    if (!ctx->s_in) {
-        ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_in, cudaStreamNonBlocking));
-        ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_out, cudaStreamNonBlocking));
-        ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_res, cudaStreamNonBlocking));
-        for (auto& e : ctx->ev) ZS_CUDA_TRY(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
+    int rc = ensure_copy_streams(ctx);
+    if (rc != ZS_OK) return rc;
     if (!ctx->h_pin) {
         ZS_CUDA_TRY(ctx, cudaMallocHost(&ctx->h_pin, 4096));
         ctx->h_pin_cap = 4096;
@@ -522,16 +532,8 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
     if (!d_in_base || !d_out || !d_ooff || !d_obits || !d_cks || !d_res) return ZS_MEM_ERROR;
     uint8_t* d_in = d_in_base + 32768;   // the history of the first slice lies before it
     const bool want_checks = checks != nullptr || wrap != ZS_WRAP_RAW;
-    cudaEvent_t* ev_in = ctx->ev;          // [s]      slice s is on the device
-    cudaEvent_t* ev_k = ctx->ev + 16;      // [s]      kernels of slice s are done
-    cudaEvent_t* ev_r = ctx->ev + 32;      // [s]      result of slice s is on the host
-    // everything issued so far on the context stream (e.g. the caller's producers) comes first
-    ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev[48], ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_in, ctx->ev[48], 0));
-    ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_out, ctx->ev[48], 0));
-    ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_res, ctx->ev[48], 0));
-    struct HintGuard { zs_ctx* c; ~HintGuard() { c->seg_hint = 0; } } guard{ctx};
-    ctx->seg_hint = seg;
+    rc = fence_copy_streams(ctx);
+    if (rc != ZS_OK) return rc;
     if (history) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in - history, in - history, history, cudaMemcpyHostToDevice, ctx->s_in));
     const uint32_t part_mask = ZS_FLAG_NOT_FIRST | ZS_FLAG_NOT_LAST;
     for (int s = 0; s < n_slices; s++) {
@@ -540,8 +542,8 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         const uint64_t b0 = (uint64_t)c0 * chunk_size;
         const uint64_t len = (b0 + (uint64_t)nc * chunk_size <= in_len) ? (uint64_t)nc * chunk_size : in_len - b0;
         if (len) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + b0, in + b0, len, cudaMemcpyHostToDevice, ctx->s_in));
-        ZS_CUDA_TRY(ctx, cudaEventRecord(ev_in[s], ctx->s_in));
-        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ev_in[s], 0));
+        ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_in[s], ctx->s_in));
+        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
         uint32_t hist = 0, sflags = flags;
         if (stitched) {
             hist = (uint32_t)(b0 + history < 32768 ? b0 + history : 32768);
@@ -551,16 +553,16 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         } else if (flags & ZS_FLAG_PRIME) {
             hist = (uint32_t)(b0 < 32768 ? b0 : 32768);
         }
-        int rc = deflate_batch_dev(ctx, dict, d_in + b0, len, nullptr, nc, chunk_size, chunk_size, hist, level, wrap,
-                                   mode, sflags, d_out + region_al * s, region, d_ooff + c0 + s,
-                                   d_obits + c0, want_checks ? d_cks + c0 : nullptr, d_res + s);
+        rc = deflate_batch_dev(ctx, dict, d_in + b0, len, nullptr, nc, chunk_size, chunk_size, hist, level, wrap, mode, sflags,
+                               d_out + region_al * s, region, d_ooff + c0 + s, d_obits + c0,
+                               want_checks ? d_cks + c0 : nullptr, d_res + s, seg);
         if (rc != ZS_OK) return rc;
-        ZS_CUDA_TRY(ctx, cudaEventRecord(ev_k[s], ctx->stream));
+        ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_kern[s], ctx->stream));
         // The 24-byte results come back on their own stream: the bulk D2H copies below are issued as
         // each result arrives and must not queue behind the waits for later slices.
-        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_res, ev_k[s], 0));
+        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_res, ctx->ev_kern[s], 0));
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(h_res + s, d_res + s, sizeof(zs_deflate_result), cudaMemcpyDeviceToHost, ctx->s_res));
-        ZS_CUDA_TRY(ctx, cudaEventRecord(ev_r[s], ctx->s_res));
+        ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_res[s], ctx->s_res));
     }
     uint64_t host_off = 0;
     uint64_t base[kMaxSlices];
@@ -572,7 +574,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         const uint32_t nc = cb[s + 1] - cb[s];
         const uint64_t b0 = (uint64_t)c0 * chunk_size;
         const uint64_t len = (b0 + (uint64_t)nc * chunk_size <= in_len) ? (uint64_t)nc * chunk_size : in_len - b0;
-        ZS_CUDA_TRY(ctx, cudaEventSynchronize(ev_r[s]));
+        ZS_CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev_res[s]));
         const uint64_t total = h_res[s].total_out_bytes;
         base[s] = host_off;
         if (total > region || host_off + total > out_cap) { rc_final = ZS_BUF_ERROR; break; }
@@ -667,7 +669,7 @@ static int deflate_batch_host(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
     if (in_off)
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_off, in_off, (size_t)(n_chunks + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
     int rc = deflate_batch_dev(ctx, dict, d_in, in_len, in_off ? d_off : nullptr, n_chunks, chunk_size, max_chunk, history,
-                               level, wrap, mode, flags, d_out, out_cap, d_ooff, d_ooff + n_chunks + 1, d_checks, d_result);
+                               level, wrap, mode, flags, d_out, out_cap, d_ooff, d_ooff + n_chunks + 1, d_checks, d_result, 0);
     if (rc != ZS_OK) return rc;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(result, d_result, sizeof(zs_deflate_result), cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -726,12 +728,15 @@ int zs_bit_concat_dev(zs_ctx* ctx, uint8_t* d_dst, uint64_t dst_bit_off, const u
     return zs_launch_bit_concat(ctx, d_dst, dst_bit_off, d_src, n_bits);
 }
 
+}  // extern "C"
+
 // ---- inflate ------------------------------------------------------------------------------------------
-int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_off, uint32_t n, int window_bits,
-                         uint8_t* d_out, const uint64_t* d_out_off, uint64_t* d_out_len, uint64_t* d_in_used,
-                         uint32_t* d_checks, int32_t* d_status, const uint8_t* d_dict, const uint64_t* d_dict_rng) {
-    if (ctx) bind_device(ctx);
-    if (!ctx) return ZS_STREAM_ERROR;
+// zs_inflate_batch_dev with options.  o.resume: res->mark receives the block mark (copied on the context stream);
+// `res` may be null otherwise.
+static int inflate_batch_dev_impl(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_off, uint32_t n, int window_bits,
+                                  uint8_t* d_out, const uint64_t* d_out_off, uint64_t* d_out_len, uint64_t* d_in_used,
+                                  uint32_t* d_checks, int32_t* d_status, const uint8_t* d_dict, const uint64_t* d_dict_rng,
+                                  const InflateOpts& o, InflateOut* res) {
     if (n == 0) return ZS_OK;
     if (!d_in || !d_in_off || !d_out || !d_out_off || !d_out_len || !d_status) return bad_arg(ctx, "inflate: null buffer");
     if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return bad_arg(ctx, "inflate: d_in must be 8-byte aligned");
@@ -770,12 +775,13 @@ int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_
         a.d_dict_adler = d_da;
     }
     a.d_start_bit = nullptr; a.d_block_mark = nullptr;
-    if (ctx->inflate_resume && n == 1) {
+    const bool resume = o.resume && n == 1;
+    if (resume) {
         // one stream of the streaming shim: [0] start bit (in), [1..2] block mark (out)
         uint64_t* d_rs = (uint64_t*)zs_scratch_get(ctx, SCR_I_RESUME, 64);
         if (!d_rs) return ZS_MEM_ERROR;
-        ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_rs, &ctx->inflate_start_bit, 8, cudaMemcpyHostToDevice, ctx->stream));
-        if (ctx->inflate_start_bit != ~0ull) a.d_start_bit = d_rs;
+        ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_rs, &o.start_bit, 8, cudaMemcpyHostToDevice, ctx->stream));
+        if (o.start_bit != ~0ull) a.d_start_bit = d_rs;
         a.d_block_mark = d_rs + 1;
     }
     // test hooks: force the thread-per-stream (1) or the warp-per-stream (-1) kernel
@@ -787,24 +793,23 @@ int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_
     // One long stream whose sizes the caller knows on the host: cut it at its flush points and decode the
     // segments in parallel (zs_inflate_par.cu); inflate_kernel then continues behind them -- the trailer
     // and the final status, or whatever the parallel part had to leave.
-    const bool par = ctx->par.on && n == 1 && !d64 && ctx->par.in_len >= kParMinInput && ((ctx->par.in_off & 7u) == 0) &&
+    const bool par = o.par.on && n == 1 && !d64 && o.par.in_len >= kParMinInput && ((o.par.in_off & 7u) == 0) &&
                      !getenv("ZS_INFLATE_SERIAL");
-    ctx->par.on = false;
-    const uint64_t par_out_cap = ctx->par.out_cap;
+    const uint32_t n_choice = o.batch_n > n ? o.batch_n : n;
     if (par) {
         uint64_t* d_ps = (uint64_t*)zs_scratch_get(ctx, SCR_P_STATE, 16 * 8);
         if (!d_ps) return ZS_MEM_ERROR;
         zs_inflate_args h = a;
         h.d_hdr_state = d_ps;
         h.d_block_mark = nullptr;
-        rc = zs_launch_inflate(ctx, h);
+        rc = zs_launch_inflate(ctx, h, n_choice);
         if (rc != ZS_OK) return rc;
-        rc = zs_launch_inflate_parallel(ctx, d_in + ctx->par.in_off, ctx->par.in_len, d_out + ctx->par.out_off, ctx->par.out_cap,
-                                        d_dict ? d_dict + ctx->par.dict_off : nullptr, d_dict ? ctx->par.dict_len : 0, d_ps, d_ps + 8);
+        rc = zs_launch_inflate_parallel(ctx, d_in + o.par.in_off, o.par.in_len, d_out + o.par.out_off, o.par.out_cap,
+                                        d_dict ? d_dict + o.par.dict_off : nullptr, d_dict ? o.par.dict_len : 0, d_ps, d_ps + 8);
         if (rc != ZS_OK) return rc;
         a.d_resume = d_ps + 8;
     }
-    rc = zs_launch_inflate(ctx, a);
+    rc = zs_launch_inflate(ctx, a, n_choice);
     if (rc != ZS_OK) return rc;
     ctx->d_last_detail = a.d_detail;
     ctx->last_detail_n = n;
@@ -814,8 +819,8 @@ int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_
     if (par) {
         // one long stream: its output is cut into pieces for the checksum too (a warp per stream would take
         // 0.5 s per GiB)
-        if (want_adler) rc = zs_launch_checksum_stream(ctx, 0, d_out, d_out_off, d_out_len, par_out_cap, d_adler);
-        if (rc == ZS_OK && want_crc) rc = zs_launch_checksum_stream(ctx, 1, d_out, d_out_off, d_out_len, par_out_cap, d_crc);
+        if (want_adler) rc = zs_launch_checksum_stream(ctx, 0, d_out, d_out_off, d_out_len, o.par.out_cap, d_adler);
+        if (rc == ZS_OK && want_crc) rc = zs_launch_checksum_stream(ctx, 1, d_out, d_out_off, d_out_len, o.par.out_cap, d_crc);
         if (rc != ZS_OK) return rc;
     } else {
         if (want_adler) {
@@ -827,14 +832,17 @@ int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_
             if (rc != ZS_OK) return rc;
         }
     }
-    return zs_launch_inflate_verify(ctx, n, want_adler ? d_adler : nullptr, want_crc ? d_crc : nullptr, a.d_trailer,
-                                    a.d_flags, d_out_len, d_checks, d_status, a.d_detail);
+    rc = zs_launch_inflate_verify(ctx, n, want_adler ? d_adler : nullptr, want_crc ? d_crc : nullptr, a.d_trailer, a.d_flags,
+                                  d_out_len, d_checks, d_status, a.d_detail);
+    if (rc == ZS_OK && resume)
+        ZS_CUDA_TRY(ctx, cudaMemcpyAsync(res->mark, a.d_block_mark, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    return rc;
 }
 
 // Host-buffer inflate of a large batch, pipelined like deflate_batch_pipelined: the streams are cut into slices
 // of about equal input + output bytes; slice s+1 is copied in while the kernels of slice s run and the output of
 // slice s-1 is copied out (three streams, events between them).  Every slice is decoded by the kernel the
-// whole batch would have used (ctx->inflate_batch_n), so the results are those of the unsliced call.
+// whole batch would have used (InflateOpts::batch_n), so the results are those of the unsliced call.
 static int inflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uint32_t n, int window_bits,
                                    uint8_t* out, const uint64_t* out_off, uint64_t* out_len, uint64_t* in_used,
                                    uint32_t* checks, int32_t* status, uint8_t* d_in, uint8_t* d_out, uint64_t* d_ioff,
@@ -842,15 +850,12 @@ static int inflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, const uint64_
     // a slice must still fill the GPU: 32768 streams for the thread-per-stream kernel, one warp per stream and
     // 32 resident warps per SM otherwise
     constexpr int kMaxSlices = 8;
+    static_assert(kMaxSlices <= kMaxPipeSlices, "one event per slice");
     const uint32_t fill = n >= 32768 ? 32768u : (uint32_t)ctx->sm_count * 32u;
     int kSlices = (int)(n / fill);
     kSlices = kSlices < 2 ? 2 : kSlices > kMaxSlices ? kMaxSlices : kSlices;
-    if (!ctx->s_in) {
-        ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_in, cudaStreamNonBlocking));
-        ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_out, cudaStreamNonBlocking));
-        ZS_CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_res, cudaStreamNonBlocking));
-        for (auto& e : ctx->ev) ZS_CUDA_TRY(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
+    int rc = ensure_copy_streams(ctx);
+    if (rc != ZS_OK) return rc;
     // slice boundaries: stream index at which the running input + output bytes pass s/kSlices of the total
     uint32_t b[kMaxSlices + 1];
     const uint64_t total = in_off[n] + out_off[n];
@@ -871,30 +876,26 @@ static int inflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, const uint64_
     int32_t* d_status = (int32_t*)(d_checks + n);
     int32_t* d_det = (int32_t*)zs_scratch_get(ctx, SCR_H_DETAIL, (size_t)n * 4);
     if (!d_det) return ZS_MEM_ERROR;
-    cudaEvent_t* ev_in = ctx->ev;          // [s] slice s is on the device
-    cudaEvent_t* ev_k = ctx->ev + 16;      // [s] kernels of slice s are done
-    // the offsets (and whatever the caller queued on the context stream) come first
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_ioff, in_off, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_ooff, out_off, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev[48], ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_in, ctx->ev[48], 0));
-    ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_out, ctx->ev[48], 0));
-    struct Guard { zs_ctx* c; ~Guard() { c->inflate_batch_n = 0; } } guard{ctx};
-    ctx->inflate_batch_n = n;
+    rc = fence_copy_streams(ctx);
+    if (rc != ZS_OK) return rc;
+    InflateOpts o;
+    o.batch_n = n;
     for (int s = 0; s < kSlices; s++) {
         const uint32_t lo = b[s], ns = b[s + 1] - b[s];
         if (ns == 0) continue;
         // whole 8-byte words around the slice's input (the decoders read aligned words)
         const uint64_t i0 = in_off[lo] & ~7ull, i1 = in_off[lo + ns];
         if (i1 > i0) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in + i0, in + i0, i1 - i0, cudaMemcpyHostToDevice, ctx->s_in));
-        ZS_CUDA_TRY(ctx, cudaEventRecord(ev_in[s], ctx->s_in));
-        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ev_in[s], 0));
-        const int rc = zs_inflate_batch_dev(ctx, d_in, d_ioff + lo, ns, window_bits, d_out, d_ooff + lo, d_olen + lo, d_used + lo,
-                                            d_checks + lo, d_status + lo, d_dict, d_rng ? d_rng + 2 * (size_t)lo : nullptr);
+        ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_in[s], ctx->s_in));
+        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
+        rc = inflate_batch_dev_impl(ctx, d_in, d_ioff + lo, ns, window_bits, d_out, d_ooff + lo, d_olen + lo, d_used + lo,
+                                    d_checks + lo, d_status + lo, d_dict, d_rng ? d_rng + 2 * (size_t)lo : nullptr, o, nullptr);
         if (rc != ZS_OK) return rc;
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_det + lo, ctx->d_last_detail, (size_t)ns * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-        ZS_CUDA_TRY(ctx, cudaEventRecord(ev_k[s], ctx->stream));
-        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_out, ev_k[s], 0));
+        ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_kern[s], ctx->stream));
+        ZS_CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_out, ctx->ev_kern[s], 0));
         const uint64_t o0 = out_off[lo], o1 = out_off[lo + ns];
         if (o1 > o0) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(out + o0, d_out + o0, o1 - o0, cudaMemcpyDeviceToHost, ctx->s_out));
     }
@@ -909,11 +910,10 @@ static int inflate_batch_pipelined(zs_ctx* ctx, const uint8_t* in, const uint64_
     return ZS_OK;
 }
 
-int zs_inflate_batch(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uint32_t n, int window_bits, uint8_t* out,
-                     const uint64_t* out_off, uint64_t* out_len, uint64_t* in_used, uint32_t* checks, int32_t* status,
-                     const uint8_t* dict, const uint64_t* dict_rng, uint64_t dict_total) {
-    if (ctx) bind_device(ctx);
-    if (!ctx) return ZS_STREAM_ERROR;
+int inflate_batch_host_impl(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uint32_t n, int window_bits, uint8_t* out,
+                            const uint64_t* out_off, uint64_t* out_len, uint64_t* in_used, uint32_t* checks, int32_t* status,
+                            const uint8_t* dict, const uint64_t* dict_rng, uint64_t dict_total, const InflateOpts& opts,
+                            InflateOut* res) {
     if (n == 0) return ZS_OK;
     if (!in_off || !out_off || !out_len || !status) return bad_arg(ctx, "inflate: null buffer");
     const uint64_t in_total = in_off[n], out_total = out_off[n];
@@ -939,22 +939,25 @@ int zs_inflate_batch(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uin
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_rng, dict_rng, (size_t)n * 16, cudaMemcpyHostToDevice, ctx->stream));
     }
     // large batches: copies and kernels overlap slice by slice
-    if (n >= 2u * (uint32_t)ctx->sm_count * 32u && in_total + out_total >= (64ull << 20) && !ctx->inflate_resume && !getenv("ZS_INFLATE_UNPIPELINED"))
+    if (n >= 2u * (uint32_t)ctx->sm_count * 32u && in_total + out_total >= (64ull << 20) && !opts.resume && !getenv("ZS_INFLATE_UNPIPELINED"))
         return inflate_batch_pipelined(ctx, in, in_off, n, window_bits, out, out_off, out_len, in_used, checks, status, d_in,
                                        d_out, d_ioff, d_ooff, d_res, d_dict, d_rng);
     if (in_total) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, in, in_total, cudaMemcpyHostToDevice, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_ioff, in_off, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_ooff, out_off, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->last_inflate_out = n == 1 ? d_out + out_off[0] : nullptr;
+    InflateOpts o = opts;
     if (n == 1) {
-        ctx->par.on = true;
-        ctx->par.in_off = in_off[0]; ctx->par.in_len = in_off[1] - in_off[0];
-        ctx->par.out_off = out_off[0]; ctx->par.out_cap = out_off[1] - out_off[0];
-        ctx->par.dict_off = d_rng ? dict_rng[0] : 0; ctx->par.dict_len = d_rng ? dict_rng[1] - dict_rng[0] : 0;
+        o.par.on = true;
+        o.par.in_off = in_off[0]; o.par.in_len = in_off[1] - in_off[0];
+        o.par.out_off = out_off[0]; o.par.out_cap = out_off[1] - out_off[0];
+        o.par.dict_off = d_rng ? dict_rng[0] : 0; o.par.dict_len = d_rng ? dict_rng[1] - dict_rng[0] : 0;
+        if (res) {
+            res->d_out = d_out + out_off[0];
+            res->out_gen = ctx->scr[SCR_H_OUT].gen;
+        }
     }
-    int rc = zs_inflate_batch_dev(ctx, d_in, d_ioff, n, window_bits, d_out, d_ooff, d_olen, d_used, d_checks, d_status,
-                                  d_dict, d_rng);
-    ctx->par.on = false;
+    int rc = inflate_batch_dev_impl(ctx, d_in, d_ioff, n, window_bits, d_out, d_ooff, d_olen, d_used, d_checks, d_status,
+                                    d_dict, d_rng, o, res);
     if (rc != ZS_OK) return rc;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(out_len, d_olen, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     if (n == 1 && out_total > (1u << 20)) {
@@ -968,12 +971,29 @@ int zs_inflate_batch(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uin
     if (in_used) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(in_used, d_used, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     if (checks) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(checks, d_checks, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(status, d_status, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (ctx->inflate_resume && n == 1) {
-        const uint64_t* d_rs = (const uint64_t*)zs_scratch_get(ctx, SCR_I_RESUME, 64);
-        ZS_CUDA_TRY(ctx, cudaMemcpyAsync(ctx->inflate_mark, d_rs + 1, 16, cudaMemcpyDeviceToHost, ctx->stream));
-    }
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return ZS_OK;
+}
+
+extern "C" {
+
+int zs_inflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, const uint64_t* d_in_off, uint32_t n, int window_bits,
+                         uint8_t* d_out, const uint64_t* d_out_off, uint64_t* d_out_len, uint64_t* d_in_used,
+                         uint32_t* d_checks, int32_t* d_status, const uint8_t* d_dict, const uint64_t* d_dict_rng) {
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    // (no segment-parallel decode here, even for one stream: its sizes are on the device)
+    return inflate_batch_dev_impl(ctx, d_in, d_in_off, n, window_bits, d_out, d_out_off, d_out_len, d_in_used, d_checks,
+                                  d_status, d_dict, d_dict_rng, InflateOpts(), nullptr);
+}
+
+int zs_inflate_batch(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uint32_t n, int window_bits, uint8_t* out,
+                     const uint64_t* out_off, uint64_t* out_len, uint64_t* in_used, uint32_t* checks, int32_t* status,
+                     const uint8_t* dict, const uint64_t* dict_rng, uint64_t dict_total) {
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    return inflate_batch_host_impl(ctx, in, in_off, n, window_bits, out, out_off, out_len, in_used, checks, status, dict,
+                                   dict_rng, dict_total, InflateOpts(), nullptr);
 }
 
 int zs_inflate_stream_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int window_bits, uint8_t* d_out, uint64_t out_cap,
@@ -987,13 +1007,11 @@ int zs_inflate_stream_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int
     const uint64_t h[6] = {0, in_len, 0, out_cap, 0, dict_len};
     // (pageable source: the copy is staged before the call returns)
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_o, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
-    ctx->par.on = true;
-    ctx->par.in_off = 0; ctx->par.in_len = in_len; ctx->par.out_off = 0; ctx->par.out_cap = out_cap;
-    ctx->par.dict_off = 0; ctx->par.dict_len = d_dict ? dict_len : 0;
-    const int rc = zs_inflate_batch_dev(ctx, d_in, d_o, 1, window_bits, d_out, d_o + 2, d_out_len, d_in_used, d_check, d_status,
-                                        d_dict && dict_len ? d_dict : nullptr, d_dict && dict_len ? d_o + 4 : nullptr);
-    ctx->par.on = false;
-    return rc;
+    InflateOpts o;
+    o.par.on = true;
+    o.par.in_len = in_len; o.par.out_cap = out_cap; o.par.dict_len = d_dict ? dict_len : 0;
+    return inflate_batch_dev_impl(ctx, d_in, d_o, 1, window_bits, d_out, d_o + 2, d_out_len, d_in_used, d_check, d_status,
+                                  d_dict && dict_len ? d_dict : nullptr, d_dict && dict_len ? d_o + 4 : nullptr, o, nullptr);
 }
 
 int zs_inflate_last_details(zs_ctx* ctx, int32_t* detail, uint32_t n) {

@@ -421,8 +421,8 @@ int zs_launch_checksum_stream(zs_ctx* ctx, int kind, const uint8_t* d_buf, const
         return ZS_STREAM_ERROR;
     }
     const uint32_t n = (uint32_t)n64;
-    uint64_t* d_off = (uint64_t*)zs_scratch_get(ctx, 0, (size_t)(n + 1) * sizeof(uint64_t));
-    uint32_t* d_part = (uint32_t*)zs_scratch_get(ctx, 1, (size_t)n * sizeof(uint32_t));
+    uint64_t* d_off = (uint64_t*)zs_scratch_get(ctx, SCR_CK_OFF, (size_t)(n + 1) * sizeof(uint64_t));
+    uint32_t* d_part = (uint32_t*)zs_scratch_get(ctx, SCR_CK_PART, (size_t)n * sizeof(uint32_t));
     if (!d_off || !d_part) return ZS_MEM_ERROR;
     ZS_KERNEL(ctx, "make_offsets_dev_kernel", make_offsets_dev_kernel<<<(n + 1 + 255) / 256, 256, 0, ctx->stream>>>(d_off, d_base, d_len, piece, n));
     int rc = zs_launch_checksum_segments(ctx, kind, d_buf, d_off, nullptr, n, d_part);
@@ -440,8 +440,8 @@ int zs_launch_checksum_whole(zs_ctx* ctx, int kind, const uint8_t* d_buf, uint64
         return ZS_STREAM_ERROR;
     }
     uint32_t n = (uint32_t)n64;
-    uint64_t* d_off = (uint64_t*)zs_scratch_get(ctx, 0, (size_t)(n + 1) * sizeof(uint64_t));
-    uint32_t* d_part = (uint32_t*)zs_scratch_get(ctx, 1, (size_t)n * sizeof(uint32_t));
+    uint64_t* d_off = (uint64_t*)zs_scratch_get(ctx, SCR_CK_OFF, (size_t)(n + 1) * sizeof(uint64_t));
+    uint32_t* d_part = (uint32_t*)zs_scratch_get(ctx, SCR_CK_PART, (size_t)n * sizeof(uint32_t));
     if (!d_off || !d_part) return ZS_MEM_ERROR;
     ZS_KERNEL(ctx, "make_offsets_kernel", make_offsets_kernel<<<(n + 1 + 255) / 256, 256, 0, ctx->stream>>>(d_off, len, piece, n));
     int rc = zs_launch_checksum_segments(ctx, kind, d_buf, d_off, nullptr, n, d_part);

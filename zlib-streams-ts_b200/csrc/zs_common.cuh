@@ -8,10 +8,41 @@
 #define ZS_FULL_MASK 0xffffffffu
 
 // ---- context (host side) -------------------------------------------------------------------------
+// Device scratch of a context: one grow-only buffer per slot (zs_scratch_get).  Every user of a slot works in
+// order on the context stream, and a slot that has to grow synchronises that stream before it frees its old
+// buffer, so users that share a slot never see each other's work in flight.
+enum zs_scratch_slot {
+    // zs_launch_checksum_whole and zs_launch_checksum_stream (offsets, partial sums of the pieces): shared by both
+    SCR_CK_OFF = 0, SCR_CK_PART,
+    // 256 bytes shared by zs_checksum_dev (the result), deflate_batch_dev (segment counter, total check, error
+    // flag) and zs_deflate_dict_create (DICTID): each reads its values back or consumes them in its own kernels
+    SCR_SMALL,
+    // deflate_batch_dev
+    SCR_D_SYM, SCR_D_NBLK, SCR_D_DESC, SCR_D_FREQ, SCR_D_CODE, SCR_D_HDR, SCR_D_BITS, SCR_D_PR, SCR_D_OFF,
+    SCR_D_CHECKS, SCR_D_OUTOFF, SCR_D_OUTBITS,
+    // staged input, output and results of the host-buffer calls (zs_checksum, zs_deflate_batch*, zs_inflate_batch),
+    // shared with the deflate stream's parts (zs_stream.cu: run_part), around a zs_deflate_batch_dev that uses none
+    SCR_H_IN, SCR_H_OUT, SCR_H_RES,
+    // the rest of the host-buffer calls
+    SCR_H_OFF, SCR_H_OFF2, SCR_H_DICT, SCR_H_RNG, SCR_H_CHECKS, SCR_H_DETAIL,
+    // batch inflate: details / trailers / checksums, the streaming shim's resume record, zs_inflate_stream_dev's offsets
+    SCR_I_MISC, SCR_I_RESUME, SCR_I_STREAM,
+    // one-stream segment-parallel inflate.  SCR_P_STATE is taken by the API layer and shared with the parallel
+    // decoder: the header pass writes it, zs_launch_inflate_parallel reads and extends it, inflate_kernel resumes from it
+    SCR_P_STATE,
+    // zs_inflate_par.cu
+    SCR_P_CAND, SCR_P_SEG, SCR_P_PLAN, SCR_P_SYM, SCR_P_WIN, SCR_P_GMAP,
+    ZS_SCR_COUNT
+};
+
 struct zs_scratch {
     void* p = nullptr;
     size_t cap = 0;
+    uint64_t gen = 0;   // bumped by every zs_scratch_get of the slot: what a call left there is intact while it is unchanged
 };
+
+// slices of one pipelined host-buffer call: deflate cuts a batch into at most 16, inflate into at most 8
+constexpr int kMaxPipeSlices = 16;
 
 struct zs_ctx {
     int device = 0;
@@ -20,33 +51,25 @@ struct zs_ctx {
     char err[256] = {0};
     uint64_t launches = 0;
     int sm_count = 148;
-    // grow-only device scratch, one slot per purpose (see zs_api.cu)
-    zs_scratch scr[40];
+    zs_scratch scr[ZS_SCR_COUNT];
     // pinned host staging for small results
     void* h_pin = nullptr;
     size_t h_pin_cap = 0;
     // last inflate details (device ptr into scratch) for zs_inflate_last_details
     int32_t* d_last_detail = nullptr;
     uint32_t last_detail_n = 0;
-    // copy streams + events of the pipelined host-buffer path (zs_deflate_batch)
-    cudaStream_t s_in = nullptr, s_out = nullptr, s_res = nullptr;   // host-buffer path: H2D, bulk D2H, small result readbacks
-    // streaming shim -> zs_inflate_batch (one stream): resume request and the block mark that comes back
-    bool inflate_resume = false;
-    uint64_t inflate_start_bit = 0;
-    uint64_t inflate_mark[2] = {0, 0};
-    uint64_t h_out_gen = 0;                      // bumped whenever the host-path output scratch is handed out again
-    const uint8_t* last_inflate_out = nullptr;   // device copy of the output of the last one-stream zs_inflate_batch (valid until the next call)
-    uint32_t seg_hint = 0;   // segment size (chunks) forced for the next deflate calls (slices of one batch)
-    uint32_t inflate_batch_n = 0;   // streams of the whole batch while its slices are decoded (kernel choice), 0 = not sliced
-    // one-stream inflate with sizes known on the host: lets zs_inflate_batch_dev use the segment-parallel decoder
-    struct { bool on = false; uint64_t in_off = 0, in_len = 0, out_off = 0, out_cap = 0, dict_off = 0, dict_len = 0; } par;
-    cudaEvent_t ev[64] = {nullptr};
+    // copy streams and events of the pipelined host-buffer paths (ensure_copy_streams, zs_api.cu)
+    cudaStream_t s_in = nullptr, s_out = nullptr, s_res = nullptr;   // H2D, bulk D2H, small result readbacks
+    cudaEvent_t ev_in[kMaxPipeSlices] = {nullptr};     // [s] slice s is on the device
+    cudaEvent_t ev_kern[kMaxPipeSlices] = {nullptr};   // [s] kernels of slice s are done
+    cudaEvent_t ev_res[kMaxPipeSlices] = {nullptr};    // [s] result of slice s is on the host
+    cudaEvent_t ev_fence = nullptr;                    // the caller's work queued before the call
     // profiling (zs_ctx_profile)
     bool prof_on = false;
     void* prof = nullptr;  // zs_profile*, zs_api.cu
 };
 
-void* zs_scratch_get(zs_ctx* ctx, int slot, size_t bytes);  // nullptr on failure (err set)
+void* zs_scratch_get(zs_ctx* ctx, zs_scratch_slot slot, size_t bytes);  // nullptr on failure (err set)
 int zs_set_cuda_error(zs_ctx* ctx, cudaError_t e, const char* where);
 #define ZS_CUDA_TRY(ctx, expr)                                                   \
     do {                                                                         \
@@ -193,12 +216,36 @@ struct zs_inflate_args {
     uint64_t* d_hdr_state;
     const uint64_t* d_resume;
 };
-int zs_launch_inflate(zs_ctx* ctx, const zs_inflate_args& a);
+// n_choice: the stream count that picks the kernel (a slice of a batch decodes like the whole batch)
+int zs_launch_inflate(zs_ctx* ctx, const zs_inflate_args& a, uint32_t n_choice);
 int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
                                const uint8_t* d_hist, uint64_t hist_len, uint64_t* d_state, uint64_t* d_resume);
 int zs_launch_inflate_verify(zs_ctx* ctx, uint32_t n, const uint32_t* d_adler, const uint32_t* d_crc,
                              const uint32_t* d_trailer, const uint32_t* d_flags, const uint64_t* d_out_len,
                              uint32_t* d_checks, int32_t* d_status, int32_t* d_detail);
+
+// Options of one batch inflate call (zs_api.cu) that the public entry points do not take.
+struct InflateOpts {
+    // one stream whose sizes the host knows: it may take the segment-parallel decoder (zs_inflate_par.cu).
+    // inflate_batch_host_impl sets it for every one-stream call.
+    struct { bool on = false; uint64_t in_off = 0, in_len = 0, out_off = 0, out_cap = 0, dict_off = 0, dict_len = 0; } par;
+    // one stream of the streaming shim: decode raw blocks from start_bit (~0: from the wrapper header on) and
+    // report the block mark
+    bool resume = false;
+    uint64_t start_bit = 0;
+    uint32_t batch_n = 0;   // streams of the whole batch when this call decodes a slice of it (kernel choice), or 0
+};
+// What a one-stream call leaves for its caller.
+struct InflateOut {
+    uint64_t mark[2] = {0, 0};        // resume: (bit offset, bytes produced before it) of the last block begun
+    const uint8_t* d_out = nullptr;   // host-buffer call: the stream's output, still on the device ...
+    uint64_t out_gen = 0;             // ... while ctx->scr[SCR_H_OUT].gen equals this
+};
+// zs_inflate_batch with options; `res` may be null.  The caller has bound the context's device.
+int inflate_batch_host_impl(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uint32_t n, int window_bits, uint8_t* out,
+                            const uint64_t* out_off, uint64_t* out_len, uint64_t* in_used, uint32_t* checks, int32_t* status,
+                            const uint8_t* dict, const uint64_t* dict_rng, uint64_t dict_total, const InflateOpts& o,
+                            InflateOut* res);
 
 // deflate
 struct zs_deflate_plan {

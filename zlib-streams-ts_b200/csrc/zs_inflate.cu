@@ -323,12 +323,11 @@ int zs_launch_inflate_tps(zs_ctx* ctx, const zs_inflate_args& a);  // zs_inflate
 // Batches of many streams go to the thread-per-stream kernel (32 streams per warp instruction;
 // measured 29 GB/s vs 12.5 GB/s on 128 K x 4 KiB gzip records); fewer / larger streams keep a whole
 // warp each (cooperative copies, big lookup tables: 21.6 vs 7.3 GB/s on 8 K x 64 KiB streams).
-int zs_launch_inflate(zs_ctx* ctx, const zs_inflate_args& a) {
+int zs_launch_inflate(zs_ctx* ctx, const zs_inflate_args& a, uint32_t n_choice) {
     if (a.n == 0) return ZS_OK;
     // thread per stream needs >= 32 k streams to fill the GPU (1024 warps); measured (tools/infmatrix.py):
     // 28-29 GB/s from 32768 streams up whatever the record size, 16-18 GB/s at 16384, where a warp per
     // stream gives 14 (4 KiB records) to 21 GB/s (64 KiB)
-    const uint32_t n_choice = ctx->inflate_batch_n > a.n ? ctx->inflate_batch_n : a.n;   // slices of one batch decode like the batch
     if (!a.d_start_bit && !a.d_block_mark && a.force_tps >= 0 && (n_choice >= 32768 || (a.force_tps > 0 && a.n >= 32)))
         return zs_launch_inflate_tps(ctx, a);
     unsigned ctas = (a.n + kWarps - 1) / kWarps;

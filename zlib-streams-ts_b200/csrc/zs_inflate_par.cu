@@ -649,9 +649,6 @@ __global__ void par_finish_kernel(ParArgs a) {
 
 }  // namespace
 
-// scratch slots of zs_api.cu reserved for this path
-enum { SCR_P_CAND = 25, SCR_P_SEG = 26, SCR_P_PLAN = 27, SCR_P_SYM = 28, SCR_P_WIN = 29, SCR_P_STATE = 30, SCR_P_GMAP = 33 };
-
 // One stream, wrapper header already located: a.d_resume receives where inflate_kernel continues.
 int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
                                const uint8_t* d_hist, uint64_t hist_len, uint64_t* d_state, uint64_t* d_resume) {

@@ -203,7 +203,6 @@ double now_s() {
 }
 
 enum { ST_INIT = 1, ST_BUSY = 2, ST_FINISH = 3 };
-enum { kScrHostIn = 14, kScrHostOut = 15, kScrHostRes = 18 };   // SCR_H_IN / SCR_H_OUT / SCR_H_RES of zs_api.cu
 constexpr size_t kPartThreshold = 16u << 20;
 constexpr size_t kPartOutHint = 2 * kPartThreshold;   // a part's output (the stored-block bound and change) behind what is still waiting
 // inflate: while a stream has brought less input than this it is decoded on EVERY call, so the call that brings the
@@ -252,8 +251,9 @@ struct InflateState {
     // resumes there in raw mode with the last 64 KiB of output as its window.
     HostBuf in;                     // input not yet consumed: from the byte that holds the next block header on
     HostBuf out;                    // output of the latest attempt (from the resume point); page-locked once it is large
-    bool out_on_device = false;     // `out` is byte for byte what the last attempt left on the device ...
-    uint64_t out_gen = 0;           // ... as long as the context has not handed that scratch out again (h_out_gen)
+    bool out_on_device = false;     // `out` is byte for byte what the last attempt left on the device at out_dev ...
+    const uint8_t* out_dev = nullptr;
+    uint64_t out_gen = 0;           // ... as long as the context has not handed that scratch out again (InflateOut)
     HostBuf ready;                  // decoded, not yet delivered
     std::vector<uint8_t> hist;      // window: the last <= 64 KiB of final output, or the preset dictionary
     std::vector<uint8_t> leftover;  // input after the end of the stream that could not be handed back
@@ -407,9 +407,9 @@ int run_part(zs_stream* strm, DeflateState* st, bool finish, bool full_flush, bo
     // cudaMalloc at its first part, cudaFree at deflateEnd -- and the driver took up to 19 ms for the one and 17 ms for
     // the other: as much as the whole 64 MiB stream (ZS_STREAM_PROF).
     const double t_alloc0 = now_s();
-    uint8_t* d_in_buf = (uint8_t*)zs_scratch_get(ctx, kScrHostIn, hist_len + n + 64 + 16);
-    uint8_t* d_out_buf = (uint8_t*)zs_scratch_get(ctx, kScrHostOut, cap + 64);
-    uint8_t* d_res_buf = (uint8_t*)zs_scratch_get(ctx, kScrHostRes, 256);
+    uint8_t* d_in_buf = (uint8_t*)zs_scratch_get(ctx, SCR_H_IN, hist_len + n + 64 + 16);
+    uint8_t* d_out_buf = (uint8_t*)zs_scratch_get(ctx, SCR_H_OUT, cap + 64);
+    uint8_t* d_res_buf = (uint8_t*)zs_scratch_get(ctx, SCR_H_RES, 256);
     st->t_alloc += now_s() - t_alloc0;
     if (!d_in_buf || !d_out_buf || !d_res_buf) return ZS_MEM_ERROR;
     // history and input are contiguous on the device; keep the input 16-byte aligned
@@ -831,11 +831,11 @@ static void push_ready(InflateState* st, size_t upto) {
     }
 }
 
-// Running checksum continued over the first n bytes of `out`.  The attempt that produced them has just run: its
-// output is still on the device (ctx->last_inflate_out), so the bytes are not uploaded a second time.
+// Running checksum continued over the first n bytes of `out`.  While the output of the attempt that produced them is
+// still on the device (out_dev), the bytes are not uploaded a second time.
 static int out_checksum(InflateState* st, size_t n, uint32_t* result) {
     const int kind = st->trailer == 1 ? 0 : 1;
-    if (st->out_on_device && st->out_gen == st->ctx->h_out_gen && st->ctx->last_inflate_out) return zs_checksum_dev(st->ctx, kind, st->ctx->last_inflate_out, n, st->run_check, result);
+    if (st->out_on_device && st->out_gen == st->ctx->scr[SCR_H_OUT].gen && st->out_dev) return zs_checksum_dev(st->ctx, kind, st->out_dev, n, st->run_check, result);
     return zs_checksum(st->ctx, kind, st->out.data(), n, st->run_check, result);
 }
 
@@ -907,23 +907,25 @@ static int inflate_attempt(zs_stream* strm, InflateState* st) {
         uint64_t out_len = 0, in_used = 0, rng[2] = {0, st->hist.size()};
         uint32_t check = 0;
         int32_t status = 0, detail = 0;
-        ctx->inflate_resume = true;
-        ctx->inflate_start_bit = st->body ? st->start_bit : ~0ull;
+        InflateOpts opts;
+        opts.resume = true;
+        opts.start_bit = st->body ? st->start_bit : ~0ull;
+        InflateOut io;
         const double t_eng0 = now_s();
-        int rc = zs_inflate_batch(ctx, st->in.data(), in_off, 1, st->body ? raw_wb : st->window_bits, st->out.data(), out_off,
-                                  &out_len, &in_used, &check, &status, st->hist.empty() ? nullptr : st->hist.data(),
-                                  st->hist.empty() ? nullptr : rng, st->hist.size());
-        ctx->inflate_resume = false;
+        int rc = inflate_batch_host_impl(ctx, st->in.data(), in_off, 1, st->body ? raw_wb : st->window_bits, st->out.data(),
+                                         out_off, &out_len, &in_used, &check, &status, st->hist.empty() ? nullptr : st->hist.data(),
+                                         st->hist.empty() ? nullptr : rng, st->hist.size(), opts, &io);
         st->t_engine += now_s() - t_eng0;
         if (rc != ZS_OK) { strm->msg = zs_last_error(ctx); return rc; }
         if (status == ZS_BUF_ERROR && out_len == st->out_cap_hint) {  // output full: grow and decode again
             st->out_cap_hint *= 4;
             continue;
         }
-        const uint64_t mark_bit = ctx->inflate_mark[0], mark_out = ctx->inflate_mark[1];
+        const uint64_t mark_bit = io.mark[0], mark_out = io.mark[1];
         st->out.resize(out_len);
         st->out_on_device = true;
-        st->out_gen = ctx->h_out_gen;
+        st->out_dev = io.d_out;
+        st->out_gen = io.out_gen;
         if (status == ZS_STREAM_END) {
             if (!st->body) {
                 // the whole stream in one attempt: wrapper and trailer were checked on the device
