@@ -1,5 +1,5 @@
 # what page-locking host memory costs on this box: cudaHostAlloc / cudaFreeHost of 16 and 128 MiB, and a pageable against a
-# page-locked H2D copy of 64 MiB (the numbers behind the stream shim's buffer policy, zs_stream.cu: HostBuf / PinPool)
+# page-locked H2D copy of 64 MiB (the numbers behind the stream shim's buffer policy, zs_stream.cu: HostBuf / BufPool)
 import ctypes, time, torch
 rt = ctypes.CDLL("libcudart.so.12")
 torch.cuda.init(); torch.zeros(1, device="cuda")

@@ -589,8 +589,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         blocks += h_res[s].n_blocks;
         if (want_checks) {
             if (!have_check) { check = h_res[s].check; have_check = true; }
-            else check = wrap == ZS_WRAP_ZLIB ? zs_host_adler32_combine(check, h_res[s].check, len)
-                                              : zs_host_crc32_combine(check, h_res[s].check, len);
+            else check = zs_host_check_combine(wrap, check, h_res[s].check, len);
         }
     }
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->s_out));
@@ -602,13 +601,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         if (host_off + T > out_cap) {
             rc_final = ZS_BUF_ERROR;
         } else {
-            uint8_t* tp = out + host_off;
-            if (wrap == ZS_WRAP_ZLIB) {
-                tp[0] = (uint8_t)(check >> 24); tp[1] = (uint8_t)(check >> 16); tp[2] = (uint8_t)(check >> 8); tp[3] = (uint8_t)check;
-            } else {
-                for (int k = 0; k < 4; k++) { tp[k] = (uint8_t)(check >> (8 * k)); tp[4 + k] = (uint8_t)(in_len >> (8 * k)); }
-            }
-            host_off += T;
+            host_off += zs_put_trailer(out + host_off, wrap, check, in_len);
         }
     }
     if (rc_final != ZS_OK) {
@@ -740,18 +733,8 @@ static int inflate_batch_dev_impl(zs_ctx* ctx, const uint8_t* d_in, const uint64
     if (n == 0) return ZS_OK;
     if (!d_in || !d_in_off || !d_out || !d_out_off || !d_out_len || !d_status) return bad_arg(ctx, "inflate: null buffer");
     if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return bad_arg(ctx, "inflate: d_in must be 8-byte aligned");
-    // inflateReset2, inflate.ts:138-172
-    int wrap, d64 = 0;
-    if (window_bits < 0) {
-        if (window_bits < -16) return bad_arg(ctx, "inflate: windowBits out of range");
-        wrap = 0;
-        d64 = window_bits == -16;
-        window_bits = -window_bits;
-    } else {
-        wrap = ((window_bits >> 4) + 5) & 3;  // bit0 zlib, bit1 gzip
-        if (window_bits < 48) window_bits &= 15;
-    }
-    if (window_bits && (window_bits < 8 || window_bits > (d64 ? 16 : 15))) return bad_arg(ctx, "inflate: windowBits out of range");
+    int wrap, d64;
+    if (!zs_inflate_window_bits(window_bits, &wrap, &d64)) return bad_arg(ctx, "inflate: windowBits out of range");
 
     // misc scratch: detail[n] trailer[2n] flags[n] adler[n] crc[n] dict_adler[n] | dict off[n] len[n] (u64)
     uint32_t* misc = (uint32_t*)zs_scratch_get(ctx, SCR_I_MISC, (size_t)n * 7 * 4 + 16 + (size_t)n * 16);

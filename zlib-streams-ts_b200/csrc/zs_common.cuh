@@ -183,6 +183,68 @@ int zs_launch_checksum_fold(zs_ctx* ctx, int kind, const uint32_t* d_part, const
                             uint32_t init, uint32_t* d_result);
 uint32_t zs_host_crc32_combine(uint32_t c1, uint32_t c2, uint64_t len2);
 uint32_t zs_host_adler32_combine(uint32_t a1, uint32_t a2, uint64_t len2);
+// The check of a stream continued by len2 bytes whose own check is c2: adler32 for zlib, crc32 for gzip.
+inline uint32_t zs_host_check_combine(int wrap, uint32_t c1, uint32_t c2, uint64_t len2) {
+    return wrap == ZS_WRAP_ZLIB ? zs_host_adler32_combine(c1, c2, len2) : zs_host_crc32_combine(c1, c2, len2);
+}
+
+// ---- wrapper framing (deflate.ts:750-832, 964-988): the device's frame_kernel and the host paths --------
+__host__ __device__ inline void zs_put_be32(uint8_t* p, uint32_t x) {
+    p[0] = (uint8_t)(x >> 24); p[1] = (uint8_t)(x >> 16); p[2] = (uint8_t)(x >> 8); p[3] = (uint8_t)x;
+}
+// zlib header: CMF/FLG with FLEVEL from level and strategy (level_flags, deflate.ts:757-765), and with a preset
+// dictionary FDICT + DICTID (big-endian, putShortMSB twice).  Returns its length.
+__host__ __device__ inline unsigned zs_put_zlib_header(uint8_t* p, int level, int strategy, bool fdict, uint32_t dict_id) {
+    unsigned header = (8u + (7u << 4)) << 8;
+    const unsigned lf = (strategy >= ZS_STRATEGY_HUFFMAN_ONLY || level < 2) ? 0u : level < 6 ? 1u : level == 6 ? 2u : 3u;
+    header |= lf << 6;
+    if (fdict) header |= 0x20u;   // PRESET_DICT
+    header += 31u - header % 31u;
+    p[0] = (uint8_t)(header >> 8); p[1] = (uint8_t)header;
+    if (!fdict) return 2;
+    zs_put_be32(p + 2, dict_id);
+    return 6;
+}
+// gzip XFL, deflate.ts:796
+__host__ __device__ inline uint8_t zs_gzip_xfl(int level, int strategy) {
+    return level == 9 ? 2 : (strategy >= ZS_STRATEGY_HUFFMAN_ONLY || level < 2) ? 4 : 0;
+}
+// The trailer of a `wrap` stream: adler32 big-endian (zlib), crc32 and the input size mod 2^32 little-endian (gzip),
+// nothing (raw).  Returns its length.
+__host__ __device__ inline unsigned zs_put_trailer(uint8_t* p, int wrap, uint32_t check, uint64_t isize) {
+    if (wrap == ZS_WRAP_ZLIB) {
+        zs_put_be32(p, check);
+        return 4;
+    }
+    if (wrap != ZS_WRAP_GZIP) return 0;
+    p[0] = (uint8_t)check; p[1] = (uint8_t)(check >> 8); p[2] = (uint8_t)(check >> 16); p[3] = (uint8_t)(check >> 24);
+    p[4] = (uint8_t)isize; p[5] = (uint8_t)(isize >> 8); p[6] = (uint8_t)(isize >> 16); p[7] = (uint8_t)(isize >> 24);
+    return 8;
+}
+
+// inflateReset2's windowBits rules (inflate.ts:138-172), and raw deflate64 at -16: false for a value out of range.
+// `wrap` (bit0 zlib, bit1 gzip, 0 raw) and `deflate64` may be null.
+inline bool zs_inflate_window_bits(int window_bits, int* wrap, int* deflate64) {
+    int w, d64 = 0;
+    if (window_bits < 0) {
+        if (window_bits < -16) return false;
+        w = 0;
+        d64 = window_bits == -16;
+        window_bits = -window_bits;
+    } else {
+        w = ((window_bits >> 4) + 5) & 3;
+        if (window_bits < 48) window_bits &= 15;
+    }
+    if (window_bits && (window_bits < 8 || window_bits > (d64 ? 16 : 15))) return false;
+    if (wrap) *wrap = w;
+    if (deflate64) *deflate64 = d64;
+    return true;
+}
+// strm->adler after inflateInit2 / inflateReset2: 1 when a zlib header may come, else 0 (the window size then comes
+// from the header, or there is none)
+inline uint32_t zs_inflate_initial_adler(int window_bits) {
+    return (window_bits >= 0 && (((window_bits >> 4) + 5) & 1)) ? 1u : 0u;
+}
 
 // inflate
 struct zs_inflate_args {

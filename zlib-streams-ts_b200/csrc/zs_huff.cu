@@ -1041,24 +1041,14 @@ __global__ void frame_kernel(EncodeArgs a) {
     const bool last = stitched ? (c + 1 == a.n_chunks && !(a.flags & ZS_FLAG_NOT_LAST)) : true;
     uint8_t* hp = stitched ? a.out : a.out + a.out_off[c];
     if (first) {
+        const int strategy = (int)((a.flags >> 8) & 7u);
         if (a.wrap == ZS_WRAP_ZLIB) {
-            unsigned header = (8u + (7u << 4)) << 8;
-            // level_flags, deflate.ts:757-765
-            const int strategy = (int)((a.flags >> 8) & 7u);
-            unsigned lf = (strategy >= ZS_STRATEGY_HUFFMAN_ONLY || a.level < 2) ? 0u : a.level < 6 ? 1u : a.level == 6 ? 2u : 3u;
-            header |= lf << 6;
-            if (a.fdict) header |= 0x20u;   // PRESET_DICT: deflate() sets it when a dictionary was given (strstart != 0)
-            header += 31u - header % 31u;
-            hp[0] = (uint8_t)(header >> 8); hp[1] = (uint8_t)header;
-            if (a.fdict) {   // DICTID, big-endian (putShortMSB twice)
-                hp[2] = (uint8_t)(a.dict_id >> 24); hp[3] = (uint8_t)(a.dict_id >> 16);
-                hp[4] = (uint8_t)(a.dict_id >> 8); hp[5] = (uint8_t)a.dict_id;
-            }
+            // FDICT: deflate() sets it when a dictionary was given (strstart != 0)
+            zs_put_zlib_header(hp, a.level, strategy, a.fdict, a.dict_id);
         } else if (a.wrap == ZS_WRAP_GZIP) {
             hp[0] = 0x1f; hp[1] = 0x8b; hp[2] = 8;
             for (int k = 3; k < 8; k++) hp[k] = 0;
-            const int strategy = (int)((a.flags >> 8) & 7u);
-            hp[8] = a.level == 9 ? 2 : (strategy >= ZS_STRATEGY_HUFFMAN_ONLY || a.level < 2) ? 4 : 0;   // XFL, deflate.ts:796
+            hp[8] = zs_gzip_xfl(a.level, strategy);
             hp[9] = 255;  // OS_CODE of the reference, deflate/constants.ts:30
         }
     }
@@ -1077,12 +1067,7 @@ __global__ void frame_kernel(EncodeArgs a) {
             ck = a.checks[c];
             isize = a.in_off[c + 1] - a.in_off[c];
         }
-        if (a.wrap == ZS_WRAP_ZLIB) {
-            tp[0] = (uint8_t)(ck >> 24); tp[1] = (uint8_t)(ck >> 16); tp[2] = (uint8_t)(ck >> 8); tp[3] = (uint8_t)ck;
-        } else {
-            tp[0] = (uint8_t)ck; tp[1] = (uint8_t)(ck >> 8); tp[2] = (uint8_t)(ck >> 16); tp[3] = (uint8_t)(ck >> 24);
-            tp[4] = (uint8_t)isize; tp[5] = (uint8_t)(isize >> 8); tp[6] = (uint8_t)(isize >> 16); tp[7] = (uint8_t)(isize >> 24);
-        }
+        zs_put_trailer(tp, a.wrap, ck, isize);
     }
     (void)out32;
 }

@@ -36,52 +36,18 @@ namespace {
 // costs about as much as one such copy, so the large buffers are handed from stream to stream through a small
 // pool: the first long stream of a process pays for them, the following ones do not.
 constexpr size_t kPinAbove = 1u << 20;
-struct PinPool {
-    std::mutex mu;
-    struct Item { uint8_t* p; size_t cap; };
-    std::vector<Item> free_list;
-    uint8_t* take(size_t want, size_t* cap) {
-        {
-            std::lock_guard<std::mutex> g(mu);
-            size_t best = free_list.size();
-            for (size_t i = 0; i < free_list.size(); i++)
-                if (free_list[i].cap >= want && (best == free_list.size() || free_list[i].cap < free_list[best].cap)) best = i;
-            if (best < free_list.size()) {
-                Item it = free_list[best];
-                free_list.erase(free_list.begin() + best);
-                *cap = it.cap;
-                return it.p;
-            }
-        }
-        void* q = nullptr;
-        if (cudaHostAlloc(&q, want, cudaHostAllocPortable) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        *cap = want;
-        return (uint8_t*)q;
-    }
-    void give(uint8_t* p, size_t cap) {
-        {
-            std::lock_guard<std::mutex> g(mu);
-            size_t held = 0;
-            for (const Item& it : free_list) held += it.cap;
-            if (free_list.size() < kMaxItems && held + cap <= kMaxBytes) { free_list.push_back({p, cap}); return; }
-        }
-        cudaFreeHost(p);
-    }
-    static constexpr size_t kMaxItems = 8, kMaxBytes = 768u << 20;   // what the pool keeps page-locked between streams
-};
-PinPool& pin_pool() { static PinPool* pool = new PinPool(); return *pool; }   // never destroyed: outlives the CUDA runtime's teardown
 
-// The same for large buffers in ORDINARY memory (the inflate side): what is expensive about them is the first touch --
-// a device-to-host copy of 64 MiB into freshly mapped pages takes 41 ms on the B200 box, 3.7 ms into pages that have
-// been touched (profiles/pincost_r2.txt) -- so a stream's large buffers go to the next stream instead of back to the
-// allocator.  take() hands out the best fit, or the largest buffer there is (the caller grows it with realloc, which
-// keeps the touched pages).
-struct PagePool {
+// Large host buffers handed from stream to stream: take() hands out the best fit for `want` (or, with
+// `else_largest`, the largest buffer there is when none fits), give() keeps at most max_items buffers of max_bytes in
+// all and releases the rest.
+struct BufPool {
+    const size_t max_items, max_bytes;
+    void (*const release)(void*);
     std::mutex mu;
     struct Item { uint8_t* p; size_t cap; };
     std::vector<Item> free_list;
-    static constexpr size_t kMaxItems = 4, kMaxBytes = 512u << 20;
-    uint8_t* take(size_t want, size_t* cap) {
+    BufPool(size_t items, size_t bytes, void (*rel)(void*)) : max_items(items), max_bytes(bytes), release(rel) {}
+    uint8_t* take(size_t want, bool else_largest, size_t* cap) {
         std::lock_guard<std::mutex> g(mu);
         if (free_list.empty()) return nullptr;
         size_t best = free_list.size(), largest = 0;
@@ -89,7 +55,10 @@ struct PagePool {
             if (free_list[i].cap >= want && (best == free_list.size() || free_list[i].cap < free_list[best].cap)) best = i;
             if (free_list[i].cap > free_list[largest].cap) largest = i;
         }
-        if (best == free_list.size()) best = largest;
+        if (best == free_list.size()) {
+            if (!else_largest) return nullptr;
+            best = largest;
+        }
         Item it = free_list[best];
         free_list.erase(free_list.begin() + best);
         *cap = it.cap;
@@ -100,12 +69,19 @@ struct PagePool {
             std::lock_guard<std::mutex> g(mu);
             size_t held = 0;
             for (const Item& it : free_list) held += it.cap;
-            if (free_list.size() < kMaxItems && held + cap <= kMaxBytes) { free_list.push_back({p, cap}); return; }
+            if (free_list.size() < max_items && held + cap <= max_bytes) { free_list.push_back({p, cap}); return; }
         }
-        free(p);
+        release(p);
     }
 };
-PagePool& page_pool() { static PagePool* pool = new PagePool(); return *pool; }
+// Both pools are never destroyed: they outlive the CUDA runtime's teardown.
+// Page-locked buffers: what the pool keeps page-locked between streams.
+BufPool& pin_pool() { static BufPool* pool = new BufPool(8, 768u << 20, [](void* p) { cudaFreeHost(p); }); return *pool; }
+// The same for large buffers in ORDINARY memory (the inflate side): what is expensive about them is the first touch --
+// a device-to-host copy of 64 MiB into freshly mapped pages takes 41 ms on the B200 box, 3.7 ms into pages that have
+// been touched (profiles/pincost_r2.txt) -- so a stream's large buffers go to the next stream instead of back to the
+// allocator.
+BufPool& page_pool() { static BufPool* pool = new BufPool(4, 512u << 20, free); return *pool; }
 
 struct HostBuf {
     uint8_t* p = nullptr;
@@ -137,8 +113,13 @@ struct HostBuf {
         if (c < want) c = want;
         if (may_pin && c > kPinAbove) {
             if (c < part_hint) c = part_hint;
-            size_t got = 0;
-            uint8_t* q = pin_pool().take(c, &got);
+            size_t got = c;
+            uint8_t* q = pin_pool().take(c, false, &got);
+            if (!q) {   // none in the pool fits: page-lock a new one
+                void* h = nullptr;
+                if (cudaHostAlloc(&h, c, cudaHostAllocPortable) == cudaSuccess) q = (uint8_t*)h;
+                else cudaGetLastError();
+            }
             if (q) {
                 if (n) memcpy(q, p, n);
                 if (p) { if (pinned) pin_pool().give(p, cap); else free(p); }
@@ -155,8 +136,8 @@ struct HostBuf {
             return true;
         }
         if (cap <= kPinAbove && c > kPinAbove) {   // becoming large: a buffer whose pages have been touched, if there is one
-            size_t got = 0;
-            uint8_t* q = page_pool().take(c, &got);
+            size_t got = 0;   // (the largest one when none holds c: growing it with realloc keeps the touched pages)
+            uint8_t* q = page_pool().take(c, true, &got);
             if (q) {
                 if (n) memcpy(q, p, n);
                 free(p);
@@ -216,22 +197,26 @@ constexpr size_t kEveryCallBelow = 64u << 10;
 struct DeflateState {
     uint32_t magic = 0x44464c54;  // 'DFLT'
     zs_ctx* ctx = nullptr;
-    int level = 6, strategy = 0, wrap = 1, status = ST_INIT, last_flush = -2;
-    std::vector<uint8_t> hist;      // last <= 32 KiB already compressed (or the preset dictionary)
+    int level = 6, strategy = 0, wrap = 1;
     HostBuf in;                     // buffered, not yet compressed: at most one part (kPartThreshold)
     HostBuf out;                    // compressed, not yet delivered
-    size_t out_pos = 0;
     // A part that was started because a whole part of input had piled up runs in the BACKGROUND: its copies and
     // kernels are queued on the context's stream and the call returns, so the caller buffers the next part while the
     // GPU compresses this one (the zlib contract lets deflate(Z_NO_FLUSH) hold output back).  Its input stays in
     // `in_flight`, its output lands in `out` behind the bytes that are waiting there, followed by the result record;
     // harvest() -- before the next part, on any flush, on a call without input, at deflateEnd -- waits for it.
     HostBuf in_flight;
-    bool pending = false, p_first = false;
-    size_t p_old = 0, p_cap = 0, p_cap_al = 0, p_n = 0;
-    bool header_done = false, any_part = false, trailer_done = false, have_dict = false;
-    uint32_t check = 0, dict_id = 0;
-    uint64_t total_in_len = 0;
+    // What deflateReset starts afresh (the buffers above keep their memory)
+    struct Progress {
+        int status = ST_INIT, last_flush = -2;
+        std::vector<uint8_t> hist;      // last <= 32 KiB already compressed (or the preset dictionary)
+        size_t out_pos = 0;
+        bool pending = false;           // a part is in flight: p_old, p_cap, p_cap_al, p_n describe it
+        size_t p_old = 0, p_cap = 0, p_cap_al = 0, p_n = 0;
+        bool header_done = false, any_part = false, trailer_done = false, have_dict = false;
+        uint32_t check = 0, dict_id = 0;
+        uint64_t total_in_len = 0;
+    } prog;
     // deflateSetHeader: a copy of the caller's gzip header fields
     bool gz_custom = false, gz_has_extra = false, gz_has_name = false, gz_has_comment = false;
     int gz_text = 0, gz_os = 0, gz_hcrc = 0;
@@ -251,32 +236,35 @@ struct InflateState {
     // resumes there in raw mode with the last 64 KiB of output as its window.
     HostBuf in;                     // input not yet consumed: from the byte that holds the next block header on
     HostBuf out;                    // output of the latest attempt (from the resume point); page-locked once it is large
-    bool out_on_device = false;     // `out` is byte for byte what the last attempt left on the device at out_dev ...
-    const uint8_t* out_dev = nullptr;
-    uint64_t out_gen = 0;           // ... as long as the context has not handed that scratch out again (InflateOut)
     HostBuf ready;                  // decoded, not yet delivered
-    std::vector<uint8_t> hist;      // window: the last <= 64 KiB of final output, or the preset dictionary
-    std::vector<uint8_t> leftover;  // input after the end of the stream that could not be handed back
-    size_t ready_pos = 0;           // delivered part of `ready`
-    size_t out_pushed = 0;          // bytes of `out` already copied to `ready`
-    size_t next_attempt = 0;
-    bool fresh_input = false;       // input has arrived since the last attempt
-    uint32_t in_tail = 1;           // the last 4 input bytes received, across calls (big endian; 1 = none yet)
-    double attempt_end = 0.0;       // monotonic clock at the end of the last attempt ...
-    double attempt_cost = 0.0;      // ... and how long it took (seconds): the pacing of a long stream's attempts
-    size_t out_cap_hint = 1 << 20;
-    bool body = false;              // the wrapper header is behind us: raw blocks from start_bit
-    uint64_t start_bit = 0;         // of the next block header inside `in`
-    int trailer = 0;                // 0 none (raw), 1 zlib (adler32), 2 gzip (crc32 + isize)
-    uint32_t run_check = 0;         // checksum of the final output so far (adler32 for zlib, crc32 otherwise)
-    uint64_t run_len = 0;           // its length
-    bool await_trailer = false;     // the last block is decoded, the trailer bytes are not all here yet
-    size_t trailer_pos = 0;         // where they start inside `in`
-    bool done = false, failed = false, need_dict = false, have_dict = false;
-    int fail_code = 0;
-    const char* fail_msg = "";
-    uint32_t check = 0;
-    zs_gz_header* gzhead = nullptr;   // inflateGetHeader
+    std::vector<uint8_t> leftover;  // input after the end of the stream that could not be handed back (inflateReset keeps it)
+    size_t out_cap_hint = 1 << 20;  // (a capacity hint: inflateReset keeps it, a smaller one would cost a re-decode)
+    // What inflateReset starts afresh (the buffers above keep their memory)
+    struct Progress {
+        bool out_on_device = false;     // `out` is byte for byte what the last attempt left on the device at out_dev ...
+        const uint8_t* out_dev = nullptr;
+        uint64_t out_gen = 0;           // ... as long as the context has not handed that scratch out again (InflateOut)
+        std::vector<uint8_t> hist;      // window: the last <= 64 KiB of final output, or the preset dictionary
+        size_t ready_pos = 0;           // delivered part of `ready`
+        size_t out_pushed = 0;          // bytes of `out` already copied to `ready`
+        size_t next_attempt = 0;
+        bool fresh_input = false;       // input has arrived since the last attempt
+        uint32_t in_tail = 1;           // the last 4 input bytes received, across calls (big endian; 1 = none yet)
+        double attempt_end = 0.0;       // monotonic clock at the end of the last attempt ...
+        double attempt_cost = 0.0;      // ... and how long it took (seconds): the pacing of a long stream's attempts
+        bool body = false;              // the wrapper header is behind us: raw blocks from start_bit
+        uint64_t start_bit = 0;         // of the next block header inside `in`
+        int trailer = 0;                // 0 none (raw), 1 zlib (adler32), 2 gzip (crc32 + isize)
+        uint32_t run_check = 0;         // checksum of the final output so far (adler32 for zlib, crc32 otherwise)
+        uint64_t run_len = 0;           // its length
+        bool await_trailer = false;     // the last block is decoded, the trailer bytes are not all here yet
+        size_t trailer_pos = 0;         // where they start inside `in`
+        bool done = false, failed = false, need_dict = false, have_dict = false;
+        int fail_code = 0;
+        const char* fail_msg = "";
+        uint32_t check = 0;
+        zs_gz_header* gzhead = nullptr;   // inflateGetHeader (inflateReset drops the request)
+    } prog;
     // The inflate buffers stay in ordinary memory: their sizes follow the stream (four times the buffered input, what
     // is waiting for delivery), so page-locked ones would rarely be reusable from stream to stream, and page-locking
     // 100 MiB anew costs more than the pageable copy it replaces (measured through the stream API: 0.39-0.91 GB/s,
@@ -306,15 +294,6 @@ InflateState* istate(zs_stream* s) {
 }
 
 
-void put_be32(HostBuf& v, uint32_t x) {
-    const uint8_t b[4] = {(uint8_t)(x >> 24), (uint8_t)(x >> 16), (uint8_t)(x >> 8), (uint8_t)x};
-    v.append(b, 4, 0);
-}
-void put_le32(HostBuf& v, uint32_t x) {
-    const uint8_t b[4] = {(uint8_t)x, (uint8_t)(x >> 8), (uint8_t)(x >> 16), (uint8_t)(x >> 24)};
-    v.append(b, 4, 0);
-}
-
 // crc32 of a few header bytes on the host (framing only; payload checksums are computed on the GPU)
 uint32_t host_crc32(const uint8_t* p, size_t n) {
     uint32_t c = 0xffffffffu;
@@ -332,7 +311,7 @@ void put_gzip_header(DeflateState* st) {
     h.push_back((uint8_t)((st->gz_text ? 1 : 0) + (st->gz_hcrc ? 2 : 0) + (st->gz_has_extra ? 4 : 0) +
                           (st->gz_has_name ? 8 : 0) + (st->gz_has_comment ? 16 : 0)));
     for (int k = 0; k < 4; k++) h.push_back((uint8_t)(st->gz_time >> (8 * k)));
-    h.push_back((uint8_t)(st->level == 9 ? 2 : (st->strategy >= 2 || st->level < 2) ? 4 : 0));
+    h.push_back(zs_gzip_xfl(st->level, st->strategy));
     h.push_back((uint8_t)st->gz_os);
     if (st->gz_has_extra) {
         const uint32_t n = (uint32_t)st->gz_extra.size() & 0xffffu;
@@ -348,29 +327,63 @@ void put_gzip_header(DeflateState* st) {
     st->out.append(h.data(), h.size(), 0);
 }
 
+// A part is done and `res` is its result: fold its check into the stream's running check (read_buf,
+// deflate.ts:155-159) and count its n bytes of input.
+int end_part(zs_stream* strm, DeflateState* st, const zs_deflate_result& res, uint64_t cap, size_t n) {
+    DeflateState::Progress& p = st->prog;
+    if (res.total_out_bytes > cap) return ZS_BUF_ERROR;
+    if (st->wrap != ZS_WRAP_RAW) {
+        p.check = p.total_in_len || p.any_part ? zs_host_check_combine(st->wrap, p.check, res.check, n) : res.check;
+        strm->adler = p.check;
+    }
+    p.total_in_len += n;
+    p.header_done = true;
+    p.any_part = true;
+    return ZS_OK;
+}
+
+// History for the next part: the last 32 KiB of (history + the part's input).
+void keep_history(std::vector<uint8_t>& hist, const HostBuf& in) {
+    const size_t hist_len = hist.size(), total = hist_len + in.size(), keep = total < 32768 ? total : 32768;
+    std::vector<uint8_t> h(keep);
+    for (size_t i = 0; i < keep; i++) {
+        size_t idx = total - keep + i;
+        h[i] = idx < hist_len ? hist[idx] : in[idx - hist_len];
+    }
+    hist.swap(h);
+}
+
 // Wait for the part in flight (if any) and take its output and checksum.
 int harvest(zs_stream* strm, DeflateState* st) {
-    if (!st->pending) return ZS_OK;
+    DeflateState::Progress& p = st->prog;
+    if (!p.pending) return ZS_OK;
     zs_ctx* ctx = st->ctx;
-    st->pending = false;
+    p.pending = false;
     const double t0 = now_s();
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     st->t_part += now_s() - t0;
     zs_deflate_result res;
-    memcpy(&res, st->out.data() + st->p_old + st->p_cap_al, sizeof(res));
-    if (res.total_out_bytes > st->p_cap) return ZS_BUF_ERROR;
-    st->out.n = st->p_old + (size_t)res.total_out_bytes;
-    if (st->wrap == ZS_WRAP_ZLIB) st->check = st->p_first ? res.check : zs_host_adler32_combine(st->check, res.check, st->p_n);
-    else if (st->wrap == ZS_WRAP_GZIP) st->check = st->p_first ? res.check : zs_host_crc32_combine(st->check, res.check, st->p_n);
-    if (st->wrap != ZS_WRAP_RAW) strm->adler = st->check;
+    memcpy(&res, st->out.data() + p.p_old + p.p_cap_al, sizeof(res));
+    const int rc = end_part(strm, st, res, p.p_cap, p.p_n);
+    if (rc != ZS_OK) return rc;
+    st->out.n = p.p_old + (size_t)res.total_out_bytes;
     st->in_flight.clear();
     return ZS_OK;
 }
 
+// Wait for the part in flight (if any) without taking its output: before its buffers are cleared or released.
+void wait_part(DeflateState* st) {
+    if (!st->prog.pending) return;
+    cudaSetDevice(st->ctx->device);
+    cudaStreamSynchronize(st->ctx->stream);
+    st->prog.pending = false;
+}
+
 // Compress everything buffered as one part.  `finish` makes it the last part of the stream; `background`: queue it
-// and return (see DeflateState::pending).
+// and return (see DeflateState::in_flight).
 int run_part(zs_stream* strm, DeflateState* st, bool finish, bool full_flush, bool background = false) {
     zs_ctx* ctx = st->ctx;
+    DeflateState::Progress& p = st->prog;
     cudaSetDevice(ctx->device);
     {
         const int rc = harvest(strm, st);
@@ -378,26 +391,20 @@ int run_part(zs_stream* strm, DeflateState* st, bool finish, bool full_flush, bo
     }
     const double t_part0 = now_s();
     struct PartTimer { DeflateState* s; double t0; ~PartTimer() { s->t_part += now_s() - t0; s->n_parts++; } } part_timer{st, t_part0};
-    const size_t hist_len = st->hist.size(), n = st->in.size();
+    const size_t hist_len = p.hist.size(), n = st->in.size();
     // zlib header with a preset dictionary carries FDICT + DICTID: host framing (deflate.ts:754-777)
-    if (!st->header_done && st->wrap == ZS_WRAP_ZLIB && st->have_dict) {
-        unsigned header = (8u + (7u << 4)) << 8;
-        unsigned lf = (st->strategy >= 2 || st->level < 2) ? 0u : st->level < 6 ? 1u : st->level == 6 ? 2u : 3u;
-        header |= lf << 6;
-        header |= 0x20;
-        header += 31u - header % 31u;
-        st->out.push_back((uint8_t)(header >> 8));
-        st->out.push_back((uint8_t)header);
-        put_be32(st->out, st->dict_id);
-        st->header_done = true;
+    if (!p.header_done && st->wrap == ZS_WRAP_ZLIB && p.have_dict) {
+        uint8_t h[6];
+        st->out.append(h, zs_put_zlib_header(h, st->level, st->strategy, true, p.dict_id), 0);
+        p.header_done = true;
     }
-    if (!st->header_done && st->wrap == ZS_WRAP_GZIP && st->gz_custom) {
+    if (!p.header_done && st->wrap == ZS_WRAP_GZIP && st->gz_custom) {
         put_gzip_header(st);
-        st->header_done = true;
+        p.header_done = true;
     }
-    const bool whole = !st->any_part && finish && !st->header_done;  // the GPU frames a single-part stream completely
+    const bool whole = !p.any_part && finish && !p.header_done;  // the GPU frames a single-part stream completely
     uint32_t flags = ZS_FLAG_SYNC | ZS_FLAG_STRATEGY(st->strategy);
-    if (st->header_done || st->any_part) flags |= ZS_FLAG_NOT_FIRST;
+    if (p.header_done || p.any_part) flags |= ZS_FLAG_NOT_FIRST;
     if (!finish) flags |= ZS_FLAG_NOT_LAST;
     const uint32_t chunk = n >= (148u * 4u * 262144u) ? 262144u : 65536u;
     const uint32_t n_chunks = n ? (uint32_t)((n + chunk - 1) / chunk) : 1u;
@@ -415,7 +422,7 @@ int run_part(zs_stream* strm, DeflateState* st, bool finish, bool full_flush, bo
     // history and input are contiguous on the device; keep the input 16-byte aligned
     const size_t pad = (16 - (hist_len & 15)) & 15;
     uint8_t* d_hist = d_in_buf + pad;
-    if (hist_len) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_hist, st->hist.data(), hist_len, cudaMemcpyHostToDevice, ctx->stream));
+    if (hist_len) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_hist, p.hist.data(), hist_len, cudaMemcpyHostToDevice, ctx->stream));
     if (n) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_hist + hist_len, st->in.data(), n, cudaMemcpyHostToDevice, ctx->stream));
     zs_deflate_result* d_result = (zs_deflate_result*)d_res_buf;
     int rc = zs_deflate_batch_dev(ctx, d_hist + hist_len, n, nullptr, n_chunks, chunk, chunk, (uint32_t)hist_len, st->level,
@@ -423,30 +430,17 @@ int run_part(zs_stream* strm, DeflateState* st, bool finish, bool full_flush, bo
     if (rc != ZS_OK) return rc;
     if (background && !finish && !full_flush) {
         // what is still waiting in `out` moves to its front, the part's output (as much as it can be: its size is
-        // known only when the kernels are done) and the result record are copied behind it
-        if (st->out_pos == st->out.size()) st->out.clear();
-        else if (st->out_pos) st->out.erase_front(st->out_pos);
-        st->out_pos = 0;
+        // known only when the kernels are done) and the result record are copied behind it; harvest() ends the part
+        if (p.out_pos == st->out.size()) st->out.clear();
+        else if (p.out_pos) st->out.erase_front(p.out_pos);
+        p.out_pos = 0;
         const size_t old = st->out.size(), cap_al = ((size_t)cap + 15) & ~(size_t)15;
         if (!st->out.reserve(old + cap_al + 64, kPartOutHint)) return ZS_MEM_ERROR;
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(st->out.data() + old + cap_al, d_result, sizeof(zs_deflate_result), cudaMemcpyDeviceToHost, ctx->stream));
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(st->out.data() + old, d_out_buf, cap, cudaMemcpyDeviceToHost, ctx->stream));
-        st->pending = true;
-        st->p_old = old; st->p_cap = (size_t)cap; st->p_cap_al = cap_al; st->p_n = n;
-        st->p_first = !(st->total_in_len || st->any_part);
-        st->total_in_len += n;
-        st->header_done = true;
-        st->any_part = true;
-        {   // history for the next part: the last 32 KiB of (history + input)
-            std::vector<uint8_t> h;
-            const size_t total = hist_len + n, keep = total < 32768 ? total : 32768;
-            h.resize(keep);
-            for (size_t i = 0; i < keep; i++) {
-                size_t idx = total - keep + i;
-                h[i] = idx < hist_len ? st->hist[idx] : st->in[idx - hist_len];
-            }
-            st->hist.swap(h);
-        }
+        p.pending = true;
+        p.p_old = old; p.p_cap = (size_t)cap; p.p_cap_al = cap_al; p.p_n = n;
+        keep_history(p.hist, st->in);
         st->in.swap(st->in_flight);   // the copy engine is still reading it
         st->in.clear();
         return ZS_OK;
@@ -454,39 +448,22 @@ int run_part(zs_stream* strm, DeflateState* st, bool finish, bool full_flush, bo
     zs_deflate_result res;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&res, d_result, sizeof(res), cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (res.total_out_bytes > cap) return ZS_BUF_ERROR;
+    rc = end_part(strm, st, res, cap, n);
+    if (rc != ZS_OK) return rc;
     const size_t old = st->out.size();
     const double t_d2h0 = now_s();
     if (!st->out.grow(res.total_out_bytes, kPartOutHint)) return ZS_MEM_ERROR;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(st->out.data() + old, d_out_buf, res.total_out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     st->t_d2h += now_s() - t_d2h0;
-    // running check over the uncompressed data (read_buf, deflate.ts:155-159)
-    if (st->wrap == ZS_WRAP_ZLIB) st->check = st->total_in_len || st->any_part ? zs_host_adler32_combine(st->check, res.check, n) : res.check;
-    else if (st->wrap == ZS_WRAP_GZIP) st->check = st->total_in_len || st->any_part ? zs_host_crc32_combine(st->check, res.check, n) : res.check;
-    st->total_in_len += n;
-    if (st->wrap != ZS_WRAP_RAW) strm->adler = st->check;
-    st->header_done = true;
-    st->any_part = true;
-    if (finish && !whole && !st->trailer_done) {
-        // trailer of a multi-part stream (deflate.ts:964-988)
-        if (st->wrap == ZS_WRAP_ZLIB) put_be32(st->out, st->check);
-        else if (st->wrap == ZS_WRAP_GZIP) { put_le32(st->out, st->check); put_le32(st->out, (uint32_t)st->total_in_len); }
+    if (finish && !whole && !p.trailer_done) {   // trailer of a multi-part stream (deflate.ts:964-988)
+        uint8_t t[8];
+        st->out.append(t, zs_put_trailer(t, st->wrap, p.check, p.total_in_len), 0);
     }
-    if (finish) st->trailer_done = true;
-    // history for the next part: the last 32 KiB of (history + input); none after Z_FULL_FLUSH
-    if (full_flush || finish) {
-        st->hist.clear();
-    } else {
-        std::vector<uint8_t> h;
-        const size_t total = hist_len + n, keep = total < 32768 ? total : 32768;
-        h.resize(keep);
-        for (size_t i = 0; i < keep; i++) {
-            size_t idx = total - keep + i;
-            h[i] = idx < hist_len ? st->hist[idx] : st->in[idx - hist_len];
-        }
-        st->hist.swap(h);
-    }
+    if (finish) p.trailer_done = true;
+    // none after Z_FULL_FLUSH
+    if (full_flush || finish) p.hist.clear();
+    else keep_history(p.hist, st->in);
     st->in.clear();
     return ZS_OK;
 }
@@ -531,7 +508,7 @@ int zs_stream_deflate_init(zs_ctx* ctx, zs_stream* strm, int level, int method, 
     st->level = level;
     st->strategy = strategy;
     st->wrap = wrap;
-    st->status = ST_INIT;
+    st->prog.status = ST_INIT;
     st->t_created = now_s();
     strm->state = st;
     strm->total_in = strm->total_out = 0;
@@ -544,24 +521,24 @@ int zs_stream_deflate_set_dictionary(zs_stream* strm, const uint8_t* dict, uint3
     DeflateState* st = dstate(strm);
     if (!st || !dict) return ZS_STREAM_ERROR;
     // deflate.ts:372-375: not for gzip, for zlib only before the first deflate call, never mid-block
-    if (st->wrap == 2 || (st->wrap == 1 && st->status != ST_INIT) || !st->in.empty()) return ZS_STREAM_ERROR;
+    if (st->wrap == 2 || (st->wrap == 1 && st->prog.status != ST_INIT) || !st->in.empty()) return ZS_STREAM_ERROR;
     if (st->wrap == 1) {
         uint32_t id = 0;
         int rc = zs_checksum(st->ctx, 0, dict, dict_len, strm->adler, &id);
         if (rc != ZS_OK) return rc;
         strm->adler = id;
-        st->dict_id = id;
-        st->have_dict = true;
+        st->prog.dict_id = id;
+        st->prog.have_dict = true;
     }
     const uint32_t keep = dict_len < 32768 ? dict_len : 32768;
-    st->hist.assign(dict + (dict_len - keep), dict + dict_len);
+    st->prog.hist.assign(dict + (dict_len - keep), dict + dict_len);
     return ZS_OK;
 }
 
 int zs_stream_deflate(zs_stream* strm, int flush) {
     DeflateState* st = dstate(strm);
     if (!st || flush > ZS_BLOCK || flush < 0) return ZS_STREAM_ERROR;
-    if (!strm->next_out || (strm->avail_in != 0 && !strm->next_in) || (st->status == ST_FINISH && flush != ZS_FINISH)) {
+    if (!strm->next_out || (strm->avail_in != 0 && !strm->next_in) || (st->prog.status == ST_FINISH && flush != ZS_FINISH)) {
         strm->msg = "stream error";
         return ZS_STREAM_ERROR;
     }
@@ -569,23 +546,23 @@ int zs_stream_deflate(zs_stream* strm, int flush) {
     cudaSetDevice(st->ctx->device);   // (the buffers below may be page-locked: on this context's device, not on device 0)
     st->n_calls++;
     // a part in flight is waited for when the caller asks for output (a call without input, any flush request)
-    if (st->pending && (strm->avail_in == 0 || flush != ZS_NO_FLUSH)) {
+    if (st->prog.pending && (strm->avail_in == 0 || flush != ZS_NO_FLUSH)) {
         const int rc = harvest(strm, st);
         if (rc != ZS_OK) { strm->msg = zs_last_error(st->ctx); return rc; }
     }
-    const int old_flush = st->last_flush;
-    st->last_flush = flush;
-    if (st->out_pos < st->out.size()) {
-        drain(strm, st->out, st->out_pos, st->pending);
-        if (strm->avail_out == 0) { st->last_flush = -1; return ZS_OK; }
+    const int old_flush = st->prog.last_flush;
+    st->prog.last_flush = flush;
+    if (st->prog.out_pos < st->out.size()) {
+        drain(strm, st->out, st->prog.out_pos, st->prog.pending);
+        if (strm->avail_out == 0) { st->prog.last_flush = -1; return ZS_OK; }
     } else if (strm->avail_in == 0 && rank_of(flush) <= rank_of(old_flush) && flush != ZS_FINISH) {
         strm->msg = "buffer error";
         return ZS_BUF_ERROR;
     }
-    if (st->status == ST_FINISH && strm->avail_in != 0) { strm->msg = "buffer error"; return ZS_BUF_ERROR; }
-    if (st->status == ST_INIT) {
-        if (st->wrap == 1 && !st->have_dict) strm->adler = 1u;
-        st->status = ST_BUSY;
+    if (st->prog.status == ST_FINISH && strm->avail_in != 0) { strm->msg = "buffer error"; return ZS_BUF_ERROR; }
+    if (st->prog.status == ST_INIT) {
+        if (st->wrap == 1 && !st->prog.have_dict) strm->adler = 1u;
+        st->prog.status = ST_BUSY;
     }
     // Input is buffered one part at a time: a call that brings more than a part compresses full parts as it goes
     // and comes back for output room when a part's output does not fit (Z_OK with avail_in > 0, as in the reference).
@@ -598,28 +575,28 @@ int zs_stream_deflate(zs_stream* strm, int flush) {
         strm->next_in += take;
         strm->total_in += take;
         strm->avail_in -= take;
-        if (strm->avail_in == 0 || st->status != ST_BUSY) break;
+        if (strm->avail_in == 0 || st->prog.status != ST_BUSY) break;
         const int rc = run_part(strm, st, false, false, true);
         if (rc != ZS_OK) {
             strm->msg = zs_last_error(st->ctx);
             return rc;
         }
-        drain(strm, st->out, st->out_pos, st->pending);
-        if (st->out_pos < st->out.size()) { st->last_flush = -1; return ZS_OK; }
+        drain(strm, st->out, st->prog.out_pos, st->prog.pending);
+        if (st->prog.out_pos < st->out.size()) { st->prog.last_flush = -1; return ZS_OK; }
     }
-    if (st->status == ST_BUSY) {
+    if (st->prog.status == ST_BUSY) {
         int rc = ZS_OK;
         if (flush == ZS_FINISH) {
             rc = run_part(strm, st, true, false);
-            if (rc == ZS_OK) st->status = ST_FINISH;
+            if (rc == ZS_OK) st->prog.status = ST_FINISH;
         } else if (flush != ZS_NO_FLUSH) {
-            if (!st->in.empty() || !st->any_part) {
+            if (!st->in.empty() || !st->prog.any_part) {
                 rc = run_part(strm, st, false, flush == ZS_FULL_FLUSH);
             } else {
                 // nothing new since the last flush point: just the marker (deflate.ts:945-946)
                 static const uint8_t marker[5] = {0, 0, 0, 0xff, 0xff};
                 st->out.append(marker, 5, 0);
-                if (flush == ZS_FULL_FLUSH) st->hist.clear();
+                if (flush == ZS_FULL_FLUSH) st->prog.hist.clear();
             }
         } else if (st->in.size() >= kPartThreshold) {
             rc = run_part(strm, st, false, false, true);
@@ -631,10 +608,10 @@ int zs_stream_deflate(zs_stream* strm, int flush) {
     }
     {
         const double t0 = now_s();
-        drain(strm, st->out, st->out_pos, st->pending);
+        drain(strm, st->out, st->prog.out_pos, st->prog.pending);
         st->t_drain += now_s() - t0;
     }
-    if (flush == ZS_FINISH && st->status == ST_FINISH && st->out_pos >= st->out.size()) return ZS_STREAM_END;
+    if (flush == ZS_FINISH && st->prog.status == ST_FINISH && st->prog.out_pos >= st->out.size()) return ZS_STREAM_END;
     return ZS_OK;
 }
 
@@ -642,14 +619,9 @@ int zs_stream_deflate(zs_stream* strm, int flush) {
 int zs_stream_deflate_reset(zs_stream* strm) {
     DeflateState* st = dstate(strm);
     if (!st) return ZS_STREAM_ERROR;
-    if (st->pending) { cudaSetDevice(st->ctx->device); cudaStreamSynchronize(st->ctx->stream); st->pending = false; }   // (nobody writes the buffers any more)
-    st->hist.clear(); st->in.clear(); st->in_flight.clear(); st->out.clear();
-    st->out_pos = 0;
-    st->header_done = st->any_part = st->trailer_done = st->have_dict = false;
-    st->check = st->dict_id = 0;
-    st->total_in_len = 0;
-    st->status = ST_INIT;
-    st->last_flush = -2;
+    wait_part(st);
+    st->in.clear(); st->in_flight.clear(); st->out.clear();
+    st->prog = {};
     strm->total_in = strm->total_out = 0;
     strm->msg = "";
     strm->data_type = 2;
@@ -667,10 +639,10 @@ int zs_stream_deflate_params(zs_stream* strm, int level, int strategy) {
     if (level < 0 || level > 9 || strategy < 0 || strategy > 4) return ZS_STREAM_ERROR;
     const bool lazy_old = st->level >= 4, lazy_new = level >= 4;
     const bool func_changes = (st->level == 0) != (level == 0) || lazy_old != lazy_new;
-    if ((strategy != st->strategy || func_changes) && st->last_flush != -2) {
+    if ((strategy != st->strategy || func_changes) && st->prog.last_flush != -2) {
         const int err = zs_stream_deflate(strm, ZS_BLOCK);
         if (err == ZS_STREAM_ERROR) return err;
-        if (strm->avail_in || !st->in.empty() || st->out_pos < st->out.size()) return ZS_BUF_ERROR;
+        if (strm->avail_in || !st->in.empty() || st->prog.out_pos < st->out.size()) return ZS_BUF_ERROR;
     }
     st->level = level;
     st->strategy = strategy;
@@ -684,7 +656,7 @@ int zs_stream_deflate_pending(zs_stream* strm, uint32_t* pending, int* bits) {
     DeflateState* st = dstate(strm);
     if (!st) return ZS_STREAM_ERROR;
     if (pending) {
-        const size_t n = st->out.size() - st->out_pos;
+        const size_t n = st->out.size() - st->prog.out_pos;
         *pending = n > 0xffffffffull ? 0xffffffffu : (uint32_t)n;
     }
     if (bits) *bits = 0;
@@ -711,8 +683,8 @@ int zs_stream_deflate_set_header(zs_stream* strm, const zs_gz_header* head) {
 int zs_stream_deflate_end(zs_stream* strm) {
     DeflateState* st = dstate(strm);
     if (!st) return ZS_STREAM_ERROR;
-    const int status = st->status;
-    if (st->pending) { cudaSetDevice(st->ctx->device); cudaStreamSynchronize(st->ctx->stream); st->pending = false; }   // before the buffers go back to the pool
+    const int status = st->prog.status;
+    wait_part(st);   // before the buffers go back to the pool
     if (getenv("ZS_STREAM_PROF")) {
         const double t0 = now_s();
         const unsigned long long tin = strm->total_in;
@@ -732,58 +704,54 @@ int zs_stream_deflate_end(zs_stream* strm) {
 int zs_stream_inflate_init(zs_ctx* ctx, zs_stream* strm, int window_bits) {
     if (!strm || !ctx) return ZS_STREAM_ERROR;
     strm->msg = "";
-    // inflateReset2, inflate.ts:138-172
-    int wb = window_bits;
-    if (wb < 0) {
-        if (wb < -16) return ZS_STREAM_ERROR;
-        wb = -wb;
-        if (wb < 8) return ZS_STREAM_ERROR;
-    } else {
-        if (wb < 48) wb &= 15;
-        if (wb && (wb < 8 || wb > 15)) return ZS_STREAM_ERROR;
-    }
+    if (!zs_inflate_window_bits(window_bits, nullptr, nullptr)) return ZS_STREAM_ERROR;
     InflateState* st = new InflateState();
     st->ctx = ctx;
     st->window_bits = window_bits;
     strm->state = st;
     strm->total_in = strm->total_out = 0;
-    strm->adler = (window_bits >= 0 && (((window_bits >> 4) + 5) & 1)) ? 1u : 0u;   // 0 = window size from the zlib header
+    strm->adler = zs_inflate_initial_adler(window_bits);
     strm->data_type = 0;
     return ZS_OK;
+}
+
+// DICTID of a zlib stream that asks for a dictionary: bytes 2..5 of the buffered stream (0 while they are not all here)
+static uint32_t dict_id(const InflateState* st) {
+    const HostBuf& b = st->in;
+    return b.size() >= 6 ? ((uint32_t)b[2] << 24 | (uint32_t)b[3] << 16 | (uint32_t)b[4] << 8 | b[5]) : 0u;
 }
 
 int zs_stream_inflate_set_dictionary(zs_stream* strm, const uint8_t* dict, uint32_t dict_len) {
     InflateState* st = istate(strm);
     if (!st || !dict) return ZS_STREAM_ERROR;
     // inflate.ts:1229: raw streams any time before data, wrapped streams only when Z_NEED_DICT was returned
-    if (st->window_bits >= 0 && !st->need_dict) return ZS_STREAM_ERROR;
-    if (st->need_dict) {
-        // DICTID check (inflate.ts:1233-1238): bytes 2..5 of the zlib stream
+    if (st->window_bits >= 0 && !st->prog.need_dict) return ZS_STREAM_ERROR;
+    if (st->prog.need_dict) {
+        // DICTID check (inflate.ts:1233-1238)
         uint32_t id = 0;
         int rc = zs_checksum(st->ctx, 0, dict, dict_len, 1u, &id);
         if (rc != ZS_OK) return rc;
-        uint32_t want = st->in.size() >= 6 ? ((uint32_t)st->in[2] << 24 | (uint32_t)st->in[3] << 16 | (uint32_t)st->in[4] << 8 | st->in[5]) : 0u;
-        if (id != want) return ZS_DATA_ERROR;
-        st->need_dict = false;
+        if (id != dict_id(st)) return ZS_DATA_ERROR;
+        st->prog.need_dict = false;
         // the 2-byte header and the DICTID are behind us: raw blocks from byte 6, adler32 trailer
-        st->body = true;
-        st->start_bit = 48;
-        st->trailer = 1;
-        st->run_check = 1u;
-        st->run_len = 0;
+        st->prog.body = true;
+        st->prog.start_bit = 48;
+        st->prog.trailer = 1;
+        st->prog.run_check = 1u;
+        st->prog.run_len = 0;
     }
     const uint32_t keep = dict_len < 65536 ? dict_len : 65536;
-    st->hist.assign(dict + (dict_len - keep), dict + dict_len);
-    st->have_dict = true;
-    st->next_attempt = 0;
+    st->prog.hist.assign(dict + (dict_len - keep), dict + dict_len);
+    st->prog.have_dict = true;
+    st->prog.next_attempt = 0;
     return ZS_OK;
 }
 
 // inflateGetHeader: fill the caller's struct from the buffered start of the stream (host framing; the
 // kernel parses and checks the header on its own, inflate.ts:423-580).
 static void fill_gz_header(InflateState* st) {
-    zs_gz_header* g = st->gzhead;
-    if (!g || g->done != 0 || st->body) return;   // `in` starts at the stream start only until the first resume
+    zs_gz_header* g = st->prog.gzhead;
+    if (!g || g->done != 0 || st->prog.body) return;   // `in` starts at the stream start only until the first resume
     const HostBuf& b = st->in;
     if (b.size() < 2) return;
     if (!(b[0] == 0x1f && b[1] == 0x8b)) { g->done = -1; return; }   // a zlib stream (windowBits 32+), inflate.ts:404
@@ -825,18 +793,18 @@ static void fill_gz_header(InflateState* st) {
 
 // Everything of `out` below `upto` that has not been queued for delivery yet goes to `ready`.
 static void push_ready(InflateState* st, size_t upto) {
-    if (upto > st->out_pushed) {
-        st->ready.append(st->out.data() + st->out_pushed, upto - st->out_pushed, 0);
-        st->out_pushed = upto;
+    if (upto > st->prog.out_pushed) {
+        st->ready.append(st->out.data() + st->prog.out_pushed, upto - st->prog.out_pushed, 0);
+        st->prog.out_pushed = upto;
     }
 }
 
 // Running checksum continued over the first n bytes of `out`.  While the output of the attempt that produced them is
 // still on the device (out_dev), the bytes are not uploaded a second time.
 static int out_checksum(InflateState* st, size_t n, uint32_t* result) {
-    const int kind = st->trailer == 1 ? 0 : 1;
-    if (st->out_on_device && st->out_gen == st->ctx->scr[SCR_H_OUT].gen && st->out_dev) return zs_checksum_dev(st->ctx, kind, st->out_dev, n, st->run_check, result);
-    return zs_checksum(st->ctx, kind, st->out.data(), n, st->run_check, result);
+    const int kind = st->prog.trailer == 1 ? 0 : 1;
+    if (st->prog.out_on_device && st->prog.out_gen == st->ctx->scr[SCR_H_OUT].gen && st->prog.out_dev) return zs_checksum_dev(st->ctx, kind, st->prog.out_dev, n, st->prog.run_check, result);
+    return zs_checksum(st->ctx, kind, st->out.data(), n, st->prog.run_check, result);
 }
 
 // The blocks before (mark_bit, mark_out) are final: fold their output into the running checksum and
@@ -844,50 +812,50 @@ static int out_checksum(InflateState* st, size_t n, uint32_t* result) {
 static int advance_to_mark(InflateState* st, uint64_t mark_bit, uint64_t mark_out) {
     if (mark_out) {
         push_ready(st, (size_t)mark_out);
-        int rc = out_checksum(st, (size_t)mark_out, &st->run_check);
+        int rc = out_checksum(st, (size_t)mark_out, &st->prog.run_check);
         if (rc != ZS_OK) return rc;
-        st->run_len += mark_out;
+        st->prog.run_len += mark_out;
         // the window: the last 64 KiB of final output (only those are copied: mark_out is the whole batch of a paced stream)
         if (mark_out >= 65536) {
-            st->hist.assign(st->out.data() + (size_t)mark_out - 65536, st->out.data() + (size_t)mark_out);
+            st->prog.hist.assign(st->out.data() + (size_t)mark_out - 65536, st->out.data() + (size_t)mark_out);
         } else {
-            st->hist.insert(st->hist.end(), st->out.data(), st->out.data() + (size_t)mark_out);
-            if (st->hist.size() > 65536) st->hist.erase(st->hist.begin(), st->hist.end() - 65536);
+            st->prog.hist.insert(st->prog.hist.end(), st->out.data(), st->out.data() + (size_t)mark_out);
+            if (st->prog.hist.size() > 65536) st->prog.hist.erase(st->prog.hist.begin(), st->prog.hist.end() - 65536);
         }
         st->out.erase_front((size_t)mark_out);
-        st->out_on_device = false;
-        st->out_pushed -= (size_t)mark_out;
+        st->prog.out_on_device = false;
+        st->prog.out_pushed -= (size_t)mark_out;
     }
     const size_t bytes = (size_t)(mark_bit >> 3);
     st->in.erase_front(bytes);
-    st->start_bit = mark_bit & 7u;
-    st->body = true;
+    st->prog.start_bit = mark_bit & 7u;
+    st->prog.body = true;
     return ZS_OK;
 }
 
 // The last block is decoded and `out` holds its output: check the trailer (CHECK / LENGTH,
 // inflate.ts:1006-1037) if its bytes are here.
 static int finish_stream(InflateState* st) {
-    const size_t T = st->trailer == 1 ? 4 : st->trailer == 2 ? 8 : 0;
-    if (st->in.size() < st->trailer_pos + T) { st->await_trailer = true; return ZS_OK; }
-    st->await_trailer = false;
-    uint32_t total = st->run_check;
+    const size_t T = st->prog.trailer == 1 ? 4 : st->prog.trailer == 2 ? 8 : 0;
+    if (st->in.size() < st->prog.trailer_pos + T) { st->prog.await_trailer = true; return ZS_OK; }
+    st->prog.await_trailer = false;
+    uint32_t total = st->prog.run_check;
     int rc = out_checksum(st, st->out.size(), &total);
     if (rc != ZS_OK) return rc;
-    const uint64_t total_len = st->run_len + st->out.size();
-    const uint8_t* t = st->in.data() + st->trailer_pos;
-    if (st->trailer == 1) {
+    const uint64_t total_len = st->prog.run_len + st->out.size();
+    const uint8_t* t = st->in.data() + st->prog.trailer_pos;
+    if (st->prog.trailer == 1) {
         const uint32_t want = (uint32_t)t[0] << 24 | (uint32_t)t[1] << 16 | (uint32_t)t[2] << 8 | t[3];
-        if (want != total) { st->failed = true; st->fail_code = ZS_DATA_ERROR; st->fail_msg = "incorrect data check"; return ZS_OK; }
-    } else if (st->trailer == 2) {
+        if (want != total) { st->prog.failed = true; st->prog.fail_code = ZS_DATA_ERROR; st->prog.fail_msg = "incorrect data check"; return ZS_OK; }
+    } else if (st->prog.trailer == 2) {
         const uint32_t want = (uint32_t)t[0] | (uint32_t)t[1] << 8 | (uint32_t)t[2] << 16 | (uint32_t)t[3] << 24;
         const uint32_t isize = (uint32_t)t[4] | (uint32_t)t[5] << 8 | (uint32_t)t[6] << 16 | (uint32_t)t[7] << 24;
-        if (want != total) { st->failed = true; st->fail_code = ZS_DATA_ERROR; st->fail_msg = "incorrect data check"; return ZS_OK; }
-        if (isize != (uint32_t)total_len) { st->failed = true; st->fail_code = ZS_DATA_ERROR; st->fail_msg = "incorrect length check"; return ZS_OK; }
+        if (want != total) { st->prog.failed = true; st->prog.fail_code = ZS_DATA_ERROR; st->prog.fail_msg = "incorrect data check"; return ZS_OK; }
+        if (isize != (uint32_t)total_len) { st->prog.failed = true; st->prog.fail_code = ZS_DATA_ERROR; st->prog.fail_msg = "incorrect length check"; return ZS_OK; }
     }
-    st->check = total;
-    st->done = true;
-    const size_t used = st->trailer_pos + T;
+    st->prog.check = total;
+    st->prog.done = true;
+    const size_t used = st->prog.trailer_pos + T;
     if (st->in.size() > used) st->leftover.assign(st->in.data() + used, st->in.data() + st->in.size());
     st->in.clear();
     return ZS_OK;
@@ -895,7 +863,7 @@ static int finish_stream(InflateState* st) {
 
 static int inflate_attempt(zs_stream* strm, InflateState* st) {
     zs_ctx* ctx = st->ctx;
-    if (st->await_trailer) return finish_stream(st);
+    if (st->prog.await_trailer) return finish_stream(st);
     const int raw_wb = st->window_bits == -16 ? -16 : -15;
     for (;;) {
         // `out` is rebuilt by every attempt; what was queued from it stays in `ready`
@@ -904,17 +872,17 @@ static int inflate_attempt(zs_stream* strm, InflateState* st) {
         // the line above, a large attempt stopped at the old capacity and was mistaken for "input ran dry")
         const uint64_t in_off[2] = {0, st->in.size()}, out_off[2] = {0, st->out_cap_hint};
         if (!st->out.resize(st->out_cap_hint)) return ZS_MEM_ERROR;
-        uint64_t out_len = 0, in_used = 0, rng[2] = {0, st->hist.size()};
+        uint64_t out_len = 0, in_used = 0, rng[2] = {0, st->prog.hist.size()};
         uint32_t check = 0;
         int32_t status = 0, detail = 0;
         InflateOpts opts;
         opts.resume = true;
-        opts.start_bit = st->body ? st->start_bit : ~0ull;
+        opts.start_bit = st->prog.body ? st->prog.start_bit : ~0ull;
         InflateOut io;
         const double t_eng0 = now_s();
-        int rc = inflate_batch_host_impl(ctx, st->in.data(), in_off, 1, st->body ? raw_wb : st->window_bits, st->out.data(),
-                                         out_off, &out_len, &in_used, &check, &status, st->hist.empty() ? nullptr : st->hist.data(),
-                                         st->hist.empty() ? nullptr : rng, st->hist.size(), opts, &io);
+        int rc = inflate_batch_host_impl(ctx, st->in.data(), in_off, 1, st->prog.body ? raw_wb : st->window_bits, st->out.data(),
+                                         out_off, &out_len, &in_used, &check, &status, st->prog.hist.empty() ? nullptr : st->prog.hist.data(),
+                                         st->prog.hist.empty() ? nullptr : rng, st->prog.hist.size(), opts, &io);
         st->t_engine += now_s() - t_eng0;
         if (rc != ZS_OK) { strm->msg = zs_last_error(ctx); return rc; }
         if (status == ZS_BUF_ERROR && out_len == st->out_cap_hint) {  // output full: grow and decode again
@@ -923,43 +891,43 @@ static int inflate_attempt(zs_stream* strm, InflateState* st) {
         }
         const uint64_t mark_bit = io.mark[0], mark_out = io.mark[1];
         st->out.resize(out_len);
-        st->out_on_device = true;
-        st->out_dev = io.d_out;
-        st->out_gen = io.out_gen;
+        st->prog.out_on_device = true;
+        st->prog.out_dev = io.d_out;
+        st->prog.out_gen = io.out_gen;
         if (status == ZS_STREAM_END) {
-            if (!st->body) {
+            if (!st->prog.body) {
                 // the whole stream in one attempt: wrapper and trailer were checked on the device
                 push_ready(st, out_len);
-                st->check = check;
-                st->done = true;
+                st->prog.check = check;
+                st->prog.done = true;
                 if (st->in.size() > (size_t)in_used) st->leftover.assign(st->in.data() + (size_t)in_used, st->in.data() + st->in.size());
                 st->in.clear();
                 return ZS_OK;
             }
             push_ready(st, out_len);
-            st->trailer_pos = (size_t)in_used;
+            st->prog.trailer_pos = (size_t)in_used;
             return finish_stream(st);
         }
-        if (status == ZS_NEED_DICT) { st->need_dict = true; return ZS_OK; }
+        if (status == ZS_NEED_DICT) { st->prog.need_dict = true; return ZS_OK; }
         if (status == ZS_DATA_ERROR) {
             zs_inflate_last_details(ctx, &detail, 1);
             push_ready(st, out_len);   // what was decoded before the error is delivered first, like the reference
-            st->failed = true;
-            st->fail_code = ZS_DATA_ERROR;
-            st->fail_msg = zs_inflate_message(detail);
+            st->prog.failed = true;
+            st->prog.fail_code = ZS_DATA_ERROR;
+            st->prog.fail_msg = zs_inflate_message(detail);
             return ZS_OK;
         }
         // the input ran dry (Z_BUF_ERROR / Z_OK): everything decoded so far is final output
         push_ready(st, out_len);
-        if (!st->body) {
+        if (!st->prog.body) {
             // mark_bit > 0 means the wrapper header is complete and the block loop was entered
             if (mark_bit == 0 && st->window_bits >= 0) return ZS_OK;
             const bool gz = st->window_bits > 15 && st->in.size() >= 2 && st->in[0] == 0x1f && st->in[1] == 0x8b;
-            st->trailer = st->window_bits < 0 ? 0 : gz ? 2 : 1;
-            st->run_check = st->trailer == 1 ? 1u : 0u;
-            st->run_len = 0;
+            st->prog.trailer = st->window_bits < 0 ? 0 : gz ? 2 : 1;
+            st->prog.run_check = st->prog.trailer == 1 ? 1u : 0u;
+            st->prog.run_len = 0;
         }
-        if (mark_bit > st->start_bit || !st->body) return advance_to_mark(st, mark_bit, mark_out);
+        if (mark_bit > st->prog.start_bit || !st->prog.body) return advance_to_mark(st, mark_bit, mark_out);
         return ZS_OK;
     }
 }
@@ -972,26 +940,26 @@ int zs_stream_inflate(zs_stream* strm, int flush) {
     // Like inflate(), which stops consuming input when the output buffer is full: while more decoded bytes
     // are waiting than this call can deliver, no new input is taken (the reference's driver loop,
     // streams.ts:86 `while (strm.avail_in > 0)`, then keeps calling with fresh output buffers).
-    const bool backlog = st->ready.size() - st->ready_pos > strm->avail_out;
-    if (!st->done && !st->failed && !backlog) {
+    const bool backlog = st->ready.size() - st->prog.ready_pos > strm->avail_out;
+    if (!st->prog.done && !st->prog.failed && !backlog) {
         // input left over from the previous member is consumed first (inflateReset flow)
         if (!st->leftover.empty() && st->in.empty()) {
             st->in.clear();
             st->in.append(st->leftover.data(), st->leftover.size(), 0);
             st->leftover.clear();
-            st->next_attempt = 0;
+            st->prog.next_attempt = 0;
         }
         if (strm->avail_in) {
             const double t_ins0 = now_s();
             if (!st->in.append(strm->next_in, (size_t)strm->avail_in, 0)) { strm->msg = "insufficient memory"; return ZS_MEM_ERROR; }
             for (size_t i = strm->avail_in > 4 ? (size_t)strm->avail_in - 4 : 0; i < strm->avail_in; i++)
-                st->in_tail = st->in_tail << 8 | strm->next_in[i];
+                st->prog.in_tail = st->prog.in_tail << 8 | strm->next_in[i];
             st->t_insert += now_s() - t_ins0;
             strm->next_in += strm->avail_in;
             strm->total_in += strm->avail_in;
             strm->avail_in = 0;
         }
-        if (st->need_dict) return ZS_NEED_DICT;
+        if (st->prog.need_dict) return ZS_NEED_DICT;
         fill_gz_header(st);
         // `in` holds only what follows the last resume point, so an attempt costs the current block plus the new
         // input (a single huge block is decoded from its start each time).  When is one due?
@@ -1017,25 +985,25 @@ int zs_stream_inflate(zs_stream* strm, int flush) {
         //  * and on a call that brings input while the last block is decoded and only the trailer is missing: finishing
         //    the stream is host work plus one checksum, and Z_STREAM_END with the hand-back of what follows the
         //    trailer through avail_in belongs to the call that brings its last byte.
-        if (in0) st->fresh_input = true;
-        bool due = flush != ZS_NO_FLUSH || st->in.size() >= st->next_attempt || (in0 == 0 && st->fresh_input) ||
-                   (in0 && (st->in_tail == 0x0000ffffu || st->await_trailer));
-        if (!due && st->fresh_input && now_s() - st->attempt_end >= kPaceFactor * st->attempt_cost) due = true;
+        if (in0) st->prog.fresh_input = true;
+        bool due = flush != ZS_NO_FLUSH || st->in.size() >= st->prog.next_attempt || (in0 == 0 && st->prog.fresh_input) ||
+                   (in0 && (st->prog.in_tail == 0x0000ffffu || st->prog.await_trailer));
+        if (!due && st->prog.fresh_input && now_s() - st->prog.attempt_end >= kPaceFactor * st->prog.attempt_cost) due = true;
         if (due && !st->in.empty()) {
             const double t_begin = now_s();
             int rc = inflate_attempt(strm, st);
             if (rc != ZS_OK) return rc;
-            st->fresh_input = false;
-            st->attempt_end = now_s();
-            st->attempt_cost = st->attempt_end - t_begin;
-            st->t_attempts += st->attempt_cost;
+            st->prog.fresh_input = false;
+            st->prog.attempt_end = now_s();
+            st->prog.attempt_cost = st->prog.attempt_end - t_begin;
+            st->t_attempts += st->prog.attempt_cost;
             st->n_attempts++;
-            st->next_attempt = st->in.size() + ((size_t)strm->total_in < kEveryCallBelow ? 1 : kAttemptAtLeastEvery);
-            if (st->need_dict) {
-                strm->adler = st->in.size() >= 6 ? ((uint32_t)st->in[2] << 24 | (uint32_t)st->in[3] << 16 | (uint32_t)st->in[4] << 8 | st->in[5]) : 0u;
+            st->prog.next_attempt = st->in.size() + ((size_t)strm->total_in < kEveryCallBelow ? 1 : kAttemptAtLeastEvery);
+            if (st->prog.need_dict) {
+                strm->adler = dict_id(st);
                 return ZS_NEED_DICT;
             }
-            if (st->done && !st->leftover.empty()) {
+            if (st->prog.done && !st->leftover.empty()) {
                 // hand back what the caller gave us in this call and we did not need
                 const size_t give = st->leftover.size() <= in0 ? st->leftover.size() : (size_t)in0;
                 strm->next_in -= give;
@@ -1053,27 +1021,27 @@ int zs_stream_inflate(zs_stream* strm, int flush) {
     st->n_calls++;
     const double t_del0 = now_s();
     struct DeliverTimer { InflateState* s; double t0; ~DeliverTimer() { s->t_deliver += now_s() - t0; } } deliver_timer{st, t_del0};
-    if (st->ready_pos < st->ready.size()) {
-        size_t c = st->ready.size() - st->ready_pos;
+    if (st->prog.ready_pos < st->ready.size()) {
+        size_t c = st->ready.size() - st->prog.ready_pos;
         if (c > strm->avail_out) c = (size_t)strm->avail_out;
-        memcpy(strm->next_out, st->ready.data() + st->ready_pos, c);
+        memcpy(strm->next_out, st->ready.data() + st->prog.ready_pos, c);
         strm->next_out += c;
         strm->avail_out -= c;
         strm->total_out += c;
-        st->ready_pos += c;
-        if (st->ready_pos == st->ready.size()) { st->ready.clear(); st->ready_pos = 0; }
-        else if (st->ready_pos > (8u << 20) && st->ready_pos >= st->ready.size() / 2) {   // (amortised: the delivered half goes, the rest moves once)
-            st->ready.erase_front(st->ready_pos);
-            st->ready_pos = 0;
+        st->prog.ready_pos += c;
+        if (st->prog.ready_pos == st->ready.size()) { st->ready.clear(); st->prog.ready_pos = 0; }
+        else if (st->prog.ready_pos > (8u << 20) && st->prog.ready_pos >= st->ready.size() / 2) {   // (amortised: the delivered half goes, the rest moves once)
+            st->ready.erase_front(st->prog.ready_pos);
+            st->prog.ready_pos = 0;
         }
     }
-    const bool all_out = st->ready_pos >= st->ready.size();
-    if (st->failed && all_out) {
-        strm->msg = st->fail_msg;
-        return st->fail_code;
+    const bool all_out = st->prog.ready_pos >= st->ready.size();
+    if (st->prog.failed && all_out) {
+        strm->msg = st->prog.fail_msg;
+        return st->prog.fail_code;
     }
-    if (st->done && all_out) {
-        strm->adler = st->check;
+    if (st->prog.done && all_out) {
+        strm->adler = st->prog.check;
         return ZS_STREAM_END;
     }
     // inf_leave, inflate.ts:1092-1098: no progress, or Z_FINISH without reaching the end
@@ -1092,7 +1060,7 @@ int zs_stream_inflate_get_header(zs_stream* strm, zs_gz_header* head) {
     if (!st || !head) return ZS_STREAM_ERROR;
     const int wb = st->window_bits;
     if (wb < 16) return ZS_STREAM_ERROR;   // (state._wrap & 2) == 0: raw or zlib-only
-    st->gzhead = head;
+    st->prog.gzhead = head;
     head->done = 0;
     return ZS_OK;
 }
@@ -1103,20 +1071,7 @@ int zs_stream_inflate_reset(zs_stream* strm) {
     st->in.clear();
     st->out.clear();
     st->ready.clear();
-    st->hist.clear();
-    st->ready_pos = st->out_pushed = 0;
-    st->next_attempt = 0;
-    st->fresh_input = false;
-    st->in_tail = 1;
-    st->attempt_end = st->attempt_cost = 0.0;
-    st->body = st->await_trailer = false;
-    st->start_bit = 0;
-    st->trailer = 0;
-    st->run_check = 0;
-    st->run_len = 0;
-    st->trailer_pos = 0;
-    st->done = st->failed = st->need_dict = st->have_dict = false;
-    st->gzhead = nullptr;   // inflateResetKeep drops the header request
+    st->prog = {};   // (inflateResetKeep drops the header request too)
     strm->total_in = strm->total_out = 0;
     strm->msg = "";
     return ZS_OK;
@@ -1126,19 +1081,11 @@ int zs_stream_inflate_reset(zs_stream* strm) {
 int zs_stream_inflate_reset2(zs_stream* strm, int window_bits) {
     InflateState* st = istate(strm);
     if (!st) return ZS_STREAM_ERROR;
-    int wb = window_bits;
-    if (wb < 0) {
-        if (wb < -16) return ZS_STREAM_ERROR;
-        wb = -wb;
-        if (wb < 8) return ZS_STREAM_ERROR;
-    } else {
-        if (wb < 48) wb &= 15;
-        if (wb && (wb < 8 || wb > 15)) return ZS_STREAM_ERROR;
-    }
+    if (!zs_inflate_window_bits(window_bits, nullptr, nullptr)) return ZS_STREAM_ERROR;
     st->window_bits = window_bits;
     st->leftover.clear();
     const int rc = zs_stream_inflate_reset(strm);
-    strm->adler = (window_bits >= 0 && (((window_bits >> 4) + 5) & 1)) ? 1u : 0u;   // 0 = window size from the zlib header
+    strm->adler = zs_inflate_initial_adler(window_bits);
     return rc;
 }
 
