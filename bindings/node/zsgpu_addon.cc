@@ -112,6 +112,38 @@ napi_value InflateBatch(napi_env env, napi_callback_info info) {
     return rc == ZS_OK ? nullptr : throw_code(env, rc, "zs_inflate_batch");
 }
 
+// gunzip(input: Uint8Array, out: Uint8Array[, members: BigUint64Array, 5 per member: inOff, inLen, outOff, outLen,
+//        crc32]) -> {outLen, inUsed, members, status, msg: Buffer}        zs_gunzip
+napi_value Gunzip(napi_env env, napi_callback_info info) {
+    size_t argc = 3; napi_value a[3];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    uint8_t *in, *out; size_t n_in, n_out;
+    if (argc < 2 || !u8(env, a[0], &in, &n_in) || !u8(env, a[1], &out, &n_out)) return throw_code(env, ZS_STREAM_ERROR, "gunzip");
+    uint64_t* tab = nullptr; size_t n_tab = 0;
+    napi_typedarray_type t; napi_value ab; size_t bo;
+    if (argc >= 3 && (napi_get_typedarray_info(env, a[2], &t, &n_tab, (void**)&tab, &ab, &bo) != napi_ok || t != napi_biguint64_array))
+        n_tab = 0;
+    std::vector<zs_gz_member> table(n_tab / 5);
+    zs_gunzip_result r;
+    int rc = zs_gunzip(g_ctx, in, n_in, out, n_out, &r, table.empty() ? nullptr : table.data(), table.size());
+    if (rc != ZS_OK) return throw_code(env, rc, "zs_gunzip");
+    for (size_t i = 0; i < table.size() && i < r.n_members; ++i) {
+        const zs_gz_member& e = table[i];
+        const uint64_t f[5] = {e.in_off, e.in_len, e.out_off, e.out_len, e.crc32};
+        memcpy(tab + 5 * i, f, sizeof f);
+    }
+    const char* msg = r.status == ZS_STREAM_END ? "" : zs_inflate_message(r.detail);
+    napi_value o, m; void* dst = nullptr;
+    napi_create_object(env, &o);
+    napi_set_named_property(env, o, "outLen", num(env, (double)r.out_len));
+    napi_set_named_property(env, o, "inUsed", num(env, (double)r.in_used));
+    napi_set_named_property(env, o, "members", num(env, (double)r.n_members));
+    napi_set_named_property(env, o, "status", num(env, (double)r.status));
+    napi_create_buffer_copy(env, msg ? strlen(msg) : 0, msg ? msg : "", &dst, &m);
+    napi_set_named_property(env, o, "msg", m);
+    return o;
+}
+
 // checksum(kind, init, buf) -> number                                  zs_checksum
 napi_value Checksum(napi_env env, napi_callback_info info) {
     size_t argc = 3; napi_value a[3];
@@ -258,7 +290,7 @@ napi_value InflateHeaderState(napi_env env, napi_callback_info info) {
 
 napi_value Register(napi_env env, napi_value exports) {
     const struct { const char* name; napi_callback fn; } fns[] = {
-        {"init", Init}, {"deflateBatch", DeflateBatch}, {"inflateBatch", InflateBatch}, {"checksum", Checksum},
+        {"init", Init}, {"deflateBatch", DeflateBatch}, {"inflateBatch", InflateBatch}, {"gunzip", Gunzip}, {"checksum", Checksum},
         {"createDeflateDictionary", CreateDeflateDictionary},
         {"streamNew", StreamNew}, {"deflateInit2", DeflateInit2}, {"inflateInit2", InflateInit2}, {"process", Process},
         {"end", End}, {"setDictionary", SetDictionary}, {"inflateReset", InflateReset}, {"control", Control},

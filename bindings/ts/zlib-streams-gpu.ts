@@ -189,3 +189,21 @@ export function inflateBatch(streams: Uint8Array[], windowBits: number, outCaps:
   }
   return { out, outOff, outLen, checks, status };
 }
+// Every member of a multi-member gzip file (bgzip / BGZF, `cat a.gz b.gz`, deflateBatch's independent gzip output) in
+// one call: what inflate(Z_FINISH) / inflateReset repeated until the input is used up produces
+// (test/inflate/test-multistream.ts:16-79), strict about trailing bytes like that loop.  Without outCap the room
+// starts at four times the input (at least 64 KiB) and doubles while the call ends with Z_BUF_ERROR on a full output.
+// With `members`, `table` holds inOff, inLen, outOff, outLen, crc32 per member (the makings of a .gzi index).
+export function gunzip(input: Uint8Array, opts: { outCap?: number; members?: boolean } = {}) {
+  const grow = opts.outCap === undefined;
+  let cap = grow ? Math.max(4 * input.length, 65536) : opts.outCap!;
+  let nTab = opts.members ? Math.floor(input.length / 1024) + 1024 : 0;
+  for (;;) {
+    const out = new Uint8Array(cap + 16), table = new BigUint64Array(5 * nTab);
+    const r = addon.gunzip(input, out.subarray(0, cap), table);
+    if (grow && r.status === -5 && r.outLen === cap) { cap *= 2; continue; }
+    if (opts.members && r.members > nTab) { nTab = r.members; continue; }
+    return { data: out.subarray(0, r.outLen), inUsed: r.inUsed, members: r.members, status: r.status,
+             msg: Buffer.from(r.msg).toString(), table: opts.members ? table.subarray(0, 5 * Math.min(r.members, nTab)) : undefined };
+  }
+}

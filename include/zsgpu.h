@@ -266,6 +266,42 @@ ZS_API const char* zs_inflate_message(int detail);
  * zs_inflate_batch[_dev] call on this context, copied to the host array `detail[n]`. */
 ZS_API int zs_inflate_last_details(zs_ctx* ctx, int32_t* detail, uint32_t n);
 
+/* ---- multi-member gzip (RFC 1952 2.2: bgzip / BGZF, `cat a.gz b.gz`, appended archives, this engine's own
+ *      INDEPENDENT gzip output): every member in one call ----
+ * The result is what the reference's multi-member loop produces (test/inflate/test-multistream.ts:16-79):
+ * inflateInit2(31), then inflate(Z_FINISH) on the rest of the input; on Z_STREAM_END inflateReset and go on behind
+ * total_in, until the input is used up.  So the call is as strict as that loop: bytes after the last member that do
+ * not form a member -- garbage, and zero padding too -- end it with that member's header error ("incorrect header
+ * check"), and empty input is Z_BUF_ERROR.  On an error the output holds the members before the failing one and that
+ * member's prefix; status / detail / in_used are what inflate() reports for it (in_used counted from the file start).
+ * Only gzip members are read; concatenated zlib or raw streams are not members.
+ * The members are found on the device (candidate headers, an output plan from their ISIZE fields, a batch decode that
+ * must land exactly on the next candidate; DESIGN.md 3.3c); a member that does not, and any member of 128 KiB or more,
+ * is decoded alone by the one-stream path of zs_inflate_stream_dev.  The calls make host decisions as they go, so
+ * they SYNCHRONISE; `res` and `members` are host memory. */
+typedef struct zs_gunzip_result {
+    uint64_t out_len;   /* bytes written to out */
+    uint64_t in_used;   /* bytes consumed (total_in of the loop) */
+    uint64_t n_members; /* members that ended with Z_STREAM_END (always the true count) */
+    int32_t status;     /* Z_STREAM_END when every byte belonged to a member, else the failing member's status */
+    int32_t detail;     /* message code of the failing member: zs_inflate_message(detail) */
+} zs_gunzip_result;
+/* One decoded member: where it lies in the input and in the output, and the crc32 of its output.  A BGZF reader
+ * builds its .gzi random-access index from these. */
+typedef struct zs_gz_member {
+    uint64_t in_off, in_len;
+    uint64_t out_off, out_len;
+    uint32_t crc32;
+} zs_gz_member;
+/* d_in (8-byte aligned) and d_out are device memory; d_out may be NULL when out_cap is 0.  At most max_members entries go to `members` (may be NULL with
+ * max_members 0), in file order.  Returns ZS_OK when the input was processed (its verdict is res->status),
+ * ZS_STREAM_ERROR for bad arguments, ZS_MEM_ERROR or ZS_E_CUDA. */
+ZS_API int zs_gunzip_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
+                         zs_gunzip_result* res, zs_gz_member* members, uint64_t max_members);
+/* Host-buffer variant: copies in, runs zs_gunzip_dev, copies res->out_len bytes out. */
+ZS_API int zs_gunzip(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint8_t* out, uint64_t out_cap, zs_gunzip_result* res,
+                     zs_gz_member* members, uint64_t max_members);
+
 /* ---- streaming shim: the z_stream protocol of deflate()/inflate() over the batch engine ----
  * Mirrors createDeflateStream/deflateInit2_/deflate/deflateEnd (deflate.ts:80,253,716,991),
  * deflateSetDictionary (:367) and createInflateStream/inflateInit2_/inflate/inflateEnd/

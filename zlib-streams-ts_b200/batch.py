@@ -319,6 +319,81 @@ def inflate_batch(streams, window_bits: int = 15, out_caps=None, dictionaries=No
     return InflateBatchHost(out[: int(out_off[-1])].tobytes(), out_off, out_len, in_used, checks, status, details)
 
 
+# zs_gz_member: one decoded member of a multi-member gzip file
+GZ_MEMBER_DTYPE = np.dtype([("in_off", "<u8"), ("in_len", "<u8"), ("out_off", "<u8"), ("out_len", "<u8"),
+                            ("crc32", "<u4"), ("_pad", "<u4")])
+assert GZ_MEMBER_DTYPE.itemsize == C.sizeof(capi.GzMember)
+
+
+@dataclass
+class Gunzip:
+    data: bytes | torch.Tensor   # the output (gunzip: bytes; gunzip_dev: the device buffer, valid to out_len)
+    out_len: int
+    in_used: int
+    n_members: int
+    status: int                  # Z_STREAM_END when every byte belonged to a member
+    detail: int
+    members: np.ndarray | None   # GZ_MEMBER_DTYPE [min(n_members, table size)] when asked for
+
+    @property
+    def message(self) -> str:
+        return (capi.load().zs_inflate_message(int(self.detail)) or b"").decode()
+
+
+def _gunzip_result(res: capi.GunzipResult, data, table: np.ndarray | None) -> Gunzip:
+    members = table[: min(int(res.n_members), table.size)] if table is not None else None
+    return Gunzip(data, int(res.out_len), int(res.in_used), int(res.n_members), int(res.status), int(res.detail), members)
+
+
+def gunzip(data, out_cap: int | None = None, members: bool = False, ctx: Context | None = None) -> Gunzip:
+    """Every member of a multi-member gzip file from a host buffer (zs_gunzip): what inflate(Z_FINISH) /
+    inflateReset repeated until the input is used up produces, like gzip -d or Python's gzip.decompress -- but strict
+    about trailing bytes, as that loop is.
+
+    `out_cap` is the output room.  Without it the room starts at four times the input (at least 64 KiB) and is
+    doubled for as long as the call ends with Z_BUF_ERROR on a full output, so the result is the one an unlimited
+    room gives.  With `members` the result carries the member table (offsets, sizes and crc32 of each member)."""
+    ctx = ctx or default_context()
+    src = _as_u8(data)
+    n = src.size
+    lib = capi.load()
+    grow = out_cap is None
+    cap = max(4 * n, 1 << 16) if grow else int(out_cap)
+    n_tab = n // 1024 + 1024 if members else 0
+    while True:
+        out = np.empty(cap + 16, dtype=np.uint8)
+        table = np.zeros(n_tab, dtype=GZ_MEMBER_DTYPE) if members else None
+        res = capi.GunzipResult()
+        rc = lib.zs_gunzip(ctx.handle, src.ctypes.data if n else None, n, out.ctypes.data, cap, C.byref(res),
+                           table.ctypes.data if members else None, n_tab)
+        ctx.check(rc, "zs_gunzip")
+        if grow and res.status == capi.Z_BUF_ERROR and res.out_len == cap:
+            cap *= 2
+            continue
+        if members and res.n_members > n_tab:   # the table was too short: once more with the exact count
+            n_tab = int(res.n_members)
+            continue
+        return _gunzip_result(res, out[: res.out_len].tobytes(), table)
+
+
+def gunzip_dev(d_in: torch.Tensor, out_cap: int, members: int = 0, out: torch.Tensor | None = None,
+               ctx: Context | None = None) -> Gunzip:
+    """Every member of a multi-member gzip file in device memory (zs_gunzip_dev; synchronises).  `d_in` must start
+    8-byte aligned (a fresh tensor does); the output goes to `out` (allocated with out_cap bytes when None).
+    `members`: size of the member table to fill (0: none)."""
+    assert d_in.is_cuda and d_in.dtype == torch.uint8 and d_in.is_contiguous()
+    ctx = ctx or default_context(d_in.device.index)
+    if out is None:
+        out = torch.empty(out_cap + 16, dtype=torch.uint8, device=d_in.device)
+    assert out.numel() >= out_cap
+    table = np.zeros(members, dtype=GZ_MEMBER_DTYPE) if members else None
+    res = capi.GunzipResult()
+    rc = capi.load().zs_gunzip_dev(ctx.handle, _ptr(d_in), d_in.numel(), _ptr(out), out_cap, C.byref(res),
+                                   table.ctypes.data if members else None, members)
+    ctx.check(rc, "zs_gunzip_dev")
+    return _gunzip_result(res, out, table)
+
+
 def checksum(data, kind: int, init: int | None = None, ctx: Context | None = None) -> int:
     """adler32(adler, buf, len) / crc32(crc, buf, len) of a host buffer, computed on the GPU."""
     ctx = ctx or default_context()

@@ -36,6 +36,18 @@ class ZStream(C.Structure):
                 ("msg", C.c_char_p), ("adler", C.c_uint32), ("data_type", C.c_int32), ("state", C.c_void_p)]
 
 
+class GunzipResult(C.Structure):
+    """zs_gunzip_result of include/zsgpu.h"""
+    _fields_ = [("out_len", C.c_uint64), ("in_used", C.c_uint64), ("n_members", C.c_uint64), ("status", C.c_int32),
+                ("detail", C.c_int32)]
+
+
+class GzMember(C.Structure):
+    """zs_gz_member of include/zsgpu.h"""
+    _fields_ = [("in_off", C.c_uint64), ("in_len", C.c_uint64), ("out_off", C.c_uint64), ("out_len", C.c_uint64),
+                ("crc32", C.c_uint32)]
+
+
 class ZsError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ""):
         super().__init__(f"{where} failed with {code}" + (f": {detail}" if detail else ""))
@@ -87,6 +99,9 @@ _PROTOTYPES = {
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]),
     "zs_inflate_message": (C.c_char_p, [C.c_int]),
     "zs_inflate_last_details": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32]),
+    "zs_gunzip_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                C.c_uint64]),
+    "zs_gunzip": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64]),
     "zs_stream_deflate_init": (C.c_int, [C.c_void_p, C.POINTER(ZStream), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "zs_stream_deflate_set_dictionary": (C.c_int, [C.POINTER(ZStream), C.c_void_p, C.c_uint32]),
     "zs_stream_deflate": (C.c_int, [C.POINTER(ZStream), C.c_int]),

@@ -32,6 +32,10 @@ enum zs_scratch_slot {
     SCR_P_STATE,
     // zs_inflate_par.cu
     SCR_P_CAND, SCR_P_SEG, SCR_P_PLAN, SCR_P_SYM, SCR_P_WIN, SCR_P_GMAP,
+    // zs_gunzip.cu: tile counts, member candidates, one pass's plan and results, member-table entries, and the aligned
+    // copy of a member decoded alone.  Its own: the batch and one-stream inflate calls it makes use none of them, and
+    // zs_gunzip stages its input and output in SCR_H_IN / SCR_H_OUT around them
+    SCR_G_TILE, SCR_G_CAND, SCR_G_PASS, SCR_G_MEMB, SCR_G_ALIGN,
     ZS_SCR_COUNT
 };
 
