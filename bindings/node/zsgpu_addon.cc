@@ -58,6 +58,101 @@ napi_value CreateDeflateDictionary(napi_env env, napi_callback_info info) {
     return o;
 }
 
+// ---- random access into one stream (zs_inflate_index_*); an index handle is destroyed when it is garbage collected ----
+void FreeIndex(napi_env, void* data, void*) { zs_inflate_index_destroy((zs_inflate_index*)data); }
+bool u64s(napi_env env, napi_value v, uint64_t** p, size_t* n) {
+    napi_typedarray_type t; napi_value ab; size_t off;
+    return napi_get_typedarray_info(env, v, &t, n, (void**)p, &ab, &off) == napi_ok && t == napi_biguint64_array;
+}
+napi_value index_object(napi_env env, zs_inflate_index* x) {
+    zs_inflate_index_info inf;
+    zs_inflate_index_info_get(x, &inf);
+    napi_value h, o;
+    napi_create_external(env, x, FreeIndex, nullptr, &h);
+    napi_create_object(env, &o);
+    napi_set_named_property(env, o, "handle", h);
+    napi_set_named_property(env, o, "points", num(env, (double)inf.n_points));
+    napi_set_named_property(env, o, "outLen", num(env, (double)inf.out_len));
+    return o;
+}
+
+// inflateIndexBuild(input: Uint8Array, windowBits, span, out: Uint8Array[, dict: Uint8Array])
+//   -> {index: {handle, points, outLen} | null, outLen, inUsed, check, status, msg: Buffer}      zs_inflate_index_build
+napi_value InflateIndexBuild(napi_env env, napi_callback_info info) {
+    size_t argc = 5; napi_value a[5];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    uint8_t *in, *out, *dict = nullptr; size_t n_in, n_out, n_dict = 0;
+    if (argc < 4 || !u8(env, a[0], &in, &n_in) || !u8(env, a[3], &out, &n_out)) return throw_code(env, ZS_STREAM_ERROR, "inflateIndexBuild");
+    if (argc >= 5 && !u8(env, a[4], &dict, &n_dict)) n_dict = 0;
+    uint32_t span = 0;
+    napi_get_value_uint32(env, a[2], &span);
+    zs_inflate_index_result r;
+    zs_inflate_index* x = nullptr;
+    int rc = zs_inflate_index_build(g_ctx, in, n_in, i32(env, a[1]), span, out, n_out, n_dict ? dict : nullptr, n_dict, &r, &x);
+    if (rc != ZS_OK) return throw_code(env, rc, "zs_inflate_index_build");
+    const char* msg = r.status == ZS_STREAM_END ? "" : zs_inflate_message(r.detail);
+    napi_value o, m, ix; void* dst = nullptr;
+    napi_create_object(env, &o);
+    if (x) ix = index_object(env, x);
+    else napi_create_object(env, &ix);   // (no index: an object without a handle)
+    napi_set_named_property(env, o, "index", ix);
+    napi_set_named_property(env, o, "outLen", num(env, (double)r.out_len));
+    napi_set_named_property(env, o, "inUsed", num(env, (double)r.in_used));
+    napi_set_named_property(env, o, "check", num(env, (double)r.check));
+    napi_set_named_property(env, o, "status", num(env, (double)r.status));
+    napi_create_buffer_copy(env, strlen(msg), msg, &dst, &m);
+    napi_set_named_property(env, o, "msg", m);
+    return o;
+}
+
+// inflateIndexExtract(handle, input: Uint8Array, off: BigUint64Array, len: BigUint64Array, out: Uint8Array,
+//                     outOff: BigUint64Array, got: BigUint64Array, status: Int32Array) -> void   zs_inflate_index_extract
+// (status is read as an Int32Array, like inflateBatch's)
+napi_value InflateIndexExtract(napi_env env, napi_callback_info info) {
+    size_t argc = 8; napi_value a[8];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    void* x = nullptr;
+    uint8_t *in, *out; size_t n_in, n_out;
+    uint64_t *off, *len, *out_off, *got; size_t n1, n2, n3, n4;
+    void* status; size_t n5; napi_typedarray_type t; napi_value ab; size_t bo;
+    if (argc < 8 || napi_get_value_external(env, a[0], &x) != napi_ok || !u8(env, a[1], &in, &n_in) || !u64s(env, a[2], &off, &n1) ||
+        !u64s(env, a[3], &len, &n2) || !u8(env, a[4], &out, &n_out) || !u64s(env, a[5], &out_off, &n3) ||
+        !u64s(env, a[6], &got, &n4) || napi_get_typedarray_info(env, a[7], &t, &n5, &status, &ab, &bo) != napi_ok ||
+        n2 < n1 || n3 < n1 || n4 < n1 || n5 < n1)
+        return throw_code(env, ZS_STREAM_ERROR, "inflateIndexExtract");
+    int rc = zs_inflate_index_extract(g_ctx, (const zs_inflate_index*)x, in, n_in, off, len, (uint32_t)n1, out, n_out, out_off, got,
+                                      (int32_t*)status);
+    return rc == ZS_OK ? nullptr : throw_code(env, rc, "zs_inflate_index_extract");
+}
+
+// inflateIndexExport(handle) -> Buffer (the format of zsgpu.h)                   zs_inflate_index_export
+napi_value InflateIndexExport(napi_env env, napi_callback_info info) {
+    size_t argc = 1; napi_value a[1];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    void* x = nullptr;
+    if (argc < 1 || napi_get_value_external(env, a[0], &x) != napi_ok) return throw_code(env, ZS_STREAM_ERROR, "inflateIndexExport");
+    uint64_t n = 0;
+    int rc = zs_inflate_index_export((const zs_inflate_index*)x, nullptr, 0, &n);
+    std::vector<uint8_t> blob(n);
+    if (rc == ZS_OK) rc = zs_inflate_index_export((const zs_inflate_index*)x, blob.data(), n, &n);
+    if (rc != ZS_OK) return throw_code(env, rc, "zs_inflate_index_export");
+    napi_value b; void* dst = nullptr;
+    napi_create_buffer_copy(env, blob.size(), blob.data(), &dst, &b);
+    return b;
+}
+
+// inflateIndexImport(blob: Uint8Array) -> {handle, points, outLen}                zs_inflate_index_import
+napi_value InflateIndexImport(napi_env env, napi_callback_info info) {
+    size_t argc = 1; napi_value a[1];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    uint8_t* p; size_t n;
+    if (argc < 1 || !u8(env, a[0], &p, &n)) return throw_code(env, ZS_STREAM_ERROR, "inflateIndexImport");
+    zs_inflate_index* x = nullptr;
+    int rc = zs_inflate_index_import(g_ctx, p, n, &x);
+    if (rc != ZS_OK) return throw_code(env, rc, "zs_inflate_index_import");
+    return index_object(env, x);
+}
+
 // deflateBatch(input: Uint8Array, chunkSize, level, wrap, mode, flags, out: Uint8Array, outOff: BigUint64Array
 //              [, dictionary handle]) -> {bytes, bits, check, blocks}   zs_deflate_batch / zs_deflate_batch_dict
 napi_value DeflateBatch(napi_env env, napi_callback_info info) {
@@ -292,6 +387,8 @@ napi_value Register(napi_env env, napi_value exports) {
     const struct { const char* name; napi_callback fn; } fns[] = {
         {"init", Init}, {"deflateBatch", DeflateBatch}, {"inflateBatch", InflateBatch}, {"gunzip", Gunzip}, {"checksum", Checksum},
         {"createDeflateDictionary", CreateDeflateDictionary},
+        {"inflateIndexBuild", InflateIndexBuild}, {"inflateIndexExtract", InflateIndexExtract},
+        {"inflateIndexExport", InflateIndexExport}, {"inflateIndexImport", InflateIndexImport},
         {"streamNew", StreamNew}, {"deflateInit2", DeflateInit2}, {"inflateInit2", InflateInit2}, {"process", Process},
         {"end", End}, {"setDictionary", SetDictionary}, {"inflateReset", InflateReset}, {"control", Control},
         {"deflatePending", DeflatePending}, {"deflateSetHeader", DeflateSetHeader},

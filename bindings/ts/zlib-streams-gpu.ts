@@ -207,3 +207,40 @@ export function gunzip(input: Uint8Array, opts: { outCap?: number; members?: boo
              msg: Buffer.from(r.msg).toString(), table: opts.members ? table.subarray(0, 5 * Math.min(r.members, nTab)) : undefined };
   }
 }
+// Random access into one zlib / gzip / raw deflate stream (zs_inflate_index_*): access points about every `span` bytes of
+// output, each with the 32 KiB window before it, kept on the GPU.  build() decodes the whole stream once (as inflate with
+// Z_FINISH would) and returns the index with the output; extract() then reads any byte ranges of the stream without
+// decoding what comes before them.  toBytes() / fromBytes() carry an index across processes (the format of zsgpu.h).
+export class InflateIndex {
+  private constructor(private readonly h: { handle: unknown; points: number; outLen: number }) {}
+  get points(): number { return this.h.points; }
+  get outLen(): number { return this.h.outLen; }
+  static build(input: Uint8Array, opts: { windowBits?: number; span?: number; dictionary?: Uint8Array; outCap?: number } = {}) {
+    const grow = opts.outCap === undefined;
+    let cap = grow ? Math.max(4 * input.length, 65536) : opts.outCap!;
+    for (;;) {
+      const out = new Uint8Array(cap + 16);
+      const args = [input, opts.windowBits ?? 15, opts.span ?? (1 << 20), out.subarray(0, cap)];
+      const r = opts.dictionary ? addon.inflateIndexBuild(...args, opts.dictionary) : addon.inflateIndexBuild(...args);
+      if (grow && r.status === -5 && r.outLen === cap) { cap *= 2; continue; }
+      return { index: r.index.handle ? new InflateIndex(r.index) : undefined, data: out.subarray(0, r.outLen),
+               inUsed: r.inUsed, check: r.check, status: r.status, msg: Buffer.from(r.msg).toString() };
+    }
+  }
+  static fromBytes(blob: Uint8Array): InflateIndex { return new InflateIndex(addon.inflateIndexImport(blob)); }
+  toBytes(): Uint8Array { return addon.inflateIndexExport(this.h.handle); }
+  // ranges: [offset, length] in the uncompressed stream; `input` is the indexed stream.  A range past the end comes back
+  // short with status Z_BUF_ERROR; one the input does not decode for has status Z_DATA_ERROR.
+  extract(input: Uint8Array, ranges: [number, number][]) {
+    const n = ranges.length;
+    const off = new BigUint64Array(n), len = new BigUint64Array(n), outOff = new BigUint64Array(n);
+    let total = 0;
+    ranges.forEach(([o, l], i) => {
+      off[i] = BigInt(o); len[i] = BigInt(l); outOff[i] = BigInt(total);
+      total += Math.max(0, Math.min(l, this.h.outLen - o));
+    });
+    const out = new Uint8Array(total + 16), got = new BigUint64Array(n), status = new Int32Array(n);
+    addon.inflateIndexExtract(this.h.handle, input, off, len, out.subarray(0, total), outOff, got, status);
+    return ranges.map((_, i) => ({ data: out.subarray(Number(outOff[i]), Number(outOff[i]) + Number(got[i])), status: status[i] }));
+  }
+}

@@ -266,6 +266,88 @@ ZS_API const char* zs_inflate_message(int detail);
  * zs_inflate_batch[_dev] call on this context, copied to the host array `detail[n]`. */
 ZS_API int zs_inflate_last_details(zs_ctx* ctx, int32_t* detail, uint32_t n);
 
+/* ---- random access into one stream: an index of access points (the method of zlib's examples/zran.c) ----
+ * Reading bytes from the middle of a long zlib, gzip or raw deflate stream otherwise means decoding everything before
+ * them.  An index records ACCESS POINTS: deflate block starts, each with its input bit, its output offset and the
+ * 32 KiB window before it.  A read then decodes from the nearest point at or before it.
+ *
+ * Block starts are every point where a deflate block begins (what inflate(Z_BLOCK) stops at: data_type & 128 set, the
+ * last block not yet seen): input bit total_in * 8 - (bits held) and output offset total_out.  The first is right after
+ * the wrapper header.  For a span S >= 1, the access points are, without duplicates, "the first block start, in stream
+ * order, whose output offset is >= m" for m = 0, S, 2S, ... with m < out_len; the first block start is always a point.
+ * This depends on the stream's block structure and S alone.  Any byte is then at most S plus one block's output after
+ * its point.  The window of a point at output offset o is the last min(32768, dict_len + o) bytes of the preset
+ * dictionary (when the stream uses one: raw, or zlib with FDICT) followed by out[0, o).
+ *
+ * The index lives on the device of the context that made it: its point table and n_points windows of up to 32 KiB,
+ * with a host copy of the table.  Any context on that device may use it; destroy it before that context.  Only the first
+ * gzip member is indexed (zs_gunzip's member table serves multi-member files).  Deflate64 has no index. */
+typedef struct zs_inflate_index zs_inflate_index;
+typedef struct zs_inflate_index_info {
+    uint64_t in_len, out_len, span, n_points;
+    uint32_t check;      /* adler32 (zlib) / crc32 (gzip, raw) of the whole output */
+    int32_t window_bits;
+} zs_inflate_index_info;
+typedef struct zs_inflate_index_result {
+    uint64_t out_len;    /* total_out */
+    uint64_t in_used;    /* total_in */
+    uint32_t check;
+    int32_t status;      /* what zs_inflate_stream_dev reports */
+    int32_t detail;      /* message code: zs_inflate_message(detail) */
+} zs_inflate_index_result;
+/* inflate(Z_FINISH) of one stream, exactly as zs_inflate_stream_dev: same output, out_len, in_used, check, status and
+ * detail.  When the status is Z_STREAM_END, *out also receives an index of the points above for span `span`; otherwise
+ * *out is NULL.  window_bits 15 / -15 / 31 / 47; -16 (deflate64) and span 0 are ZS_STREAM_ERROR.  d_in 8-byte aligned,
+ * d_dict optional as in zs_inflate_stream_dev.  Makes host decisions, so it SYNCHRONISES; res is host memory.  After the
+ * decode, the stream is walked once more for its block starts: in parallel over the segments the one-stream decoder
+ * cut it into, by one warp over the part it decoded serially (DESIGN.md 3.3d). */
+ZS_API int zs_inflate_index_build_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int window_bits, uint64_t span,
+                                      uint8_t* d_out, uint64_t out_cap, const uint8_t* d_dict, uint64_t dict_len,
+                                      zs_inflate_index_result* res, zs_inflate_index** out);
+/* Host-buffer variant: copies in, runs zs_inflate_index_build_dev, copies res->out_len bytes out. */
+ZS_API int zs_inflate_index_build(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, int window_bits, uint64_t span, uint8_t* out,
+                                  uint64_t out_cap, const uint8_t* dict, uint64_t dict_len, zs_inflate_index_result* res,
+                                  zs_inflate_index** index);
+ZS_API int zs_inflate_index_info_get(const zs_inflate_index* index, zs_inflate_index_info* info);
+/* The first min(n_points, max) points into host arrays (either may be NULL), in stream order. */
+ZS_API int zs_inflate_index_points(const zs_inflate_index* index, uint64_t* in_bit, uint64_t* out_off, uint64_t max);
+/* Serialised index, format version 1, little-endian (synchronises):
+ *   offset  0  "ZSIX"
+ *           4  u32 version (1)
+ *           8  i32 window_bits
+ *          12  u32 reserved (0)
+ *          16  u64 in_len        24  u64 out_len        32  u64 span
+ *          40  u32 check         44  u32 reserved (0)   48  u64 n_points
+ *          56  n_points x { u64 in_bit, u64 out_off, u32 win_len, u32 reserved (0) }
+ *          then the windows back to back, win_len bytes each, in point order.
+ * cap 0: *len receives the size only.  A smaller non-zero cap is ZS_BUF_ERROR. */
+ZS_API int zs_inflate_index_export(const zs_inflate_index* index, uint8_t* buf, uint64_t cap, uint64_t* len);
+/* Rebuilds an index on the context's device from an export.  Everything is validated before the device is touched:
+ * magic, version, window_bits, reserved fields, a length that is exactly header + points + windows, a first point at
+ * output offset 0, points strictly increasing in bit and non-decreasing in output, in_bit < 8 * in_len,
+ * out_off <= out_len, win_len <= 32768 and consistent with out_off and one dictionary length.  Anything else is
+ * ZS_DATA_ERROR (zs_last_error names the check). */
+ZS_API int zs_inflate_index_import(zs_ctx* ctx, const uint8_t* buf, uint64_t len, zs_inflate_index** out);
+/* Frees the index (waits for the device). */
+ZS_API void zs_inflate_index_destroy(zs_inflate_index* index);
+/* Range i is the uncompressed bytes [off[i], off[i] + len[i]) of the indexed stream, written to d_out + d_out_off[i].
+ * d_got[i] = bytes written; d_status[i] = Z_OK (the whole range), Z_BUF_ERROR (clipped at out_len: got < len) or
+ * Z_DATA_ERROR (the input does not decode from a point: a wrong or damaged stream).  On Z_DATA_ERROR got counts the
+ * range's bytes before the failure, and zs_inflate_last_details gives the message code per range (0 when the input
+ * or the stream ended first).  A range spanning k intervals between points is k work items decoded in parallel.
+ * d_in must hold the same stream (8-byte aligned); in_len must equal the index's, else ZS_STREAM_ERROR.  Device
+ * arrays; asynchronous like the other _dev calls. */
+ZS_API int zs_inflate_index_extract_dev(zs_ctx* ctx, const zs_inflate_index* index, const uint8_t* d_in, uint64_t in_len,
+                                        const uint64_t* d_off, const uint64_t* d_len, uint32_t n, uint8_t* d_out,
+                                        const uint64_t* d_out_off, uint64_t* d_got, int32_t* d_status);
+/* Host-buffer variant (synchronises).  It copies in only the input the ranges need -- from the byte of each range's
+ * first point to the byte of the point after its last one, or to in_len, plus the bit reader's read-ahead -- not the
+ * whole stream, and copies back only the bytes written.  Every range as clipped must fit: out_off[i] + its bytes <=
+ * out_cap, else ZS_STREAM_ERROR. */
+ZS_API int zs_inflate_index_extract(zs_ctx* ctx, const zs_inflate_index* index, const uint8_t* in, uint64_t in_len,
+                                    const uint64_t* off, const uint64_t* len, uint32_t n, uint8_t* out, uint64_t out_cap,
+                                    const uint64_t* out_off, uint64_t* got, int32_t* status);
+
 /* ---- multi-member gzip (RFC 1952 2.2: bgzip / BGZF, `cat a.gz b.gz`, appended archives, this engine's own
  *      INDEPENDENT gzip output): every member in one call ----
  * The result is what the reference's multi-member loop produces (test/inflate/test-multistream.ts:16-79):

@@ -394,6 +394,199 @@ def gunzip_dev(d_in: torch.Tensor, out_cap: int, members: int = 0, out: torch.Te
     return _gunzip_result(res, out, table)
 
 
+@dataclass
+class IndexBuild:
+    """What zs_inflate_index_build_dev decoded: the zs_inflate_stream_dev result of the stream."""
+    data: torch.Tensor   # device output, valid to out_len
+    out_len: int
+    in_used: int
+    check: int
+    status: int
+    detail: int
+
+    @property
+    def message(self) -> str:
+        return (capi.load().zs_inflate_message(int(self.detail)) or b"").decode()
+
+
+@dataclass
+class IndexExtract:
+    """Ranges read from an index: range i is data[out_off[i]: out_off[i] + got[i]]."""
+    data: bytes
+    out_off: np.ndarray
+    got: np.ndarray
+    status: np.ndarray   # Z_OK, Z_BUF_ERROR (clipped at the end of the stream), Z_DATA_ERROR
+    details: np.ndarray  # message codes (zs_inflate_message)
+
+    def range(self, i: int) -> bytes:
+        o = int(self.out_off[i])
+        return self.data[o: o + int(self.got[i])]
+
+    def message(self, i: int) -> str:
+        return (capi.load().zs_inflate_message(int(self.details[i])) or b"").decode()
+
+
+class InflateIndex:
+    """Access points into one zlib, gzip or raw deflate stream (zs_inflate_index_*): block starts about every `span`
+    bytes of output, each with the 32 KiB window before it, on the device.  Byte ranges of the stream are then read
+    without decoding what comes before them, many at once.  Close it (or let it be collected) before its context goes.
+
+    `source` is the stream the index was built from when build() had it (host bytes or a device tensor); extract()
+    reads from it unless it is given another copy of the same stream."""
+
+    def __init__(self, handle, ctx: Context, source=None):
+        self._lib = capi.load()
+        self._h = handle
+        self.ctx = ctx
+        self.source = source
+        info = capi.InflateIndexInfo()
+        ctx.check(self._lib.zs_inflate_index_info_get(handle, C.byref(info)), "zs_inflate_index_info_get")
+        self.info = info
+
+    @classmethod
+    def build(cls, data, window_bits: int = 15, span: int = 1 << 20, dictionary=None, out_cap: int | None = None,
+              ctx: Context | None = None):
+        """Decode a whole stream (bytes or a CUDA uint8 tensor) as zs_inflate_stream_dev does and index it.  Returns
+        (index, IndexBuild); the index is None unless the status is Z_STREAM_END.  Without `out_cap` the output room
+        grows until a full-output Z_BUF_ERROR no longer occurs, as gunzip() does."""
+        if isinstance(data, torch.Tensor):
+            assert data.is_cuda and data.dtype == torch.uint8 and data.is_contiguous()
+            ctx = ctx or default_context(data.device.index)
+            d_in, source = data, data
+        else:
+            ctx = ctx or default_context()
+            source = _as_u8(data)
+            # (an empty stream still needs a real pointer: a slice of a small buffer)
+            d_in = torch.from_numpy(source.copy()).to(f"cuda:{ctx.device}") if source.size else \
+                torch.zeros(8, dtype=torch.uint8, device=f"cuda:{ctx.device}")[:0]
+        d_dict = None
+        if dictionary is not None and len(dictionary):
+            d_dict = torch.from_numpy(_as_u8(dictionary).copy()).to(d_in.device)
+        n = d_in.numel()
+        grow = out_cap is None
+        cap = max(4 * n, 1 << 16) if grow else int(out_cap)
+        lib = capi.load()
+        while True:
+            out = torch.empty(cap + 16, dtype=torch.uint8, device=d_in.device)
+            res = capi.InflateIndexResult()
+            h = C.c_void_p()
+            rc = lib.zs_inflate_index_build_dev(ctx.handle, _ptr(d_in), n, window_bits, span, _ptr(out),
+                                                cap, _ptr(d_dict), d_dict.numel() if d_dict is not None else 0, C.byref(res),
+                                                C.byref(h))
+            ctx.check(rc, "zs_inflate_index_build_dev")
+            if grow and res.status == capi.Z_BUF_ERROR and res.out_len == cap:
+                cap *= 2
+                continue
+            built = IndexBuild(out, int(res.out_len), int(res.in_used), int(res.check), int(res.status), int(res.detail))
+            return (cls(h, ctx, source) if h.value else None), built
+
+    @classmethod
+    def from_bytes(cls, blob, ctx: Context | None = None, source=None) -> "InflateIndex":
+        """An index from to_bytes() output (zs_inflate_index_import): a malformed blob raises with Z_DATA_ERROR."""
+        ctx = ctx or default_context()
+        src = _as_u8(blob)
+        h = C.c_void_p()
+        rc = capi.load().zs_inflate_index_import(ctx.handle, src.ctypes.data if src.size else None, src.size, C.byref(h))
+        ctx.check(rc, "zs_inflate_index_import")
+        return cls(h, ctx, source)
+
+    @property
+    def handle(self):
+        if not self._h:
+            raise ValueError("InflateIndex is closed")
+        return self._h
+
+    @property
+    def points(self) -> np.ndarray:
+        """(n_points, 2) uint64: input bit and output offset of every access point."""
+        n = int(self.info.n_points)
+        bit = np.zeros(n, dtype=np.uint64)
+        off = np.zeros(n, dtype=np.uint64)
+        self.ctx.check(self._lib.zs_inflate_index_points(self.handle, bit.ctypes.data, off.ctypes.data, n),
+                       "zs_inflate_index_points")
+        return np.stack([bit, off], axis=1)
+
+    def to_bytes(self) -> bytes:
+        """The export format of include/zsgpu.h (version 1)."""
+        n = C.c_uint64(0)
+        self.ctx.check(self._lib.zs_inflate_index_export(self.handle, None, 0, C.byref(n)), "zs_inflate_index_export")
+        buf = np.zeros(n.value, dtype=np.uint8)
+        self.ctx.check(self._lib.zs_inflate_index_export(self.handle, buf.ctypes.data, n.value, C.byref(n)),
+                       "zs_inflate_index_export")
+        return buf.tobytes()
+
+    def extract_dev(self, d_in: torch.Tensor, off: torch.Tensor, length: torch.Tensor, out: torch.Tensor,
+                    out_off: torch.Tensor, got: torch.Tensor | None = None, status: torch.Tensor | None = None):
+        """zs_inflate_index_extract_dev on device arrays (int64 off / length / out_off); no synchronisation.
+        Returns (got, status) device tensors."""
+        n = off.numel()
+        got = got if got is not None else torch.zeros(n, dtype=torch.int64, device=off.device)
+        status = status if status is not None else torch.zeros(n, dtype=torch.int32, device=off.device)
+        rc = self._lib.zs_inflate_index_extract_dev(self.ctx.handle, self.handle, _ptr(d_in), d_in.numel(), _ptr(off),
+                                                    _ptr(length), n, _ptr(out), _ptr(out_off), _ptr(got), _ptr(status))
+        self.ctx.check(rc, "zs_inflate_index_extract_dev")
+        return got, status
+
+    def extract_ranges(self, off, length, data=None) -> IndexExtract:
+        """Ranges [off[i], off[i] + length[i]) of the stream, packed one after the other, with their statuses and
+        message codes.  A device source goes through extract_dev, a host one through zs_inflate_index_extract."""
+        src = self.source if data is None else data
+        if src is None:
+            raise ValueError("the index has no source stream: pass the stream as `data`")
+        off = np.ascontiguousarray(np.asarray(off, dtype=np.uint64).reshape(-1))
+        length = np.ascontiguousarray(np.asarray(length, dtype=np.uint64).reshape(-1))
+        n = off.size
+        out_len = int(self.info.out_len)
+        clipped = np.minimum(length, np.uint64(out_len) - np.minimum(off, np.uint64(out_len)))   # the bytes each range gets
+        out_off = np.zeros(n, dtype=np.uint64)
+        if n > 1:
+            np.cumsum(clipped[:-1], out=out_off[1:])
+        cap = int(clipped.sum()) if n else 0
+        details = np.zeros(n, dtype=np.int32)
+        if isinstance(src, torch.Tensor):
+            dev = src.device
+            t = lambda a: torch.from_numpy(a.view(np.int64)).to(dev)
+            out = torch.zeros(cap + 16, dtype=torch.uint8, device=dev)
+            got_t, status_t = self.extract_dev(src, t(off), t(length), out, t(out_off))
+            got = got_t.cpu().numpy().view(np.uint64)
+            status = status_t.cpu().numpy()
+            data_out = out[:cap].cpu().numpy().tobytes()
+        else:
+            s = _as_u8(src)
+            outb = np.zeros(cap + 16, dtype=np.uint8)
+            got = np.zeros(n, dtype=np.uint64)
+            status = np.zeros(n, dtype=np.int32)
+            rc = self._lib.zs_inflate_index_extract(self.ctx.handle, self.handle, s.ctypes.data if s.size else None, s.size,
+                                                    off.ctypes.data, length.ctypes.data, n, outb.ctypes.data, cap,
+                                                    out_off.ctypes.data, got.ctypes.data, status.ctypes.data)
+            self.ctx.check(rc, "zs_inflate_index_extract")
+            data_out = outb[:cap].tobytes()
+        if n:
+            self.ctx.check(self._lib.zs_inflate_last_details(self.ctx.handle, details.ctypes.data, n), "zs_inflate_last_details")
+        return IndexExtract(data_out, out_off, got, status, details)
+
+    def extract(self, ranges, data=None) -> list:
+        """[(off, length), ...] -> the bytes of each range (shorter where it runs past the end of the stream).  A range
+        the stream does not decode for raises ZsError with Z_DATA_ERROR."""
+        ranges = list(ranges)
+        r = self.extract_ranges([o for o, _ in ranges], [n for _, n in ranges], data)
+        bad = np.nonzero(r.status == capi.Z_DATA_ERROR)[0]
+        if bad.size:
+            raise capi.ZsError(capi.Z_DATA_ERROR, "zs_inflate_index_extract", f"range {int(bad[0])}: {r.message(int(bad[0]))}")
+        return [r.range(i) for i in range(len(ranges))]
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.zs_inflate_index_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def checksum(data, kind: int, init: int | None = None, ctx: Context | None = None) -> int:
     """adler32(adler, buf, len) / crc32(crc, buf, len) of a host buffer, computed on the GPU."""
     ctx = ctx or default_context()

@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libzsgpu.so")
-SOURCES = ["zs_api.cu", "zs_checksum.cu", "zs_inflate.cu", "zs_inflate_par.cu", "zs_inflate_tps.cu", "zs_lz77.cu", "zs_huff.cu", "zs_stream.cu", "zs_gunzip.cu"]
+SOURCES = ["zs_api.cu", "zs_checksum.cu", "zs_inflate.cu", "zs_inflate_par.cu", "zs_inflate_tps.cu", "zs_lz77.cu", "zs_huff.cu", "zs_stream.cu", "zs_gunzip.cu", "zs_inflate_index.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--use_fast_math",

@@ -48,6 +48,18 @@ class GzMember(C.Structure):
                 ("crc32", C.c_uint32)]
 
 
+class InflateIndexInfo(C.Structure):
+    """zs_inflate_index_info of include/zsgpu.h"""
+    _fields_ = [("in_len", C.c_uint64), ("out_len", C.c_uint64), ("span", C.c_uint64), ("n_points", C.c_uint64),
+                ("check", C.c_uint32), ("window_bits", C.c_int32)]
+
+
+class InflateIndexResult(C.Structure):
+    """zs_inflate_index_result of include/zsgpu.h"""
+    _fields_ = [("out_len", C.c_uint64), ("in_used", C.c_uint64), ("check", C.c_uint32), ("status", C.c_int32),
+                ("detail", C.c_int32)]
+
+
 class ZsError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ""):
         super().__init__(f"{where} failed with {code}" + (f": {detail}" if detail else ""))
@@ -99,6 +111,19 @@ _PROTOTYPES = {
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]),
     "zs_inflate_message": (C.c_char_p, [C.c_int]),
     "zs_inflate_last_details": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32]),
+    "zs_inflate_index_build_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_uint64, C.c_void_p, C.c_uint64,
+                                             C.c_void_p, C.c_uint64, C.POINTER(InflateIndexResult), C.POINTER(C.c_void_p)]),
+    "zs_inflate_index_build": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_uint64, C.c_void_p, C.c_uint64,
+                                         C.c_void_p, C.c_uint64, C.POINTER(InflateIndexResult), C.POINTER(C.c_void_p)]),
+    "zs_inflate_index_info_get": (C.c_int, [C.c_void_p, C.POINTER(InflateIndexInfo)]),
+    "zs_inflate_index_points": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]),
+    "zs_inflate_index_export": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "zs_inflate_index_import": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]),
+    "zs_inflate_index_destroy": (None, [C.c_void_p]),
+    "zs_inflate_index_extract_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                               C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "zs_inflate_index_extract": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32,
+                                           C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "zs_gunzip_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                 C.c_uint64]),
     "zs_gunzip": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64]),

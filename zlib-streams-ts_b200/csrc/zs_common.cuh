@@ -36,6 +36,10 @@ enum zs_scratch_slot {
     // copy of a member decoded alone.  Its own: the batch and one-stream inflate calls it makes use none of them, and
     // zs_gunzip stages its input and output in SCR_H_IN / SCR_H_OUT around them
     SCR_G_TILE, SCR_G_CAND, SCR_G_PASS, SCR_G_MEMB, SCR_G_ALIGN,
+    // zs_inflate_index.cu.  Build: the one-stream call's results and the record pass's start record and counters.
+    // Extract: per-range plan and verdicts, per-warp history rings, and the staged input of the host-buffer call (its
+    // output goes to SCR_H_OUT)
+    SCR_X_BUILD, SCR_X_PLAN, SCR_X_RING, SCR_X_IN,
     ZS_SCR_COUNT
 };
 
@@ -286,6 +290,9 @@ struct zs_inflate_args {
 int zs_launch_inflate(zs_ctx* ctx, const zs_inflate_args& a, uint32_t n_choice);
 int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
                                const uint8_t* d_hist, uint64_t hist_len, uint64_t* d_state, uint64_t* d_resume);
+int zs_launch_inflate_record(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint64_t out_cap, bool planned, uint64_t* d_state,
+                             const uint64_t* d_tail, int wrap, uint64_t span, uint64_t* d_rec, uint64_t rec_cap,
+                             unsigned long long* d_cnt);
 int zs_launch_inflate_verify(zs_ctx* ctx, uint32_t n, const uint32_t* d_adler, const uint32_t* d_crc,
                              const uint32_t* d_trailer, const uint32_t* d_flags, const uint64_t* d_out_len,
                              uint32_t* d_checks, int32_t* d_status, int32_t* d_detail);

@@ -28,7 +28,11 @@
 //                       the end of the stream, or for whatever the parallel part could not prove (an error,
 //                       truncated input, output space running out, a distance beyond the start of the
 //                       stream), so that status, message and output prefix stay the reference's.
+//   par_record_kernel   launched only by the index build (zs_inflate_index.cu), after a decode: the planned segments
+//                       and the serial decoder's part walked again, lengths only, keeping the block starts an index
+//                       of access points may use.
 #include <cstdio>
+#include <cstring>
 
 #include "zs_inflate_common.cuh"
 
@@ -296,11 +300,25 @@ __global__ void par_spec_merge_kernel(ParArgs a) {
     }
 }
 
+// Where the index build's pass (kRecord) appends the block starts it keeps: (bit, output offset) pairs at
+// rec[2i], rec[2i + 1], i taken from cnt[0]; cnt[1] counts the walks that reached their end.
+struct RecordSink {
+    uint64_t* rec;
+    uint64_t cap;        // pairs
+    unsigned long long* cnt;
+    uint64_t span;
+};
+
 // One segment, decoded by a warp from bit `start_bit`.  kWrite = false: lengths only (count pass), stops on a
-// later candidate; true: symbols to a.sym + out_base, stops at end_bit.
-template <bool kWrite>
+// later candidate; true: symbols to a.sym + out_base, stops at end_bit.  kRecord (with kWrite = false): lengths
+// only from start_bit to stop_bit or the end of the last block, the index build's pass (zs_inflate_index.cu): it
+// keeps the first block start and every later one that some multiple of the span falls on -- one whose output
+// offset o has a multiple of rs->span in (o of the block start before it, o].  A block start the access-point
+// rule selects is always kept, whichever walk it falls in.
+template <bool kWrite, bool kRecord = false>
 __device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, const FixedTables& F, uint32_t slot, uint64_t start_bit,
-                                               uint64_t stop_bit, uint64_t out_base, uint64_t avail_hist, SegInfo* info, uint32_t* err) {
+                                               uint64_t stop_bit, uint64_t out_base, uint64_t avail_hist, SegInfo* info, uint32_t* err,
+                                               const RecordSink* rs = nullptr) {
     const unsigned lane = zs_lane();
     BitReader br;
     br.base = a.in;
@@ -322,10 +340,22 @@ __device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, c
     uint64_t end_bit = 0;
     uint32_t next_slot = 0;
     bool last = false;
+    uint64_t rec_prev = 0;   // kRecord: output offset of the block start before this one (none yet: ~0)
+    if (kRecord) rec_prev = ~0ull;
     while (!bad) {
         // ---- a block boundary ----
         const uint64_t here_bit = br.pos * 8 - br.bits;
-        if (kWrite) {
+        if (kRecord) {
+            if (here_bit >= stop_bit || last) { status = SEG_LANDED; break; }
+            const uint64_t o = out_base + op;
+            if (rec_prev == ~0ull || o / rs->span > rec_prev / rs->span) {
+                if (lane == 0) {
+                    const unsigned long long i = atomicAdd(rs->cnt, 1ull);
+                    if (i < rs->cap) { rs->rec[2 * i] = here_bit; rs->rec[2 * i + 1] = o; }
+                }
+            }
+            rec_prev = o;
+        } else if (kWrite) {
             if (here_bit >= stop_bit) { status = SEG_LANDED; break; }
         } else if (here_bit > start_bit) {
             if (last) { status = SEG_FINAL; end_bit = here_bit; break; }
@@ -365,7 +395,7 @@ __device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, c
                 for (uint64_t j = lane; j < n; j += 32) sym[op + j] = a.in[br.pos + j];
             br.pos += n;
             op += n;
-            if (!kWrite && op > a.out_cap) break;
+            if (!kWrite && !kRecord && op > a.out_cap) break;
             continue;
         } else if (type == 1) {
             lcode = F.len; dcode = F.dist; lenbits = 9; distbits = 5;
@@ -418,11 +448,12 @@ __device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, c
                 __syncwarp();
             }
             op += len;
-            if (!kWrite && op > a.out_cap) break;
+            if (!kWrite && !kRecord && op > a.out_cap) break;
         }
         if (!block_ok) break;
     }
-    if (!kWrite && lane == 0) {
+    if (kRecord && lane == 0 && status == SEG_LANDED) atomicAdd(rs->cnt + 1, 1ull);
+    if (!kWrite && !kRecord && lane == 0) {
         SegInfo r;
         r.end_bit = end_bit; r.out_len = op; r.status = status; r.next_slot = next_slot;
         *info = r;
@@ -647,12 +678,47 @@ __global__ void par_finish_kernel(ParArgs a) {
     }
 }
 
-}  // namespace
+// The index build's pass (zs_inflate_index.cu).  Warp item 0 walks what the serial decoder decoded: from bit tail[0]
+// (~0: the first block, behind the wrapper header) with tail[1] bytes before it -- nothing when tail[2] & 4 says the
+// planned segments reached the last block.  Items 1..n are the planned segments of the decode that ran before.  The
+// walk goes first: it is the longest item whenever the parallel part gave up early.
+__global__ void __launch_bounds__(kWarps * 32) par_record_kernel(ParArgs a, RecordSink rs, const uint64_t* tail, int wrap) {
+    __shared__ WarpArena s_arena[kWarps];
+    __shared__ FixedTables s_fixed;
+    const unsigned wid = threadIdx.x >> 5;
+    if (wid == 0) build_fixed_tables(s_fixed, s_arena[0], false);
+    __syncthreads();
+    const uint64_t n = a.state ? a.state[0] : 0;
+    for (uint64_t k = (uint64_t)blockIdx.x * kWarps + wid; k <= n; k += (uint64_t)gridDim.x * kWarps) {
+        if (k == 0) {
+            if (tail[2] & 4u) {
+                if (zs_lane() == 0) atomicAdd(rs.cnt + 1, 1ull);
+                continue;
+            }
+            uint64_t bit = tail[0], out = tail[1];
+            if (bit == ~0ull) {
+                BitReader br;
+                br.base = a.in; br.pos = 0; br.end = a.in_len; br.safe_end = (a.in_len + 7) & ~7ull; br.hold = 0; br.bits = 0;
+                int status = ZS_OK, detail = D_NONE;
+                unsigned tflags = 0;
+                // (a zlib header with FDICT reports Z_NEED_DICT here: the stream decoded with its dictionary already)
+                if (wrap) read_wrapper_header(br, wrap, status, detail, tflags, nullptr);
+                bit = br.pos * 8 - br.bits;
+                out = 0;
+            }
+            decode_segment<false, true>(a, s_arena[wid], s_fixed, 0, bit, ~0ull, out, 0, nullptr, nullptr, &rs);
+        } else {
+            const uint32_t slot = a.plan_slot[k - 1];
+            decode_segment<false, true>(a, s_arena[wid], s_fixed, slot, a.cand[slot], a.seg[slot].end_bit, a.plan_off[k - 1], 0,
+                                        nullptr, nullptr, &rs);
+        }
+        __syncwarp();
+    }
+}
 
-// One stream, wrapper header already located: a.d_resume receives where inflate_kernel continues.
-int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
-                               const uint8_t* d_hist, uint64_t hist_len, uint64_t* d_state, uint64_t* d_resume) {
-    ParArgs p;
+// The decoder's view of its scratch for one stream of in_len bytes and out_cap bytes of output room.  The same sizes
+// give the same buffers, so a later call finds there what the decode left.
+int par_args(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint64_t out_cap, uint64_t* d_state, ParArgs& p, unsigned& n_groups) {
     p.in = d_in; p.in_len = in_len;
     // At most 6144 candidates (1.3 waves of warps); for shorter inputs the tiles shrink to 8 KiB so that every flush
     // point of a stream cut every 64 KiB is a candidate: what an attempt costs is the slowest warp, and a warp that
@@ -671,7 +737,7 @@ int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len
     uint8_t* plan = (uint8_t*)zs_scratch_get(ctx, SCR_P_PLAN, (size_t)p.n_slots * 16 + 64);
     p.sym = (uint16_t*)zs_scratch_get(ctx, SCR_P_SYM, (size_t)out_cap * 2 + 64);
     p.windows = (uint8_t*)zs_scratch_get(ctx, SCR_P_WIN, ((size_t)p.n_slots + 1) * kWin);
-    const unsigned n_groups = (p.n_slots + kWinGroup - 1) / kWinGroup;
+    n_groups = (p.n_slots + kWinGroup - 1) / kWinGroup;
     p.gmap = (uint16_t*)zs_scratch_get(ctx, SCR_P_GMAP, (size_t)n_groups * kWin * 2);
     if (!p.cand || !p.seg || !plan || !p.sym || !p.windows || !p.gmap) return ZS_MEM_ERROR;
     p.plan_off = (uint64_t*)plan;                                   // [n_slots + 1]
@@ -679,6 +745,19 @@ int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len
     p.plan_err = p.plan_slot + p.n_slots;                           // [n_slots]  (16 bytes per slot + 8 in all)
     p.state = d_state;
     p.out_cap = out_cap;
+    p.hist_len = 0; p.hist = nullptr; p.out = nullptr; p.resume = nullptr;
+    return ZS_OK;
+}
+
+}  // namespace
+
+// One stream, wrapper header already located: a.d_resume receives where inflate_kernel continues.
+int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap,
+                               const uint8_t* d_hist, uint64_t hist_len, uint64_t* d_state, uint64_t* d_resume) {
+    ParArgs p;
+    unsigned n_groups = 0;
+    const int rc = par_args(ctx, d_in, in_len, out_cap, d_state, p, n_groups);
+    if (rc != ZS_OK) return rc;
     p.hist_len = hist_len > kWin ? kWin : hist_len;
     p.hist = d_hist + (hist_len > kWin ? hist_len - kWin : 0);
     p.out = d_out;
@@ -715,5 +794,30 @@ int zs_launch_inflate_parallel(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len
     ZS_KERNEL(ctx, "par_window_kernel", par_window_kernel<<<n_groups, 1024, 2 * kWin, ctx->stream>>>(p));
     ZS_KERNEL(ctx, "par_resolve_kernel", par_resolve_kernel<<<sms * 8u, 256, 0, ctx->stream>>>(p));
     ZS_KERNEL(ctx, "par_finish_kernel", par_finish_kernel<<<1, 32, 0, ctx->stream>>>(p));
+    return ZS_OK;
+}
+
+// The index build's record pass (par_record_kernel) over one stream that zs_inflate_stream_dev decoded just before
+// with the same in_len and out_cap.  planned: that decode took the segment-parallel path, whose plan is still in its
+// scratch and whose state (SCR_P_STATE) is d_state; otherwise the whole stream is walked from its wrapper header.
+// d_tail: the walk's start record (see par_record_kernel); d_cnt[2] zeroed by the caller.
+int zs_launch_inflate_record(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint64_t out_cap, bool planned, uint64_t* d_state,
+                             const uint64_t* d_tail, int wrap, uint64_t span, uint64_t* d_rec, uint64_t rec_cap,
+                             unsigned long long* d_cnt) {
+    ParArgs p;
+    memset(&p, 0, sizeof(p));
+    unsigned ctas = 1;
+    if (planned) {
+        unsigned n_groups = 0;
+        const int rc = par_args(ctx, d_in, in_len, out_cap, d_state, p, n_groups);
+        if (rc != ZS_OK) return rc;
+        ctas = (p.n_slots + 1 + kWarps - 1) / kWarps;
+        if (ctas > (unsigned)ctx->sm_count * 8u) ctas = (unsigned)ctx->sm_count * 8u;
+    } else {
+        p.in = d_in; p.in_len = in_len; p.tile = 1; p.out_cap = ~0ull;
+    }
+    RecordSink rs;
+    rs.rec = d_rec; rs.cap = rec_cap; rs.cnt = d_cnt; rs.span = span;
+    ZS_KERNEL(ctx, "par_record_kernel", par_record_kernel<<<ctas, kWarps * 32, 0, ctx->stream>>>(p, rs, d_tail, wrap));
     return ZS_OK;
 }
