@@ -8,6 +8,8 @@
 #include "zs_common.cuh"
 
 constexpr uint64_t kParMinInput = 128u << 10;   // shorter streams are decoded by one warp
+// SCR_I_STREAM: zs_inflate_stream_dev's offsets (in [2], out [2], dictionary [2]), then inflate_stream_one's results
+constexpr size_t kStreamScratch = 9 * 8;
 
 // ---- scratch (slots: zs_common.cuh) -----------------------------------------------------------------
 void* zs_scratch_get(zs_ctx* ctx, zs_scratch_slot slot, size_t bytes) {
@@ -73,6 +75,11 @@ int zs_set_cuda_error(zs_ctx* ctx, cudaError_t e, const char* where) {
     return ZS_E_CUDA;
 }
 
+int zs_bad_arg(zs_ctx* ctx, const char* msg) {
+    if (ctx) snprintf(ctx->err, sizeof(ctx->err), "%s", msg);
+    return ZS_STREAM_ERROR;
+}
+
 namespace {
 
 // dictionary ranges [begin, end) -> (begin, length) for the checksum kernels
@@ -91,11 +98,6 @@ __global__ void make_chunk_offsets_kernel(uint64_t* off, uint64_t len, uint64_t 
 
 // Every entry point works on the context's device, whatever the caller's current device is.
 inline void bind_device(zs_ctx* ctx) { cudaSetDevice(ctx->device); }
-
-int bad_arg(zs_ctx* ctx, const char* msg) {
-    if (ctx) snprintf(ctx->err, sizeof(ctx->err), "%s", msg);
-    return ZS_STREAM_ERROR;
-}
 
 // The copy streams and events of the pipelined host-buffer paths, created by the first such call.
 int ensure_copy_streams(zs_ctx* ctx) {
@@ -241,13 +243,13 @@ uint32_t zs_adler32_combine(uint32_t a1, uint32_t a2, uint64_t len2) { return zs
 int zs_checksum_batch_dev(zs_ctx* ctx, int kind, const uint8_t* d_buf, const uint64_t* d_off, uint32_t n,
                           uint32_t* d_out) {
     if (ctx) bind_device(ctx);
-    if (!ctx || (kind != 0 && kind != 1) || (n && (!d_buf || !d_off || !d_out))) return bad_arg(ctx, "checksum: bad arguments");
+    if (!ctx || (kind != 0 && kind != 1) || (n && (!d_buf || !d_off || !d_out))) return zs_bad_arg(ctx, "checksum: bad arguments");
     return zs_launch_checksum_segments(ctx, kind, d_buf, d_off, nullptr, n, d_out);
 }
 
 int zs_checksum_dev(zs_ctx* ctx, int kind, const uint8_t* d_buf, uint64_t len, uint32_t init, uint32_t* result) {
     if (ctx) bind_device(ctx);
-    if (!ctx || (kind != 0 && kind != 1) || !result || (len && !d_buf)) return bad_arg(ctx, "checksum: bad arguments");
+    if (!ctx || (kind != 0 && kind != 1) || !result || (len && !d_buf)) return zs_bad_arg(ctx, "checksum: bad arguments");
     uint32_t* d_res = (uint32_t*)zs_scratch_get(ctx, SCR_SMALL, 256);
     if (!d_res) return ZS_MEM_ERROR;
     int rc = zs_launch_checksum_whole(ctx, kind, d_buf, len, init, d_res);
@@ -259,7 +261,7 @@ int zs_checksum_dev(zs_ctx* ctx, int kind, const uint8_t* d_buf, uint64_t len, u
 
 int zs_checksum(zs_ctx* ctx, int kind, const uint8_t* buf, uint64_t len, uint32_t init, uint32_t* result) {
     if (ctx) bind_device(ctx);
-    if (!ctx || !result || (len && !buf)) return bad_arg(ctx, "checksum: bad arguments");
+    if (!ctx || !result || (len && !buf)) return zs_bad_arg(ctx, "checksum: bad arguments");
     uint8_t* d_in = (uint8_t*)zs_scratch_get(ctx, SCR_H_IN, len + 64);
     if (!d_in) return ZS_MEM_ERROR;
     if (len) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in, buf, len, cudaMemcpyHostToDevice, ctx->stream));
@@ -278,28 +280,28 @@ static int deflate_batch_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uin
                              zs_deflate_result* d_result, uint32_t seg_hint) {
     if (level == -1) level = 6;
     // argument rules of deflateInit2_ (deflate.ts:263-297) that apply to the batch form
-    if (level < 0 || level > 9) return bad_arg(ctx, "deflate: level must be 0..9");
+    if (level < 0 || level > 9) return zs_bad_arg(ctx, "deflate: level must be 0..9");
     const int strategy = (int)((flags >> 8) & 7u);
-    if (strategy > ZS_STRATEGY_FIXED) return bad_arg(ctx, "deflate: unknown strategy");
+    if (strategy > ZS_STRATEGY_FIXED) return zs_bad_arg(ctx, "deflate: unknown strategy");
     if (wrap < 0 || wrap > 2 || (mode != ZS_MODE_INDEPENDENT && mode != ZS_MODE_STITCHED))
-        return bad_arg(ctx, "deflate: bad wrap or mode");
-    if (!d_out || !d_result || (in_len && !d_in) || n_chunks == 0) return bad_arg(ctx, "deflate: null buffer or zero chunks");
-    if ((reinterpret_cast<uintptr_t>(d_out) & 15u) != 0) return bad_arg(ctx, "deflate: d_out must be 16-byte aligned");
+        return zs_bad_arg(ctx, "deflate: bad wrap or mode");
+    if (!d_out || !d_result || (in_len && !d_in) || n_chunks == 0) return zs_bad_arg(ctx, "deflate: null buffer or zero chunks");
+    if ((reinterpret_cast<uintptr_t>(d_out) & 15u) != 0) return zs_bad_arg(ctx, "deflate: d_out must be 16-byte aligned");
     if ((flags & ZS_FLAG_PRIME) && (mode != ZS_MODE_INDEPENDENT || wrap != ZS_WRAP_RAW))
-        return bad_arg(ctx, "deflate: ZS_FLAG_PRIME needs INDEPENDENT mode and the raw wrapper (deflate.ts:373)");
+        return zs_bad_arg(ctx, "deflate: ZS_FLAG_PRIME needs INDEPENDENT mode and the raw wrapper (deflate.ts:373)");
     if (history > 32768) history = 32768;
     // an empty part still names its position (its history lies before it): a null pointer with history is
     // a caller error, never a device fault
-    if (!d_in && history) return bad_arg(ctx, "deflate: history given without an input pointer");
+    if (!d_in && history) return zs_bad_arg(ctx, "deflate: history given without an input pointer");
     if (mode == ZS_MODE_INDEPENDENT && !(flags & ZS_FLAG_PRIME)) history = 0;
     if (!d_in_off) {
-        if (chunk_size == 0) return bad_arg(ctx, "deflate: chunk_size is zero");
+        if (chunk_size == 0) return zs_bad_arg(ctx, "deflate: chunk_size is zero");
         uint64_t want = in_len ? (in_len + chunk_size - 1) / chunk_size : 1;
-        if (want != n_chunks) return bad_arg(ctx, "deflate: n_chunks does not match in_len / chunk_size");
+        if (want != n_chunks) return zs_bad_arg(ctx, "deflate: n_chunks does not match in_len / chunk_size");
         max_chunk = chunk_size;
     }
     if (max_chunk == 0) max_chunk = 1;
-    if (in_len > 0xffffffff00ull) return bad_arg(ctx, "deflate: input too large for one call");
+    if (in_len > 0xffffffff00ull) return zs_bad_arg(ctx, "deflate: input too large for one call");
 
     zs_deflate_plan p;
     memset(&p, 0, sizeof(p));
@@ -387,7 +389,7 @@ int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, cons
 // ---- preset dictionaries ------------------------------------------------------------------------------
 int zs_deflate_dict_create(zs_ctx* ctx, const uint8_t* dict, uint64_t dict_len, zs_deflate_dict** out) {
     if (ctx) bind_device(ctx);
-    if (!ctx || !out || (dict_len && !dict)) return bad_arg(ctx, "deflate_dict_create: bad arguments");
+    if (!ctx || !out || (dict_len && !dict)) return zs_bad_arg(ctx, "deflate_dict_create: bad arguments");
     *out = nullptr;
     // deflateSetDictionary (deflate.ts:367-424): only the last w_size bytes are used; DICTID covers them all
     const uint64_t used = dict_len < 32768 ? dict_len : 32768;
@@ -442,10 +444,10 @@ void zs_deflate_dict_destroy(zs_deflate_dict* d) {
 // the arguments zlib refuses with a dictionary (deflateSetDictionary, deflate.ts:372) and those the batch form
 // has no meaning for: every chunk is one whole independent stream
 static int check_dict_call(zs_ctx* ctx, const zs_deflate_dict* dict, int wrap, uint32_t flags) {
-    if (!dict) return bad_arg(ctx, "deflate_batch_dict: no dictionary");
-    if (dict->device != ctx->device) return bad_arg(ctx, "deflate_batch_dict: dictionary prepared for another device");
-    if (wrap != ZS_WRAP_RAW && wrap != ZS_WRAP_ZLIB) return bad_arg(ctx, "deflate_batch_dict: gzip streams take no dictionary (deflate.ts:372)");
-    if (flags & ~(7u << 8)) return bad_arg(ctx, "deflate_batch_dict: flags carry the strategy only");
+    if (!dict) return zs_bad_arg(ctx, "deflate_batch_dict: no dictionary");
+    if (dict->device != ctx->device) return zs_bad_arg(ctx, "deflate_batch_dict: dictionary prepared for another device");
+    if (wrap != ZS_WRAP_RAW && wrap != ZS_WRAP_ZLIB) return zs_bad_arg(ctx, "deflate_batch_dict: gzip streams take no dictionary (deflate.ts:372)");
+    if (flags & ~(7u << 8)) return zs_bad_arg(ctx, "deflate_batch_dict: flags carry the strategy only");
     return ZS_OK;
 }
 
@@ -502,7 +504,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         const bool grow = level >= 4 && !getenv("ZS_SLICE_WAVES");
         uint32_t w = waves_per_slice;
         while (cb[n_slices] < n_chunks) {
-            if (n_slices >= kMaxSlices) return bad_arg(ctx, "deflate: internal slicing error");
+            if (n_slices >= kMaxSlices) return zs_bad_arg(ctx, "deflate: internal slicing error");
             uint64_t next = (uint64_t)cb[n_slices] + (uint64_t)seg * wave * w;
             if (next > n_chunks || n_slices + 1 == kMaxSlices) next = n_chunks;
             cb[++n_slices] = (uint32_t)next;
@@ -629,17 +631,17 @@ static int deflate_batch_host(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
                               uint32_t history, const uint64_t* in_off, uint32_t n_chunks, uint32_t chunk_size, int level,
                               int wrap, int mode, uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off,
                               uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result) {
-    if (!out || !result || (in_len && !in) || n_chunks == 0) return bad_arg(ctx, "deflate: null buffer or zero chunks");
-    if (history && !in) return bad_arg(ctx, "deflate: history without an input pointer");
+    if (!out || !result || (in_len && !in) || n_chunks == 0) return zs_bad_arg(ctx, "deflate: null buffer or zero chunks");
+    if (history && !in) return zs_bad_arg(ctx, "deflate: history without an input pointer");
     if (history > 32768) history = 32768;
     uint32_t max_chunk = chunk_size;
     if (in_off) {
         max_chunk = 1;
-        if (in_off[0] != 0 || in_off[n_chunks] != in_len) return bad_arg(ctx, "deflate: in_off must span [0, in_len]");
+        if (in_off[0] != 0 || in_off[n_chunks] != in_len) return zs_bad_arg(ctx, "deflate: in_off must span [0, in_len]");
         for (uint32_t i = 0; i < n_chunks; i++) {
-            if (in_off[i + 1] < in_off[i]) return bad_arg(ctx, "deflate: in_off must be non-decreasing");
+            if (in_off[i + 1] < in_off[i]) return zs_bad_arg(ctx, "deflate: in_off must be non-decreasing");
             uint64_t l = in_off[i + 1] - in_off[i];
-            if (l > 0xffffffffull) return bad_arg(ctx, "deflate: chunk too large");
+            if (l > 0xffffffffull) return zs_bad_arg(ctx, "deflate: chunk too large");
             if (l > max_chunk) max_chunk = (uint32_t)l;
         }
     }
@@ -707,17 +709,17 @@ int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t hi
                     int wrap, uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_bits, zs_deflate_result* result) {
     if (ctx) bind_device(ctx);
     if (!ctx) return ZS_STREAM_ERROR;
-    if (chunk_size == 0) return bad_arg(ctx, "deflate: chunk_size is zero");
-    if (flags & ZS_FLAG_PRIME) return bad_arg(ctx, "deflate: ZS_FLAG_PRIME does not apply to a part of a stream");
+    if (chunk_size == 0) return zs_bad_arg(ctx, "deflate: chunk_size is zero");
+    if (flags & ZS_FLAG_PRIME) return zs_bad_arg(ctx, "deflate: ZS_FLAG_PRIME does not apply to a part of a stream");
     const uint64_t nc = in_len ? (in_len + chunk_size - 1) / chunk_size : 1;
-    if (nc > 0xffffffffull) return bad_arg(ctx, "deflate: too many chunks");
+    if (nc > 0xffffffffull) return zs_bad_arg(ctx, "deflate: too many chunks");
     return deflate_batch_host(ctx, nullptr, in, in_len, history, nullptr, (uint32_t)nc, chunk_size, level, wrap, ZS_MODE_STITCHED,
                               flags, out, out_cap, nullptr, out_bits, nullptr, result);
 }
 
 int zs_bit_concat_dev(zs_ctx* ctx, uint8_t* d_dst, uint64_t dst_bit_off, const uint8_t* d_src, uint64_t n_bits) {
     if (ctx) bind_device(ctx);
-    if (!ctx || !d_dst || (n_bits && !d_src)) return bad_arg(ctx, "bit_concat: bad arguments");
+    if (!ctx || !d_dst || (n_bits && !d_src)) return zs_bad_arg(ctx, "bit_concat: bad arguments");
     return zs_launch_bit_concat(ctx, d_dst, dst_bit_off, d_src, n_bits);
 }
 
@@ -731,10 +733,10 @@ static int inflate_batch_dev_impl(zs_ctx* ctx, const uint8_t* d_in, const uint64
                                   uint32_t* d_checks, int32_t* d_status, const uint8_t* d_dict, const uint64_t* d_dict_rng,
                                   const InflateOpts& o, InflateOut* res) {
     if (n == 0) return ZS_OK;
-    if (!d_in || !d_in_off || !d_out || !d_out_off || !d_out_len || !d_status) return bad_arg(ctx, "inflate: null buffer");
-    if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return bad_arg(ctx, "inflate: d_in must be 8-byte aligned");
+    if (!d_in || !d_in_off || !d_out || !d_out_off || !d_out_len || !d_status) return zs_bad_arg(ctx, "inflate: null buffer");
+    if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return zs_bad_arg(ctx, "inflate: d_in must be 8-byte aligned");
     int wrap, d64;
-    if (!zs_inflate_window_bits(window_bits, &wrap, &d64)) return bad_arg(ctx, "inflate: windowBits out of range");
+    if (!zs_inflate_window_bits(window_bits, &wrap, &d64)) return zs_bad_arg(ctx, "inflate: windowBits out of range");
 
     // misc scratch: detail[n] trailer[2n] flags[n] adler[n] crc[n] dict_adler[n] | dict off[n] len[n] (u64)
     uint32_t* misc = (uint32_t*)zs_scratch_get(ctx, SCR_I_MISC, (size_t)n * 7 * 4 + 16 + (size_t)n * 16);
@@ -898,9 +900,9 @@ int inflate_batch_host_impl(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_o
                             const uint8_t* dict, const uint64_t* dict_rng, uint64_t dict_total, const InflateOpts& opts,
                             InflateOut* res) {
     if (n == 0) return ZS_OK;
-    if (!in_off || !out_off || !out_len || !status) return bad_arg(ctx, "inflate: null buffer");
+    if (!in_off || !out_off || !out_len || !status) return zs_bad_arg(ctx, "inflate: null buffer");
     const uint64_t in_total = in_off[n], out_total = out_off[n];
-    if ((in_total && !in) || (out_total && !out)) return bad_arg(ctx, "inflate: null buffer");
+    if ((in_total && !in) || (out_total && !out)) return zs_bad_arg(ctx, "inflate: null buffer");
     uint8_t* d_in = (uint8_t*)zs_scratch_get(ctx, SCR_H_IN, in_total + 64);
     uint8_t* d_out = (uint8_t*)zs_scratch_get(ctx, SCR_H_OUT, out_total + 64);
     uint64_t* d_ioff = (uint64_t*)zs_scratch_get(ctx, SCR_H_OFF, (size_t)(n + 1) * 8);
@@ -984,8 +986,8 @@ int zs_inflate_stream_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int
                           uint64_t dict_len) {
     if (ctx) bind_device(ctx);
     if (!ctx) return ZS_STREAM_ERROR;
-    if (!d_in || !d_out || !d_out_len || !d_status) return bad_arg(ctx, "inflate: null buffer");
-    uint64_t* d_o = (uint64_t*)zs_scratch_get(ctx, SCR_I_STREAM, 8 * 8);
+    if (!d_in || !d_out || !d_out_len || !d_status) return zs_bad_arg(ctx, "inflate: null buffer");
+    uint64_t* d_o = (uint64_t*)zs_scratch_get(ctx, SCR_I_STREAM, kStreamScratch);
     if (!d_o) return ZS_MEM_ERROR;
     const uint64_t h[6] = {0, in_len, 0, out_cap, 0, dict_len};
     // (pageable source: the copy is staged before the call returns)
@@ -997,10 +999,34 @@ int zs_inflate_stream_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int
                                   d_dict && dict_len ? d_dict : nullptr, d_dict && dict_len ? d_o + 4 : nullptr, o, nullptr);
 }
 
+}  // extern "C"
+
+int inflate_stream_one(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int window_bits, uint8_t* d_out, uint64_t out_cap,
+                       const uint8_t* d_dict, uint64_t dict_len, InflateOneResult* r) {
+    // the results go to SCR_I_STREAM behind the call's offsets: u64 out_len, in_used | u32 check, i32 status
+    uint64_t* d_r = (uint64_t*)zs_scratch_get(ctx, SCR_I_STREAM, kStreamScratch);
+    if (!d_r) return ZS_MEM_ERROR;
+    d_r += 6;
+    const int rc = zs_inflate_stream_dev(ctx, d_in, in_len, window_bits, d_out, out_cap, d_r, d_r + 1, (uint32_t*)(d_r + 2),
+                                         (int32_t*)(d_r + 2) + 1, d_dict, dict_len);
+    if (rc != ZS_OK) return rc;
+    uint64_t h[3];
+    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(h, d_r, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&r->detail, ctx->d_last_detail, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    r->out_len = h[0];
+    r->in_used = h[1];
+    r->check = (uint32_t)h[2];
+    r->status = (int32_t)(h[2] >> 32);
+    return ZS_OK;
+}
+
+extern "C" {
+
 int zs_inflate_last_details(zs_ctx* ctx, int32_t* detail, uint32_t n) {
     if (ctx) bind_device(ctx);
     if (!ctx || !detail) return ZS_STREAM_ERROR;
-    if (!ctx->d_last_detail || n > ctx->last_detail_n) return bad_arg(ctx, "inflate: no details available");
+    if (!ctx->d_last_detail || n > ctx->last_detail_n) return zs_bad_arg(ctx, "inflate: no details available");
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(detail, ctx->d_last_detail, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return ZS_OK;

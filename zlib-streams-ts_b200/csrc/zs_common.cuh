@@ -25,18 +25,19 @@ enum zs_scratch_slot {
     SCR_H_IN, SCR_H_OUT, SCR_H_RES,
     // the rest of the host-buffer calls
     SCR_H_OFF, SCR_H_OFF2, SCR_H_DICT, SCR_H_RNG, SCR_H_CHECKS, SCR_H_DETAIL,
-    // batch inflate: details / trailers / checksums, the streaming shim's resume record, zs_inflate_stream_dev's offsets
+    // batch inflate: details / trailers / checksums, the streaming shim's resume record, and zs_inflate_stream_dev's
+    // offsets followed by the results inflate_stream_one reads back
     SCR_I_MISC, SCR_I_RESUME, SCR_I_STREAM,
     // one-stream segment-parallel inflate.  SCR_P_STATE is taken by the API layer and shared with the parallel
     // decoder: the header pass writes it, zs_launch_inflate_parallel reads and extends it, inflate_kernel resumes from it
     SCR_P_STATE,
     // zs_inflate_par.cu
     SCR_P_CAND, SCR_P_SEG, SCR_P_PLAN, SCR_P_SYM, SCR_P_WIN, SCR_P_GMAP,
-    // zs_gunzip.cu: tile counts, member candidates, one pass's plan and results, member-table entries, and the aligned
+    // zs_gunzip.cu: tile counts, member candidates, one pass's plan and verdict, member-table entries, and the aligned
     // copy of a member decoded alone.  Its own: the batch and one-stream inflate calls it makes use none of them, and
     // zs_gunzip stages its input and output in SCR_H_IN / SCR_H_OUT around them
     SCR_G_TILE, SCR_G_CAND, SCR_G_PASS, SCR_G_MEMB, SCR_G_ALIGN,
-    // zs_inflate_index.cu.  Build: the one-stream call's results and the record pass's start record and counters.
+    // zs_inflate_index.cu.  Build: the record pass's start record and counters.
     // Extract: per-range plan and verdicts, per-warp history rings, and the staged input of the host-buffer call (its
     // output goes to SCR_H_OUT)
     SCR_X_BUILD, SCR_X_PLAN, SCR_X_RING, SCR_X_IN,
@@ -79,6 +80,7 @@ struct zs_ctx {
 
 void* zs_scratch_get(zs_ctx* ctx, zs_scratch_slot slot, size_t bytes);  // nullptr on failure (err set)
 int zs_set_cuda_error(zs_ctx* ctx, cudaError_t e, const char* where);
+int zs_bad_arg(zs_ctx* ctx, const char* msg);   // an argument error: msg to ctx->err (ctx may be null), ZS_STREAM_ERROR
 #define ZS_CUDA_TRY(ctx, expr)                                                   \
     do {                                                                         \
         cudaError_t _e = (expr);                                                 \
@@ -136,6 +138,45 @@ __device__ __forceinline__ uint32_t zs_ld32(const uint8_t* __restrict__ base, ui
     uint32_t lo = (a < safe_end) ? __ldg(reinterpret_cast<const unsigned*>(base + a)) : 0u;
     uint32_t hi = (sh != 0 && a + 4 < safe_end) ? __ldg(reinterpret_cast<const unsigned*>(base + a + 4)) : 0u;
     return __funnelshift_r(lo, hi, sh);
+}
+
+// Exclusive scan of n values by one block (<= 1024 threads): out[i] = min(base + sum of val(j) for j < i, clip) for
+// i = 0..n.  A thread reads val(i) and writes out[i] for its own [lo, hi) only, and out[n] is never read, so out may
+// hold the values themselves (an in-place scan).
+template <class Val>
+__device__ void block_scan(uint32_t n, const Val& val, uint64_t base, uint64_t clip, uint64_t* out) {
+    __shared__ uint64_t s_warp[32];
+    const uint32_t per = (n + blockDim.x - 1) / blockDim.x;
+    const uint32_t lo = min(n, threadIdx.x * per), hi = min(n, lo + per);
+    uint64_t sum = 0;
+    for (uint32_t i = lo; i < hi; i++) sum += val(i);
+    const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    uint64_t incl = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint64_t v = __shfl_up_sync(ZS_FULL_MASK, incl, o);
+        if ((int)lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        const uint64_t w = lane < blockDim.x / 32 ? s_warp[lane] : 0;
+        uint64_t wi = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint64_t v = __shfl_up_sync(ZS_FULL_MASK, wi, o);
+            if ((int)lane >= o) wi += v;
+        }
+        s_warp[lane] = wi - w;
+    }
+    __syncthreads();
+    uint64_t run = base + s_warp[warp] + incl - sum;
+    for (uint32_t i = lo; i < hi; i++) {
+        const uint64_t v = val(i);
+        out[i] = run < clip ? run : clip;
+        run += v;
+    }
+    if (threadIdx.x == blockDim.x - 1) out[n] = run < clip ? run : clip;
 }
 
 __device__ __forceinline__ unsigned zs_bitrev(unsigned code, unsigned len) { return __brev(code) >> (32u - len); }
@@ -314,6 +355,15 @@ struct InflateOut {
     const uint8_t* d_out = nullptr;   // host-buffer call: the stream's output, still on the device ...
     uint64_t out_gen = 0;             // ... while ctx->scr[SCR_H_OUT].gen equals this
 };
+// What zs_inflate_stream_dev reports for its one stream.
+struct InflateOneResult {
+    uint64_t out_len, in_used;
+    uint32_t check;
+    int32_t status, detail;
+};
+// zs_inflate_stream_dev, then its results and message code read back in one synchronise.
+int inflate_stream_one(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, int window_bits, uint8_t* d_out, uint64_t out_cap,
+                       const uint8_t* d_dict, uint64_t dict_len, InflateOneResult* r);
 // zs_inflate_batch with options; `res` may be null.  The caller has bound the context's device.
 int inflate_batch_host_impl(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_off, uint32_t n, int window_bits, uint8_t* out,
                             const uint64_t* out_off, uint64_t* out_len, uint64_t* in_used, uint32_t* checks, int32_t* status,

@@ -45,8 +45,7 @@ constexpr uint64_t kHeaderCheck = 1024;
 // A gzip header that does not fail inside [p, min(in_len, p + kHeaderCheck)): it parses, or it goes on past the bound.
 __device__ bool header_plausible(const uint8_t* in, uint64_t in_len, uint64_t safe_end, uint64_t p) {
     zsinf::BitReader br;
-    br.base = in; br.pos = p; br.end = in_len - p > kHeaderCheck ? p + kHeaderCheck : in_len; br.safe_end = safe_end;
-    br.hold = 0; br.bits = 0;
+    br.open(in, p, in_len - p > kHeaderCheck ? p + kHeaderCheck : in_len, safe_end);
     int status = ZS_OK, detail = 0;
     unsigned tflags = 0;
     zsinf::read_wrapper_header(br, 2, status, detail, tflags, nullptr);
@@ -96,54 +95,9 @@ __global__ void __launch_bounds__(kLocThreads) gunzip_locate_kernel(const uint8_
     if (threadIdx.x == 0) tile_cnt[blockIdx.x] = s_cnt;
 }
 
-// Exclusive scan of n values in one block: out[i] = min(base + sum of values before i, clip), i = 0..n.
-template <class Val>
-__device__ void block_scan(uint32_t n, const Val& val, uint64_t base, uint64_t clip, uint64_t* out) {
-    __shared__ uint64_t s_warp[32];
-    const uint32_t per = (n + blockDim.x - 1) / blockDim.x;
-    const uint32_t lo = min(n, threadIdx.x * per), hi = min(n, lo + per);
-    uint64_t sum = 0;
-    for (uint32_t i = lo; i < hi; i++) sum += val(i);
-    const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-    uint64_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint64_t v = __shfl_up_sync(ZS_FULL_MASK, incl, o);
-        if ((int)lane >= o) incl += v;
-    }
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    if (warp == 0) {
-        const uint64_t w = lane < blockDim.x / 32 ? s_warp[lane] : 0;
-        uint64_t wi = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint64_t v = __shfl_up_sync(ZS_FULL_MASK, wi, o);
-            if ((int)lane >= o) wi += v;
-        }
-        s_warp[lane] = wi - w;
-    }
-    __syncthreads();
-    uint64_t run = base + s_warp[warp] + incl - sum;
-    for (uint32_t i = lo; i < hi; i++) {
-        out[i] = run < clip ? run : clip;
-        run += val(i);
-    }
-    if (threadIdx.x == blockDim.x - 1) out[n] = run < clip ? run : clip;
-}
-
-struct TileCount {
-    const uint64_t* cnt;
-    __device__ uint64_t operator()(uint32_t i) const { return cnt[i]; }
-};
-struct PlannedSize {
-    const uint32_t* isz;   // isz[i + 1]: ISIZE before the end of member i
-    __device__ uint64_t operator()(uint32_t i) const { return isz[i + 1]; }
-};
-
 // tile counts [n_tiles] -> tile offsets [n_tiles + 1] behind them; the last is the candidate count
 __global__ void __launch_bounds__(kScanThreads) gunzip_scan_tiles_kernel(uint64_t* tile, uint32_t n_tiles) {
-    block_scan(n_tiles, TileCount{tile}, 0, ~0ull, tile + n_tiles + 1);
+    block_scan(n_tiles, [=](uint32_t i) { return tile[i]; }, 0, ~0ull, tile + n_tiles + 1);
 }
 
 // Candidates in position order: cand[m] = in_len closes the last one; isz[k] = the ISIZE field before cand[k].
@@ -185,7 +139,7 @@ __global__ void __launch_bounds__(kLocThreads) gunzip_compact_kernel(const uint8
 __global__ void __launch_bounds__(kScanThreads) gunzip_plan_kernel(const uint32_t* isz, uint32_t nb, uint64_t produced,
                                                                    uint64_t out_cap, uint64_t* out_off, uint32_t* first_bad) {
     if (threadIdx.x == 0) *first_bad = nb;
-    block_scan(nb, PlannedSize{isz}, produced, out_cap, out_off);
+    block_scan(nb, [=](uint32_t i) { return isz[i + 1]; }, produced, out_cap, out_off);   // the ISIZE that ends member i
 }
 
 // The trust rule of a planned member, and its member-table entry.
@@ -211,22 +165,9 @@ __global__ void gunzip_pass_kernel(const uint32_t* first_bad, const uint64_t* ou
     res[1] = out_off[u];
 }
 
-int bad_arg(zs_ctx* ctx, const char* msg) {
-    if (ctx) snprintf(ctx->err, sizeof(ctx->err), "%s", msg);
-    return ZS_STREAM_ERROR;
-}
-
-// What one member decoded alone returned.
-struct One {
-    uint64_t out_len, in_used;
-    uint32_t check;
-    int32_t status, detail;
-};
-
 // inflate(Z_FINISH) of d_in[pos, end) into d_out with `room` bytes, by the one-stream path (zs_inflate_stream_dev).
 // That path wants an 8-byte aligned start: a member elsewhere is copied to scratch first.
-int decode_one(zs_ctx* ctx, const uint8_t* d_in, uint64_t pos, uint64_t end, uint8_t* d_out, uint64_t room, uint64_t* d_res,
-               One* r) {
+int decode_one(zs_ctx* ctx, const uint8_t* d_in, uint64_t pos, uint64_t end, uint8_t* d_out, uint64_t room, InflateOneResult* r) {
     const uint64_t len = end - pos;
     const uint8_t* src = d_in + pos;
     if (pos & 7u) {
@@ -235,24 +176,13 @@ int decode_one(zs_ctx* ctx, const uint8_t* d_in, uint64_t pos, uint64_t end, uin
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(al, src, len, cudaMemcpyDeviceToDevice, ctx->stream));
         src = al;
     }
-    int rc = zs_inflate_stream_dev(ctx, src, len, 31, d_out, room, d_res, d_res + 1, (uint32_t*)(d_res + 2),
-                                   (int32_t*)(d_res + 3), nullptr, 0);
-    if (rc != ZS_OK) return rc;
-    uint64_t h[4];
-    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(h, d_res, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&r->detail, ctx->d_last_detail, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    r->out_len = h[0];
-    r->in_used = h[1];
-    r->check = (uint32_t)h[2];
-    r->status = (int32_t)(uint32_t)h[3];
-    return ZS_OK;
+    return inflate_stream_one(ctx, src, len, 31, d_out, room, nullptr, 0, r);
 }
 
 int gunzip_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out, uint64_t out_cap, zs_gunzip_result* res,
                zs_gz_member* members, uint64_t max_members) {
-    if (!res || (in_len && !d_in) || (out_cap && !d_out) || (max_members && !members)) return bad_arg(ctx, "gunzip: null buffer");
-    if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return bad_arg(ctx, "gunzip: d_in must be 8-byte aligned");
+    if (!res || (in_len && !d_in) || (out_cap && !d_out) || (max_members && !members)) return zs_bad_arg(ctx, "gunzip: null buffer");
+    if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return zs_bad_arg(ctx, "gunzip: d_in must be 8-byte aligned");
     memset(res, 0, sizeof(*res));
     if (in_len == 0) {   // inflate() without input makes no progress
         res->status = ZS_BUF_ERROR;
@@ -263,7 +193,7 @@ int gunzip_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out
 
     // 1. locate: candidate count, then the candidates in position order with the ISIZE field before each
     const uint64_t n_tiles64 = (in_len + kLocTile - 1) / kLocTile;
-    if (n_tiles64 > 0x7fffffffull) return bad_arg(ctx, "gunzip: input too large for one call");
+    if (n_tiles64 > 0x7fffffffull) return zs_bad_arg(ctx, "gunzip: input too large for one call");
     const uint32_t n_tiles = (uint32_t)n_tiles64;
     uint64_t* d_tile = (uint64_t*)zs_scratch_get(ctx, SCR_G_TILE, ((size_t)n_tiles * 2 + 2) * 8);
     if (!d_tile) return ZS_MEM_ERROR;
@@ -274,9 +204,9 @@ int gunzip_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out
     uint64_t m = 0;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&m, d_tile_off + n_tiles, 8, cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (m > 0xfffffffeull) return bad_arg(ctx, "gunzip: too many member candidates");
+    if (m > 0xfffffffeull) return zs_bad_arg(ctx, "gunzip: too many member candidates");
     uint8_t* cand_blob = (uint8_t*)zs_scratch_get(ctx, SCR_G_CAND, (size_t)(m + 1) * 12 + 16);
-    // one pass: out_off [m+1], out_len [m], in_used [m] (u64) | checks [m], status [m], first untrusted | results [4] (u64)
+    // one pass: out_off [m+1], out_len [m], in_used [m] (u64) | checks [m], status [m], first untrusted | verdict [2] (u64)
     uint8_t* pass = (uint8_t*)zs_scratch_get(ctx, SCR_G_PASS, (size_t)m * 32 + 128);
     zs_gz_member* d_mem = nullptr;
     if (max_members) d_mem = (zs_gz_member*)zs_scratch_get(ctx, SCR_G_MEMB, (size_t)m * sizeof(zs_gz_member));
@@ -360,13 +290,13 @@ int gunzip_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out
         // stops for want of input or of the planned room (false candidates inside the member, a false ISIZE before one).
         // A Z_STREAM_END over any range is final.  Anything else is decided over the whole rest of the input with all
         // the room: one step of the reference's loop.
-        One r;
+        InflateOneResult r;
         bool final_ = false;
         const uint64_t room = out_cap - produced;
         for (uint64_t step = tried ? 2 : 1; at_cand && j + step <= m && cand[j + step] < in_len; step *= 2) {
             const uint64_t end = cand[j + step];
             const uint64_t cap = step == 1 && isz[j + 1] < room ? isz[j + 1] : room;
-            const int rc = decode_one(ctx, d_in, pos, end, d_out + produced, cap, d_res, &r);
+            const int rc = decode_one(ctx, d_in, pos, end, d_out + produced, cap, &r);
             if (rc != ZS_OK) return rc;
             final_ = r.status == ZS_STREAM_END;
             const bool short_in = r.in_used == end - pos && r.out_len < cap;
@@ -374,7 +304,7 @@ int gunzip_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, uint8_t* d_out
             if (final_ || r.status != ZS_BUF_ERROR || !(short_in || short_room)) break;
         }
         if (!final_) {
-            const int rc = decode_one(ctx, d_in, pos, in_len, d_out + produced, room, d_res, &r);
+            const int rc = decode_one(ctx, d_in, pos, in_len, d_out + produced, room, &r);
             if (rc != ZS_OK) return rc;
         }
         if (r.status != ZS_STREAM_END) {
@@ -416,7 +346,7 @@ int zs_gunzip(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint8_t* out, uin
               zs_gz_member* members, uint64_t max_members) {
     if (!ctx) return ZS_STREAM_ERROR;
     cudaSetDevice(ctx->device);
-    if (!res || (in_len && !in) || (out_cap && !out)) return bad_arg(ctx, "gunzip: null buffer");
+    if (!res || (in_len && !in) || (out_cap && !out)) return zs_bad_arg(ctx, "gunzip: null buffer");
     uint8_t* d_in = (uint8_t*)zs_scratch_get(ctx, SCR_H_IN, in_len + 64);
     uint8_t* d_out = (uint8_t*)zs_scratch_get(ctx, SCR_H_OUT, out_cap + 64);
     if (!d_in || !d_out) return ZS_MEM_ERROR;

@@ -1,8 +1,9 @@
 // zs_inflate_common.cuh -- pieces shared by the warp-per-stream inflate kernel (zs_inflate.cu), the
-// thread-per-stream kernel (zs_inflate_tps.cu) and the segment-parallel decoder of one stream
-// (zs_inflate_par.cu): decode-table entries and their lookup, the warp-parallel table construction, the bit
-// reader, the dynamic block header, and the stream setup, wrapper header, trailer and result record of a
-// batch stream.
+// thread-per-stream kernel (zs_inflate_tps.cu), the segment-parallel decoder of one stream (zs_inflate_par.cu)
+// and the inflate index (zs_inflate_index.cu): decode-table entries and their lookup, the warp-parallel table
+// construction, the bit reader, the dynamic block header, the stream setup, wrapper header, trailer and result
+// record of a batch stream, and walk_blocks, the warp-uniform block walk behind the segment-parallel passes and
+// the index extract.
 //
 // The decode tables have the layout of the reference's inflate_table (src/mod/inflate/inftrees.ts:62-307):
 // a root table of `root` bits whose entries are symbols (replicated for shorter codes) or pointers to
@@ -17,6 +18,7 @@ namespace zsinf {
 constexpr int kEnoughLens = 852;
 constexpr int kEnoughDists = 592;
 constexpr int kEnoughDists9 = 594;
+constexpr unsigned kWin = 32768;   // the window of a deflate stream (deflate64's is not used by the block walk)
 
 // detail codes -> reference messages (zs_inflate_message, zs_inflate.cu)
 enum {
@@ -224,6 +226,17 @@ struct BitReader {
     uint64_t pos, end, safe_end;
     uint64_t hold;
     unsigned bits;
+    // empty, at byte p of [b, e); safe_end as for zs_ld32 (the readable words, which may reach past e)
+    __device__ __forceinline__ void open(const uint8_t* b, uint64_t p, uint64_t e, uint64_t se) {
+        base = b; pos = p; end = e; safe_end = se; hold = 0; bits = 0;
+    }
+    // drop the first k < 8 bits of a just opened reader; false when the byte that holds them is not there
+    __device__ __forceinline__ bool skip(unsigned k) {
+        if (k == 0) return true;
+        if (!need(8)) return false;
+        drop(k);
+        return true;
+    }
     __device__ __forceinline__ void refill() {
         if (bits <= 32) {
             if (end - pos >= 4) {
@@ -280,12 +293,7 @@ __device__ __forceinline__ uint32_t table_lookup(const uint32_t* table, unsigned
 // inflate_kernel's fast loop computes the addresses of its match copies.)
 __device__ __forceinline__ void open_stream(const zs_inflate_args& a, uint64_t sidx, uint64_t safe_end, BitReader& br,
                                             uint64_t& cap, const uint8_t*& dict, uint64_t& dict_len) {
-    br.base = a.d_in;
-    br.pos = a.d_in_off[sidx];
-    br.end = a.d_in_off[sidx + 1];
-    br.safe_end = safe_end;
-    br.hold = 0;
-    br.bits = 0;
+    br.open(a.d_in, a.d_in_off[sidx], a.d_in_off[sidx + 1], safe_end);
     cap = a.d_out_off[sidx + 1] - a.d_out_off[sidx];
     dict = nullptr;
     dict_len = 0;
@@ -509,6 +517,90 @@ __device__ __forceinline__ void build_fixed_tables(FixedTables& F, WarpArena& A,
     bits = 5; idx = 0;
     build_table_warp(2, A.lens, 32, F.dist, &bits, A.scratch, &idx, d64);
     __syncwarp();
+}
+
+// ---- the block walk of the segment-parallel passes (zs_inflate_par.cu) and the index extract (zs_inflate_index.cu) ----
+// A warp walks the deflate blocks (32 KiB window) of a positioned reader in lock-step; the dynamic header is built in
+// `A`, the fixed tables are `F`.  What it decodes goes to the sink, whose hooks the whole warp calls with warp-uniform
+// arguments:
+//   bool at_block(bit, last)   a block boundary at input bit `bit`, before the next header (last: the block that ended
+//                              there was the final one); true stops the walk
+//   bool full()                tested at every boundary and before every symbol; true stops the walk, mid-block too
+//   int stored(pos, n)         the n bytes of a stored block at input byte pos: 0, or a code that ends the walk
+//   void literal(byte)
+//   int match(len, dist)       0, or a code that ends the walk
+// The walk synchronises nothing: each sink has the __syncwarp()s its own writes need.  Returns 0 when the sink stopped
+// it, a detail code on a data error (or the sink's code), -1 when the input ran out or the last block ended first.
+template <class Sink>
+__device__ __forceinline__ int walk_blocks(BitReader& br, WarpArena& A, const FixedTables& F, Sink& s) {
+    for (bool last = false;;) {
+        if (s.at_block(br.pos * 8 - br.bits, last) || s.full()) return 0;
+        if (last || !br.need(3)) return -1;
+        last = br.take(1) != 0;
+        const unsigned type = br.take(2);
+        const uint32_t* lcode;
+        const uint32_t* dcode;
+        unsigned lenbits, distbits;
+        if (type == 1) {
+            lcode = F.len; dcode = F.dist; lenbits = 9; distbits = 5;
+        } else if (type == 2) {
+            unsigned dist_at = 0;
+            lenbits = distbits = 0;
+            if (const int rc = read_dynamic_header(br, A, false, lenbits, distbits, dist_at)) return rc;
+            lcode = A.codes; dcode = A.codes + dist_at;
+        } else if (type == 0) {
+            br.align_byte();
+            if (!br.need(32)) return -1;
+            const unsigned w = (unsigned)br.hold;
+            if ((w & 0xffffu) != ((w >> 16) ^ 0xffffu)) return D_STORED_LEN;
+            br.drop(32);
+            br.unload();
+            const uint64_t n = w & 0xffffu;
+            if (n > br.end - br.pos) return -1;
+            if (const int rc = s.stored(br.pos, n)) return rc;
+            br.pos += n;
+            continue;
+        } else {
+            return D_BLOCK_TYPE;
+        }
+        const unsigned lmask = (1u << lenbits) - 1u, dmask = (1u << distbits) - 1u;
+        for (;;) {
+            if (s.full()) return 0;
+            br.refill();
+            unsigned used;
+            uint32_t here = table_lookup<true>(lcode, lmask, br.hold, used);
+            if (used > br.bits) return -1;
+            const unsigned lop = E_OP(here);
+            if (lop == 0) {
+                br.drop(used);
+                s.literal(E_VAL(here));
+                continue;
+            }
+            if (lop & 32) { br.drop(used); break; }
+            if (lop & 64) return D_LITLEN_CODE;
+            unsigned xb = lop & 15u;
+            if (used + xb > br.bits) return -1;
+            br.drop(used);
+            const unsigned len = E_VAL(here) + br.take(xb);
+            br.refill();
+            here = table_lookup<false>(dcode, dmask, br.hold, used);
+            if (used > br.bits) return -1;
+            if (E_OP(here) & 64) return D_DIST_CODE;
+            xb = E_OP(here) & 15u;
+            if (used + xb > br.bits) return -1;
+            br.drop(used);
+            if (const int rc = s.match(len, E_VAL(here) + br.take(xb))) return rc;
+        }
+    }
+}
+
+// walk_blocks from bit `bit` of in[0, in_len) (8-byte aligned, readable to in_len rounded up to 8)
+template <class Sink>
+__device__ __forceinline__ int walk_blocks_at(const uint8_t* in, uint64_t in_len, uint64_t bit, WarpArena& A, const FixedTables& F,
+                                              Sink& s) {
+    BitReader br;
+    br.open(in, bit >> 3, in_len, (in_len + 7) & ~7ull);
+    return br.skip((unsigned)(bit & 7u)) ? walk_blocks(br, A, F, s) : -1;
 }
 
 }  // namespace zsinf

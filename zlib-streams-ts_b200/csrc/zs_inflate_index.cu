@@ -10,9 +10,11 @@
 //   ix_gather_kernel    copies every point's window (dictionary, then output) out of the decoded output.
 // Extract (zs_inflate_index_extract_dev):
 //   ix_plan_kernel      per range: the first point at or before its start and the number of intervals it spans;
-//   ix_scan_kernel      exclusive scan of those counts: work item g belongs to range r with base[r] <= g < base[r+1];
+//   ix_scan_kernel      exclusive scan of those counts (block_scan, zs_common.cuh): work item g belongs to range r with
+//                       base[r] <= g < base[r+1];
 //   ix_extract_kernel   persistent warps take items from a counter; a warp decodes raw deflate from the item's point
-//                       against its window through a private 64 KiB history ring, writing only the item's bytes;
+//                       against its window through a private 64 KiB history ring, writing only the item's bytes (the
+//                       block walk of zs_inflate_common.cuh, walk_blocks, with ExtractSink);
 //   ix_finish_kernel    per range: bytes, status and message code.
 #include <algorithm>
 #include <cstdio>
@@ -43,15 +45,9 @@ namespace {
 using namespace zsinf;
 
 constexpr int kWarps = 4;
-constexpr unsigned kWin = 32768;
 constexpr uint64_t kRing = 65536;             // per-warp history: a 32 KiB distance plus a 258-byte match never alias
 constexpr uint64_t kExportHeader = 56;
 constexpr uint64_t kExportPoint = 24;
-
-int bad_arg(zs_ctx* ctx, const char* msg) {
-    if (ctx) snprintf(ctx->err, sizeof(ctx->err), "%s", msg);
-    return ZS_STREAM_ERROR;
-}
 
 // ---- build ---------------------------------------------------------------------------------------------------------
 
@@ -116,131 +112,67 @@ __global__ void ix_plan_kernel(IxTables t, IxRanges r) {
     r.fail[i] = ~0ull;
 }
 
+// exclusive scan of the counts, in place: base[n] = items in all
 __global__ void __launch_bounds__(1024) ix_scan_kernel(uint64_t* base, uint32_t n) {
-    __shared__ uint64_t s[1024];
-    const unsigned t = threadIdx.x;
-    const uint64_t per = (n + 1023u) / 1024u;
-    const uint64_t lo = t * per < n ? t * per : n, hi = lo + per < n ? lo + per : n;
-    uint64_t sum = 0;
-    for (uint64_t i = lo; i < hi; i++) sum += base[i];
-    s[t] = sum;
-    __syncthreads();
-    for (unsigned d = 1; d < 1024; d <<= 1) {
-        const uint64_t v = t >= d ? s[t - d] : 0;
-        __syncthreads();
-        s[t] += v;
-        __syncthreads();
-    }
-    uint64_t run = s[t] - sum;
-    for (uint64_t i = lo; i < hi; i++) {
-        const uint64_t c = base[i];
-        base[i] = run;
-        run += c;
-    }
-    if (t == 1023) base[n] = s[1023];
+    block_scan(n, [=](uint32_t i) { return base[i]; }, 0, ~0ull, base);
 }
+
+// An item's bytes: every byte decoded from the point goes to the warp's ring, those from `skip` on to dest as well, and
+// the walk stops once `want` bytes are out.
+struct ExtractSink {
+    static constexpr uint64_t M = kRing - 1;
+    const uint8_t* in;
+    uint8_t* ring;
+    uint8_t* dest;
+    uint64_t skip, want;
+    uint64_t r, h;   // bytes decoded from the point; history bytes in the ring
+    __device__ bool at_block(uint64_t, bool) const { return false; }
+    __device__ bool full() const { return r >= want; }
+    __device__ int stored(uint64_t pos, uint64_t n) {
+        const uint64_t c = n < want - r ? n : want - r;
+        for (uint64_t j = zs_lane(); j < c; j += 32) {
+            const uint8_t b = __ldg(in + pos + j);
+            ring[(h + j) & M] = b;
+            if (r + j >= skip) dest[r + j - skip] = b;
+        }
+        __syncwarp();
+        r += c; h += c;
+        return 0;
+    }
+    __device__ void literal(unsigned byte) {
+        if (zs_lane() == 0) {
+            ring[h & M] = (uint8_t)byte;
+            if (r >= skip) dest[r - skip] = (uint8_t)byte;
+        }
+        r++; h++;
+    }
+    __device__ int match(unsigned len, uint64_t dist) {
+        if (dist > h) return D_TOO_FAR;
+        const uint64_t c = len < want - r ? len : want - r;
+        __syncwarp();
+        for (unsigned j = zs_lane(); j < c; j += 32) {
+            const uint8_t b = ring[(h - dist + (dist >= c ? j : j % dist)) & M];
+            ring[(h + j) & M] = b;
+            if (r + j >= skip) dest[r + j - skip] = b;
+        }
+        __syncwarp();
+        r += c; h += c;
+        return 0;
+    }
+};
 
 // One item: raw deflate from bit `bit` against the wl-byte window `win`, through the warp's ring, until `want` bytes
 // have been decoded; bytes from `skip` on go to dest.  Returns 0, the detail code of the error, or -1 when the input or
-// the stream ended first; *made = bytes decoded.  Warp-uniform, like decode_segment (zs_inflate_par.cu).
+// the stream ended first; *made = bytes decoded.  Warp-uniform.
 __device__ int extract_item(const uint8_t* in, uint64_t in_len, uint64_t bit, const uint8_t* win, uint64_t wl, uint8_t* ring,
                             uint64_t skip, uint64_t want, uint8_t* dest, WarpArena& A, const FixedTables& F, uint64_t* made) {
-    const unsigned lane = zs_lane();
-    constexpr uint64_t M = kRing - 1;
     // windows start 16-byte aligned in the index (and the ring bytes past wl are written before they are read)
-    for (uint64_t j = lane; j < (wl + 15) / 16; j += 32) reinterpret_cast<uint4*>(ring)[j] = reinterpret_cast<const uint4*>(win)[j];
+    for (uint64_t j = zs_lane(); j < (wl + 15) / 16; j += 32) reinterpret_cast<uint4*>(ring)[j] = reinterpret_cast<const uint4*>(win)[j];
     __syncwarp();
-    BitReader br;
-    br.base = in; br.pos = bit >> 3; br.end = in_len; br.safe_end = (in_len + 7) & ~7ull; br.hold = 0; br.bits = 0;
-    uint64_t r = 0, h = wl;   // bytes decoded from the point; history bytes in the ring
-    int rc = 0;
-    if (bit & 7u) {
-        if (!br.need(8)) rc = -1;
-        else br.drop((unsigned)(bit & 7u));
-    }
-    bool last = false;
-    while (rc == 0 && r < want) {
-        if (last || !br.need(3)) { rc = -1; break; }
-        last = br.take(1) != 0;
-        const unsigned type = br.take(2);
-        const uint32_t* lcode;
-        const uint32_t* dcode;
-        unsigned lenbits, distbits;
-        if (type == 0) {
-            br.align_byte();
-            if (!br.need(32)) { rc = -1; break; }
-            const unsigned w = (unsigned)br.hold;
-            if ((w & 0xffffu) != ((w >> 16) ^ 0xffffu)) { rc = D_STORED_LEN; break; }
-            br.drop(32);
-            br.unload();
-            const uint64_t n = w & 0xffffu;
-            if (n > br.end - br.pos) { rc = -1; break; }
-            const uint64_t c = n < want - r ? n : want - r;
-            for (uint64_t j = lane; j < c; j += 32) {
-                const uint8_t b = __ldg(in + br.pos + j);
-                ring[(h + j) & M] = b;
-                if (r + j >= skip) dest[r + j - skip] = b;
-            }
-            __syncwarp();
-            br.pos += n;
-            r += c; h += c;
-            continue;
-        } else if (type == 1) {
-            lcode = F.len; dcode = F.dist; lenbits = 9; distbits = 5;
-        } else if (type == 2) {
-            unsigned dist_at = 0;
-            lenbits = distbits = 0;
-            const int hr = read_dynamic_header(br, A, false, lenbits, distbits, dist_at);
-            if (hr) { rc = hr; break; }
-            lcode = A.codes; dcode = A.codes + dist_at;
-        } else {
-            rc = D_BLOCK_TYPE;
-            break;
-        }
-        const unsigned lmask = (1u << lenbits) - 1u, dmask = (1u << distbits) - 1u;
-        while (r < want) {
-            br.refill();
-            unsigned used;
-            uint32_t here = table_lookup<true>(lcode, lmask, br.hold, used);
-            if (used > br.bits) { rc = -1; break; }
-            const unsigned lop = E_OP(here);
-            if (lop == 0) {
-                br.drop(used);
-                if (lane == 0) {
-                    ring[h & M] = (uint8_t)E_VAL(here);
-                    if (r >= skip) dest[r - skip] = (uint8_t)E_VAL(here);
-                }
-                r++; h++;
-                continue;
-            }
-            if (lop & 32) { br.drop(used); break; }
-            if (lop & 64) { rc = D_LITLEN_CODE; break; }
-            unsigned xb = lop & 15u;
-            if (used + xb > br.bits) { rc = -1; break; }
-            br.drop(used);
-            const unsigned len = E_VAL(here) + br.take(xb);
-            br.refill();
-            here = table_lookup<false>(dcode, dmask, br.hold, used);
-            if (used > br.bits) { rc = -1; break; }
-            if (E_OP(here) & 64) { rc = D_DIST_CODE; break; }
-            xb = E_OP(here) & 15u;
-            if (used + xb > br.bits) { rc = -1; break; }
-            br.drop(used);
-            const uint64_t dist = E_VAL(here) + br.take(xb);
-            if (dist > h) { rc = D_TOO_FAR; break; }
-            const uint64_t c = len < want - r ? len : want - r;
-            __syncwarp();
-            for (unsigned j = lane; j < c; j += 32) {
-                const uint8_t b = ring[(h - dist + (dist >= c ? j : j % dist)) & M];
-                ring[(h + j) & M] = b;
-                if (r + j >= skip) dest[r + j - skip] = b;
-            }
-            __syncwarp();
-            r += c; h += c;
-        }
-    }
+    ExtractSink s{in, ring, dest, skip, want, 0, wl};
+    const int rc = walk_blocks_at(in, in_len, bit, A, F, s);
     __syncwarp();
-    *made = r;
+    *made = s.r;
     return rc;
 }
 
@@ -359,38 +291,27 @@ int zs_inflate_index_build_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len
     if (!ctx) return ZS_STREAM_ERROR;
     cudaSetDevice(ctx->device);
     int wrap = 0, d64 = 0;
-    if (!res || !out || !d_in || !d_out) return bad_arg(ctx, "inflate_index_build: null argument");
-    if (!zs_inflate_window_bits(window_bits, &wrap, &d64) || d64) return bad_arg(ctx, "inflate_index_build: windowBits out of range (deflate64 has no index)");
-    if (span == 0) return bad_arg(ctx, "inflate_index_build: span is zero");
+    if (!res || !out || !d_in || !d_out) return zs_bad_arg(ctx, "inflate_index_build: null argument");
+    if (!zs_inflate_window_bits(window_bits, &wrap, &d64) || d64) return zs_bad_arg(ctx, "inflate_index_build: windowBits out of range (deflate64 has no index)");
+    if (span == 0) return zs_bad_arg(ctx, "inflate_index_build: span is zero");
     if (!d_dict) dict_len = 0;
-    // results (u64 out_len, in_used; u32 check; i32 status) | the walk's start record [4] | counters [2]
-    uint64_t* scr = (uint64_t*)zs_scratch_get(ctx, SCR_X_BUILD, 16 * 8);
+    // the walk's start record [4] | counters [2]
+    uint64_t* scr = (uint64_t*)zs_scratch_get(ctx, SCR_X_BUILD, 6 * 8);
     if (!scr) return ZS_MEM_ERROR;
     const uint64_t gen0 = ctx->scr[SCR_P_STATE].gen;
-    int rc = zs_inflate_stream_dev(ctx, d_in, in_len, window_bits, d_out, out_cap, scr, scr + 1, (uint32_t*)(scr + 2),
-                                   (int32_t*)(scr + 2) + 1, d_dict, dict_len);
+    InflateOneResult one;
+    int rc = inflate_stream_one(ctx, d_in, in_len, window_bits, d_out, out_cap, d_dict, dict_len, &one);
     if (rc != ZS_OK) return rc;
     // the segment-parallel path took this stream when it used its state slot in this call
     const bool planned = ctx->scr[SCR_P_STATE].gen != gen0;
-    uint64_t h[3] = {0, 0, 0};
-    int32_t detail = 0;
-    uint8_t head[2] = {0, 0};
-    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(h, scr, 24, cudaMemcpyDeviceToHost, ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&detail, ctx->d_last_detail, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (in_len >= 2) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(head, d_in, 2, cudaMemcpyDeviceToHost, ctx->stream));
-    ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    res->out_len = h[0];
-    res->in_used = h[1];
-    res->check = (uint32_t)h[2];
-    res->status = (int32_t)(h[2] >> 32);
-    res->detail = detail;
+    *res = {one.out_len, one.in_used, one.check, one.status, one.detail};
     if (res->status != ZS_STREAM_END) return ZS_OK;
-    const uint64_t out_len = h[0];
+    const uint64_t out_len = one.out_len;
 
     // the block starts the rule may select
     uint64_t* d_state = planned ? (uint64_t*)ctx->scr[SCR_P_STATE].p : nullptr;
-    uint64_t* tail = scr + 4;
-    unsigned long long* cnt = (unsigned long long*)(scr + 8);
+    uint64_t* tail = scr;
+    unsigned long long* cnt = (unsigned long long*)(scr + 4);
     const uint64_t tail0[4] = {~0ull, 0, 0, 0};
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(tail, tail0, sizeof(tail0), cudaMemcpyHostToDevice, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaMemsetAsync(cnt, 0, 16, ctx->stream));
@@ -403,8 +324,10 @@ int zs_inflate_index_build_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len
     rc = zs_launch_inflate_record(ctx, d_in, in_len, out_cap, planned, d_state, planned ? d_state + 8 : tail, wrap, span, d_rec,
                                   rec_cap, cnt);
     uint64_t c[2] = {0, 0}, n_planned = 0;
+    uint8_t head[2] = {0, 0};
     cudaError_t e = rc == ZS_OK ? cudaMemcpyAsync(c, cnt, 16, cudaMemcpyDeviceToHost, ctx->stream) : cudaSuccess;
     if (rc == ZS_OK && e == cudaSuccess && planned) e = cudaMemcpyAsync(&n_planned, d_state, 8, cudaMemcpyDeviceToHost, ctx->stream);
+    if (rc == ZS_OK && e == cudaSuccess && in_len >= 2) e = cudaMemcpyAsync(head, d_in, 2, cudaMemcpyDeviceToHost, ctx->stream);
     if (rc == ZS_OK && e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     std::vector<uint64_t> rec;
     if (rc == ZS_OK && e == cudaSuccess && c[0] <= rec_cap) {
@@ -459,7 +382,7 @@ int zs_inflate_index_build(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, int 
     if (index) *index = nullptr;
     if (!ctx) return ZS_STREAM_ERROR;
     cudaSetDevice(ctx->device);
-    if ((in_len && !in) || (out_cap && !out) || (dict_len && !dict) || !res) return bad_arg(ctx, "inflate_index_build: null buffer");
+    if ((in_len && !in) || (out_cap && !out) || (dict_len && !dict) || !res) return zs_bad_arg(ctx, "inflate_index_build: null buffer");
     uint8_t* d_in = (uint8_t*)zs_scratch_get(ctx, SCR_X_IN, in_len + 64);
     uint8_t* d_out = (uint8_t*)zs_scratch_get(ctx, SCR_H_OUT, out_cap + 64);
     uint8_t* d_dict = dict_len ? (uint8_t*)zs_scratch_get(ctx, SCR_H_DICT, dict_len + 64) : nullptr;
@@ -537,7 +460,7 @@ int zs_inflate_index_import(zs_ctx* ctx, const uint8_t* buf, uint64_t len, zs_in
     if (out) *out = nullptr;
     if (!ctx) return ZS_STREAM_ERROR;
     cudaSetDevice(ctx->device);
-    if (!out || (len && !buf)) return bad_arg(ctx, "inflate_index_import: null argument");
+    if (!out || (len && !buf)) return zs_bad_arg(ctx, "inflate_index_import: null argument");
     auto bad = [&](const char* msg) {
         snprintf(ctx->err, sizeof(ctx->err), "inflate_index_import: %s", msg);
         return ZS_DATA_ERROR;
@@ -627,12 +550,12 @@ int zs_inflate_index_extract_dev(zs_ctx* ctx, const zs_inflate_index* x, const u
                                  int32_t* d_status) {
     if (!ctx) return ZS_STREAM_ERROR;
     cudaSetDevice(ctx->device);
-    if (!x) return bad_arg(ctx, "inflate_index_extract: no index");
-    if (x->device != ctx->device) return bad_arg(ctx, "inflate_index_extract: index built for another device");
-    if (in_len != x->in_len) return bad_arg(ctx, "inflate_index_extract: in_len is not the indexed stream's");
+    if (!x) return zs_bad_arg(ctx, "inflate_index_extract: no index");
+    if (x->device != ctx->device) return zs_bad_arg(ctx, "inflate_index_extract: index built for another device");
+    if (in_len != x->in_len) return zs_bad_arg(ctx, "inflate_index_extract: in_len is not the indexed stream's");
     if (n == 0) return ZS_OK;
-    if (!d_in || !d_off || !d_len || !d_out || !d_out_off || !d_got || !d_status) return bad_arg(ctx, "inflate_index_extract: null buffer");
-    if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return bad_arg(ctx, "inflate_index_extract: d_in must be 8-byte aligned");
+    if (!d_in || !d_off || !d_len || !d_out || !d_out_off || !d_got || !d_status) return zs_bad_arg(ctx, "inflate_index_extract: null buffer");
+    if ((reinterpret_cast<uintptr_t>(d_in) & 7u) != 0) return zs_bad_arg(ctx, "inflate_index_extract: d_in must be 8-byte aligned");
     uint8_t* plan = (uint8_t*)zs_scratch_get(ctx, SCR_X_PLAN, (size_t)n * 28 + 64);
     const unsigned ctas = (unsigned)ctx->sm_count * 8u;
     uint8_t* rings = (uint8_t*)zs_scratch_get(ctx, SCR_X_RING, (size_t)ctas * kWarps * kRing);
@@ -663,10 +586,10 @@ int zs_inflate_index_extract(zs_ctx* ctx, const zs_inflate_index* x, const uint8
                              uint64_t* got, int32_t* status) {
     if (!ctx) return ZS_STREAM_ERROR;
     cudaSetDevice(ctx->device);
-    if (!x) return bad_arg(ctx, "inflate_index_extract: no index");
-    if (in_len != x->in_len) return bad_arg(ctx, "inflate_index_extract: in_len is not the indexed stream's");
+    if (!x) return zs_bad_arg(ctx, "inflate_index_extract: no index");
+    if (in_len != x->in_len) return zs_bad_arg(ctx, "inflate_index_extract: in_len is not the indexed stream's");
     if (n == 0) return ZS_OK;
-    if (!in || !off || !len || !out_off || !got || !status) return bad_arg(ctx, "inflate_index_extract: null buffer");
+    if (!in || !off || !len || !out_off || !got || !status) return zs_bad_arg(ctx, "inflate_index_extract: null buffer");
     // the input each range needs: from its first point's byte to the byte of the point after its last one (or the end),
     // plus the bit reader's read-ahead; output room for every range as clipped to the stream
     std::vector<std::pair<uint64_t, uint64_t>> span;
@@ -674,7 +597,7 @@ int zs_inflate_index_extract(zs_ctx* ctx, const zs_inflate_index* x, const uint8
     for (uint32_t i = 0; i < n; i++) {
         const uint64_t o = off[i], e = o >= x->out_len ? o : (len[i] > x->out_len - o ? x->out_len : o + len[i]);
         if (e <= o) continue;
-        if (!out || out_off[i] > out_cap || e - o > out_cap - out_off[i]) return bad_arg(ctx, "inflate_index_extract: a range does not fit out_cap");
+        if (!out || out_off[i] > out_cap || e - o > out_cap - out_off[i]) return zs_bad_arg(ctx, "inflate_index_extract: a range does not fit out_cap");
         const uint64_t p0 = (uint64_t)(std::upper_bound(x->off.begin(), x->off.end(), o) - x->off.begin()) - 1;
         const uint64_t p1 = (uint64_t)(std::lower_bound(x->off.begin(), x->off.end(), e) - x->off.begin());   // the point after the last
         const uint64_t lo = (x->bit[p0] >> 3) & ~7ull;

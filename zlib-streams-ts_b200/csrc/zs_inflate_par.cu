@@ -31,6 +31,8 @@
 //   par_record_kernel   launched only by the index build (zs_inflate_index.cu), after a decode: the planned segments
 //                       and the serial decoder's part walked again, lengths only, keeping the block starts an index
 //                       of access points may use.
+// The count, decode and record passes are one block walk (walk_blocks, zs_inflate_common.cuh) with three sinks:
+// CountSink, SymbolSink and RecordSink.
 #include <cstdio>
 #include <cstring>
 
@@ -41,7 +43,6 @@ namespace {
 using namespace zsinf;
 
 constexpr int kWarps = 4;
-constexpr unsigned kWin = 32768;            // window of a deflate stream (the parallel path is not used for deflate64)
 constexpr unsigned kMaxPassed = 48;         // candidates a count pass may run over before it gives up
 constexpr uint64_t kMaxTiles = 64;          // ... and tiles of input it may consume
 constexpr uint64_t kMaxSpan = 2u << 20;     // (but not fewer bytes than this: the tiles of a short input are small)
@@ -300,167 +301,111 @@ __global__ void par_spec_merge_kernel(ParArgs a) {
     }
 }
 
-// Where the index build's pass (kRecord) appends the block starts it keeps: (bit, output offset) pairs at
-// rec[2i], rec[2i + 1], i taken from cnt[0]; cnt[1] counts the walks that reached their end.
-struct RecordSink {
+// The count pass: lengths only, until the walk stands at a block boundary exactly on a later candidate (LANDED), ends
+// the stream (FINAL), or fails, runs out of input or gives up (STOPPED).
+struct CountSink {
+    const ParArgs& a;
+    uint64_t start_bit;
+    uint64_t t_seen;     // candidate slots up to here have been looked at
+    unsigned passed;
+    SegInfo r;           // r.out_len: the output so far
+    __device__ bool at_block(uint64_t bit, bool last) {
+        if (bit <= start_bit) return false;
+        const uint64_t byte = bit >> 3, t = byte / a.tile + 1;
+        if (last) {
+            r.status = SEG_FINAL;
+        } else if ((bit & 7u) == 0 && byte == a.in_len) {
+            r.status = SEG_LANDED; r.next_slot = kEndOfInput;
+        } else if (t < a.n_slots && a.cand[t] == bit) {   // a candidate of this tile at exactly this bit (markers are
+            r.status = SEG_LANDED; r.next_slot = (uint32_t)t;   // byte aligned, speculative cuts are not)
+        }
+        if (r.status != SEG_STOPPED) { r.end_bit = bit; return true; }
+        // A wrong guess decodes garbage until it fails; bound what it may cost: candidates run over without standing
+        // on one, and input consumed.  (A true segment that long is left to the serial decoder, together with what
+        // follows it.)
+        while (t_seen < t && t_seen + 1 < a.n_slots) {
+            ++t_seen;
+            const uint64_t c = a.cand[t_seen];
+            if (c != ~0ull && c < bit) ++passed;
+        }
+        return passed > kMaxPassed || byte - (start_bit >> 3) > (kMaxTiles * a.tile > kMaxSpan ? kMaxTiles * a.tile : kMaxSpan);
+    }
+    __device__ bool full() const { return false; }
+    __device__ int stored(uint64_t, uint64_t n) { r.out_len += n; return r.out_len > a.out_cap; }
+    __device__ void literal(unsigned) { r.out_len++; }
+    __device__ int match(unsigned len, uint64_t) { r.out_len += len; return r.out_len > a.out_cap; }
+};
+
+// The decode pass: 16-bit symbols to `sym` until the walk reaches stop_bit (the candidate the count pass landed on) or
+// ends the stream.  A reference to byte w of the 32 KiB window before the segment is the symbol 256 + w.
+struct SymbolSink {
+    const ParArgs& a;
+    uint16_t* sym;
+    uint64_t stop_bit;
+    uint64_t avail_hist;   // bytes of stream, dictionary or earlier output before the segment
+    uint64_t op;
+    __device__ bool at_block(uint64_t bit, bool last) { return bit >= stop_bit || last; }
+    __device__ bool full() const { return false; }
+    __device__ int stored(uint64_t pos, uint64_t n) {
+        for (uint64_t j = zs_lane(); j < n; j += 32) sym[op + j] = a.in[pos + j];
+        op += n;
+        return 0;
+    }
+    __device__ void literal(unsigned byte) {
+        if (zs_lane() == 0) sym[op] = (uint16_t)byte;
+        op++;
+    }
+    __device__ int match(unsigned len, uint64_t dist) {
+        // a distance that reaches before the start of the stream (and its dictionary) is the reference's "invalid
+        // distance too far back": left to the serial decoder
+        if (dist > op + avail_hist) return 1;
+        __syncwarp();
+        const int64_t s0 = (int64_t)op - (int64_t)dist;
+        for (unsigned j = zs_lane(); j < len; j += 32) {
+            const int64_t si = s0 + (int64_t)(dist >= len ? j : j % dist);
+            sym[op + j] = si >= 0 ? sym[si] : (uint16_t)(256 + kWin + si);
+        }
+        __syncwarp();
+        op += len;
+        return 0;
+    }
+};
+
+// Where the index build's pass appends the block starts it keeps: (bit, output offset) pairs at rec[2i], rec[2i + 1],
+// i taken from cnt[0]; cnt[1] counts the walks that reached their end.
+struct RecordOut {
     uint64_t* rec;
     uint64_t cap;        // pairs
     unsigned long long* cnt;
     uint64_t span;
 };
 
-// One segment, decoded by a warp from bit `start_bit`.  kWrite = false: lengths only (count pass), stops on a
-// later candidate; true: symbols to a.sym + out_base, stops at end_bit.  kRecord (with kWrite = false): lengths
-// only from start_bit to stop_bit or the end of the last block, the index build's pass (zs_inflate_index.cu): it
-// keeps the first block start and every later one that some multiple of the span falls on -- one whose output
-// offset o has a multiple of rs->span in (o of the block start before it, o].  A block start the access-point
-// rule selects is always kept, whichever walk it falls in.
-template <bool kWrite, bool kRecord = false>
-__device__ __forceinline__ void decode_segment(const ParArgs& a, WarpArena& A, const FixedTables& F, uint32_t slot, uint64_t start_bit,
-                                               uint64_t stop_bit, uint64_t out_base, uint64_t avail_hist, SegInfo* info, uint32_t* err,
-                                               const RecordSink* rs = nullptr) {
-    const unsigned lane = zs_lane();
-    BitReader br;
-    br.base = a.in;
-    br.pos = start_bit >> 3;
-    br.end = a.in_len;
-    br.safe_end = (a.in_len + 7) & ~7ull;
-    br.hold = 0;
-    br.bits = 0;
-    bool bad = false;
-    if (start_bit & 7u) {
-        if (!br.need(8)) bad = true;
-        else br.drop((unsigned)(start_bit & 7u));
-    }
-    uint64_t op = 0;
-    uint16_t* sym = kWrite ? a.sym + out_base : nullptr;
-    unsigned passed = 0;
-    uint64_t t_seen = (start_bit >> 3) / a.tile + 1;   // candidate slots up to here have been looked at
-    uint32_t status = SEG_STOPPED;
-    uint64_t end_bit = 0;
-    uint32_t next_slot = 0;
-    bool last = false;
-    uint64_t rec_prev = 0;   // kRecord: output offset of the block start before this one (none yet: ~0)
-    if (kRecord) rec_prev = ~0ull;
-    while (!bad) {
-        // ---- a block boundary ----
-        const uint64_t here_bit = br.pos * 8 - br.bits;
-        if (kRecord) {
-            if (here_bit >= stop_bit || last) { status = SEG_LANDED; break; }
-            const uint64_t o = out_base + op;
-            if (rec_prev == ~0ull || o / rs->span > rec_prev / rs->span) {
-                if (lane == 0) {
-                    const unsigned long long i = atomicAdd(rs->cnt, 1ull);
-                    if (i < rs->cap) { rs->rec[2 * i] = here_bit; rs->rec[2 * i + 1] = o; }
-                }
+// The index build's pass (zs_inflate_index.cu): lengths only, from a walk's start to stop_bit or the end of the last
+// block.  It keeps the first block start and every later one that some multiple of the span falls on -- one whose output
+// offset o has a multiple of the span in (o of the block start before it, o].  A block start the access-point rule
+// selects is always kept, whichever walk it falls in.
+struct RecordSink {
+    const RecordOut& out;
+    uint64_t stop_bit;
+    uint64_t o;          // output offset in the stream
+    uint64_t prev;       // o of the block start before this one (none yet: ~0)
+    bool landed;         // the walk reached its end (a flag, not the walk's result: that cost a move per symbol here)
+    __device__ bool at_block(uint64_t bit, bool last) {
+        if (bit >= stop_bit || last) { landed = true; return true; }
+        if (prev == ~0ull || o / out.span > prev / out.span) {
+            if (zs_lane() == 0) {
+                const unsigned long long i = atomicAdd(out.cnt, 1ull);
+                if (i < out.cap) { out.rec[2 * i] = bit; out.rec[2 * i + 1] = o; }
             }
-            rec_prev = o;
-        } else if (kWrite) {
-            if (here_bit >= stop_bit) { status = SEG_LANDED; break; }
-        } else if (here_bit > start_bit) {
-            if (last) { status = SEG_FINAL; end_bit = here_bit; break; }
-            const uint64_t byte = here_bit >> 3;
-            if ((here_bit & 7u) == 0 && byte == a.in_len) { status = SEG_LANDED; end_bit = here_bit; next_slot = kEndOfInput; break; }
-            {   // a candidate of this tile at exactly this bit (markers are byte aligned, speculative cuts are not)
-                const uint64_t t = byte / a.tile + 1;
-                if (t < a.n_slots && a.cand[t] == here_bit) { status = SEG_LANDED; end_bit = here_bit; next_slot = (uint32_t)t; break; }
-            }
-            // A wrong guess decodes garbage until it fails; bound what it may cost: candidates run over
-            // without standing on one, and input consumed.  (A true segment that long is left to the
-            // serial decoder, together with what follows it.)
-            for (uint64_t t = byte / a.tile + 1; t_seen < t && t_seen + 1 < a.n_slots; ) {
-                ++t_seen;
-                const uint64_t c = a.cand[t_seen];
-                if (c != ~0ull && c < here_bit) ++passed;
-            }
-            if (passed > kMaxPassed || byte - (start_bit >> 3) > (kMaxTiles * a.tile > kMaxSpan ? kMaxTiles * a.tile : kMaxSpan)) break;
         }
-        if (kWrite && last) { status = SEG_FINAL; break; }
-        if (!br.need(3)) break;
-        last = br.take(1) != 0;
-        const unsigned type = br.take(2);
-        const uint32_t* lcode;
-        const uint32_t* dcode;
-        unsigned lenbits, distbits;
-        if (type == 0) {
-            br.align_byte();
-            if (!br.need(32)) break;
-            const unsigned w = (unsigned)br.hold;
-            if ((w & 0xffffu) != ((w >> 16) ^ 0xffffu)) break;
-            br.drop(32);
-            br.unload();
-            const uint64_t n = w & 0xffffu;
-            if (n > br.end - br.pos) break;
-            if (kWrite)
-                for (uint64_t j = lane; j < n; j += 32) sym[op + j] = a.in[br.pos + j];
-            br.pos += n;
-            op += n;
-            if (!kWrite && !kRecord && op > a.out_cap) break;
-            continue;
-        } else if (type == 1) {
-            lcode = F.len; dcode = F.dist; lenbits = 9; distbits = 5;
-        } else if (type == 2) {
-            unsigned dist_at = 0;
-            lenbits = distbits = 0;
-            if (read_dynamic_header(br, A, false, lenbits, distbits, dist_at) != 0) break;
-            lcode = A.codes; dcode = A.codes + dist_at;
-        } else {
-            break;
-        }
-        const unsigned lmask = (1u << lenbits) - 1u, dmask = (1u << distbits) - 1u;
-        bool block_ok = false;
-        for (;;) {
-            br.refill();
-            unsigned used;
-            uint32_t here = table_lookup<true>(lcode, lmask, br.hold, used);
-            if (used > br.bits) break;
-            const unsigned lop = E_OP(here);
-            if (lop == 0) {
-                br.drop(used);
-                if (kWrite && lane == 0) sym[op] = (uint16_t)E_VAL(here);
-                op++;
-                continue;
-            }
-            if (lop & 32) { br.drop(used); block_ok = true; break; }
-            if (lop & 64) break;
-            unsigned xb = lop & 15u;
-            if (used + xb > br.bits) break;
-            br.drop(used);
-            const unsigned len = E_VAL(here) + br.take(xb);
-            br.refill();
-            here = table_lookup<false>(dcode, dmask, br.hold, used);
-            if (used > br.bits) break;
-            if (E_OP(here) & 64) break;
-            xb = E_OP(here) & 15u;
-            if (used + xb > br.bits) break;
-            br.drop(used);
-            const uint64_t dist = E_VAL(here) + br.take(xb);
-            if (kWrite) {
-                // a distance that reaches before the start of the stream (and its dictionary) is the
-                // reference's "invalid distance too far back": left to the serial decoder
-                if (dist > op + avail_hist) { *err = 1u; break; }
-                __syncwarp();
-                const int64_t s0 = (int64_t)op - (int64_t)dist;
-                for (unsigned j = lane; j < len; j += 32) {
-                    const int64_t si = s0 + (int64_t)(dist >= len ? j : j % dist);
-                    sym[op + j] = si >= 0 ? sym[si] : (uint16_t)(256 + kWin + si);
-                }
-                __syncwarp();
-            }
-            op += len;
-            if (!kWrite && !kRecord && op > a.out_cap) break;
-        }
-        if (!block_ok) break;
+        prev = o;
+        return false;
     }
-    if (kRecord && lane == 0 && status == SEG_LANDED) atomicAdd(rs->cnt + 1, 1ull);
-    if (!kWrite && !kRecord && lane == 0) {
-        SegInfo r;
-        r.end_bit = end_bit; r.out_len = op; r.status = status; r.next_slot = next_slot;
-        *info = r;
-    }
-    if (kWrite && status == SEG_STOPPED) *err = 1u;   // the count pass got through: cannot happen, but never trust it
-    (void)slot;
-}
+    __device__ bool full() const { return false; }
+    __device__ int stored(uint64_t, uint64_t n) { o += n; return 0; }
+    __device__ void literal(unsigned) { o++; }
+    __device__ int match(unsigned len, uint64_t) { o += len; return 0; }
+};
 
 __global__ void __launch_bounds__(kWarps * 32) par_count_kernel(ParArgs a) {
     __shared__ WarpArena s_arena[kWarps];
@@ -477,7 +422,9 @@ __global__ void __launch_bounds__(kWarps * 32) par_count_kernel(ParArgs a) {
             if (zs_lane() == 0) { SegInfo r; r.end_bit = 0; r.out_len = 0; r.status = SEG_STOPPED; r.next_slot = 0; a.seg[slot] = r; }
             continue;
         }
-        decode_segment<false>(a, s_arena[wid], s_fixed, (uint32_t)slot, start, 0, 0, 0, &a.seg[slot], nullptr);
+        CountSink cs{a, start, (start >> 3) / a.tile + 1, 0, {0, 0, SEG_STOPPED, 0}};
+        walk_blocks_at(a.in, a.in_len, start, s_arena[wid], s_fixed, cs);
+        if (zs_lane() == 0) a.seg[slot] = cs.r;
         __syncwarp();
     }
 }
@@ -522,8 +469,9 @@ __global__ void __launch_bounds__(kWarps * 32) par_decode_kernel(ParArgs a) {
         const uint32_t slot = a.plan_slot[k];
         const SegInfo s = a.seg[slot];
         const uint64_t off = a.plan_off[k];
-        const uint64_t avail = off + a.hist_len;
-        decode_segment<true>(a, s_arena[wid], s_fixed, slot, a.cand[slot], s.end_bit, off, avail, nullptr, &a.plan_err[k]);
+        SymbolSink ss{a, a.sym + off, s.end_bit, off + a.hist_len, 0};
+        // a walk that does not reach the end the count pass reached: cannot happen, but never trust it
+        if (walk_blocks_at(a.in, a.in_len, a.cand[slot], s_arena[wid], s_fixed, ss) != 0) a.plan_err[k] = 1u;
         __syncwarp();
     }
 }
@@ -682,7 +630,7 @@ __global__ void par_finish_kernel(ParArgs a) {
 // (~0: the first block, behind the wrapper header) with tail[1] bytes before it -- nothing when tail[2] & 4 says the
 // planned segments reached the last block.  Items 1..n are the planned segments of the decode that ran before.  The
 // walk goes first: it is the longest item whenever the parallel part gave up early.
-__global__ void __launch_bounds__(kWarps * 32) par_record_kernel(ParArgs a, RecordSink rs, const uint64_t* tail, int wrap) {
+__global__ void __launch_bounds__(kWarps * 32) par_record_kernel(ParArgs a, RecordOut ro, const uint64_t* tail, int wrap) {
     __shared__ WarpArena s_arena[kWarps];
     __shared__ FixedTables s_fixed;
     const unsigned wid = threadIdx.x >> 5;
@@ -690,15 +638,16 @@ __global__ void __launch_bounds__(kWarps * 32) par_record_kernel(ParArgs a, Reco
     __syncthreads();
     const uint64_t n = a.state ? a.state[0] : 0;
     for (uint64_t k = (uint64_t)blockIdx.x * kWarps + wid; k <= n; k += (uint64_t)gridDim.x * kWarps) {
+        uint64_t bit, stop = ~0ull, out;
         if (k == 0) {
             if (tail[2] & 4u) {
-                if (zs_lane() == 0) atomicAdd(rs.cnt + 1, 1ull);
+                if (zs_lane() == 0) atomicAdd(ro.cnt + 1, 1ull);
                 continue;
             }
-            uint64_t bit = tail[0], out = tail[1];
+            bit = tail[0]; out = tail[1];
             if (bit == ~0ull) {
                 BitReader br;
-                br.base = a.in; br.pos = 0; br.end = a.in_len; br.safe_end = (a.in_len + 7) & ~7ull; br.hold = 0; br.bits = 0;
+                br.open(a.in, 0, a.in_len, (a.in_len + 7) & ~7ull);
                 int status = ZS_OK, detail = D_NONE;
                 unsigned tflags = 0;
                 // (a zlib header with FDICT reports Z_NEED_DICT here: the stream decoded with its dictionary already)
@@ -706,12 +655,13 @@ __global__ void __launch_bounds__(kWarps * 32) par_record_kernel(ParArgs a, Reco
                 bit = br.pos * 8 - br.bits;
                 out = 0;
             }
-            decode_segment<false, true>(a, s_arena[wid], s_fixed, 0, bit, ~0ull, out, 0, nullptr, nullptr, &rs);
         } else {
             const uint32_t slot = a.plan_slot[k - 1];
-            decode_segment<false, true>(a, s_arena[wid], s_fixed, slot, a.cand[slot], a.seg[slot].end_bit, a.plan_off[k - 1], 0,
-                                        nullptr, nullptr, &rs);
+            bit = a.cand[slot]; stop = a.seg[slot].end_bit; out = a.plan_off[k - 1];
         }
+        RecordSink rs{ro, stop, out, ~0ull, false};
+        walk_blocks_at(a.in, a.in_len, bit, s_arena[wid], s_fixed, rs);
+        if (rs.landed && zs_lane() == 0) atomicAdd(ro.cnt + 1, 1ull);
         __syncwarp();
     }
 }
@@ -816,8 +766,8 @@ int zs_launch_inflate_record(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, 
     } else {
         p.in = d_in; p.in_len = in_len; p.tile = 1; p.out_cap = ~0ull;
     }
-    RecordSink rs;
-    rs.rec = d_rec; rs.cap = rec_cap; rs.cnt = d_cnt; rs.span = span;
-    ZS_KERNEL(ctx, "par_record_kernel", par_record_kernel<<<ctas, kWarps * 32, 0, ctx->stream>>>(p, rs, d_tail, wrap));
+    RecordOut ro;
+    ro.rec = d_rec; ro.cap = rec_cap; ro.cnt = d_cnt; ro.span = span;
+    ZS_KERNEL(ctx, "par_record_kernel", par_record_kernel<<<ctas, kWarps * 32, 0, ctx->stream>>>(p, ro, d_tail, wrap));
     return ZS_OK;
 }
