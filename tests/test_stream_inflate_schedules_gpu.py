@@ -18,6 +18,7 @@ import zlib
 
 import pytest
 
+import deflate_craft as D
 from conftest import make_mixed, make_text, pkg, rand_bytes
 
 pytestmark = pytest.mark.gpu
@@ -281,57 +282,6 @@ def test_flush_points_every_call_forced_and_through_the_c_abi(gpu_ctx, oracle):
         check_schedule(oracle, stream, wbits, sched, seed=seed, expect=data, marks=marks, party=_CAbi)
 
 
-class _Bits:
-    """Deflate bit writer, enough for fixed-Huffman and stored blocks."""
-
-    def __init__(self):
-        self.out, self.acc, self.n = bytearray(), 0, 0
-
-    def put(self, v, n):
-        self.acc |= v << self.n
-        self.n += n
-        while self.n >= 8:
-            self.out.append(self.acc & 255)
-            self.acc >>= 8
-            self.n -= 8
-
-    def code(self, c, n):                     # Huffman codes go most significant bit first
-        self.put(int(format(c, f"0{n}b")[::-1], 2), n)
-
-    def literal(self, b):
-        if b < 144:
-            self.code(0x30 + b, 8)
-        else:
-            self.code(0x190 + b - 144, 9)
-
-    def fixed(self, lits, final=False, matches=()):
-        self.put(int(final), 1)
-        self.put(1, 2)
-        for b in lits:
-            self.literal(b)
-        for (lsym, lextra, lxbits, dcode, dextra, dxbits) in matches:
-            self.code(0xC0 + lsym - 280, 8) if lsym >= 280 else self.code(lsym - 256, 7)
-            self.put(lextra, lxbits)
-            self.code(dcode, 5)
-            self.put(dextra, dxbits)
-        self.code(0, 7)
-
-    def stored(self, data, final=False):
-        """Returns the offset of the byte holding the block header."""
-        at = len(self.out)
-        self.put(int(final), 1)
-        self.put(0, 2)
-        if self.n:
-            self.put(0, 8 - self.n)
-        self.out += len(data).to_bytes(2, "little") + (len(data) ^ 0xFFFF).to_bytes(2, "little") + data
-        return at
-
-    def done(self):
-        if self.n:
-            self.put(0, 8 - self.n)
-        return bytes(self.out)
-
-
 def test_stored_block_length_field_and_header_bits(gpu_ctx, oracle):
     """A 65 535-byte stored block whose header starts at each of the 8 bit positions of a byte, behind a fixed
     block, followed by a fixed block and a final block that copies 258 bytes from 32 768 back, into the stored
@@ -340,13 +290,14 @@ def test_stored_block_length_field_and_header_bits(gpu_ctx, oracle):
     rng = random.Random(65535)
     payload = rng.randbytes(65535)
     for high in range(8):                       # literals of 9 bits move the stored header's bit position
-        w = _Bits()
-        w.fixed(b"abc" + bytes([200] * high))
-        hdr = w.stored(payload)
-        next_hdr = len(w.out)
-        w.fixed(b"xyz" + bytes([150, 250]))
-        w.fixed(b"!", final=True, matches=[(285, 0, 0, 29, 32768 - 24577, 13), (265, 0, 1, 13, 100 - 97, 5)])
-        stream = w.done()
+        d = D.Deflate()
+        d.fixed(b"abc" + bytes([200] * high))
+        hdr = d.w.n // 8                        # the byte holding the stored block's header
+        d.stored(payload)
+        next_hdr = d.w.n // 8
+        d.fixed(b"xyz" + bytes([150, 250]))
+        d.fixed([33, D.Match(258, 32768), D.Match(11, 100)], final=True)
+        stream = d.data()
         expect = zlib.decompressobj(-15).decompress(stream)
         assert len(expect) == 3 + high + 65535 + 5 + 1 + 258 + 11
         cuts = list(range(hdr, hdr + 7)) + list(range(next_hdr - 1, next_hdr + 4))

@@ -3,7 +3,8 @@
 // One warp per stream.  Results must be bit-exact with the reference decoder: inflate_fast
 // (src/mod/inflate/inffast.ts:5), inflate_table (inftrees.ts:62), the block / header / trailer modes
 // of inflate() (inflate.ts:332-1100) when called as inflate(strm, Z_FINISH) on a whole stream: same
-// output bytes, same total_in / total_out, same return code and message.
+// output bytes, same total_in / total_out, same return code and message.  (One known difference: total_in after
+// a Z_BUF_ERROR for want of output room, see store_result in zs_inflate_common.cuh.)
 //
 // Layout: every warp owns a private decode-table arena in shared memory (852 length + 594 distance
 // entries of 32 bits, the reference's ENOUGH bounds).  The run-length coded code lengths of a dynamic

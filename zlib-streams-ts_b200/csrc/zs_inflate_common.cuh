@@ -406,7 +406,9 @@ __device__ __forceinline__ void read_trailer(BitReader& br, unsigned tflags, int
 }
 
 // The per-stream result record.  A Z_BUF_ERROR with output space left means the input ran dry: the reference
-// has pulled every available byte by then (PULLBYTE, inflate.ts:1147-1158).
+// has pulled every available byte by then (PULLBYTE, inflate.ts:1147-1158).  A known difference: on a Z_BUF_ERROR
+// with the output full, the count leaves out the whole bytes still in the bit buffer, while the reference's total_in
+// keeps the bytes it pulled for the symbol that did not fit.
 __device__ __forceinline__ void store_result(const zs_inflate_args& a, uint64_t sidx, const BitReader& br, uint64_t in_start,
                                              uint64_t op, uint64_t cap, int status, int detail, unsigned tflags,
                                              uint32_t check, uint32_t isize) {
@@ -465,7 +467,8 @@ static __device__ __noinline__ int read_dynamic_header(BitReader& br, WarpArena&
             br.refill();
             const uint32_t here = A.codes[br.peek(cbits)];
             if (E_BITS(here) > br.bits) { rc = -1; break; }
-            if (E_OP(here) & 64) { rc = D_CODE_LENGTHS; break; }  // unreachable: the code-length code is complete
+            // (a code-length code without codes has only invalid-code entries of 1 bit and value 0; like the
+            // reference, which never tests their op here, the loop reads them as lengths of 0)
             const unsigned v = E_VAL(here);
             if (v < 16) {
                 br.drop(E_BITS(here));

@@ -3,7 +3,8 @@
 // Same contract as inflate_kernel (zs_inflate.cu): bit-exact with the reference's inflate() called as
 // inflate(strm, Z_FINISH) on a whole stream -- inflate_fast (src/mod/inflate/inffast.ts:5),
 // inflate_table (inftrees.ts:62), block / header / trailer modes (inflate.ts:332-1100), including
-// raw deflate64 -- same output, total_in / total_out, return code and message.
+// raw deflate64 -- same output, total_in / total_out, return code and message (total_in after a Z_BUF_ERROR for
+// want of output room excepted, see store_result in zs_inflate_common.cuh).
 //
 // Why a second kernel: symbol decoding is serial inside a stream.  The warp-per-stream kernel spends
 // a full warp instruction per scalar decode step (31 of 32 lanes redundant), which bounds it near
@@ -70,6 +71,13 @@ __device__ int build_canon(const Tab& T, unsigned first, unsigned n, int type, b
         if (d64) return -1;                       // PARAMS_9._createTableWhenNoCodes = false
         for (int l = 1; l <= 15; l++) { T.at(t_lim + l) = 0; T.at(t_base + l) = 0; }
         *minlen = 1;                              // every code is invalid (inftrees.ts:113-123)
+        if (type == 0) {
+            // ... but the code-length loop never tests an entry's op: it reads the reference's two invalid
+            // entries (1 bit, value 0) as lengths of 0.  Two 1-bit codes of symbol 0 decode the same way.
+            T.at(t_lim + 1) = 0x8000;
+            T.sym(t_sym) = 0;
+            T.sym(t_sym + 1) = 0;
+        }
         return 0;
     }
     int left = 1;
@@ -253,7 +261,6 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
                     br.refill();
                     unsigned nb;
                     const int sym = decode_sym(T, br.hold, T_LSYM, T_LLIM, T_LBASE, cmin, &nb);
-                    if (sym < 0) { err = nb > br.bits ? -1 : D_CODE_LENGTHS; break; }
                     if (nb > br.bits) { err = -1; break; }
                     if (sym < 16) {
                         br.drop(nb);
@@ -296,7 +303,9 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
                 unsigned nb;
                 const int sym = decode_sym_fast<true>(T, LL, br.hold, T_LSYM, T_LBASE, &nb);
                 if (sym < 0) {
-                    if (nb > br.bits && br.bits < 15) status = ZS_BUF_ERROR;
+                    // only an incomplete or empty set has invalid codes, and the reference's entry for them is one
+                    // bit wide: one bit of input is enough for the verdict
+                    if (br.bits == 0) status = ZS_BUF_ERROR;
                     else { status = ZS_DATA_ERROR; detail = D_LITLEN_CODE; }
                     break;
                 }
@@ -318,7 +327,7 @@ __global__ void __launch_bounds__(32 * kWarpsPerCta) inflate_tps_kernel(zs_infla
                 br.refill();
                 const int ds = decode_sym_fast<false>(T, DL, br.hold, T_DSYM, T_DBASE, &nb);
                 if (ds < 0) {
-                    if (nb > br.bits && br.bits < 15) status = ZS_BUF_ERROR;
+                    if (br.bits == 0) status = ZS_BUF_ERROR;
                     else { status = ZS_DATA_ERROR; detail = D_DIST_CODE; }
                     break;
                 }
