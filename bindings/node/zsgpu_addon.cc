@@ -181,6 +181,33 @@ napi_value DeflateBatch(napi_env env, napi_callback_info info) {
     return o;
 }
 
+// deflateIndexed(input: Uint8Array, chunkSize, level, wrap, flags, span, out: Uint8Array[, outOff: BigUint64Array])
+//   -> {outLen, check, index: {handle, points, outLen}}                zs_deflate_indexed
+// One stitched stream and its index for `span`, made from the encoder's block layout (no decode).
+napi_value DeflateIndexed(napi_env env, napi_callback_info info) {
+    size_t argc = 8; napi_value a[8];
+    napi_get_cb_info(env, info, &argc, a, nullptr, nullptr);
+    uint8_t *in, *out; size_t n, cap;
+    if (argc < 7 || !u8(env, a[0], &in, &n) || !u8(env, a[6], &out, &cap)) return throw_code(env, ZS_STREAM_ERROR, "deflateIndexed");
+    uint32_t chunk = (uint32_t)i32(env, a[1]);
+    if (chunk == 0) return throw_code(env, ZS_STREAM_ERROR, "deflateIndexed");
+    uint32_t n_chunks = n ? (uint32_t)((n + chunk - 1) / chunk) : 1;
+    uint32_t span = 0;
+    napi_get_value_uint32(env, a[5], &span);
+    uint64_t* off = nullptr; size_t off_n = 0;
+    if (argc >= 8 && !u64s(env, a[7], &off, &off_n)) off_n = 0;
+    zs_deflate_result r;
+    zs_inflate_index* x = nullptr;
+    int rc = zs_deflate_indexed(g_ctx, in, n, nullptr, n_chunks, chunk, i32(env, a[2]), i32(env, a[3]), (uint32_t)i32(env, a[4]),
+                                span, out, cap, off_n >= n_chunks + 1 ? off : nullptr, nullptr, nullptr, &r, &x);
+    if (rc != ZS_OK) return throw_code(env, rc, "zs_deflate_indexed");
+    napi_value o; napi_create_object(env, &o);
+    napi_set_named_property(env, o, "outLen", num(env, (double)r.total_out_bytes));
+    napi_set_named_property(env, o, "check", num(env, (double)r.check));
+    napi_set_named_property(env, o, "index", index_object(env, x));
+    return o;
+}
+
 // inflateBatch(input, inOff: BigUint64Array, windowBits, out, outOff: BigUint64Array, outLen: BigUint64Array,
 //              checks: Uint32Array, status: Int32Array[, dicts: Uint8Array, dictRng: BigUint64Array (2 per stream)])
 //   -> void                                                            zs_inflate_batch
@@ -387,7 +414,7 @@ napi_value Register(napi_env env, napi_value exports) {
     const struct { const char* name; napi_callback fn; } fns[] = {
         {"init", Init}, {"deflateBatch", DeflateBatch}, {"inflateBatch", InflateBatch}, {"gunzip", Gunzip}, {"checksum", Checksum},
         {"createDeflateDictionary", CreateDeflateDictionary},
-        {"inflateIndexBuild", InflateIndexBuild}, {"inflateIndexExtract", InflateIndexExtract},
+        {"deflateIndexed", DeflateIndexed}, {"inflateIndexBuild", InflateIndexBuild}, {"inflateIndexExtract", InflateIndexExtract},
         {"inflateIndexExport", InflateIndexExport}, {"inflateIndexImport", InflateIndexImport},
         {"streamNew", StreamNew}, {"deflateInit2", DeflateInit2}, {"inflateInit2", InflateInit2}, {"process", Process},
         {"end", End}, {"setDictionary", SetDictionary}, {"inflateReset", InflateReset}, {"control", Control},

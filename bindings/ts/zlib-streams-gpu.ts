@@ -212,7 +212,7 @@ export function gunzip(input: Uint8Array, opts: { outCap?: number; members?: boo
 // Z_FINISH would) and returns the index with the output; extract() then reads any byte ranges of the stream without
 // decoding what comes before them.  toBytes() / fromBytes() carry an index across processes (the format of zsgpu.h).
 export class InflateIndex {
-  private constructor(private readonly h: { handle: unknown; points: number; outLen: number }) {}
+  constructor(private readonly h: { handle: unknown; points: number; outLen: number }) {}
   get points(): number { return this.h.points; }
   get outLen(): number { return this.h.outLen; }
   static build(input: Uint8Array, opts: { windowBits?: number; span?: number; dictionary?: Uint8Array; outCap?: number } = {}) {
@@ -243,4 +243,15 @@ export class InflateIndex {
     addon.inflateIndexExtract(this.h.handle, input, off, len, out.subarray(0, total), outOff, got, status);
     return ranges.map((_, i) => ({ data: out.subarray(Number(outOff[i]), Number(outOff[i]) + Number(got[i])), status: status[i] }));
   }
+}
+// One stitched stream (deflateBatch with stitched: true) and its InflateIndex, made in the same call from the encoder's
+// block layout without decoding the stream: the index equals InflateIndex.build(data, {windowBits, span}).index.
+// flags: the strategy (bits 8..10) and 8 (a sync marker after every chunk).
+export function deflateIndexed(input: Uint8Array, opts: { chunkSize?: number; level?: number; wrap?: 0 | 1 | 2; flags?: number;
+                                                         span?: number } = {}) {
+  const chunkSize = opts.chunkSize ?? 65536;
+  const nChunks = Math.max(1, Math.ceil(input.length / chunkSize));
+  const out = new Uint8Array(input.length + 6 * nChunks * (Math.floor(chunkSize / 16351) + 2) + 26 * nChunks + 64);
+  const r = addon.deflateIndexed(input, chunkSize, opts.level ?? 6, opts.wrap ?? 1, opts.flags ?? 0, opts.span ?? (1 << 20), out);
+  return { data: out.subarray(0, r.outLen), check: r.check, index: new InflateIndex(r.index) };
 }

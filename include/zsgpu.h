@@ -78,6 +78,7 @@ extern "C" {
 #define ZS_FLAG_STRATEGY(s) (((uint32_t)(s) & 7u) << 8)
 
 typedef struct zs_ctx zs_ctx;
+typedef struct zs_inflate_index zs_inflate_index;   /* random access into one stream: see zs_inflate_index_build */
 
 #if defined(__GNUC__)
 #define ZS_API __attribute__((visibility("default")))
@@ -165,6 +166,30 @@ ZS_API int zs_deflate_batch(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, con
 ZS_API int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t history, uint32_t chunk_size,
                     int level, int wrap, uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_bits,
                     zs_deflate_result* result);
+
+/* ---- deflate one stream and index it in the same call ----
+ * The arguments of zs_deflate_batch_dev / zs_deflate_batch without mode (always ZS_MODE_STITCHED: one stream) and
+ * history, with the span of an index (zs_inflate_index_*, below) and the index itself.  The compressed bytes, out_off,
+ * out_bits, checks and the result are those zs_deflate_batch_dev / zs_deflate_batch write with ZS_MODE_STITCHED and the
+ * same arguments (the host call's slices and their sync markers included): indexing does not change the stream.
+ * *index receives the index zs_inflate_index_build makes from that output with window_bits 15 / 31 / -15 (zlib / gzip /
+ * raw) and the same span -- header, points and windows alike, with crc32 as the check of a raw stream -- without
+ * decoding it: the encoder's block layout gives every block start (DESIGN.md 3.3e), the input is the output before it.
+ * flags: the strategy and ZS_FLAG_SYNC.  ZS_FLAG_PRIME, ZS_FLAG_NOT_FIRST, ZS_FLAG_NOT_LAST (a part is not a whole
+ * stream), span 0, a null index pointer and whatever the batch call refuses are ZS_STREAM_ERROR; an out_cap too small
+ * for the stream is ZS_BUF_ERROR.  *index is NULL unless the call returns ZS_OK.  The calls make host decisions, so they
+ * SYNCHRONISE.  The device call writes d_result (device memory) as zs_deflate_batch_dev does; d_in must stay valid and
+ * unchanged until it returns (the windows are read from it). */
+ZS_API int zs_deflate_indexed_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, const uint64_t* d_in_off,
+                                  uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk, int level, int wrap,
+                                  uint32_t flags, uint64_t span, uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off,
+                                  uint64_t* d_out_bits, uint32_t* d_checks, zs_deflate_result* d_result,
+                                  zs_inflate_index** index);
+/* Host-buffer variant: `result` is host memory, as in zs_deflate_batch. */
+ZS_API int zs_deflate_indexed(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, const uint64_t* in_off, uint32_t n_chunks,
+                              uint32_t chunk_size, int level, int wrap, uint32_t flags, uint64_t span, uint8_t* out,
+                              uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits, uint32_t* checks,
+                              zs_deflate_result* result, zs_inflate_index** index);
 
 /* ---- preset dictionary for batch deflate (deflateSetDictionary, deflate.ts:367-424, once for many
  *      records).  Many small records compress far better against a shared dictionary; the batch calls
@@ -282,7 +307,6 @@ ZS_API int zs_inflate_last_details(zs_ctx* ctx, int32_t* detail, uint32_t n);
  * The index lives on the device of the context that made it: its point table and n_points windows of up to 32 KiB,
  * with a host copy of the table.  Any context on that device may use it; destroy it before that context.  Only the first
  * gzip member is indexed (zs_gunzip's member table serves multi-member files).  Deflate64 has no index. */
-typedef struct zs_inflate_index zs_inflate_index;
 typedef struct zs_inflate_index_info {
     uint64_t in_len, out_len, span, n_points;
     uint32_t check;      /* adler32 (zlib) / crc32 (gzip, raw) of the whole output */

@@ -212,6 +212,72 @@ def deflate_batch(data, chunk_size: int = 65536, level: int = 6, wrap: int = WRA
                             res.total_out_bits, res.check, res.n_blocks)
 
 
+def deflate_indexed_dev(d_in: torch.Tensor, chunk_size: int, level: int = 6, wrap: int = WRAP_ZLIB, flags: int = 0,
+                        span: int = 1 << 20, in_off: torch.Tensor | None = None, max_chunk: int | None = None,
+                        out: torch.Tensor | None = None, want_checks: bool = False,
+                        ctx: Context | None = None) -> tuple[DeflateBatchDev, "InflateIndex"]:
+    """One STITCHED stream from device-resident input and its index for `span` (zs_deflate_indexed_dev), without a
+    decode: the DeflateBatchDev that deflate_batch_dev(mode=MODE_STITCHED) returns, and an InflateIndex whose source
+    is the stream out[:total_out_bytes].  Synchronises."""
+    assert d_in.is_cuda and d_in.dtype == torch.uint8 and d_in.is_contiguous()
+    ctx = ctx or default_context(d_in.device.index)
+    n = d_in.numel()
+    if in_off is None:
+        n_chunks = n_chunks_for(n, chunk_size)
+        mc = chunk_size
+    else:
+        n_chunks = in_off.numel() - 1
+        mc = max_chunk if max_chunk is not None else int((in_off[1:] - in_off[:-1]).max().item())
+    dev = d_in.device
+    if out is None:
+        out = torch.empty(int(capi.load().zs_deflate_batch_bound(n, n_chunks, mc, wrap, MODE_STITCHED)), dtype=torch.uint8,
+                          device=dev)
+    out_off = torch.empty(n_chunks + 1, dtype=torch.int64, device=dev)
+    out_bits = torch.empty(n_chunks, dtype=torch.int64, device=dev)
+    checks = torch.empty(n_chunks, dtype=torch.int32, device=dev) if (want_checks or wrap != WRAP_RAW) else None
+    result = torch.zeros(24, dtype=torch.uint8, device=dev)
+    h = C.c_void_p()
+    rc = capi.load().zs_deflate_indexed_dev(ctx.handle, _ptr(d_in), n, _ptr(in_off), n_chunks, chunk_size, mc, level, wrap,
+                                            flags, span, _ptr(out), out.numel(), _ptr(out_off), _ptr(out_bits), _ptr(checks),
+                                            _ptr(result), C.byref(h))
+    ctx.check(rc, "zs_deflate_indexed_dev")
+    batch = DeflateBatchDev(out, out_off, out_bits, checks, result)
+    return batch, InflateIndex(h, ctx, out[: batch.read_result().total_out_bytes])
+
+
+def deflate_indexed(data, chunk_size: int = 65536, level: int = 6, wrap: int = WRAP_ZLIB, flags: int = 0,
+                    span: int = 1 << 20, in_off=None, ctx: Context | None = None) -> tuple[DeflateBatchHost, "InflateIndex"]:
+    """One STITCHED stream from a host buffer and its index for `span` (zs_deflate_indexed), without a decode: the
+    DeflateBatchHost that deflate_batch(mode=MODE_STITCHED) returns, and an InflateIndex whose source is its bytes."""
+    ctx = ctx or default_context()
+    src = _as_u8(data)
+    n = src.size
+    if in_off is None:
+        n_chunks = n_chunks_for(n, chunk_size)
+        mc = chunk_size
+        off_arr = None
+    else:
+        off_arr = np.ascontiguousarray(np.asarray(in_off, dtype=np.uint64))
+        n_chunks = off_arr.size - 1
+        mc = int((off_arr[1:] - off_arr[:-1]).max()) if n_chunks else 1
+    lib = capi.load()
+    cap = int(lib.zs_deflate_batch_bound(n, n_chunks, max(mc, 1), wrap, MODE_STITCHED))
+    out = np.empty(cap, dtype=np.uint8)
+    out_off = np.zeros(n_chunks + 1, dtype=np.uint64)
+    out_bits = np.zeros(n_chunks, dtype=np.uint64)
+    checks = np.zeros(n_chunks, dtype=np.uint32)
+    res = DeflateResult()
+    h = C.c_void_p()
+    rc = lib.zs_deflate_indexed(ctx.handle, src.ctypes.data if n else None, n,
+                                off_arr.ctypes.data if off_arr is not None else None, n_chunks, chunk_size, level, wrap, flags,
+                                span, out.ctypes.data, cap, out_off.ctypes.data, out_bits.ctypes.data, checks.ctypes.data,
+                                C.byref(res), C.byref(h))
+    ctx.check(rc, "zs_deflate_indexed")
+    stream = out[: res.total_out_bytes].tobytes()
+    return (DeflateBatchHost(stream, out_off, out_bits, checks, res.total_out_bytes, res.total_out_bits, res.check,
+                             res.n_blocks), InflateIndex(h, ctx, stream))
+
+
 @dataclass
 class InflateBatchDev:
     out: torch.Tensor

@@ -88,6 +88,12 @@ _PROTOTYPES = {
     "zs_deflate_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32, C.c_int,
                                    C.c_int, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.POINTER(DeflateResult)]),
+    "zs_deflate_indexed_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32,
+                                         C.c_uint32, C.c_int, C.c_int, C.c_uint32, C.c_uint64, C.c_void_p, C.c_uint64,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "zs_deflate_indexed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32, C.c_int,
+                                     C.c_int, C.c_uint32, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.POINTER(DeflateResult), C.POINTER(C.c_void_p)]),
     "zs_deflate_part": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.c_uint32,
                                   C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(DeflateResult)]),
     "zs_deflate_dict_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]),

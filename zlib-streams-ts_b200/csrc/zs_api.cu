@@ -273,11 +273,12 @@ int zs_checksum(zs_ctx* ctx, int kind, const uint8_t* buf, uint64_t len, uint32_
 // ---- deflate ------------------------------------------------------------------------------------------
 // zs_deflate_batch_dev, and zs_deflate_batch_dict_dev with `dict` (INDEPENDENT, no history, checked by the caller).
 // seg_hint: 0, or the LZ77 segment size (chunks) of the whole batch when this call compresses a slice of it.
+// record: the indexed calls' request to keep block starts (deflate_record_kernel), or nullptr.
 static int deflate_batch_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* d_in, uint64_t in_len,
                              const uint64_t* d_in_off, uint32_t n_chunks, uint32_t chunk_size, uint32_t max_chunk,
                              uint32_t history, int level, int wrap, int mode, uint32_t flags, uint8_t* d_out,
                              uint64_t out_cap, uint64_t* d_out_off, uint64_t* d_out_bits, uint32_t* d_checks,
-                             zs_deflate_result* d_result, uint32_t seg_hint) {
+                             zs_deflate_result* d_result, uint32_t seg_hint, const DeflateRecord* record) {
     if (level == -1) level = 6;
     // argument rules of deflateInit2_ (deflate.ts:263-297) that apply to the batch form
     if (level < 0 || level > 9) return zs_bad_arg(ctx, "deflate: level must be 0..9");
@@ -310,6 +311,7 @@ static int deflate_batch_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const uin
     p.level = level; p.wrap = wrap; p.mode = mode; p.flags = flags; p.strategy = strategy;
     p.seg_hint = seg_hint;
     p.dict = dict;
+    p.record = record;
     const size_t slots = (size_t)n_chunks * p.max_bpc;
 
     uint64_t* off = (uint64_t*)zs_scratch_get(ctx, SCR_D_OFF, (size_t)(n_chunks + 1) * 8);
@@ -383,7 +385,7 @@ int zs_deflate_batch_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, cons
     if (ctx) bind_device(ctx);
     if (!ctx) return ZS_STREAM_ERROR;
     return deflate_batch_dev(ctx, nullptr, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, history, level, wrap,
-                             mode, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0);
+                             mode, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0, nullptr);
 }
 
 // ---- preset dictionaries ------------------------------------------------------------------------------
@@ -460,8 +462,60 @@ int zs_deflate_batch_dict_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
     const int rc = check_dict_call(ctx, dict, wrap, flags);
     if (rc != ZS_OK) return rc;
     return deflate_batch_dev(ctx, dict, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, 0, level, wrap,
-                             ZS_MODE_INDEPENDENT, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0);
+                             ZS_MODE_INDEPENDENT, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0, nullptr);
 }
+
+// The block starts an indexed call keeps (zs_deflate_indexed*), in SCR_D_REC: a counter and a region of `cap` pairs
+// per slice.  deflate_record_kernel writes bits and input offsets local to the slice's part; the call that cut the
+// slices notes where each part lies in the stream (bit) and in the input (byte) to shift them by.
+struct KeptStarts {
+    uint64_t span = 0;
+    unsigned long long* d_cnt = nullptr;   // [kMaxPipeSlices]
+    uint64_t* d_rec = nullptr;             // [n_slices][cap][2]
+    uint64_t cap = 0;
+    int n_slices = 1;
+    uint64_t bit0[kMaxPipeSlices] = {0}, byte0[kMaxPipeSlices] = {0};
+    const uint8_t* d_in = nullptr;         // host-buffer call: the whole input on the device, where the windows come from
+
+    // room for n slices of at most nc chunks and len bytes (2 * nc + len / span + 4 pairs each: a chunk keeps its first
+    // start and at most one per multiple of the span it covers, and a chunk of b bytes covers at most b / span + 1)
+    int begin(zs_ctx* ctx, int n, uint64_t nc, uint64_t len) {
+        n_slices = n;
+        cap = 2 * nc + len / span + 4;
+        uint8_t* m = (uint8_t*)zs_scratch_get(ctx, SCR_D_REC, kMaxPipeSlices * 8 + (size_t)n * cap * 16);
+        if (!m) return ZS_MEM_ERROR;
+        d_cnt = (unsigned long long*)m;
+        d_rec = (uint64_t*)(m + kMaxPipeSlices * 8);
+        ZS_CUDA_TRY(ctx, cudaMemsetAsync(d_cnt, 0, kMaxPipeSlices * 8, ctx->stream));
+        return ZS_OK;
+    }
+    DeflateRecord slice(int s) const { return {d_rec + 2 * cap * s, cap, d_cnt + s, span}; }
+    // every slice's kept starts, shifted into the stream, after the call's work on the context stream
+    int read(zs_ctx* ctx, std::vector<uint64_t>& rec) const {
+        unsigned long long cnt[kMaxPipeSlices];
+        ZS_CUDA_TRY(ctx, cudaMemcpyAsync(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, ctx->stream));
+        ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        uint64_t total = 0;
+        for (int s = 0; s < n_slices; s++) {
+            if (cnt[s] > cap) {   // cannot happen: cap bounds what the rule keeps
+                snprintf(ctx->err, sizeof(ctx->err), "deflate_indexed: more block starts kept than room for them");
+                return ZS_E_CUDA;
+            }
+            total += cnt[s];
+        }
+        rec.resize(2 * total);
+        uint64_t k = 0;
+        for (int s = 0; s < n_slices; s++) {
+            if (cnt[s]) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(rec.data() + 2 * k, d_rec + 2 * cap * s, cnt[s] * 16, cudaMemcpyDeviceToHost, ctx->stream));
+            k += cnt[s];
+        }
+        ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        k = 0;
+        for (int s = 0; s < n_slices; s++)
+            for (uint64_t i = 0; i < cnt[s]; i++, k++) { rec[2 * k] += bit0[s]; rec[2 * k + 1] += byte0[s]; }
+        return ZS_OK;
+    }
+};
 
 // Host-buffer deflate of a large batch, software-pipelined: the batch is cut into slices of whole waves of
 // LZ77 segments, and the H2D copy of slice s+1, the kernels of slice s and the D2H copy of slice s-1 run
@@ -475,7 +529,7 @@ int zs_deflate_batch_dict_dev(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
 static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len,
                                    uint32_t history, uint32_t n_chunks, uint32_t chunk_size, int level, int wrap, int mode,
                                    uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off, uint64_t* out_bits,
-                                   uint32_t* checks, zs_deflate_result* result) {
+                                   uint32_t* checks, zs_deflate_result* result, KeptStarts* kept) {
     constexpr int kMaxSlices = 16;
     static_assert(kMaxSlices <= kMaxPipeSlices, "one event per slice");
     const bool stitched = mode == ZS_MODE_STITCHED;
@@ -534,6 +588,11 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
     if (!d_in_base || !d_out || !d_ooff || !d_obits || !d_cks || !d_res) return ZS_MEM_ERROR;
     uint8_t* d_in = d_in_base + 32768;   // the history of the first slice lies before it
     const bool want_checks = checks != nullptr || wrap != ZS_WRAP_RAW;
+    if (kept) {
+        rc = kept->begin(ctx, n_slices, slice_chunks, slice_bytes);
+        if (rc != ZS_OK) return rc;
+        kept->d_in = d_in;
+    }
     rc = fence_copy_streams(ctx);
     if (rc != ZS_OK) return rc;
     if (history) ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in - history, in - history, history, cudaMemcpyHostToDevice, ctx->s_in));
@@ -555,9 +614,10 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         } else if (flags & ZS_FLAG_PRIME) {
             hist = (uint32_t)(b0 < 32768 ? b0 : 32768);
         }
+        const DeflateRecord rec = kept ? kept->slice(s) : DeflateRecord{};
         rc = deflate_batch_dev(ctx, dict, d_in + b0, len, nullptr, nc, chunk_size, chunk_size, hist, level, wrap, mode, sflags,
                                d_out + region_al * s, region, d_ooff + c0 + s, d_obits + c0,
-                               want_checks ? d_cks + c0 : nullptr, d_res + s, seg);
+                               want_checks ? d_cks + c0 : nullptr, d_res + s, seg, kept ? &rec : nullptr);
         if (rc != ZS_OK) return rc;
         ZS_CUDA_TRY(ctx, cudaEventRecord(ctx->ev_kern[s], ctx->stream));
         // The 24-byte results come back on their own stream: the bulk D2H copies below are issued as
@@ -579,6 +639,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
         ZS_CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev_res[s]));
         const uint64_t total = h_res[s].total_out_bytes;
         base[s] = host_off;
+        if (kept) { kept->bit0[s] = host_off * 8; kept->byte0[s] = b0; }
         if (total > region || host_off + total > out_cap) { rc_final = ZS_BUF_ERROR; break; }
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(out + host_off, d_out + region_al * s, total, cudaMemcpyDeviceToHost, ctx->s_out));
         if (out_off)
@@ -630,7 +691,7 @@ static int deflate_batch_pipelined(zs_ctx* ctx, const zs_deflate_dict* dict, con
 static int deflate_batch_host(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len,
                               uint32_t history, const uint64_t* in_off, uint32_t n_chunks, uint32_t chunk_size, int level,
                               int wrap, int mode, uint32_t flags, uint8_t* out, uint64_t out_cap, uint64_t* out_off,
-                              uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result) {
+                              uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result, KeptStarts* kept) {
     if (!out || !result || (in_len && !in) || n_chunks == 0) return zs_bad_arg(ctx, "deflate: null buffer or zero chunks");
     if (history && !in) return zs_bad_arg(ctx, "deflate: history without an input pointer");
     if (history > 32768) history = 32768;
@@ -648,7 +709,7 @@ static int deflate_batch_host(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
     // Large batches with fixed chunking are software-pipelined (see deflate_batch_pipelined).
     if (!in_off && n_chunks >= 512 && chunk_size >= 4096 && !(mode == ZS_MODE_STITCHED && (flags & ZS_FLAG_PRIME)))
         return deflate_batch_pipelined(ctx, dict, in, in_len, history, n_chunks, chunk_size, level, wrap, mode, flags, out,
-                                       out_cap, out_off, out_bits, checks, result);
+                                       out_cap, out_off, out_bits, checks, result, kept);
     if (mode != ZS_MODE_STITCHED) history = 0;
     uint8_t* d_in_base = (uint8_t*)zs_scratch_get(ctx, SCR_H_IN, 32768 + in_len + 64);
     uint8_t* d_out = (uint8_t*)zs_scratch_get(ctx, SCR_H_OUT, out_cap + 64);
@@ -659,12 +720,19 @@ static int deflate_batch_host(zs_ctx* ctx, const zs_deflate_dict* dict, const ui
     uint8_t* d_in = d_in_base + 32768;
     zs_deflate_result* d_result = (zs_deflate_result*)d_res;
     uint32_t* d_checks = checks ? (uint32_t*)(d_res + 64) : nullptr;
+    if (kept) {
+        const int rc = kept->begin(ctx, 1, n_chunks, in_len);
+        if (rc != ZS_OK) return rc;
+        kept->d_in = d_in;
+    }
+    const DeflateRecord rec = kept ? kept->slice(0) : DeflateRecord{};
     if (in_len + history)
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_in - history, in - history, in_len + history, cudaMemcpyHostToDevice, ctx->stream));
     if (in_off)
         ZS_CUDA_TRY(ctx, cudaMemcpyAsync(d_off, in_off, (size_t)(n_chunks + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
     int rc = deflate_batch_dev(ctx, dict, d_in, in_len, in_off ? d_off : nullptr, n_chunks, chunk_size, max_chunk, history,
-                               level, wrap, mode, flags, d_out, out_cap, d_ooff, d_ooff + n_chunks + 1, d_checks, d_result, 0);
+                               level, wrap, mode, flags, d_out, out_cap, d_ooff, d_ooff + n_chunks + 1, d_checks, d_result, 0,
+                               kept ? &rec : nullptr);
     if (rc != ZS_OK) return rc;
     ZS_CUDA_TRY(ctx, cudaMemcpyAsync(result, d_result, sizeof(zs_deflate_result), cudaMemcpyDeviceToHost, ctx->stream));
     ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -690,7 +758,7 @@ int zs_deflate_batch(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, const uint
     if (ctx) bind_device(ctx);
     if (!ctx) return ZS_STREAM_ERROR;
     return deflate_batch_host(ctx, nullptr, in, in_len, 0, in_off, n_chunks, chunk_size, level, wrap, mode, flags, out, out_cap,
-                              out_off, out_bits, checks, result);
+                              out_off, out_bits, checks, result, nullptr);
 }
 
 int zs_deflate_batch_dict(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_t* in, uint64_t in_len, const uint64_t* in_off,
@@ -702,7 +770,7 @@ int zs_deflate_batch_dict(zs_ctx* ctx, const zs_deflate_dict* dict, const uint8_
     if (rc != ZS_OK) return rc;
     // every chunk is its own segment in a dictionary call, so slicing a large batch cannot change the output
     return deflate_batch_host(ctx, dict, in, in_len, 0, in_off, n_chunks, chunk_size, level, wrap, ZS_MODE_INDEPENDENT, flags,
-                              out, out_cap, out_off, out_bits, checks, result);
+                              out, out_cap, out_off, out_bits, checks, result, nullptr);
 }
 
 int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t history, uint32_t chunk_size, int level,
@@ -714,7 +782,89 @@ int zs_deflate_part(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, uint32_t hi
     const uint64_t nc = in_len ? (in_len + chunk_size - 1) / chunk_size : 1;
     if (nc > 0xffffffffull) return zs_bad_arg(ctx, "deflate: too many chunks");
     return deflate_batch_host(ctx, nullptr, in, in_len, history, nullptr, (uint32_t)nc, chunk_size, level, wrap, ZS_MODE_STITCHED,
-                              flags, out, out_cap, nullptr, out_bits, nullptr, result);
+                              flags, out, out_cap, nullptr, out_bits, nullptr, result, nullptr);
+}
+
+}  // extern "C"
+
+// ---- deflate with an index of the stream it writes -----------------------------------------------------------
+// The arguments the batch calls take that the indexed ones refuse: a part of a stream, primed chunks, a zero span.
+static int check_indexed_call(zs_ctx* ctx, uint32_t flags, uint64_t span, zs_inflate_index** index) {
+    if (!index) return zs_bad_arg(ctx, "deflate_indexed: null index pointer");
+    if (flags & (ZS_FLAG_PRIME | ZS_FLAG_NOT_FIRST | ZS_FLAG_NOT_LAST))
+        return zs_bad_arg(ctx, "deflate_indexed: the stream is one whole stream (no PRIME or part flags)");
+    if (span == 0) return zs_bad_arg(ctx, "deflate_indexed: span is zero");
+    return ZS_OK;
+}
+
+// The index of the stream a deflate call just wrote (total_out bytes from in_len bytes of input at d_in): the kept
+// block starts, the check inflate reports, and the windows gathered from the input, which is the stream's output.
+// `check` is the deflate result's; a raw stream's is crc32, which deflate computes only for per-chunk checks.
+static int finish_indexed(zs_ctx* ctx, const KeptStarts& kept, const uint8_t* d_in, uint64_t in_len, int wrap,
+                          bool per_chunk_checks, uint64_t total_out, uint32_t check, zs_inflate_index** index) {
+    if (wrap == ZS_WRAP_RAW && !per_chunk_checks) {
+        check = 0;
+        if (in_len) {
+            uint32_t* d_crc = (uint32_t*)zs_scratch_get(ctx, SCR_SMALL, 256);
+            if (!d_crc) return ZS_MEM_ERROR;
+            const int rc = zs_launch_checksum_whole(ctx, 1, d_in, in_len, 0u, d_crc);
+            if (rc != ZS_OK) return rc;
+            ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&check, d_crc, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        }
+    }
+    std::vector<uint64_t> rec;
+    const int rc = kept.read(ctx, rec);   // synchronises
+    if (rc != ZS_OK) return rc;
+    const int wb = wrap == ZS_WRAP_ZLIB ? 15 : wrap == ZS_WRAP_GZIP ? 31 : -15;
+    return zs_index_from_starts(ctx, rec.data(), rec.size() / 2, kept.span, wb, check, total_out, in_len, d_in, nullptr, 0, 0,
+                                index);
+}
+
+extern "C" {
+
+int zs_deflate_indexed_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len, const uint64_t* d_in_off, uint32_t n_chunks,
+                           uint32_t chunk_size, uint32_t max_chunk, int level, int wrap, uint32_t flags, uint64_t span,
+                           uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off, uint64_t* d_out_bits, uint32_t* d_checks,
+                           zs_deflate_result* d_result, zs_inflate_index** index) {
+    if (index) *index = nullptr;
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    int rc = check_indexed_call(ctx, flags, span, index);
+    if (rc != ZS_OK) return rc;
+    KeptStarts kept;
+    kept.span = span;
+    rc = kept.begin(ctx, 1, n_chunks, in_len);
+    if (rc != ZS_OK) return rc;
+    const DeflateRecord r = kept.slice(0);
+    rc = deflate_batch_dev(ctx, nullptr, d_in, in_len, d_in_off, n_chunks, chunk_size, max_chunk, 0, level, wrap,
+                           ZS_MODE_STITCHED, flags, d_out, out_cap, d_out_off, d_out_bits, d_checks, d_result, 0, &r);
+    if (rc != ZS_OK) return rc;
+    zs_deflate_result res;
+    ZS_CUDA_TRY(ctx, cudaMemcpyAsync(&res, d_result, sizeof(res), cudaMemcpyDeviceToHost, ctx->stream));
+    ZS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (res.total_out_bytes > out_cap) {
+        snprintf(ctx->err, sizeof(ctx->err), "deflate_indexed: output needs %llu bytes, capacity %llu",
+                 (unsigned long long)res.total_out_bytes, (unsigned long long)out_cap);
+        return ZS_BUF_ERROR;
+    }
+    return finish_indexed(ctx, kept, d_in, in_len, wrap, d_checks != nullptr, res.total_out_bytes, res.check, index);
+}
+
+int zs_deflate_indexed(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, const uint64_t* in_off, uint32_t n_chunks,
+                       uint32_t chunk_size, int level, int wrap, uint32_t flags, uint64_t span, uint8_t* out, uint64_t out_cap,
+                       uint64_t* out_off, uint64_t* out_bits, uint32_t* checks, zs_deflate_result* result,
+                       zs_inflate_index** index) {
+    if (index) *index = nullptr;
+    if (ctx) bind_device(ctx);
+    if (!ctx) return ZS_STREAM_ERROR;
+    int rc = check_indexed_call(ctx, flags, span, index);
+    if (rc != ZS_OK) return rc;
+    KeptStarts kept;
+    kept.span = span;
+    rc = deflate_batch_host(ctx, nullptr, in, in_len, 0, in_off, n_chunks, chunk_size, level, wrap, ZS_MODE_STITCHED, flags,
+                            out, out_cap, out_off, out_bits, checks, result, &kept);
+    if (rc != ZS_OK) return rc;
+    return finish_indexed(ctx, kept, kept.d_in, in_len, wrap, checks != nullptr, result->total_out_bytes, result->check, index);
 }
 
 int zs_bit_concat_dev(zs_ctx* ctx, uint8_t* d_dst, uint64_t dst_bit_off, const uint8_t* d_src, uint64_t n_bits) {

@@ -41,6 +41,9 @@ enum zs_scratch_slot {
     // Extract: per-range plan and verdicts, per-warp history rings, and the staged input of the host-buffer call (its
     // output goes to SCR_H_OUT)
     SCR_X_BUILD, SCR_X_PLAN, SCR_X_RING, SCR_X_IN,
+    // zs_deflate_indexed*: the block starts deflate_record_kernel keeps, a counter and a region of pairs per slice.  Its
+    // own: the deflate it runs uses the deflate and host-buffer slots above, and the index it makes allocates its memory
+    SCR_D_REC,
     ZS_SCR_COUNT
 };
 
@@ -338,6 +341,14 @@ int zs_launch_inflate_verify(zs_ctx* ctx, uint32_t n, const uint32_t* d_adler, c
                              const uint32_t* d_trailer, const uint32_t* d_flags, const uint64_t* d_out_len,
                              uint32_t* d_checks, int32_t* d_status, int32_t* d_detail);
 
+// zs_inflate_index.cu: the index of a stream (in_len bytes, out_len bytes of output, its check) from its kept block
+// starts -- n_rec (bit, output offset) pairs in any order that include every access point: the points for `span`, and
+// their windows gathered from d_src (the output; when hist > 0, preceded by the last hist of dict_len bytes at d_dict).
+// Synchronises; *out is set only on success.
+int zs_index_from_starts(zs_ctx* ctx, const uint64_t* rec, uint64_t n_rec, uint64_t span, int window_bits, uint32_t check,
+                         uint64_t in_len, uint64_t out_len, const uint8_t* d_src, const uint8_t* d_dict, uint64_t dict_len,
+                         uint64_t hist, zs_inflate_index** out);
+
 // Options of one batch inflate call (zs_api.cu) that the public entry points do not take.
 struct InflateOpts {
     // one stream whose sizes the host knows: it may take the segment-parallel decoder (zs_inflate_par.cu).
@@ -371,6 +382,14 @@ int inflate_batch_host_impl(zs_ctx* ctx, const uint8_t* in, const uint64_t* in_o
                             InflateOut* res);
 
 // deflate
+// Where deflate_record_kernel (zs_huff.cu) appends the block starts of one deflate call that the access-point rule may
+// select: (bit, input offset) pairs local to the call at rec[2i], rec[2i + 1], i taken from *cnt.
+struct DeflateRecord {
+    uint64_t* rec;
+    uint64_t cap;        // pairs
+    unsigned long long* cnt;
+    uint64_t span;
+};
 struct zs_deflate_plan {
     const uint8_t* d_in;      // points at the first byte of this call's input
     uint64_t in_len;
@@ -403,6 +422,7 @@ struct zs_deflate_plan {
     zs_deflate_result* d_result;
     int32_t* d_error;         // device flag: ZS_BUF_ERROR if out_cap too small
     const zs_deflate_dict* dict;   // zs_deflate_batch_dict*: every chunk starts from this dictionary, or nullptr
+    const DeflateRecord* record;   // zs_deflate_indexed*: keep the block starts an index may select, or nullptr
 };
 int zs_launch_lz77(zs_ctx* ctx, const zs_deflate_plan& p);
 // Runs d_dict[0, len) (len <= 32768, 16-byte aligned, readable to len rounded up to 16) through the match

@@ -16,6 +16,8 @@
 //    after), chunk starts are resolved by one warp (prefix scan when no chunk of a 32-chunk group
 //    holds a stored block, shuffle-serial otherwise), then every block gets its absolute bit offset.
 //    This is the "exclusive scan of per-chunk compressed bit lengths" of the north star.
+//    For the indexed calls (zs_deflate_indexed*), deflate_record_kernel walks the same sizes once more and keeps
+//    the block starts an index of the stream may select (DESIGN.md 3.3e).
 //  * encode_kernel: one CTA per block; per 256-symbol tile a CTA-wide scan of code lengths gives
 //    every symbol its bit offset, codes are OR-ed into a shared-memory staging tile and flushed as
 //    whole 32-bit words (boundary words with atomicOr, the output having been zeroed).  Blocks
@@ -685,17 +687,27 @@ __device__ __forceinline__ uint64_t wrap_header_bytes(int wrap, int fdict) {
 
 __device__ __forceinline__ unsigned stored_pad(uint64_t bitpos_after_hdr) { return (unsigned)((8u - (bitpos_after_hdr & 7u)) & 7u); }
 
+// Z_SYNC_FLUSH marker (empty stored block) after chunk c: between chunks when ZS_FLAG_SYNC is set, and always at the
+// end of a part that is not the last one -- the next part must start byte aligned because stored blocks inside it are
+// padded relative to its own first bit
+__device__ __forceinline__ bool has_sync_marker(int mode, uint32_t flags, uint32_t c, uint32_t n_chunks) {
+    return mode == ZS_MODE_STITCHED && (c + 1 == n_chunks ? (flags & ZS_FLAG_NOT_LAST) != 0 : (flags & ZS_FLAG_SYNC) != 0);
+}
+
+// the bit after a block that starts at `pos`: h0 is its header word, bits its size without the stored padding
+__device__ __forceinline__ uint64_t block_end(uint64_t pos, uint32_t h0, uint64_t bits) {
+    if ((h0 & 0xffu) == BT_STORED) pos += 3 + stored_pad(pos + 3) + (bits - 3);
+    else pos += bits;
+    return pos;
+}
+
 // chunk summary: P = bits up to (excluding) the first stored block, R = bits from that block's
 // LEN field to the end of the chunk (later stored blocks start from a known alignment)
 __global__ void layout_chunks_kernel(LayoutArgs a) {
     const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= a.n_chunks) return;
     const uint32_t nb = a.chunk_nblk[c];
-    // Z_SYNC_FLUSH marker (empty stored block) after the chunk: between chunks when ZS_FLAG_SYNC is
-    // set, and always at the end of a part that is not the last one -- the next part must start
-    // byte aligned because stored blocks inside it are padded relative to its own first bit
-    const bool sync_marker = a.mode == ZS_MODE_STITCHED &&
-                             (c + 1 == a.n_chunks ? (a.flags & ZS_FLAG_NOT_LAST) != 0 : (a.flags & ZS_FLAG_SYNC) != 0);
+    const bool sync_marker = has_sync_marker(a.mode, a.flags, c, a.n_chunks);
     uint64_t P = 0, R = 0;
     bool seen = false;
     for (uint32_t j = 0; j < nb + (sync_marker ? 1u : 0u); j++) {
@@ -833,8 +845,30 @@ __global__ void layout_blocks_kernel(LayoutArgs a) {
         const uint64_t bits = a.blk_bits[gid];
         a.blk_bits[gid] = pos;
         if (chunk_final && j + 1 == nb) a.blk_hdr[gid * kHdrWords] = h0 | 0x80000000u;
-        if ((h0 & 0xffu) == BT_STORED) pos += 3 + stored_pad(pos + 3) + (bits - 3);
-        else pos += bits;
+        pos = block_end(pos, h0, bits);
+    }
+}
+
+// The indexed calls (zs_deflate_indexed*): every block start of the stream as (bit, input offset = output offset), per
+// chunk in stream order -- its blocks, then its sync marker -- keeping those the access-point rule may select, by the
+// rule of par_record_kernel's RecordSink: the chunk's first start, and every start whose offset o has a multiple of the
+// span in (offset of the start before it, o].  It runs between layout_scan_kernel and layout_blocks_kernel: blk_bits
+// still holds the block sizes, and the marker starts where the chunk's last block ends.
+__global__ void deflate_record_kernel(LayoutArgs a, const uint32_t* blk_desc, DeflateRecord r) {
+    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.n_chunks) return;
+    const uint32_t nb = a.chunk_nblk[c] + (has_sync_marker(a.mode, a.flags, c, a.n_chunks) ? 1u : 0u);
+    uint64_t pos = a.out_off[c], prev = ~0ull;
+    for (uint32_t j = 0; j < nb; j++) {
+        const bool marker = j == a.chunk_nblk[c];
+        const uint64_t gid = (uint64_t)c * a.max_bpc + j;
+        const uint64_t o = marker ? a.in_off[c + 1] : a.in_off[c] + blk_desc[gid * 4 + 2];
+        if (prev == ~0ull || o / r.span > prev / r.span) {
+            const unsigned long long i = atomicAdd(r.cnt, 1ull);
+            if (i < r.cap) { r.rec[2 * i] = pos; r.rec[2 * i + 1] = o; }
+        }
+        prev = o;
+        if (!marker) pos = block_end(pos, a.blk_hdr[gid * kHdrWords], a.blk_bits[gid]);
     }
 }
 
@@ -1152,6 +1186,8 @@ int zs_launch_huffman(zs_ctx* ctx, const zs_deflate_plan& p) {
     const unsigned cgrid = (p.n_chunks + 127) / 128;
     ZS_KERNEL(ctx, "layout_chunks_kernel", layout_chunks_kernel<<<cgrid, 128, 0, ctx->stream>>>(l));
     ZS_KERNEL(ctx, "layout_scan_kernel", layout_scan_kernel<<<1, kScanThreads, 0, ctx->stream>>>(l));
+    if (p.record)
+        ZS_KERNEL(ctx, "deflate_record_kernel", deflate_record_kernel<<<cgrid, 128, 0, ctx->stream>>>(l, p.d_blk_desc, *p.record));
     ZS_KERNEL(ctx, "layout_blocks_kernel", layout_blocks_kernel<<<cgrid, 128, 0, ctx->stream>>>(l));
 
     ZS_KERNEL(ctx, "zero_output_kernel", zero_output_kernel<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(p.d_out, p.d_result, p.d_error, p.out_cap));

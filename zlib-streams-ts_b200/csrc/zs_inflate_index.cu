@@ -8,6 +8,8 @@
 //                       falls on), so the kept starts are a superset of the points;
 //   (host)              the rule applied to the kept starts, sorted by bit, gives the points exactly;
 //   ix_gather_kernel    copies every point's window (dictionary, then output) out of the decoded output.
+// The host rule, the allocation and the gather are zs_index_from_starts, which the indexed deflate calls (zs_api.cu)
+// use too: their kept starts come from deflate_record_kernel (zs_huff.cu) and their windows from the input.
 // Extract (zs_inflate_index_extract_dev):
 //   ix_plan_kernel      per range: the first point at or before its start and the number of intervals it spans;
 //   ix_scan_kernel      exclusive scan of those counts (block_scan, zs_common.cuh): work item g belongs to range r with
@@ -231,8 +233,7 @@ __global__ void ix_finish_kernel(IxRanges r, uint64_t out_len) {
 // The point rule over the kept block starts (bit, output offset), in stream order: the first start, and every start
 // some m = k * span < out_len falls on -- m in (offset of the kept start before it, its offset].  The kept starts
 // include every point, so this is the rule over all block starts (DESIGN.md 3.3d).
-void select_points(std::vector<uint64_t>& rec, uint64_t span, uint64_t out_len, std::vector<uint64_t>& bit, std::vector<uint64_t>& off) {
-    const size_t m = rec.size() / 2;
+void select_points(const uint64_t* rec, size_t m, uint64_t span, uint64_t out_len, std::vector<uint64_t>& bit, std::vector<uint64_t>& off) {
     std::vector<size_t> order(m);
     for (size_t i = 0; i < m; i++) order[i] = i;
     std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return rec[2 * a] < rec[2 * b]; });
@@ -281,6 +282,39 @@ uint32_t get32(const uint8_t* p) { uint32_t v; memcpy(&v, p, 4); return v; }
 uint64_t get64(const uint8_t* p) { uint64_t v; memcpy(&v, p, 8); return v; }
 
 }  // namespace
+
+int zs_index_from_starts(zs_ctx* ctx, const uint64_t* rec, uint64_t n_rec, uint64_t span, int window_bits, uint32_t check,
+                         uint64_t in_len, uint64_t out_len, const uint8_t* d_src, const uint8_t* d_dict, uint64_t dict_len,
+                         uint64_t hist, zs_inflate_index** out) {
+    zs_inflate_index* x = new zs_inflate_index();
+    x->device = ctx->device;
+    x->window_bits = window_bits;
+    x->check = check;
+    x->in_len = in_len;
+    x->out_len = out_len;
+    x->span = span;
+    x->d_mem = nullptr;
+    select_points(rec, n_rec, span, out_len, x->bit, x->off);
+    x->n = x->bit.size();
+    x->wlen.resize(x->n);
+    for (uint64_t p = 0; p < x->n; p++) x->wlen[p] = (uint32_t)(hist + x->off[p] < kWin ? hist + x->off[p] : kWin);
+    int rc = index_alloc(ctx, x);
+    if (rc == ZS_OK && x->n)
+        ZS_KERNEL(ctx, "ix_gather_kernel",
+                  ix_gather_kernel<<<(unsigned)(x->n < 4096 ? x->n : 4096), 256, 0, ctx->stream>>>(
+                      x->d_off(), x->d_woff(), x->d_wlen(), x->n, (uint8_t*)x->d_win(), d_src, hist ? d_dict : nullptr, dict_len));
+    if (rc == ZS_OK) {
+        const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = zs_set_cuda_error(ctx, e, "inflate_index: windows");
+    }
+    if (rc != ZS_OK) {
+        cudaFree(x->d_mem);
+        delete x;
+        return rc;
+    }
+    *out = x;
+    return ZS_OK;
+}
 
 extern "C" {
 
@@ -342,38 +376,12 @@ int zs_inflate_index_build_dev(zs_ctx* ctx, const uint8_t* d_in, uint64_t in_len
         return ZS_E_CUDA;
     }
 
-    zs_inflate_index* x = new zs_inflate_index();
-    x->device = ctx->device;
-    x->window_bits = window_bits;
-    x->check = res->check;
-    x->in_len = in_len;
-    x->out_len = out_len;
-    x->span = span;
-    x->d_mem = nullptr;
-    select_points(rec, span, out_len, x->bit, x->off);
-    x->n = x->bit.size();
     // the dictionary is history only where the decoder used it: raw streams, and zlib streams that name one (FDICT)
     const bool gz = in_len >= 2 && head[0] == 0x1f && head[1] == 0x8b && (wrap & 2);
     const bool fdict = (wrap & 1) && !gz && (head[1] & 0x20);
     const uint64_t hist = (wrap == 0 || fdict) ? (dict_len < kWin ? dict_len : kWin) : 0;
-    x->wlen.resize(x->n);
-    for (uint64_t p = 0; p < x->n; p++) x->wlen[p] = (uint32_t)(hist + x->off[p] < kWin ? hist + x->off[p] : kWin);
-    rc = index_alloc(ctx, x);
-    if (rc == ZS_OK && x->n)
-        ZS_KERNEL(ctx, "ix_gather_kernel",
-                  ix_gather_kernel<<<(unsigned)(x->n < 4096 ? x->n : 4096), 256, 0, ctx->stream>>>(
-                      x->d_off(), x->d_woff(), x->d_wlen(), x->n, (uint8_t*)x->d_win(), d_out, hist ? d_dict : nullptr, dict_len));
-    if (rc == ZS_OK) {
-        const cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-        if (e2 != cudaSuccess) rc = zs_set_cuda_error(ctx, e2, "inflate_index_build: windows");
-    }
-    if (rc != ZS_OK) {
-        cudaFree(x->d_mem);
-        delete x;
-        return rc;
-    }
-    *out = x;
-    return ZS_OK;
+    return zs_index_from_starts(ctx, rec.data(), c[0], span, window_bits, res->check, in_len, out_len, d_out, d_dict, dict_len,
+                                hist, out);
 }
 
 int zs_inflate_index_build(zs_ctx* ctx, const uint8_t* in, uint64_t in_len, int window_bits, uint64_t span, uint8_t* out,
